@@ -1,7 +1,8 @@
 #!/bin/bash
 # profiles/capture_ab.sh <tag> — one gpurun call on one B200:
-#   1. GPU parity tests  2. the bench line (with e2e and the CPU baseline)  3. A/B of the single optimisations (build the
-#      one-switch-off libraries and an earlier commit HERE first: python -m rala_b200.build --variants; bash profiles/build_prev.sh)
+#   1. GPU parity tests  2. the bench line (with e2e and the CPU baseline)  3. A/B of the product against the parent commit's
+#      library and the switches of any experiment under trial (build them HERE first: bash profiles/build_prev.sh;
+#      python -m rala_b200.build --variants)
 #   4. ncu launch list of the same bench command  5. one `ncu --set full` capture of the kernels of one step
 # Numbers printed under ncu are never bench values.
 set -u

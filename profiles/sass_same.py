@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """profiles/sass_same.py <objdir A> <objdir B> — which kernels' SASS differs between two builds of rala_b200/csrc
-(e.g. rala_b200/build/<variant>/ against rala_b200/build/).  Used when code is added behind a switch without GPU time
-to re-run the parity suite: the kernels of the default path must come out bit-identical to the build that was tested."""
+(e.g. rala_b200/build/<variant>/ against rala_b200/build/, or the parent commit's build against this one).  Used when
+code is added behind a switch, or a settled switch is removed: the kernels of the default path must come out
+bit-identical to the build that was tested."""
 import hashlib
 import re
 import subprocess
@@ -23,7 +24,7 @@ def funcs(path):
 
 a_dir, b_dir = sys.argv[1], sys.argv[2]
 rc = 0
-for f in ("classify", "containment", "graph_build", "transitive"):
+for f in ("classify", "containment", "graph_build", "transitive", "fabric", "frontend"):   # every object with kernels
     a, b = funcs(f"{a_dir}/{f}.o"), funcs(f"{b_dir}/{f}.o")
     changed = sorted(k for k in a if k in b and a[k] != b[k])
     print(f"{f}: {len(a)} / {len(b)} kernels, changed: {changed or 'none'}, only in A: {sorted(set(a) - set(b)) or 'none'}, "

@@ -15,8 +15,9 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# RALA_B200_LIB: another build of the same library (rala_b200/variants/: one optimisation switched off each), for
-# bench.py's A/B lines.  Never a fallback: the file must exist.
+# RALA_B200_LIB: another build of the same library (rala_b200/variants/: an experiment's switch turned off, or the
+# parent commit's library from profiles/build_prev.sh), to compare its results and times with the product's.
+# Never a fallback: the file must exist.
 LIB_PATH = os.environ.get("RALA_B200_LIB") or os.path.join(_HERE, "librala_b200.so")
 N_STAGES = 9
 STAGE_NAMES = ("classify", "retrim", "finalize", "build", "transitive", "k1_classify_kernel", "k1b_fixpoint_kernel",

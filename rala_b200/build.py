@@ -61,18 +61,18 @@ def build(verbose: bool = False, force: bool = False) -> str:
     return _compile(LIB, os.path.join(HERE, "build"), [], verbose)
 
 
-# A/B libraries: the product with ONE optimisation switched off each (common.cuh RB_OPT_*), for bench.py --ab.
-VARIANTS = {"no_events": "RB_OPT_EVENTS", "no_reloc": "RB_OPT_RELOC", "no_aos": "RB_OPT_AOS", "no_fill": "RB_OPT_FILL",
-            "no_rank": "RB_OPT_RANK", "no_conc": "RB_OPT_CONC", "no_fuse": "RB_OPT_FUSE"}
+# A/B libraries for bench.py --ab, built by `python -m rala_b200.build --variants` into rala_b200/variants/.
+# An optimisation under trial goes behind a compile-time switch that is on by default, and gets an entry here: VARIANTS
+# maps a library name to the switch that library turns off (-D<macro>=0), TUNINGS to other -D settings of a tunable.
+# The commit that settles the experiment removes both the switch and its entry, so every kernel keeps one code path.
+# bench.py --ab also times `prev`, the parent commit's library built by profiles/build_prev.sh.
+VARIANTS: dict = {}
+TUNINGS: dict = {}
 VARIANT_DIR = os.path.join(HERE, "variants")
 
 
 def variant_path(name: str) -> str:
     return os.path.join(VARIANT_DIR, f"librala_b200_{name}.so")
-
-
-# other settings of a tunable, same product otherwise
-TUNINGS = {"no_packrow": ["-DRB_GROUP_PACKROW=0"]}
 
 
 def build_variants(verbose: bool = False):

@@ -207,9 +207,7 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
     CU(ctx, g->edges.reserve(align_up((size_t) edge_cap * 4, 256) * 3));
     CU(ctx, g->col.reserve((size_t) edge_cap * 8));
     CU(ctx, g->col_eid.reserve((size_t) edge_cap * 4));
-#if RB_OPT_RANK
     CU(ctx, g->edge_rank.reserve((size_t) edge_cap * 4));
-#endif
     CU(ctx, g->T.reserve(align_up(edge_cap, 256)));
     CU(ctx, g->marked.reserve(align_up(edge_cap, 256)));
     g->heavy_cap = edge_cap / 16 + 4096;
@@ -472,12 +470,12 @@ static int phase_resolve(rala_b200_graph* g, bool first_pass) {
     rala_b200_ctx* ctx = g->ctx;
     // the hill counters read the death times BEFORE the deaths are applied to the pile table; without hills nothing
     // sits between the resolution and k_apply_deaths, which then decodes the states itself
-    const bool fused_decode = RB_OPT_FUSE && !(first_pass && g->n_hills);
+    const bool fused_decode = !(first_pass && g->n_hills);
     CU(ctx, stage_event(g, g->ev_start[ST_K1B_KERNEL]));
     // The final pass (graph.cpp:831-866) has no events at all on clean data: scan, scatter, resolution and the sweep over the
     // pile table then return at once (nobody dies; the death times of the first pass, all "never" for the piles still
     // in the lists, stay in place).  The first pass always runs: it also builds the liveness bitmap.
-    const bool skip_if_empty = RB_OPT_FUSE && !first_pass && fused_decode;
+    const bool skip_if_empty = !first_pass && fused_decode;
     int rc = resolve_containment(g, !fused_decode, skip_if_empty);
     if (rc) return rc;
     CU(ctx, end_stage(g, ST_K1B_KERNEL));
@@ -702,7 +700,7 @@ extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
         g->download_pending = true;
     }
     scan_state(g, (uint64_t) g->n_nodes_max + 1, &status, &ticket);
-    launch_build_csr(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->cnt(), status, ticket, RB_OPT_RANK != 0);
+    launch_build_csr(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->cnt(), status, ticket, true);
     if (g->download_pending && !g->in_run) {
         join_side(ctx->L, 0);
         g->download_pending = false;

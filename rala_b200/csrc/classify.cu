@@ -31,12 +31,8 @@ namespace rb {
 // barriers in the first pass.  The second pass reads only the two id columns (8 B / record) plus one
 // bit per pile of an L1-resident liveness bitmap, and gathers the coordinates of the few survivors.
 // =============================================================================================
-#ifndef RB_EVENTS_ITEMS
-#define RB_EVENTS_ITEMS 4   // consecutive records per thread in k_classify_events (one 16-byte load per column)
-#endif
-#ifndef RB_EVENTS_MINB
-#define RB_EVENTS_MINB 3    // its resident blocks per SM
-#endif
+constexpr int kEventsItems = 4;                           // consecutive records per thread in k_classify_events (one 16-byte load per column)
+constexpr int kEventsMinBlocks = 3;                       // its resident blocks per SM
 constexpr int kRecItems = 4;                              // consecutive records per thread (one uint4 per column)
 constexpr int kRecTile = kTileThreads * kRecItems;        // records per block iteration
 constexpr uint32_t kRunRecords = 512;                     // survivors pass: records per warp iteration = one run
@@ -164,46 +160,19 @@ __global__ void __launch_bounds__(kTileThreads, MINB) k_classify_events(
         }
 #pragma unroll
         for (int r = 0; r < R; ++r) {
-            bool is_ev = false;
-            uint32_t evv = 0, evc = 0;
-#if RB_OPT_EVENTS
-            {
-                // straight-line trim + type (common.cuh event_code): a dead pile (end == 0) rejects itself
-                const uint32_t idb = b[r] & 0x7FFFFFFFu;
-                const uint32_t code = event_code(ab[r], ae[r], bb[r], be[r], b[r] >> 31, pa[r].x, pa[r].y & kEndMask,
-                                                 pb[r].x, pb[r].y & kEndMask);                              // :451-452
-                const uint32_t fa = pa[r].y >> 30, fb = pb[r].y >> 30;
-                if ((code & 1u) && ((fa | fb) & 1u)) {                                                      // :457-462, resolved by k_hill_coverage
-                    uint32_t slot = atomicAdd(&counters[C_HILL], 1u);
-                    if (slot < hill_cap) hill_rec[slot] = (uint32_t) R * q + r;
-                }
-                const bool ev_b = (code & 2u) && !(fb & 2u);                                                // :469-474
-                const bool ev_a = (code & 4u) && !(fa & 2u);                                                // :475-480
-                is_ev = ev_a | ev_b;
-                evv = ev_b ? a[r] : idb;
-                evc = ev_b ? idb : a[r];
+            // straight-line trim + type (common.cuh event_code): a dead pile (end == 0) rejects itself
+            const uint32_t idb = b[r] & 0x7FFFFFFFu;
+            const uint32_t code = event_code(ab[r], ae[r], bb[r], be[r], b[r] >> 31, pa[r].x, pa[r].y & kEndMask,
+                                             pb[r].x, pb[r].y & kEndMask);                              // :451-452
+            const uint32_t fa = pa[r].y >> 30, fb = pb[r].y >> 30;
+            if ((code & 1u) && ((fa | fb) & 1u)) {                                                      // :457-462, resolved by k_hill_coverage
+                uint32_t slot = atomicAdd(&counters[C_HILL], 1u);
+                if (slot < hill_cap) hill_rec[slot] = (uint32_t) R * q + r;
             }
-#else
-            if (live[r]) {
-                Pile A, B;
-                A.begin = pa[r].x; A.end = pa[r].y & kEndMask; A.flags = pa[r].y >> 30;
-                B.begin = pb[r].x; B.end = pb[r].y & kEndMask; B.flags = pb[r].y >> 30;
-                const uint32_t idb = b[r] & 0x7FFFFFFFu, ori = b[r] >> 31;
-                Coords c{ab[r], ae[r], bb[r], be[r]};
-                if (A.alive() && B.alive() && trim(c, ori, A, B)) {                          // :451-452
-                    if ((A.flags | B.flags) & 1u) {                                          // :457-462, resolved by k_hill_coverage
-                        uint32_t slot = atomicAdd(&counters[C_HILL], 1u);
-                        if (slot < hill_cap) hill_rec[slot] = (uint32_t) R * q + r;
-                    }
-                    const uint8_t t = classify(c, relative(c, ori, A, B));
-                    if (t == kB && !(B.flags & 2u)) {                                        // :469-474
-                        is_ev = true; evv = a[r]; evc = idb;
-                    } else if (t == kA && !(A.flags & 2u)) {                                 // :475-480
-                        is_ev = true; evv = idb; evc = a[r];
-                    }
-                }
-            }
-#endif
+            const bool ev_b = (code & 2u) && !(fb & 2u);                                                // :469-474
+            const bool ev_a = (code & 4u) && !(fa & 2u);                                                // :475-480
+            const bool is_ev = ev_a | ev_b;
+            const uint32_t evv = ev_b ? a[r] : idb, evc = ev_b ? idb : a[r];
             const uint32_t m = __ballot_sync(0xFFFFFFFFu, is_ev);
             if (m) {
                 if (is_ev) {
@@ -222,12 +191,10 @@ __global__ void __launch_bounds__(kTileThreads, MINB) k_classify_events(
     if (staged) flush();
 }
 
-#if RB_OPT_AOS
 // Scratch of the survivors pass: one 32-byte entry per slot, kept as two 16-byte halves in the two spare list buffers
 // (a list buffer holds 25 B per entry of capacity, a half needs 16): {a, b | ori << 31, ab, ae} and {bb, be, tag, -}.
 __device__ __forceinline__ uint4* scratch_lo(const List& spare_ovl) { return reinterpret_cast<uint4*>(spare_ovl.a); }
 __device__ __forceinline__ uint4* scratch_hi(const List& spare_inl) { return reinterpret_cast<uint4*>(spare_inl.a); }
-#endif
 
 // Survivors pass.  Every warp owns RUNS of 512 consecutive records (4 x 4 per lane): it writes the survivors of a
 // run, in record order, to the run's own slot range of the scratch lists (slot = record index of the run's
@@ -244,13 +211,9 @@ __device__ __forceinline__ uint4* scratch_hi(const List& spare_inl) { return rei
 // 5 resident blocks per SM (48 registers, 28 bytes of spill) and a grid of two waves: survivors stage 83 us against 91 us at
 // 4 resident blocks (64 registers); one persistent wave loses 15 us, 6 resident blocks spill 104 bytes and win nothing
 // (profiles/r02ae_ab.json, r02af_ab.json)
-#ifndef RB_SURV_MINB
-#define RB_SURV_MINB 5
-#endif
-#ifndef RB_SURV_BLOCKS
-#define RB_SURV_BLOCKS 10   // grid = this many blocks per SM at most
-#endif
-__global__ void __launch_bounds__(kTileThreads, RB_SURV_MINB) k_classify_survivors(
+constexpr int kSurvMinBlocks = 5;
+constexpr int kSurvBlocks = 10;   // grid = this many blocks per SM at most
+__global__ void __launch_bounds__(kTileThreads, kSurvMinBlocks) k_classify_survivors(
     List recs, uint32_t n, const uint2* __restrict__ piles, const uint32_t* __restrict__ alive_bits, uint32_t n_piles,
     List tmp_ovl, List tmp_inl, uint32_t cap, uint32_t* __restrict__ run_cnt) {
     __shared__ uint16_t s_queue[kTileWarps][kRunRecords];
@@ -321,7 +284,6 @@ __global__ void __launch_bounds__(kTileThreads, RB_SURV_MINB) k_classify_survivo
             }
             const uint32_t ma = __ballot_sync(0xFFFFFFFFu, dest == 1), mb = __ballot_sync(0xFFFFFFFFu, dest == 2);
             const uint32_t below = (1u << lane) - 1u;
-#if RB_OPT_AOS
             if (dest) {   // one 32-byte scratch entry, two 16-byte stores: `overlaps` fill the run's slots from the front, `internals` from the back
                 const uint32_t p = dest == 1 ? run * kRunRecords + n_a + __popc(ma & below)
                                              : run * kRunRecords + run_len - 1u - (n_b + __popc(mb & below));
@@ -330,15 +292,6 @@ __global__ void __launch_bounds__(kTileThreads, RB_SURV_MINB) k_classify_survivo
                     scratch_hi(tmp_inl)[p] = make_uint4(e.c.bb, e.c.be, tag, 0u);
                 }
             }
-#else
-            if (dest == 1) {
-                const uint32_t p = run * kRunRecords + n_a + __popc(ma & below);
-                if (p < cap) store_entry(tmp_ovl, p, e, tag);
-            } else if (dest == 2) {
-                const uint32_t p = run * kRunRecords + n_b + __popc(mb & below);
-                if (p < cap) store_entry(tmp_inl, p, e, tag);
-            }
-#endif
             n_a += __popc(ma);
             n_b += __popc(mb);
         }
@@ -410,69 +363,14 @@ __global__ void __launch_bounds__(kTileThreads) k_scan_runs(const uint32_t* __re
     }
 }
 
-// scratch run -> final position, one thread per OUTPUT entry (stores fully coalesced, gathers contiguous inside a
-// run).  The run of entry j satisfies off[run] <= j < off[run + 1]: lane 0 finds it by binary search, the other
-// lanes walk forward from there (32 consecutive entries span a handful of runs).
-__global__ void k_relocate(List tmp, List out, uint32_t cap, const uint32_t* __restrict__ off, const uint32_t* __restrict__ total_ptr,
-                           uint32_t num_runs) {
-    const uint32_t total = min(*total_ptr, cap);
-    for (uint32_t base = blockIdx.x * blockDim.x; base < total; base += gridDim.x * blockDim.x) {
-        const uint32_t j = base + threadIdx.x;
-        const uint32_t j0 = base + (threadIdx.x & ~31u);   // lane 0's entry
-        uint32_t lo = 0, hi = num_runs;                    // largest run with off[run] <= j0
-        while (hi - lo > 1) {
-            const uint32_t mid = (lo + hi) >> 1;
-            if (__ldg(off + mid) <= j0) lo = mid; else hi = mid;
-        }
-        if (j < total) {
-            uint32_t run = lo;
-            while (run + 1 < num_runs && __ldg(off + run + 1) <= j) ++run;
-            const uint32_t s = run * kRunRecords + (j - __ldg(off + run));
-            if (s < cap) {
-                out.a[j] = tmp.a[s]; out.b[j] = tmp.b[s];
-                out.ab[j] = tmp.ab[s]; out.ae[j] = tmp.ae[s];
-                out.bb[j] = tmp.bb[s]; out.be[j] = tmp.be[s];
-                out.tag[j] = tmp.tag[s];
-            }
-        }
-    }
-}
-
-// The same move, one BLOCK per 32 consecutive runs.  The survivors of 32 runs are one contiguous piece of the final list
+// Scratch runs -> final positions, one BLOCK per 32 consecutive runs.  The survivors of 32 runs are one contiguous piece of the final list
 // (~1 150 entries on clean data), so the threads take consecutive OUTPUT positions: every column is written fully
 // coalesced, and read in contiguous pieces of a run.  Each warp holds the 32 runs' offsets in its lanes and finds the
 // run of a position with a 5-step binary search over them (shuffles).  (One warp per run, ~36 entries each, was 28 000
 // short dependent chains: count / offset loads, then one and a bit half-empty iterations: 34 us, profiles/r02a.)
 constexpr uint32_t kRelocRuns = 32;
+constexpr int kRelocUnroll = 2;
 
-__device__ __forceinline__ void relocate_piece(const List& tmp, const List& out, uint32_t cap, uint32_t run0, uint32_t my_off,
-                                               uint32_t first, uint32_t total) {
-    const uint32_t lane = lane_id(), warp = warp_id();
-    for (uint32_t k = warp * 32u; k < total; k += kTileThreads) {   // block-uniform trip count per warp: all lanes shuffle
-        const uint32_t d = first + k + lane;
-        uint32_t l = 0;   // the largest run l of the 32 whose first output position is <= d
-#pragma unroll
-        for (uint32_t step = 16; step > 0; step >>= 1) {
-            const uint32_t v = __shfl_sync(0xFFFFFFFFu, my_off, (l + step) & 31u);
-            if (l + step < kRelocRuns && v <= d) l += step;
-        }
-        const uint32_t off = __shfl_sync(0xFFFFFFFFu, my_off, l);
-        if (k + lane < total) {
-            const uint32_t s = (run0 + l) * kRunRecords + (d - off);
-            if (s < cap && d < cap) {
-                out.a[d] = tmp.a[s]; out.b[d] = tmp.b[s];
-                out.ab[d] = tmp.ab[s]; out.ae[d] = tmp.ae[s];
-                out.bb[d] = tmp.bb[s]; out.be[d] = tmp.be[s];
-                out.tag[d] = tmp.tag[s];
-            }
-        }
-    }
-}
-
-#if RB_OPT_AOS
-#ifndef RB_RELOC_UNROLL
-#define RB_RELOC_UNROLL 2
-#endif
 // The move out of the 32-byte scratch entries: two 16-byte loads per entry (consecutive output positions read consecutive
 // slots of a run), seven coalesced column stores.  U positions per thread and trip: the loads of all of them are issued
 // before the first store, the trips of a block are a chain of dependent memory latencies otherwise.
@@ -514,7 +412,6 @@ __device__ __forceinline__ void relocate_scratch_piece(const uint4* __restrict__
         }
     }
 }
-#endif
 
 __global__ void __launch_bounds__(kTileThreads) k_relocate_runs(List tmp_a, List out_a, List tmp_b, List out_b, uint32_t cap,
                                                                const uint32_t* __restrict__ run_cnt, const uint32_t* __restrict__ off_a,
@@ -531,13 +428,8 @@ __global__ void __launch_bounds__(kTileThreads) k_relocate_runs(List tmp_a, List
         const uint32_t na = run <= last ? (c & 0xFFFFu) : 0u, nb = run <= last ? (c >> 16) : 0u;
         const uint32_t first_a = __shfl_sync(0xFFFFFFFFu, oa, 0), first_b = __shfl_sync(0xFFFFFFFFu, ob, 0);
         const uint32_t total_a = __shfl_sync(0xFFFFFFFFu, oa + na, 31) - first_a, total_b = __shfl_sync(0xFFFFFFFFu, ob + nb, 31) - first_b;
-#if RB_OPT_AOS
-        relocate_scratch_piece<false, RB_RELOC_UNROLL>(scratch_lo(tmp_a), scratch_hi(tmp_b), out_a, cap, n, run0, oa, first_a, total_a);
+        relocate_scratch_piece<false, kRelocUnroll>(scratch_lo(tmp_a), scratch_hi(tmp_b), out_a, cap, n, run0, oa, first_a, total_a);
         relocate_scratch_piece<true, 1>(scratch_lo(tmp_a), scratch_hi(tmp_b), out_b, cap, n, run0, ob, first_b, total_b);
-#else
-        relocate_piece(tmp_a, out_a, cap, run0, oa, first_a, total_a);
-        relocate_piece(tmp_b, out_b, cap, run0, ob, first_b, total_b);
-#endif
     }
 }
 
@@ -744,10 +636,6 @@ __global__ void k_trim_classify_aos(uint32_t* __restrict__ rec, uint32_t n, cons
     }
 }
 
-__global__ void k_fill_u32(uint32_t* __restrict__ p, uint32_t v, size_t n) {
-    for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < n; i += (size_t) gridDim.x * blockDim.x) p[i] = v;
-}
-
 // host table {begin,end} + flag bytes -> packed device table
 __global__ void k_pack_piles(const uint2* __restrict__ in, const uint8_t* __restrict__ flags, uint2* __restrict__ out,
                              uint32_t n) {
@@ -796,12 +684,6 @@ __global__ void k_list_connections(List l, const uint32_t* __restrict__ n_ptr, u
 // ---------------------------------------------------------------------------------------------
 // host-side launchers
 // ---------------------------------------------------------------------------------------------
-static inline int grid_for(uint64_t n, int per_block, int max_blocks) {
-    uint64_t b = (n + per_block - 1) / per_block;
-    if (b < 1) b = 1;
-    return (int) (b < (uint64_t) max_blocks ? b : (uint64_t) max_blocks);
-}
-
 void launch_records_to_soa(Launch& L, const uint32_t* aos, uint32_t n, List recs) {
     if (n == 0) return;
     k_records_to_soa<<<grid_for(n, 256, kNumSMs * 8), 256, 0, L.stream>>>(aos, n, recs);
@@ -819,8 +701,8 @@ void launch_classify_events(Launch& L, List recs, uint32_t n, uint32_t t0, const
                             Events ev, uint32_t ev_cap, uint32_t* vcount, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters) {
     if (n == 0) return;
     // 3 blocks / SM at 80 registers: 4 and 5 blocks (64 / 48 registers) lost 15 and 25 us per step (profiles/r02a_ab.json)
-    k_classify_events<RB_EVENTS_MINB, RB_EVENTS_ITEMS><<<grid_for(n, kTileThreads * RB_EVENTS_ITEMS, kNumSMs * RB_EVENTS_MINB), kTileThreads, 0, L.stream>>>(recs, n, t0, piles, n_piles, ev, ev_cap, vcount,
-                                                                                          hill_rec, hill_cap, counters);
+    k_classify_events<kEventsMinBlocks, kEventsItems><<<grid_for(n, kTileThreads * kEventsItems, kNumSMs * kEventsMinBlocks), kTileThreads, 0, L.stream>>>(recs, n, t0, piles, n_piles, ev, ev_cap, vcount,
+                                                                                        hill_rec, hill_cap, counters);
     L.count++;
 }
 
@@ -829,21 +711,15 @@ void launch_classify_survivors(Launch& L, List recs, uint32_t n, const uint2* pi
                                RunBufs runs, unsigned long long* status, uint32_t* ticket) {
     if (n == 0) return;   // n_ovl / n_inl were zeroed by the caller
     const uint32_t num_runs = (n + kRunRecords - 1) / kRunRecords;
-    k_classify_survivors<<<grid_for(num_runs, kTileWarps, kNumSMs * RB_SURV_BLOCKS), kTileThreads, 0, L.stream>>>(
+    k_classify_survivors<<<grid_for(num_runs, kTileWarps, kNumSMs * kSurvBlocks), kTileThreads, 0, L.stream>>>(
         recs, n, piles, alive_bits, n_piles, tmp_ovl, tmp_inl, cap, runs.cnt);
     L.count++;
     k_scan_runs<<<grid_for(num_runs, kTile, kNumSMs * 4), kTileThreads, 0, L.stream>>>(runs.cnt, num_runs, runs.off_a, runs.off_b, n_ovl,
                                                                                        n_inl, status, ticket);
     L.count++;
-#if RB_OPT_RELOC
     k_relocate_runs<<<grid_for(num_runs, kRelocRuns, kNumSMs * 8), kTileThreads, 0, L.stream>>>(tmp_ovl, ovl, tmp_inl, inl, cap, runs.cnt,
                                                                                                runs.off_a, runs.off_b, num_runs, n);
     L.count++;
-#else
-    k_relocate<<<grid_for(cap, 256, kNumSMs * 8), 256, 0, L.stream>>>(tmp_ovl, ovl, cap, runs.off_a, n_ovl, num_runs);
-    k_relocate<<<grid_for(cap, 256, kNumSMs * 8), 256, 0, L.stream>>>(tmp_inl, inl, cap, runs.off_b, n_inl, num_runs);
-    L.count += 2;
-#endif
 }
 
 uint32_t classify_num_runs(uint32_t n) { return (n + kRunRecords - 1) / kRunRecords; }
@@ -897,12 +773,6 @@ void launch_trim_classify_aos(Launch& L, uint32_t* rec, uint32_t n, const uint2*
     L.count++;
 }
 
-void launch_fill_u32(Launch& L, uint32_t* p, uint32_t v, size_t n) {
-    if (n == 0) return;
-    k_fill_u32<<<grid_for(n, 1024, kNumSMs * 8), 256, 0, L.stream>>>(p, v, n);
-    L.count++;
-}
-
 void launch_pack_piles(Launch& L, const uint2* in, const uint8_t* flags, uint2* out, uint32_t n) {
     if (n == 0) return;
     k_pack_piles<<<grid_for(n, 256, kNumSMs * 8), 256, 0, L.stream>>>(in, flags, out, n);
@@ -938,7 +808,7 @@ void preload_classify() {
     cudaFuncAttributes a;
     cudaFuncGetAttributes(&a, k_records_to_soa);
     cudaFuncGetAttributes(&a, k_unpack_records);
-    cudaFuncGetAttributes(&a, k_classify_events<RB_EVENTS_MINB, RB_EVENTS_ITEMS>);
+    cudaFuncGetAttributes(&a, k_classify_events<kEventsMinBlocks, kEventsItems>);
     cudaFuncGetAttributes(&a, k_classify_survivors);
     cudaFuncGetAttributes(&a, k_scan_runs);
     cudaFuncGetAttributes(&a, k_relocate_runs);
@@ -952,7 +822,6 @@ void preload_classify() {
     cudaFuncGetAttributes(&a, k_list_pass<kFinalInt>);
     cudaFuncGetAttributes(&a, k_classify_final);
     cudaFuncGetAttributes(&a, k_trim_classify_aos);
-    cudaFuncGetAttributes(&a, k_fill_u32);
     cudaFuncGetAttributes(&a, k_pack_piles);
     cudaFuncGetAttributes(&a, k_unpack_piles);
     cudaFuncGetAttributes(&a, k_list_to_aos);

@@ -4,38 +4,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// Compile-time switches of single optimisations (all on by default).  rala_b200/build.py builds one extra
-// library per switch turned off (rala_b200/variants/), so that bench.py can measure each contribution on the
-// GPU (RALA_B200_LIB selects the library).
-#ifndef RB_OPT_EVENTS
-#define RB_OPT_EVENTS 1   // branch-free event detection in the first pass over the records
-#endif
-#ifndef RB_OPT_RELOC
-#define RB_OPT_RELOC 1    // warp-per-run relocation of the survivors
-#endif
-#ifndef RB_OPT_AOS
-#define RB_OPT_AOS 1      // scratch of the survivors pass as 32-byte entries (two 16-byte halves) instead of seven columns
-#endif
-#if !RB_OPT_RELOC
-#undef RB_OPT_AOS
-#define RB_OPT_AOS 0
-#endif
-#ifndef RB_OPT_RANK
-#define RB_OPT_RANK 1     // the degree count in k_emit_edges hands every edge its row slot: no atomics left in the CSR fill
-#endif
-#ifndef RB_OPT_FILL
-#define RB_OPT_FILL 1     // four independent atomics in flight per thread in the CSR fill
-#endif
-#ifndef RB_OPT_FUSE
-#define RB_OPT_FUSE 1     // small dependent-free kernels of the containment resolution share a launch
-#endif
-#ifndef RB_GROUP_PACKROW
-#define RB_GROUP_PACKROW 1  // K3 group kernel: row base and edge length of a neighbour in one 8-byte smem word (-4 % per step, r01l)
-#endif
-#ifndef RB_OPT_CONC
-#define RB_OPT_CONC 1     // independent kernels of one step on forked streams
-#endif
-
 namespace rb {
 
 constexpr uint32_t kInf = 0xFFFFFFFFu;         // "never dies" death time

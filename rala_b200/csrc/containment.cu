@@ -37,65 +37,14 @@ __device__ __forceinline__ uint32_t ld_state(const uint32_t* p) {
     return v;
 }
 
-// scatter the events into their victim's segment (order inside a segment is irrelevant)
-__global__ void k_events_fill(Events ev, const uint32_t* __restrict__ n_events, uint32_t ev_cap,
-                              uint32_t* __restrict__ vcursor, uint32_t* __restrict__ seg_c, uint32_t* __restrict__ seg_t) {
-    const uint32_t n = min(*n_events, ev_cap);
-#if RB_OPT_FILL
-    const uint32_t stride = gridDim.x * blockDim.x;   // four independent load -> atomic -> store chains per thread
-    for (uint32_t i0 = blockIdx.x * blockDim.x + threadIdx.x; i0 < n; i0 += 4u * stride) {
-        uint32_t v[4], c[4], t[4], p[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t i = i0 + k * stride;
-            if (i < n) { v[k] = ev.v[i]; c[k] = ev.c[i]; t[k] = ev.t[i]; }
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-            if (i0 + k * stride < n) p[k] = atomicAdd(&vcursor[v[k]], 1u);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (i0 + k * stride < n) {
-                seg_c[p[k]] = c[k];
-                seg_t[p[k]] = t[k];
-            }
-        }
-    }
-#else
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const uint32_t p = atomicAdd(&vcursor[ev.v[i]], 1u);
-        seg_c[p] = ev.c[i];
-        seg_t[p] = ev.t[i];
-    }
-#endif
-}
-
 __global__ void k_events_hist(Events ev, const uint32_t* __restrict__ n_events, uint32_t ev_cap, uint32_t* __restrict__ vcount) {
     const uint32_t n = min(*n_events, ev_cap);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) atomicAdd(&vcount[ev.v[i]], 1u);
 }
 
-__global__ void k_resolve_init(const uint32_t* __restrict__ vstart, uint32_t n_piles, uint32_t* __restrict__ S,
-                               uint32_t* __restrict__ work, uint32_t* __restrict__ n_work) {
-    for (uint32_t base = blockIdx.x * blockDim.x; base < n_piles; base += gridDim.x * blockDim.x) {
-        const uint32_t x = base + threadIdx.x;
-        bool victim = false;
-        if (x < n_piles) {
-            victim = vstart[x + 1] != vstart[x];
-            S[x] = victim ? 0u : (kSettled | kNever);
-        }
-        const uint32_t m = __ballot_sync(0xFFFFFFFFu, victim);
-        if (m) {
-            uint32_t gb = 0;
-            if (lane_id() == 0) gb = atomicAdd(n_work, (uint32_t) __popc(m));
-            gb = __shfl_sync(0xFFFFFFFFu, gb, 0);
-            if (victim) work[gb + __popc(m & ((1u << lane_id()) - 1u))] = x;
-        }
-    }
-}
-
-// k_events_fill and k_resolve_init do not depend on each other (both follow the scan of the victim histogram): one
-// launch, the first `fill_blocks` blocks scatter the events, the others initialise the states and the worklist.
+// Two independent jobs that both follow the scan of the victim histogram, in one launch: the first `fill_blocks` blocks
+// scatter the events into their victim's segment (order inside a segment is irrelevant), the others initialise the
+// states and the worklist.
 __global__ void __launch_bounds__(256) k_resolve_prepare(Events ev, const uint32_t* __restrict__ n_events, uint32_t ev_cap,
                                                         uint32_t* __restrict__ vcursor, uint32_t* __restrict__ seg_c,
                                                         uint32_t* __restrict__ seg_t, const uint32_t* __restrict__ vstart,
@@ -282,12 +231,6 @@ __global__ void __launch_bounds__(256) k_resolve(const uint32_t* __restrict__ vs
     }
 }
 
-static inline int grid_for(uint64_t n, int per_block, int max_blocks) {
-    uint64_t b = (n + per_block - 1) / per_block;
-    if (b < 1) b = 1;
-    return (int) (b < (uint64_t) max_blocks ? b : (uint64_t) max_blocks);
-}
-
 void launch_events_hist(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_cap, uint32_t* vcount) {
     k_events_hist<<<grid_for(ev_cap, 256, kNumSMs * 8), 256, 0, L.stream>>>(ev, n_events, ev_cap, vcount);
     L.count++;
@@ -310,19 +253,10 @@ void launch_resolve(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_
     int skip = skip_if_empty ? 1 : 0;
     launch_scan_u32(L, rb.vcursor, rb.vstart, n_piles + 1, status, ticket, nullptr, skip_if_empty ? n_events : nullptr);
     cudaMemsetAsync(rb.n_work, 0, 16, L.stream);
-#if RB_OPT_FUSE
-    {
-        const int fill_blocks = grid_for(ev_cap, 1024, kNumSMs * 4), init_blocks = grid_for(n_piles, 256, kNumSMs * 4);
-        k_resolve_prepare<<<fill_blocks + init_blocks, 256, 0, L.stream>>>(ev, n_events, ev_cap, rb.vcursor, rb.seg_c, rb.seg_t, rb.vstart,
-                                                                         n_piles, rb.S, rb.work0, rb.n_work, (uint32_t) fill_blocks, skip);
-        L.count++;
-    }
-#else
-    k_events_fill<<<grid_for(ev_cap, 256, kNumSMs * 8), 256, 0, L.stream>>>(ev, n_events, ev_cap, rb.vcursor, rb.seg_c, rb.seg_t);
+    const int fill_blocks = grid_for(ev_cap, 1024, kNumSMs * 4), init_blocks = grid_for(n_piles, 256, kNumSMs * 4);
+    k_resolve_prepare<<<fill_blocks + init_blocks, 256, 0, L.stream>>>(ev, n_events, ev_cap, rb.vcursor, rb.seg_c, rb.seg_t, rb.vstart,
+                                                                     n_piles, rb.S, rb.work0, rb.n_work, (uint32_t) fill_blocks, skip);
     L.count++;
-    k_resolve_init<<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(rb.vstart, n_piles, rb.S, rb.work0, rb.n_work);
-    L.count++;
-#endif
     void* args[] = {&rb.vstart, &rb.seg_c, &rb.seg_t, &rb.S, &rb.work0, &rb.work1, &rb.n_work, &counters, &n_events, &skip};
     cudaLaunchCooperativeKernel((void*) k_resolve, dim3(coop_blocks), dim3(256), args, 0, L.stream);
     L.count++;

@@ -39,11 +39,6 @@ __device__ __forceinline__ FabricHdr* hdr_of(const Peers& P, int q) { return rei
 template <class T>
 __device__ __forceinline__ T* section(const Peers& P, int q, size_t off) { return reinterpret_cast<T*>(P.base[q] + off); }
 
-static inline int grid_for(uint64_t n, int per_block, int max_blocks) {
-    uint64_t b = (n + per_block - 1) / per_block;
-    if (b < 1) b = 1;
-    return (int) (b < (uint64_t) max_blocks ? b : (uint64_t) max_blocks);
-}
 // x-dimension of a grid whose y-dimension is the source rank: about 8 blocks per SM over the whole grid, at least one per SM
 // (with kNumSMs blocks per source the inbox kernels ran on 148 blocks at world = 1 and took 2 - 3 x their time, profiles/r02v)
 static inline int blocks_per_source(int world) {

@@ -206,12 +206,8 @@ __global__ void __launch_bounds__(kTileThreads) k_scan_degrees(uint32_t* __restr
 // (k_finalize_marks reads whole 16-byte groups): a memset of the buffer's CAPACITY (2 x the record count) would
 // write ~15 x more bytes than there are edges.
 // eight edges in flight per thread, or twice the blocks, changed nothing (profiles/r02ab_ab.json)
-#ifndef RB_FILL_INFLIGHT
-#define RB_FILL_INFLIGHT 4
-#endif
-#ifndef RB_FILL_BLOCKS
-#define RB_FILL_BLOCKS 8   // per SM
-#endif
+constexpr int kFillInflight = 4;
+constexpr int kFillBlocks = 8;   // per SM
 __global__ void k_fill_csr(const uint32_t* __restrict__ src, const uint32_t* __restrict__ dst,
                            const uint32_t* __restrict__ len, const uint32_t* __restrict__ n_edges_ptr, uint32_t edge_cap,
                            uint32_t* __restrict__ cursor, uint2* __restrict__ col, uint32_t* __restrict__ col_eid,
@@ -222,10 +218,9 @@ __global__ void k_fill_csr(const uint32_t* __restrict__ src, const uint32_t* __r
         for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += gridDim.x * blockDim.x)
             reinterpret_cast<uint4*>(T)[i] = make_uint4(0u, 0u, 0u, 0u);
     }
-#if RB_OPT_FILL
     // load -> returning atomic -> store is a chain of three dependent round trips: keep four edges of it in flight
     const uint32_t stride = gridDim.x * blockDim.x;
-    constexpr int F = RB_FILL_INFLIGHT;
+    constexpr int F = kFillInflight;
     for (uint32_t e0 = blockIdx.x * blockDim.x + threadIdx.x; e0 < n; e0 += F * stride) {
         uint32_t s[F], d[F], l[F], p[F];
 #pragma unroll
@@ -254,13 +249,6 @@ __global__ void k_fill_csr(const uint32_t* __restrict__ src, const uint32_t* __r
             }
         }
     }
-#else
-    for (uint32_t e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
-        const uint32_t p = atomicAdd(&cursor[src[e]], 1u);
-        col[p] = make_uint2(dst[e], len[e]);
-        col_eid[p] = e;
-    }
-#endif
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -382,12 +370,6 @@ __global__ void k_time_bases(const uint32_t* __restrict__ counts, uint32_t rank,
     bases[1] = total_ovl + int_before;
 }
 
-static inline int grid_for(uint64_t n, int per_block, int max_blocks) {
-    uint64_t b = (n + per_block - 1) / per_block;
-    if (b < 1) b = 1;
-    return (int) (b < (uint64_t) max_blocks ? b : (uint64_t) max_blocks);
-}
-
 void launch_adjacency_view(Launch& L, const uint32_t* key, const uint8_t* marked, const uint32_t* n_edges_ptr, uint32_t edge_cap,
                            uint32_t n_nodes, uint32_t* degree_cursor, uint32_t* row_ptr, uint32_t* ids_tmp, uint32_t* ids_sorted,
                            unsigned long long* status, uint32_t* ticket) {
@@ -414,7 +396,7 @@ void launch_node_ids(Launch& L, const uint2* piles, uint32_t n_piles, uint32_t* 
 void launch_emit_edges(Launch& L, List ovl, const uint32_t* n_ptr, uint32_t cap, const uint2* piles, GraphArrays g,
                        uint32_t edge_cap, uint32_t* counters, unsigned long long* status, uint32_t* ticket) {
     k_emit_edges<<<grid_for(cap, kEmitTile, kNumSMs * 8), kTileThreads, 0, L.stream>>>(
-        ovl, n_ptr, cap, piles, g.seq_to_node, g.src, g.dst, g.len, edge_cap, g.cursor, RB_OPT_RANK ? g.rank : nullptr, counters, status, ticket);
+        ovl, n_ptr, cap, piles, g.seq_to_node, g.src, g.dst, g.len, edge_cap, g.cursor, g.rank, counters, status, ticket);
     L.count++;
 }
 
@@ -460,7 +442,7 @@ void launch_build_csr(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t e
     k_scan_degrees<<<grid_for(n_nodes_max + 1, kTile, kNumSMs * 8), kTileThreads, 0, L.stream>>>(
         g.cursor, g.row_ptr, n_nodes_max + 1, status, ticket, nullptr, nullptr, counters + C_NODES);
     L.count++;
-    k_fill_csr<<<grid_for(edge_cap, 256, kNumSMs * RB_FILL_BLOCKS), 256, 0, L.stream>>>(g.src, g.dst, g.len, counters + C_EDGES,
+    k_fill_csr<<<grid_for(edge_cap, 256, kNumSMs * kFillBlocks), 256, 0, L.stream>>>(g.src, g.dst, g.len, counters + C_EDGES,
                                                                             edge_cap, g.cursor, g.col, g.col_eid, g.T,
                                                                             ranked ? g.rank : nullptr, g.row_ptr);
     L.count++;

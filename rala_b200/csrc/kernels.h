@@ -40,6 +40,13 @@ struct Launch {
     cudaEvent_t ev_fork[2] = {nullptr, nullptr}, ev_join[2] = {nullptr, nullptr};
 };
 
+// grid of a grid-stride kernel: one block per per_block items, at least 1, at most max_blocks
+inline int grid_for(uint64_t n, int per_block, int max_blocks) {
+    uint64_t b = (n + per_block - 1) / per_block;
+    if (b < 1) b = 1;
+    return (int) (b < (uint64_t) max_blocks ? b : (uint64_t) max_blocks);
+}
+
 // side[k] continues from the current end of the main stream; false when the context has no side streams
 inline bool fork_side(Launch& L, int k) {
     if (!L.side[k]) return false;
@@ -82,7 +89,6 @@ void launch_classify_final(Launch& L, List ovl, const uint32_t* n_ovl, const uin
                            const uint32_t* n_inl, const uint32_t* inl_time_base, uint32_t cap, const uint2* piles, Events ev,
                            uint32_t ev_cap, uint32_t* vcount, uint32_t* counters);
 void launch_trim_classify_aos(Launch& L, uint32_t* rec, uint32_t n, const uint2* piles, uint32_t n_piles, uint8_t* type_out);
-void launch_fill_u32(Launch& L, uint32_t* p, uint32_t v, size_t n);
 void launch_pack_piles(Launch& L, const uint2* in, const uint8_t* flags, uint2* out, uint32_t n);
 void launch_unpack_piles(Launch& L, const uint2* in, uint2* out, uint32_t n);
 void launch_list_to_aos(Launch& L, List l, const uint32_t* n_ptr, uint32_t cap, uint32_t* out);
@@ -126,10 +132,7 @@ void launch_node_ids(Launch& L, const uint2* piles, uint32_t n_piles, uint32_t* 
                      unsigned long long* status, uint32_t* ticket);
 // entries per thread of k_emit_edges (its tiles are 256 x this); its look-back scan needs one status word per tile.
 // 2 and 1 (more, smaller tiles: a longer look-back chain) measured no faster than 4 (profiles/r02aa_ab.json).
-#ifndef RB_EMIT_ITEMS
-#define RB_EMIT_ITEMS 4
-#endif
-constexpr int kEmitItems = RB_EMIT_ITEMS;
+constexpr int kEmitItems = 4;
 inline uint64_t emit_scan_span(uint64_t cap) { return cap * (4 / kEmitItems); }   // in units of the common 1024-entry tile
 void launch_emit_edges(Launch& L, List ovl, const uint32_t* n_ptr, uint32_t cap, const uint2* piles, GraphArrays g,
                        uint32_t edge_cap, uint32_t* counters, unsigned long long* status, uint32_t* ticket);

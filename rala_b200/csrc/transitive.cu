@@ -115,22 +115,15 @@ struct GroupSmem {
     uint32_t keys[kGroupMaxDeg];             // destinations, sorted; kEmpty behind the last one
     uint32_t eid[kGroupMaxDeg];              // edge id at that position
     uint2 iv[kGroupMaxDeg];                  // comparable(sum, len of that edge)  <=>  sum - iv.x <= iv.y
-#if RB_GROUP_PACKROW
     uint2 prow[kGroupMaxDeg];                // per neighbour b: (start of row b in col - its offset in the flat stream, len of a->b)
-#else
-    uint32_t nrow[kGroupMaxDeg];
-    uint32_t nlen[kGroupMaxDeg];
-#endif
     uint32_t noff[kGroupMaxDeg + 1];
     uint32_t hit;                            // bit j: the edge at sorted position j passed the test
 };
 
 // resident blocks per SM: 6 (40 registers) is a sharp optimum: 115 us, against 134 us at 4 or 5 and 148 us at 7 or 8
 // (profiles/r02ab_ab.json, r02ad_ab.json): the kernel lives on its shared-memory / L1 data path (69 % of peak)
-#ifndef RB_GROUP_MINB
-#define RB_GROUP_MINB 6
-#endif
-__global__ void __launch_bounds__(kLightWarps * 32, RB_GROUP_MINB) k_transitive_group(
+constexpr int kGroupMinBlocks = 6;
+__global__ void __launch_bounds__(kLightWarps * 32, kGroupMinBlocks) k_transitive_group(
     const uint32_t* __restrict__ row_ptr, const uint2* __restrict__ col, const uint32_t* __restrict__ col_eid,
     uint8_t* __restrict__ T, uint32_t node_begin, uint32_t node_end, const uint32_t* __restrict__ node_range,
     const uint32_t* __restrict__ n_nodes_ptr, uint32_t* __restrict__ work_counter, HeavyItems heavy,
@@ -167,9 +160,7 @@ __global__ void __launch_bounds__(kLightWarps * 32, RB_GROUP_MINB) k_transitive_
             // ---- this lane's (at most two) neighbours ----
             unsigned long long mine[2] = {~0ull, ~0ull};
             uint32_t dg[2] = {0u, 0u}, my_len[2] = {0u, 0u};
-#if RB_GROUP_PACKROW
             uint32_t rs2[2] = {0u, 0u};
-#endif
             if (act) {
 #pragma unroll
                 for (int h = 0; h < 2; ++h) {
@@ -180,12 +171,7 @@ __global__ void __launch_bounds__(kLightWarps * 32, RB_GROUP_MINB) k_transitive_
                         my_len[h] = e.y;
                         const uint32_t rs = row_ptr[e.x];
                         dg[h] = row_ptr[e.x + 1] - rs;
-#if RB_GROUP_PACKROW
                         rs2[h] = rs;
-#else
-                        S.nrow[i] = rs;
-                        S.nlen[i] = e.y;
-#endif
                     }
                     S.ukey[i] = mine[h];
                 }
@@ -198,11 +184,9 @@ __global__ void __launch_bounds__(kLightWarps * 32, RB_GROUP_MINB) k_transitive_
                 if (gl < d) S.noff[gl] = inc0 - dg[0];
                 if (gl + kGroupLanes < d) S.noff[gl + kGroupLanes] = tot0 + inc1 - dg[1];
                 if (gl == 0) S.noff[d] = W;
-#if RB_GROUP_PACKROW
                 // element f of the flat stream that falls into row i is col[prow[i].x + f]
                 if (gl < d) S.prow[gl] = make_uint2(rs2[0] - (inc0 - dg[0]), my_len[0]);
                 if (gl + kGroupLanes < d) S.prow[gl + kGroupLanes] = make_uint2(rs2[1] - (tot0 + inc1 - dg[1]), my_len[1]);
-#endif
             }
             __syncwarp();
             if (act && W > kGroupMaxVisits) {   // short row, very long rows behind it: give the node to a block
@@ -251,14 +235,9 @@ __global__ void __launch_bounds__(kLightWarps * 32, RB_GROUP_MINB) k_transitive_
                         lab[u] = 0u;
                         if (ok[u]) {
                             while (f >= S.noff[i + 1]) ++i;
-#if RB_GROUP_PACKROW
                             const uint2 row = S.prow[i];
                             e[u] = col[row.x + f];
                             lab[u] = row.y;
-#else
-                            e[u] = col[S.nrow[i] + (f - S.noff[i])];
-                            lab[u] = S.nlen[i];
-#endif
                         }
                     }
                     uint32_t pass = 0;   // bit j: a witness for the edge at sorted position j
@@ -602,11 +581,7 @@ void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t 
     if (blocks > (uint64_t) kNumSMs * 8) blocks = kNumSMs * 8;
     // the group and the light kernel take disjoint sets of nodes (by out-degree) and only meet in atomics (heavy work
     // list, visit counter): the light one (14 us, mostly idle SMs) runs beside the group one on a forked stream
-#if RB_OPT_CONC
     const bool forked = fork_side(L, 1);
-#else
-    const bool forked = false;
-#endif
     k_transitive_group<<<(int) blocks, kLightWarps * 32, 0, L.stream>>>(g.row_ptr, g.col, g.col_eid, g.T, node_begin, node_end,
                                                                        node_range, counters + C_NODES, work_counter + 1, heavy, counters);
     L.count++;
