@@ -61,17 +61,11 @@ def trim_type(rec, pa, pb):
 
 def trim_type_batch(rec, piles):
     """rec (n,7), piles (n_piles,2) -> (trimmed (n,7), type (n,) uint8 with 255 = rejected)."""
-    r = _u32(rec).copy()
-    piles = _u32(piles)
-    n_piles = C.c_uint32(piles.shape[0])
+    r = _u32(rec).reshape(-1, 7).copy()
+    piles = _u32(piles).reshape(-1, 2)
     types = np.full(r.shape[0], REJECT, dtype=np.uint8)
-    L = lib()
-    for i in range(r.shape[0]):
-        if r[i, 6] & 2:
-            continue
-        row = r[i]
-        if L.ora_trim(_p(row), _p(piles), n_piles):
-            types[i] = L.ora_type(_p(row), _p(piles))
+    if r.shape[0]:
+        lib().ora_trim_type_batch(_p(r), C.c_uint64(r.shape[0]), _p(piles), C.c_uint32(piles.shape[0]), _p(types, C.c_uint8))
     return r, types
 
 

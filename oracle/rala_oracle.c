@@ -91,7 +91,16 @@ int ora_type(const uint32_t* r, const uint32_t* piles) {
     return type_with_coords(r, piles, &a0, &a1, &b0, &b1, &al, &bl);
 }
 
-/* pile.cpp:457-469 (SURVEY.md A.6): note begin_ is added to coordinates that are already absolute */
+void ora_trim_type_batch(uint32_t* rec, uint64_t n, const uint32_t* piles, uint32_t n_piles, uint8_t* types) {
+    for (uint64_t i = 0; i < n; ++i) {
+        uint32_t* r = rec + REC * i;
+        types[i] = 255;
+        if (!(r[6] & 2u) && ora_trim(r, piles, n_piles)) types[i] = (uint8_t) ora_type(r, piles);
+    }
+}
+
+/* pile.cpp:457-469 (SURVEY.md A.6): note begin_ is added to coordinates that are already absolute.  The pile picks the
+ * side by comparing the overlap's a id with its own id, so a self overlap (a == b) bumps twice with the a-side span. */
 static void bump_hills(const uint32_t* hills, uint32_t n_hills, uint32_t* cov,
                        uint32_t pile, uint32_t pile_begin, uint32_t lo, uint32_t hi) {
     uint32_t begin = pile_begin + lo, end = pile_begin + hi;
@@ -129,7 +138,8 @@ void ora_classify(const uint32_t* rec, uint64_t n, uint32_t* piles, const uint8_
         if (!ora_trim(r, piles, n_piles)) continue;                                     /* :452 */
         uint32_t a = r[0], b = r[1];
         if (pflags[a] & 1u) bump_hills(hills, n_hills, hill_cov, a, piles[2 * a], r[2], r[3]);   /* :457-459 */
-        if (pflags[b] & 1u) bump_hills(hills, n_hills, hill_cov, b, piles[2 * b], r[4], r[5]);   /* :460-462 */
+        if (pflags[b] & 1u) bump_hills(hills, n_hills, hill_cov, b, piles[2 * b],
+                                       a == b ? r[2] : r[4], a == b ? r[3] : r[5]);              /* :460-462 */
         switch (ora_type(r, piles)) {                                                   /* :464-483 */
             case ORA_KX:
                 memcpy(int_out + REC * n_int++, r, sizeof(r));

@@ -454,8 +454,11 @@ __global__ void k_hill_coverage(List recs, uint32_t t0, const uint2* __restrict_
             const Pile& p = side ? pb : pa;
             if (!(p.flags & 1u)) continue;
             const uint32_t id = side ? e.b : e.a;
-            const uint32_t lo = p.begin + (side ? e.c.bb : e.c.ab);   // begin_ added to absolute coordinates, as in :459-462
-            const uint32_t hi = p.begin + (side ? e.c.be : e.c.ae);
+            // begin_ added to absolute coordinates, as in :459-462; the pile takes the b side only when it is not also the
+            // a pile (it compares the overlap's a id with its own), so a self overlap counts its a-side span twice
+            const bool b_side = side && e.a != e.b;
+            const uint32_t lo = p.begin + (b_side ? e.c.bb : e.c.ab);
+            const uint32_t hi = p.begin + (b_side ? e.c.be : e.c.ae);
             uint32_t l = 0, h = n_hills;
             while (l < h) {
                 uint32_t m = (l + h) >> 1;
