@@ -202,7 +202,8 @@ def bench_main(args):
             raise api.RalaB200Error("a capacity-bounded exchange overflowed during the timed region")
         c = sess.counts()
         E, n_nodes, n_pairs, n_two_hop = c["n_edges"], c["n_nodes"], c["n_transitive_pairs"], c["n_two_hop"]
-        n_events, n_final_events, rounds = dg.last_info["n_events"], dg.last_info["n_final_events"], [c["n_rounds"], c["n_final_rounds"]]
+        # the imported event lists are every rank's: these counts are totals over the ranks
+        n_events, n_final_events, rounds = c["n_candidates"], c["n_final_candidates"], [c["n_rounds"], c["n_final_rounds"]]
         first = 0
         e_mine, m_mine = (sess.edges(), sess.marked()) if rank == 0 else (np.zeros((0, 3), np.uint32), np.zeros(0, np.uint8))
     parity = None

@@ -226,45 +226,36 @@ int rala_b200_graph_stage_ms(rala_b200_graph* g, float* ms_out /* RALA_B200_N_ST
  * by source-node range (transitive), the event lists and the edge list all-gathered, the marks
  * merged with an all-reduce(max) (= OR on 0/1 bytes).  The collectives are the caller's
  * (rala_b200/multi.py uses torch.distributed / NCCL); every pointer below is a DEVICE pointer of
- * the caller's exchange buffer, laid out as three columns of `stride` 32-bit words
- * (events: victim | container | time;  edges: src | dst | len).
+ * the caller's exchange buffer.  No call synchronises with the host: element counts travel inside the
+ * exchange blocks and the time bases of the final pass are computed on the device.
  *
  *   set_shard; set_piles; set_overlaps(local records)
- *   phase_events              -> events_count, export_events, [all-gather], import_events (all ranks' blocks)
+ *   phase_events              -> export_padded(0), [all-gather], import_gathered(0) (all ranks' blocks)
  *   phase_resolve(1)          ordered containment of graph.cpp:469-480 on the union of the events (replicated)
- *   phase_survivors           -> list_counts, [all-gather counts]
- *   phase_final_events(ovl_base, int_base)  time = global position in overlaps ++ internals (graph.cpp:831-866)
- *                             -> events_count, export_events, [all-gather], import_events
+ *   phase_survivors           -> export_list_counts, [all-gather]
+ *   phase_final_events_gathered   time = global position in overlaps ++ internals (graph.cpp:831-866)
+ *                             -> export_padded(0), [all-gather], import_gathered(0)
  *   phase_resolve(0)
- *   phase_emit_edges          -> export_edges, [all-gather], import_edges (global edge-id order = rank order)
+ *   phase_emit_edges          -> export_padded(1), [all-gather], import_gathered(1) (global edge-id order = rank order)
  *   phase_csr                 CSR of the whole graph, replicated (two-hop lookups cross shards)
  *   phase_transitive          T(e) for candidate edges whose source node this rank owns
  *   export_marks, [all-reduce(max)], phase_marks     marked(e) = T(e) | T(e^1)
+ *
+ * Exchange blocks (rala_b200_exchange_block_words(kind, cap) = 3 * cap + 4 words):
+ *   kind 0, containment events: [n clamped to cap | overflow flag | n | 0 | victim [cap] | container [cap] | time [cap]]
+ *   kind 1, edges: the same layout with src | dst | len
+ * n is the exporting rank's element count.  d_gathered = the `world` blocks of an all-gather, in rank order.  A count
+ * beyond `cap` raises the session's overflow flag (reported by rala_b200_graph_counts); the largest word 2 of the
+ * gathered blocks is the smallest `cap` that fits.
  * ---------------------------------------------------------------------------------------------- */
 /* a context that enqueues on the caller's CUDA stream (cudaStream_t), e.g. torch's current stream */
 int rala_b200_create_on_stream(rala_b200_ctx** out, int device, void* cuda_stream);
 int rala_b200_graph_set_shard(rala_b200_graph* g, uint32_t t0, int rank, int world);
 int rala_b200_graph_phase_events(rala_b200_graph* g);
-int rala_b200_graph_events_count(rala_b200_graph* g, uint32_t* n);
-int rala_b200_graph_export_events(rala_b200_graph* g, uint32_t* d_cols, uint32_t stride, uint32_t n);
-int rala_b200_graph_import_events(rala_b200_graph* g, const uint32_t* d_cols, uint32_t stride, uint32_t n,
-                                  uint32_t offset, uint32_t total);
 int rala_b200_graph_phase_resolve(rala_b200_graph* g, int first_pass);
 int rala_b200_graph_phase_survivors(rala_b200_graph* g);
-int rala_b200_graph_list_counts(rala_b200_graph* g, uint32_t* n_ovl, uint32_t* n_int);
-int rala_b200_graph_phase_final_events(rala_b200_graph* g, uint32_t ovl_base, uint32_t int_base);
-int rala_b200_graph_phase_emit_edges(rala_b200_graph* g, uint32_t* n_local_edges);
-int rala_b200_graph_export_edges(rala_b200_graph* g, uint32_t* d_cols, uint32_t stride, uint32_t n);
-int rala_b200_graph_import_edges(rala_b200_graph* g, const uint32_t* d_cols, uint32_t stride, uint32_t n,
-                                 uint32_t offset, uint32_t total);
+int rala_b200_graph_phase_emit_edges(rala_b200_graph* g);
 int rala_b200_graph_phase_csr(rala_b200_graph* g);
-/* Capacity-bounded variants of the exchange steps: element counts travel inside the blocks and the time bases are
- * computed on the device, so no call below synchronises with the host (the sized variants above read counts back).
- *   kind 0, containment events: block (3 * cap + 4 words) = [n clamped to cap | overflow flag | 0 | 0 | victim [cap] | container [cap] | time [cap]]
- *   kind 1, edges: the same layout with src | dst | len
- *   rala_b200_exchange_block_words(kind, cap) is the block size in 32-bit words.  d_gathered = the `world` blocks of an all-gather, in rank order.
- * A count beyond `cap` raises the session's overflow flag (reported by rala_b200_graph_counts): re-run sized.
- * rala_b200_graph_phase_emit_edges accepts n_local_edges == NULL (no read-back). */
 uint64_t rala_b200_exchange_block_words(int kind, uint32_t cap);
 int rala_b200_graph_export_padded(rala_b200_graph* g, int kind, uint32_t* d_block, uint32_t cap);
 int rala_b200_graph_import_gathered(rala_b200_graph* g, int kind, const uint32_t* d_gathered, uint32_t cap, int world);

@@ -56,10 +56,8 @@ EXPORTS = [
     "rala_b200_graph_set_overlaps_packed", "rala_b200_multi_set_overlaps_packed", "rala_b200_graph_get_adjacency",
     # multi-GPU phases
     "rala_b200_create_on_stream", "rala_b200_graph_set_shard", "rala_b200_graph_phase_events",
-    "rala_b200_graph_events_count", "rala_b200_graph_export_events", "rala_b200_graph_import_events",
-    "rala_b200_graph_phase_resolve", "rala_b200_graph_phase_survivors", "rala_b200_graph_list_counts",
-    "rala_b200_graph_phase_final_events", "rala_b200_graph_phase_emit_edges", "rala_b200_graph_export_edges",
-    "rala_b200_graph_import_edges", "rala_b200_graph_phase_csr", "rala_b200_graph_phase_transitive",
+    "rala_b200_graph_phase_resolve", "rala_b200_graph_phase_survivors", "rala_b200_graph_phase_emit_edges",
+    "rala_b200_graph_phase_csr", "rala_b200_graph_phase_transitive",
     "rala_b200_graph_export_marks", "rala_b200_graph_phase_marks",
     "rala_b200_graph_export_padded", "rala_b200_graph_import_gathered", "rala_b200_graph_export_list_counts",
     "rala_b200_graph_phase_final_events_gathered", "rala_b200_exchange_block_words",

@@ -676,11 +676,10 @@ extern "C" int rala_b200_graph_finalize(rala_b200_graph* g) {
     return rc;
 }
 
-// graph.cpp:552-632
-extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
-    if (!g) return RALA_B200_ERR_ARG;
+// node ids + the edges of the overlaps in list order (graph.cpp:552-632).  In a multi-GPU phase the list is the local
+// shard's and the node ids are global: the pile table is replicated.
+static int emit_edges(rala_b200_graph* g) {
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "build: finalize first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_BUILD));
     CU(ctx, zero_counter(g, C_NODES, 4));   // C_NODES, C_ALIVE, C_DOVETAILS, C_EDGES
@@ -692,6 +691,18 @@ extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
     scan_state(g, emit_scan_span(g->cap), &status, &ticket);
     launch_emit_edges(ctx->L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), g->graph_view(),
                       g->edge_cap, g->cnt(), status, ticket);
+    return RALA_B200_OK;
+}
+
+// graph.cpp:552-632
+extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
+    if (!g) return RALA_B200_ERR_ARG;
+    rala_b200_ctx* ctx = g->ctx;
+    if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "build: finalize first");
+    int rc = emit_edges(g);
+    if (rc) return rc;
+    unsigned long long* status;
+    uint32_t* ticket;
     // the edge list is final: rows into the caller's buffer on a forked stream, beside the CSR build and (inside a
     // whole run) the transitive pass; edges beyond the caller's capacity are not written (n_edges tells)
     if (g->out_edges && g->out_edges_cap && fork_side(ctx->L, 0)) {
@@ -1187,11 +1198,13 @@ extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes,
 // Multi-GPU phases (one process per GPU).  The records are sharded by contiguous file range, the pile
 // table is replicated; the collectives between the phases belong to the caller (NCCL through
 // torch.distributed in rala_b200/multi.py), which passes DEVICE pointers of its exchange buffers:
-//   phase_events -> [all-gather events] -> import_events -> phase_resolve(1) -> phase_survivors
-//   -> [all-gather list counts] -> phase_final_events -> [all-gather events] -> import_events
-//   -> phase_final_resolve -> phase_emit_edges -> [all-gather edges] -> import_edges -> phase_csr
-//   -> phase_transitive(rank, world) -> [all-reduce(max) marks] -> phase_marks
-// Exchange blocks are three columns of `stride` words: events v | c | t, edges src | dst | len.
+//   phase_events -> export_padded -> [all-gather] -> import_gathered -> phase_resolve(1) -> phase_survivors
+//   -> export_list_counts -> [all-gather] -> phase_final_events_gathered -> export_padded -> [all-gather]
+//   -> import_gathered -> phase_resolve(0) -> phase_emit_edges -> export_padded -> [all-gather] -> import_gathered
+//   -> phase_csr -> phase_transitive -> export_marks -> [all-reduce(max)] -> phase_marks
+// No call reads a count back to the host: counts travel inside the exchange blocks (k_export_padded has the layout),
+// the time bases of the final pass are computed on the device, and a block too small for its rank's elements raises
+// the session's overflow flag.
 // ---------------------------------------------------------------------------------------------
 extern "C" int rala_b200_graph_set_shard(rala_b200_graph* g, uint32_t t0, int rank, int world) {
     if (!g || world < 1 || rank < 0 || rank >= world) return RALA_B200_ERR_ARG;
@@ -1203,59 +1216,6 @@ extern "C" int rala_b200_graph_set_shard(rala_b200_graph* g, uint32_t t0, int ra
 
 extern "C" int rala_b200_graph_phase_events(rala_b200_graph* g) { return g ? phase_events(g) : RALA_B200_ERR_ARG; }
 
-static int read_counter(rala_b200_graph* g, int slot, uint32_t* out) {
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, cudaMemcpyAsync(out, g->cnt() + slot, 4, cudaMemcpyDeviceToHost, ctx->L.stream));
-    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
-    return RALA_B200_OK;
-}
-
-extern "C" int rala_b200_graph_events_count(rala_b200_graph* g, uint32_t* n) {
-    if (!g || !n) return RALA_B200_ERR_ARG;
-    int rc = read_counter(g, C_EV, n);
-    if (!rc && *n > g->ev_cap) return fail(g->ctx, RALA_B200_ERR_LIMIT, "event list overflow (%u > %u)", *n, g->ev_cap);
-    return rc;
-}
-
-extern "C" int rala_b200_graph_export_events(rala_b200_graph* g, uint32_t* d_cols, uint32_t stride, uint32_t n) {
-    if (!g || (n && !d_cols) || n > stride) return RALA_B200_ERR_ARG;
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    Events ev = g->events_view();
-    if (n) {
-        CU(ctx, cudaMemcpyAsync(d_cols, ev.v, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(d_cols + stride, ev.c, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(d_cols + 2 * (size_t) stride, ev.t, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    }
-    return RALA_B200_OK;
-}
-
-extern "C" int rala_b200_graph_import_events(rala_b200_graph* g, const uint32_t* d_cols, uint32_t stride, uint32_t n,
-                                             uint32_t offset, uint32_t total) {
-    if (!g || (n && !d_cols) || (uint64_t) offset + n > total) return RALA_B200_ERR_ARG;
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    if (offset == 0) {
-        int rc = reserve_events(g, total);   // the local events were exported before the first import
-        if (rc) return rc;
-    }
-    Events ev = g->events_view();
-    if (n) {
-        CU(ctx, cudaMemcpyAsync(ev.v + offset, d_cols, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(ev.c + offset, d_cols + stride, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(ev.t + offset, d_cols + 2 * (size_t) stride, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    }
-    if ((uint64_t) offset + n == total) {
-        CU(ctx, cudaMemcpyAsync(g->cnt() + C_EV, &total, 4, cudaMemcpyHostToDevice, ctx->L.stream));
-        CU(ctx, cudaStreamSynchronize(ctx->L.stream));   // `total` lives on this stack frame
-        CU(ctx, clear_victim_histogram(g));
-        launch_events_hist(ctx->L, g->events_view(), g->cnt() + C_EV, g->ev_cap, resolve_bufs(g).vcursor);
-        CU(ctx, cudaGetLastError());
-    }
-    return RALA_B200_OK;
-}
-
 extern "C" int rala_b200_graph_phase_resolve(rala_b200_graph* g, int first_pass) {
     if (!g) return RALA_B200_ERR_ARG;
     return first_pass ? phase_resolve(g, true) : phase_final_resolve(g);
@@ -1263,84 +1223,17 @@ extern "C" int rala_b200_graph_phase_resolve(rala_b200_graph* g, int first_pass)
 
 extern "C" int rala_b200_graph_phase_survivors(rala_b200_graph* g) { return g ? phase_survivors(g) : RALA_B200_ERR_ARG; }
 
-extern "C" int rala_b200_graph_list_counts(rala_b200_graph* g, uint32_t* n_ovl, uint32_t* n_int) {
-    if (!g || !n_ovl || !n_int) return RALA_B200_ERR_ARG;
-    if (g->state < 2) return fail(g->ctx, RALA_B200_ERR_STATE, "list_counts: classify first");
-    uint32_t h[C_COUNT];
-    int rc = read_counters(g, h);
-    if (rc) return rc;
-    *n_ovl = h[g->slot_ovl];
-    *n_int = h[g->slot_inl];
-    return RALA_B200_OK;
-}
-
-extern "C" int rala_b200_graph_phase_final_events(rala_b200_graph* g, uint32_t ovl_base, uint32_t int_base) {
-    if (!g) return RALA_B200_ERR_ARG;
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    uint32_t bases[2] = {ovl_base, int_base};
-    CU(ctx, cudaMemcpyAsync(g->cnt() + C_TBASE_OVL, bases, 8, cudaMemcpyHostToDevice, ctx->L.stream));
-    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
-    g->final_time_base_slot = C_TBASE_INL;
-    return phase_final_events(g, g->cnt() + C_TBASE_OVL, g->cnt() + C_TBASE_INL);
-}
-
 // node ids (replicated) + the edges of the LOCAL overlaps, in local list order, with global node ids
-extern "C" int rala_b200_graph_phase_emit_edges(rala_b200_graph* g, uint32_t* n_local_edges) {
+extern "C" int rala_b200_graph_phase_emit_edges(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "emit_edges: finalize first");
-    CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, begin_stage(g, ST_BUILD));
-    CU(ctx, zero_counter(g, C_NODES, 4));
-    CU(ctx, cudaMemsetAsync(g->cursor.p, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
-    unsigned long long* status;
-    uint32_t* ticket;
-    scan_state(g, g->n_piles, &status, &ticket);
-    launch_node_ids(ctx->L, g->piles.as<uint2>(), g->n_piles, g->seq_to_node.as<uint32_t>(), g->cnt(), status, ticket);
-    scan_state(g, emit_scan_span(g->cap), &status, &ticket);
-    launch_emit_edges(ctx->L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), g->graph_view(),
-                      g->edge_cap, g->cnt(), status, ticket);
+    int rc = emit_edges(g);
+    if (rc) return rc;
     CU(ctx, cudaGetLastError());
-    return n_local_edges ? read_counter(g, C_EDGES, n_local_edges) : RALA_B200_OK;   // NULL: no host synchronisation
-}
-
-extern "C" int rala_b200_graph_export_edges(rala_b200_graph* g, uint32_t* d_cols, uint32_t stride, uint32_t n) {
-    if (!g || (n && !d_cols) || n > stride) return RALA_B200_ERR_ARG;
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    GraphArrays ga = g->graph_view();
-    if (n) {
-        CU(ctx, cudaMemcpyAsync(d_cols, ga.src, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(d_cols + stride, ga.dst, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(d_cols + 2 * (size_t) stride, ga.len, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    }
     return RALA_B200_OK;
 }
 
-extern "C" int rala_b200_graph_import_edges(rala_b200_graph* g, const uint32_t* d_cols, uint32_t stride, uint32_t n,
-                                            uint32_t offset, uint32_t total) {
-    if (!g || (n && !d_cols) || (uint64_t) offset + n > total) return RALA_B200_ERR_ARG;
-    rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, cudaSetDevice(ctx->device));
-    if (offset == 0) {
-        int rc = reserve_edges(g, total);   // the local edges were exported before the first import
-        if (rc) return rc;
-    }
-    GraphArrays ga = g->graph_view();
-    if (n) {
-        CU(ctx, cudaMemcpyAsync(ga.src + offset, d_cols, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(ga.dst + offset, d_cols + stride, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-        CU(ctx, cudaMemcpyAsync(ga.len + offset, d_cols + 2 * (size_t) stride, (size_t) n * 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    }
-    if ((uint64_t) offset + n == total) {
-        CU(ctx, cudaMemcpyAsync(g->cnt() + C_EDGES, &total, 4, cudaMemcpyHostToDevice, ctx->L.stream));
-        CU(ctx, cudaStreamSynchronize(ctx->L.stream));
-    }
-    return RALA_B200_OK;
-}
-
-// ---- capacity-bounded exchange: counts travel inside the blocks, nothing is read back by the host ------------------------
 extern "C" int rala_b200_graph_export_padded(rala_b200_graph* g, int kind, uint32_t* d_block, uint32_t cap) {
     if (!g || !d_block || cap == 0 || (kind != 0 && kind != 1)) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;

@@ -317,13 +317,14 @@ __global__ void __launch_bounds__(256) k_pack_edges(const uint32_t* __restrict__
 
 // ---------------------------------------------------------------------------------------------
 // Capacity-bounded exchange blocks of the multi-GPU path: the element count travels INSIDE the block, so the
-// host never has to read it (no synchronisation around the collectives).
-//   block = [n (clamped to cap) | overflow flag | 0 | 0 | column 0 [cap] | column 1 [cap] | column 2 [cap]]
+// host never has to read it (no synchronisation around the collectives).  Word 2 is the rank's whole count, so after an
+// overflow the caller learns from the gathered blocks how large `cap` has to be.
+//   block = [n clamped to cap | overflow flag | n | 0 | column 0 [cap] | column 1 [cap] | column 2 [cap]]
 // ---------------------------------------------------------------------------------------------
 __global__ void k_export_padded(const uint32_t* __restrict__ c0, const uint32_t* __restrict__ c1, const uint32_t* __restrict__ c2,
                                 const uint32_t* __restrict__ n_ptr, uint32_t src_cap, uint32_t cap, uint32_t* __restrict__ block) {
     const uint32_t n = min(*n_ptr, src_cap), m = min(n, cap);
-    if (blockIdx.x == 0 && threadIdx.x < 4) block[threadIdx.x] = threadIdx.x == 0 ? m : (threadIdx.x == 1 ? (n > cap ? 1u : 0u) : 0u);
+    if (blockIdx.x == 0 && threadIdx.x < 4) block[threadIdx.x] = threadIdx.x == 0 ? m : (threadIdx.x == 1 ? (n > cap ? 1u : 0u) : (threadIdx.x == 2 ? n : 0u));
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
         block[4 + i] = c0[i];
         block[4 + (size_t) cap + i] = c1[i];

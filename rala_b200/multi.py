@@ -8,7 +8,9 @@ timing reductions of the bench.  A step enqueues kernels only and is replayed as
 
 FALLBACK TRANSPORT — `DistributedGraph` over `CudaShardSession`: the round-1 path, NCCL collectives issued through
 torch.distributed between the library's phases, with the CSR built on every rank.  Used only when the GPUs cannot map
-each other's memory (no peer access / no CUDA IPC); both are checked against the oracle by the same tests.
+each other's memory (no peer access / no CUDA IPC); both are checked against the oracle by the same tests.  Every
+exchange all-gathers fixed-capacity blocks that carry their own element counts, so a pass never waits for the host;
+like the product path, `DistributedGraph.plan` sizes the capacities from real passes.
 
 Partition of the fallback transport (BASELINE.json north_star; SURVEY.md 8e):
   * overlap records are sharded by contiguous FILE RANGE (rank r holds records [t0_r, t0_r + n_r)); the
@@ -59,52 +61,26 @@ class CudaShardSession:
 
     # ---- inputs -------------------------------------------------------------------------------------------
     def set_inputs(self, records, piles, flags, t0: int, rank: int, world: int):
+        self.n_records = len(records)
         self.G.set_piles(piles, flags).set_hills(None).set_overlaps(records)
         self.G._call("rala_b200_graph_set_shard", C.c_uint32(t0), C.c_int(rank), C.c_int(world))
-
-    def _u32(self, name, *args):
-        out = C.c_uint32(0)
-        self.G._call(name, *args, C.byref(out))
-        return int(out.value)
 
     @staticmethod
     def _dp(t: torch.Tensor):
         return C.c_void_p(t.data_ptr())
 
-    # ---- phases -------------------------------------------------------------------------------------------
-    def phase_events(self) -> int:
+    # ---- phases: none reads a count back to the host (counts travel inside the exchange blocks) -------------------
+    def phase_events(self):
         self.G._call("rala_b200_graph_phase_events")
-        return self._u32("rala_b200_graph_events_count")
-
-    def export_events(self, block: torch.Tensor, n: int):
-        self.G._call("rala_b200_graph_export_events", self._dp(block), C.c_uint32(block.shape[1]), C.c_uint32(n))
-
-    def import_events(self, block: torch.Tensor, n: int, offset: int, total: int):
-        self.G._call("rala_b200_graph_import_events", self._dp(block), C.c_uint32(block.shape[1]), C.c_uint32(n),
-                     C.c_uint32(offset), C.c_uint32(total))
 
     def phase_resolve(self, first: bool):
         self.G._call("rala_b200_graph_phase_resolve", C.c_int(1 if first else 0))
 
     def phase_survivors(self):
         self.G._call("rala_b200_graph_phase_survivors")
-        a, b = C.c_uint32(0), C.c_uint32(0)
-        self.G._call("rala_b200_graph_list_counts", C.byref(a), C.byref(b))
-        return int(a.value), int(b.value)
 
-    def phase_final_events(self, ovl_base: int, int_base: int) -> int:
-        self.G._call("rala_b200_graph_phase_final_events", C.c_uint32(ovl_base), C.c_uint32(int_base))
-        return self._u32("rala_b200_graph_events_count")
-
-    def phase_emit_edges(self) -> int:
-        return self._u32("rala_b200_graph_phase_emit_edges")
-
-    def export_edges(self, block: torch.Tensor, n: int):
-        self.G._call("rala_b200_graph_export_edges", self._dp(block), C.c_uint32(block.shape[1]), C.c_uint32(n))
-
-    def import_edges(self, block: torch.Tensor, n: int, offset: int, total: int):
-        self.G._call("rala_b200_graph_import_edges", self._dp(block), C.c_uint32(block.shape[1]), C.c_uint32(n),
-                     C.c_uint32(offset), C.c_uint32(total))
+    def phase_emit_edges(self):
+        self.G._call("rala_b200_graph_phase_emit_edges")
 
     def phase_csr(self):
         self.G._call("rala_b200_graph_phase_csr")
@@ -118,18 +94,8 @@ class CudaShardSession:
     def phase_marks(self, t: torch.Tensor):
         self.G._call("rala_b200_graph_phase_marks", self._dp(t), C.c_uint32(t.shape[0]))
 
-    # ---- capacity-bounded phases: nothing below reads a count back to the host ------------------------------------
-    def phase_events_async(self):
-        self.G._call("rala_b200_graph_phase_events")
-
-    def phase_survivors_async(self):
-        self.G._call("rala_b200_graph_phase_survivors")
-
-    def phase_emit_edges_async(self):
-        self.G._call("rala_b200_graph_phase_emit_edges", None)
-
     def block_words(self, kind: int, cap: int) -> int:
-        """32-bit words of one exchange block (edges travel as reverse-complement pairs: 8 B per edge)."""
+        """32-bit words of one exchange block: a 4-word header and three columns of `cap` words."""
         return int(self.ctx.lib.rala_b200_exchange_block_words(C.c_int(kind), C.c_uint32(cap)))
 
     def export_padded(self, kind: int, block: torch.Tensor, cap: int):
@@ -167,62 +133,70 @@ class CudaShardSession:
         self.ctx.close()
 
 
+def default_caps(n_records: int, world: int) -> dict:
+    """Exchange capacities of a first planning pass over a shard of n_records, in the proportions of
+    rala_b200_multi_default_caps (the events of both containment passes share its event capacity)."""
+    align = lambda n: (n + 255) // 256 * 256   # noqa: E731
+    events = align(n_records // (4 if world > 1 else 1) + 4096)
+    edges = align(n_records // (2 if world > 1 else 1) * (1 if world > 1 else 2) + 4096)
+    return {"events": events, "final_events": events, "edges": edges}
+
+
+def _slack(n: int) -> int:
+    return int(n * 1.25) + 4096
+
+
 class DistributedGraph:
     """Drives one ShardSession per rank through the phases, with the collectives in between.
-    Like the product path it runs the frozen-pile chain only (no hills, no host pile breaking between the passes);
-    results of a capacity-bounded pass are valid only if check() says so."""
+    Like the product path it runs the frozen-pile chain only (no hills, no host pile breaking between the passes).
+    A pass never reads a count back to the host, so its results are valid only if check() says so."""
 
     def __init__(self, session, rank: int, world: int, group=None):
         self.s, self.rank, self.world, self.group = session, rank, world, group
         self.device = session.device
         self.comm_bytes = 0   # bytes this rank received through collectives in the last run
-        self.caps = None      # exchange capacities learned by the last sized run
-        self.last_info = None
+        self.caps = None      # per-rank exchange capacities, set by plan()
         self._bufs = {}
         self._graph = None    # one bounded pass (kernels + NCCL collectives) captured in a CUDA graph
         self.graph_launches = 0
         self.graph_error = None
 
-    def _gather_counts(self, values):
-        t = torch.tensor(values, dtype=torch.int64, device=self.device)
-        out = [torch.empty_like(t) for _ in range(self.world)]
-        dist.all_gather(out, t, group=self.group)
-        return torch.stack(out).cpu().numpy()   # (world, len(values))
-
-    def _exchange(self, n_local: int, export_fn, import_fn):
-        """All-gather of variable-length 3-column blocks; imports them in rank order. Returns the total."""
-        counts = self._gather_counts([n_local])[:, 0]
-        total, stride = int(counts.sum()), max(int(counts.max()), 1)
-        block = torch.zeros((3, stride), dtype=torch.int32, device=self.device)
-        export_fn(block, n_local)
-        gathered = [torch.empty_like(block) for _ in range(self.world)]
-        dist.all_gather(gathered, block, group=self.group)
-        self.comm_bytes += block.numel() * 4 * (self.world - 1)
-        off = 0
-        for k in range(self.world):
-            n_k = int(counts[k])
-            if n_k or k == self.world - 1:
-                import_fn(gathered[k], n_k, off, total)   # the last import publishes the total
-            off += n_k
-        return total, int(counts.max())
-
-    KINDS = {"events": 0, "edges": 1}
-
     def run(self):
-        """One pass of the hot path.  The first pass (and any pass after an overflow) sizes every exchange on the
-        host (`run_sized`); it leaves capacities behind with which the following passes run without a single host
-        synchronisation (`run_bounded`): counts travel inside the exchange blocks."""
+        """One pass of the hot path.  Without capacities (the first pass, and the first after check() found an
+        overflow) it plans them, which leaves the results of the pass that fitted."""
         if self.caps is None:
-            info = self.run_sized()
-            slack = lambda n: int(n * 1.25) + 4096   # noqa: E731
-            self.caps = {"events": slack(info["max_events"]), "final_events": slack(info["max_final_events"]),
-                         "edges": (slack(info["max_edges"]) + 1) // 2 * 2}
-            self.last_info = info
-            return info
-        return self.run_bounded()
+            self.plan()
+        else:
+            self.run_bounded()
+
+    def plan(self, max_attempts: int = 4):
+        """Size the exchange blocks from real passes (collective): run, read from the gathered blocks what every rank
+        needed, set each capacity to slack(need), until a pass fits.  The first events exchange depends on no capacity,
+        the final events only on it and the edges on both, so the fourth pass fits at the latest.  The capacities
+        that stay are slack(largest per-rank count) of the pass that fitted, whatever the capacities it ran with."""
+        caps = default_caps(self.s.n_records, self.world)
+        t = torch.tensor(list(caps.values()), dtype=torch.int64, device=self.device)
+        dist.all_reduce(t, op=dist.ReduceOp.MAX, group=self.group)
+        caps = dict(zip(caps, (int(v) for v in t.tolist())))
+        for _ in range(max_attempts):
+            self.caps = caps
+            self.run_bounded()
+            # word 2 of a block = its rank's count; the gathered blocks are the same on every rank, so all ranks read
+            # the same needs without another collective (the read-back synchronises)
+            need = dict(zip(caps, torch.stack([self._bufs[(name, cap)][1][:, 2].max() for name, cap in caps.items()]).tolist()))
+            fits = all(need[name] <= cap for name, cap in caps.items())
+            caps = {"events": _slack(need["events"]), "final_events": _slack(need["final_events"]),
+                    "edges": (_slack(need["edges"]) + 1) // 2 * 2}
+            if fits:
+                self.caps = caps
+                keep = set(caps.items()) | {("marks", caps["edges"] * self.world), "pair"}
+                self._bufs = {k: v for k, v in self._bufs.items() if k in keep}
+                return self
+        self.caps = None
+        raise api.RalaB200Error("plan: the exchange blocks still did not fit")
 
     def check(self) -> bool:
-        """After bounded passes: did every block fit?  (synchronises)  On overflow the next run() is sized again."""
+        """After bounded passes: did every block fit?  (synchronises)  On overflow the next run() plans again."""
         if self.caps is not None and self.s.overflowed():
             self.caps = None
             self._bufs = {}
@@ -233,10 +207,10 @@ class DistributedGraph:
     def capture(self) -> bool:
         """Capture one capacity-bounded pass, NCCL collectives included, in a CUDA graph: `replay()` then costs one
         launch per step instead of ~50 kernel launches, ~20 library calls and 5 collectives issued from Python.
-        Requires a sized pass before (capacities, buffers) and a session created on a non-default stream that is
-        torch's current stream.  Returns False (and keeps the eager path) when the capture fails."""
+        Requires planned capacities (it plans when there are none) and a session created on a non-default stream that
+        is torch's current stream.  Returns False (and keeps the eager path) when the capture fails."""
         if self.caps is None:
-            self.run()
+            self.plan()
         self.run_bounded()          # every exchange buffer exists before the capture starts
         torch.cuda.synchronize(self.device)
         stream = torch.cuda.current_stream(self.device)
@@ -254,11 +228,12 @@ class DistributedGraph:
         return self._graph is not None
 
     def replay(self):
-        """One pass: the captured graph when there is one, else the eager bounded (or sized) pass."""
+        """One pass: the captured graph when there is one, else run().  The counts of the pass stay on the device:
+        session.counts() after check() reads them."""
         if self._graph is not None:
             self._graph.replay()
-            return {"bounded": True, "graph": True}   # counts of THIS pass: session.counts() after check() (they stay on the device)
-        return self.run()
+        else:
+            self.run()
 
     def _buffers(self, name: str, cap: int, kind: int = 0):
         key = (name, cap)
@@ -268,7 +243,7 @@ class DistributedGraph:
                                torch.zeros((self.world, words), dtype=torch.int32, device=self.device))
         return self._bufs[key]
 
-    def _exchange_bounded(self, name: str, kind: int, cap: int):
+    def _exchange(self, name: str, kind: int, cap: int):
         block, gathered = self._buffers(name, cap, kind)
         self.s.export_padded(kind, block, cap)
         dist.all_gather_into_tensor(gathered.view(-1), block, group=self.group)
@@ -276,12 +251,15 @@ class DistributedGraph:
         self.s.import_gathered(kind, gathered, cap, self.world)
 
     def run_bounded(self):
+        """One pass with the current capacities; enqueues only (no count is read back)."""
         s, caps = self.s, self.caps
         self.comm_bytes = 0
-        s.phase_events_async()
-        self._exchange_bounded("events", 0, caps["events"])
+        # graph.cpp:443-518
+        s.phase_events()
+        self._exchange("events", 0, caps["events"])
         s.phase_resolve(True)
-        s.phase_survivors_async()
+        s.phase_survivors()
+        # graph.cpp:831-877 — time of a list entry = its position in the GLOBAL overlaps ++ internals order
         if "pair" not in self._bufs:
             self._bufs["pair"] = (torch.zeros(2, dtype=torch.int32, device=self.device),
                                   torch.zeros((self.world, 2), dtype=torch.int32, device=self.device))
@@ -289,11 +267,13 @@ class DistributedGraph:
         s.export_list_counts(pair)
         dist.all_gather_into_tensor(pairs.view(-1), pair, group=self.group)
         s.phase_final_events_gathered(pairs, self.world)
-        self._exchange_bounded("final_events", 0, caps["final_events"])
+        self._exchange("final_events", 0, caps["final_events"])
         s.phase_resolve(False)
-        s.phase_emit_edges_async()
-        self._exchange_bounded("edges", 1, caps["edges"])
+        # graph.cpp:552-632 — edge ids follow the global list order = rank order of the shards
+        s.phase_emit_edges()
+        self._exchange("edges", 1, caps["edges"])
         s.phase_csr()
+        # graph.cpp:1281-1318 — split by source node; marks merged with all-reduce(max)
         s.phase_transitive()
         n_marks = caps["edges"] * self.world
         if ("marks", n_marks) not in self._bufs:
@@ -303,39 +283,6 @@ class DistributedGraph:
         dist.all_reduce(marks, op=dist.ReduceOp.MAX, group=self.group)
         self.comm_bytes += marks.numel() * 2 * (self.world - 1) // self.world
         s.phase_marks(marks)
-        # no counts here: a bounded pass never reads them back (last_info describes the sized pass that set the capacities);
-        # check() tells whether this pass fit, session.counts() reads its counts
-        return {"bounded": True}
-
-    def run_sized(self):
-        s = self.s
-        self.comm_bytes = 0
-        # graph.cpp:443-518
-        n_ev = s.phase_events()
-        n_events, max_events = self._exchange(n_ev, s.export_events, s.import_events)
-        s.phase_resolve(True)
-        n_ovl, n_int = s.phase_survivors()
-        # graph.cpp:831-877 — time of a list entry = its position in the GLOBAL overlaps ++ internals order
-        counts = self._gather_counts([n_ovl, n_int])
-        total_ovl = int(counts[:, 0].sum())
-        ovl_base = int(counts[:self.rank, 0].sum())
-        int_base = total_ovl + int(counts[:self.rank, 1].sum())
-        n_ev2 = s.phase_final_events(ovl_base, int_base)
-        n_final_events, max_final_events = self._exchange(n_ev2, s.export_events, s.import_events)
-        s.phase_resolve(False)
-        # graph.cpp:552-632 — edge ids follow the global list order = rank order of the shards
-        n_e = s.phase_emit_edges()
-        n_edges, max_edges = self._exchange(n_e, s.export_edges, s.import_edges)
-        s.phase_csr()
-        # graph.cpp:1281-1318 — split by source node; marks merged with all-reduce(max)
-        s.phase_transitive()
-        marks = torch.zeros(max(n_edges, 1), dtype=torch.uint8, device=self.device)
-        s.export_marks(marks[:n_edges])
-        dist.all_reduce(marks, op=dist.ReduceOp.MAX, group=self.group)
-        self.comm_bytes += marks.numel() * 2 * (self.world - 1) // self.world
-        s.phase_marks(marks[:n_edges])
-        return dict(n_events=n_events, n_final_events=n_final_events, n_edges=n_edges, n_overlaps=total_ovl,
-                    max_events=max_events, max_final_events=max_final_events, max_edges=max_edges)
 
 
 def shard_bounds(n_records: int, world: int):

@@ -33,6 +33,7 @@ class OracleShardSession:
         self._overflow = False
         self.flags = np.zeros(len(piles), np.uint8) if flags is None else np.asarray(flags, np.uint8)
         self.t0, self.rank, self.world = t0, rank, world
+        self.n_records = len(self.rec)
         self.events = np.zeros((0, 3), np.uint32)
         self.edges_all = np.zeros((0, 3), np.uint32)
 
@@ -41,15 +42,6 @@ class OracleShardSession:
         if r[6] & 2 or a >= len(self.piles) or b >= len(self.piles) or self.piles[a, 1] == 0 or self.piles[b, 1] == 0:
             return False, r, O.REJECT
         return O.trim_type(r, self.piles[a], self.piles[b])
-
-    @staticmethod
-    def _to_block(arr, block, n):
-        if n:
-            block[:, :n] = torch.from_numpy(np.ascontiguousarray(arr[:n].T).view(np.int32))
-
-    @staticmethod
-    def _from_block(block, n):
-        return block[:, :n].numpy().view(np.uint32).T.copy()
 
     def phase_events(self):
         self.piles = self.piles0.copy()   # re-runnable, like the CUDA session
@@ -65,15 +57,7 @@ class OracleShardSession:
             elif t == O.KA and not (self.flags[a] & 2):
                 ev.append((b, a, self.t0 + i))
         self.events = np.asarray(ev, np.uint32).reshape(-1, 3)
-        return len(ev)
-
-    def export_events(self, block, n):
-        self._to_block(self.events, block, n)
-
-    def import_events(self, block, n, offset, total):
-        if offset == 0:
-            self.events_all = np.zeros((total, 3), np.uint32)
-        self.events_all[offset:offset + n] = self._from_block(block, n)
+        self.n_first_events = len(ev)
 
     def phase_resolve(self, first):
         # the reference's sequential semantics: in time order, an event fires iff both piles are still alive
@@ -96,9 +80,13 @@ class OracleShardSession:
                 (inl if t == O.KX else ovl).append(tr)
         self.ovl = np.asarray(ovl, np.uint32).reshape(-1, 7)
         self.inl = np.asarray(inl, np.uint32).reshape(-1, 7)
-        return len(ovl), len(inl)
 
-    def phase_final_events(self, ovl_base, int_base):
+    def export_list_counts(self, pair):
+        pair[0], pair[1] = len(self.ovl), len(self.inl)
+
+    def phase_final_events_gathered(self, counts, world):
+        c = counts.numpy().astype(np.int64)
+        ovl_base, int_base = int(c[:self.rank, 0].sum()), int(c[:, 0].sum() + c[:self.rank, 1].sum())
         ev = []
         for base, lst in ((ovl_base, self.ovl), (int_base, self.inl)):
             for i, r in enumerate(lst):
@@ -110,7 +98,6 @@ class OracleShardSession:
                 elif t == O.KB:
                     ev.append((int(r[0]), int(r[1]), base + i))
         self.events = np.asarray(ev, np.uint32).reshape(-1, 3)
-        return len(ev)
 
     def phase_emit_edges(self):
         alive = self.piles[:, 1] != 0
@@ -122,15 +109,6 @@ class OracleShardSession:
         P.ovl = np.asarray(keep, np.uint32).reshape(-1, 7)
         P.build_edges()      # local node numbering == global: the pile table is replicated
         self.edges = P.edges
-        return len(self.edges)
-
-    def export_edges(self, block, n):
-        self._to_block(self.edges, block, n)
-
-    def import_edges(self, block, n, offset, total):
-        if offset == 0:
-            self.edges_all = np.zeros((total, 3), np.uint32)
-        self.edges_all[offset:offset + n] = self._from_block(block, n)
 
     def phase_csr(self):
         pass
@@ -172,23 +150,13 @@ class OracleShardSession:
         m = (T[0::2] | T[1::2])
         self.marked = np.repeat(m, 2).astype(np.uint8)
 
-
-    # ---- capacity-bounded interface (counts travel inside the blocks) ---------------------------------------
-    def phase_events_async(self):
-        self.phase_events()
-
-    def phase_survivors_async(self):
-        self.phase_survivors()
-
-    def phase_emit_edges_async(self):
-        self.phase_emit_edges()
-
+    # ---- exchange blocks: [n clamped to cap | overflow flag | n | 0 | three columns of cap] ----------------------
     def export_padded(self, kind, block, cap):
         arr = self.events if kind == 0 else self.edges
         n = len(arr)
         m = min(n, cap)
         b = block.numpy().view(np.uint32)
-        b[:4] = (m, int(n > cap), 0, 0)
+        b[:4] = (m, int(n > cap), n, 0)
         for k in range(3):
             b[4 + k * cap: 4 + k * cap + m] = arr[:m, k]
 
@@ -204,13 +172,6 @@ class OracleShardSession:
             self.events_all = merged
         else:
             self.edges_all = merged
-
-    def export_list_counts(self, pair):
-        pair[0], pair[1] = len(self.ovl), len(self.inl)
-
-    def phase_final_events_gathered(self, counts, world):
-        c = counts.numpy().astype(np.int64)
-        self.phase_final_events(int(c[:self.rank, 0].sum()), int(c[:, 0].sum() + c[:self.rank, 1].sum()))
 
     def overflowed(self):
         return self._overflow
@@ -232,37 +193,66 @@ def _worker(rank, world, port, kw, out_dir):
         lo, hi = multi.shard_bounds(ds.n_overlaps, world)[rank]
         sess = OracleShardSession(ds.records[lo:hi], piles, flags, lo, rank, world)
         dg = multi.DistributedGraph(sess, rank, world)
-        info = dg.run()                                   # sized: every exchange is counted on the host first
+        passes = []
+        bounded = dg.run_bounded
+        dg.run_bounded = lambda: (passes.append(dict(dg.caps)), bounded())[1]
+
+        dg.run()                                          # plans: the default capacities fit this data
+        assert dg.check() and len(passes) == 1
+        # this rank's element count of every exchange, from the pass that fitted
+        counts = [sess.n_first_events, len(sess.events), len(sess.edges)]
+        caps = dict(dg.caps)
         first = (sess.edges_all.copy(), sess.marked.copy(), sess.piles.copy())
-        again = dg.run()                                  # bounded: counts travel inside the blocks
-        assert again.get("bounded") and dg.check()
-        for x, y in zip(first, (sess.edges_all, sess.marked, sess.piles)):
-            assert np.array_equal(x, y)
-        dg.caps = {k: 8 for k in dg.caps}                 # far too small: must be detected, and the next run sized again
+
+        def same_results():
+            return all(np.array_equal(x, y) for x, y in zip(first, (sess.edges_all, sess.marked, sess.piles)))
+
+        dg.run()                                          # one pass with the planned capacities
+        assert len(passes) == 2 and passes[-1] == caps and dg.check() and same_results()
+
+        dg.caps = {k: 8 for k in dg.caps}                 # far too small: must be detected, and the next run plans again
         dg._bufs = {}
         dg.run()
         assert not dg.check() and dg.caps is None
-        info = dg.run()
-        assert "bounded" not in info
+        dg.run()
+        assert dg.check() and dg.caps == caps and same_results()
+
+        # defaults too small for the data: plan() grows until a pass fits and ends where it would have started
+        multi.default_caps = lambda n_records, world: {"events": 8, "final_events": 8, "edges": 8}
+        del passes[:]
+        dg.caps = None
+        dg.run()
+        grown = len(passes)
+        assert dg.check() and dg.caps == caps and same_results()
+        # buffers of the sizes it grew through are dropped
+        assert set(k for k in dg._bufs if k != "pair") <= set(caps.items()) | {("marks", caps["edges"] * world)}
+
         np.savez(os.path.join(out_dir, f"r{rank}.npz"), edges=sess.edges_all, marked=sess.marked, piles=sess.piles,
-                 n_events=info["n_events"])
+                 counts=counts, caps=[caps["events"], caps["final_events"], caps["edges"]], grown=grown)
     finally:
         dist.destroy_process_group()
 
 
 @pytest.mark.parametrize("world", [2, 3])
-def test_orchestration_matches_single_process_oracle(world, tmp_path):
+def test_orchestration_plans_capacities_and_matches_single_process_oracle(world, tmp_path):
     kw = dict(genome_len=150_000, coverage=30, read_len=6000, len_sd=1500, seed=61, noise=60, dual=True, min_ovl=800)
     ds = synth.generate(**kw)
     flags = (np.random.Generator(np.random.PCG64(1)).random(ds.n_reads) < 0.05).astype(np.uint8) * 2
     want = O.Pipeline(ds.records, ds.flat_piles(), flags).run()
     assert want.edges.shape[0] > 200 and want.n_pairs > 20
     mp.spawn(_worker, args=(world, _free_port(), kw, str(tmp_path)), nprocs=world, join=True)
-    for r in range(world):
-        z = np.load(tmp_path / f"r{r}.npz")
+    got = [np.load(tmp_path / f"r{r}.npz") for r in range(world)]
+    # the capacities a pass sized on the host would choose: slack(largest per-rank count), edges rounded to even
+    most = np.max([z["counts"] for z in got], axis=0)
+    assert (most > 0).all()
+    slack = [int(n * 1.25) + 4096 for n in most.tolist()]
+    slack[2] = (slack[2] + 1) // 2 * 2
+    for r, z in enumerate(got):
         assert np.array_equal(z["edges"], want.edges), f"rank {r}: edge list"
         assert np.array_equal(z["marked"], want.marked), f"rank {r}: removed-edge set"
         assert np.array_equal(z["piles"], want.piles), f"rank {r}: pile liveness"
+        assert z["caps"].tolist() == slack, f"rank {r}: planned capacities"
+        assert 2 <= int(z["grown"]) <= 4, f"rank {r}: passes of the growing plan"
 
 
 def test_shard_bounds():

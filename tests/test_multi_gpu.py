@@ -22,7 +22,7 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 from oracle import oracle as O  # noqa: E402
-from rala_b200 import multi, synth  # noqa: E402
+from rala_b200 import api, multi, synth  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -72,13 +72,14 @@ def _worker(rank, world, port, out_dir, transport, same_device):
             sess = multi.CudaShardSession(dev)
             sess.set_inputs(shard, piles, flags, lo, rank, world)
             dg = multi.DistributedGraph(sess, rank, world)
-            for _ in range(3):   # sized, then capacity-bounded passes
+            for _ in range(3):   # planned, then capacity-bounded passes
                 dg.run()
             assert dg.check()
             c = sess.counts()
             np.savez(os.path.join(out_dir, f"r{rank}.npz"), edges=sess.edges() if rank == 0 else np.zeros((0, 3), np.uint32),
                      marked=sess.marked() if rank == 0 else np.zeros(0, np.uint8), first=0 if rank == 0 else c["n_edges"],
-                     piles=sess.G.piles(), n_edges=c["n_edges"], n_pairs=c["n_transitive_pairs"] if rank == 0 else 0, n_nodes=c["n_nodes"])
+                     piles=sess.G.piles(), n_edges=c["n_edges"], n_pairs=c["n_transitive_pairs"] if rank == 0 else 0, n_nodes=c["n_nodes"],
+                     n_candidates=c["n_candidates"], n_final_candidates=c["n_final_candidates"])
             dist.barrier()
             sess.close()
     finally:
@@ -97,6 +98,7 @@ def _run_and_compare(world, transport, same_device, tmp_path):
     for z in parts:
         assert np.array_equal(z["piles"], want.piles), "pile liveness"
         assert int(z["n_nodes"]) == want.n_nodes and int(z["n_edges"]) == want.edges.shape[0]
+    return parts
 
 
 @pytest.mark.parametrize("world", [1, 2, 4, 8])
@@ -114,4 +116,17 @@ def test_fabric_two_processes_on_one_device(tmp_path):
 def test_nccl_fallback_transport(world, tmp_path):
     if torch.cuda.device_count() < world:
         pytest.skip(f"needs {world} GPUs")
-    _run_and_compare(world, "nccl", False, tmp_path)
+    parts = _run_and_compare(world, "nccl", False, tmp_path)
+    # every rank imports all ranks' events: its containment-event counts are those of one GPU on the whole batch
+    ds = synth.generate(**KW)
+    ctx = api.Context(0)
+    G = api.Graph(ctx)
+    G.set_piles(ds.flat_piles(), _flags(ds)).set_hills(None).set_overlaps(ds.records)
+    G.run()
+    want = G.counts()
+    G.close()
+    ctx.close()
+    assert want["n_candidates"] > 0
+    for z in parts:
+        assert int(z["n_candidates"]) == want["n_candidates"], "containment events of the first pass"
+        assert int(z["n_final_candidates"]) == want["n_final_candidates"], "containment events of the final pass"
