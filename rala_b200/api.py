@@ -613,7 +613,8 @@ class Multi:
 
     def set_rounds(self, rounds: int, final_rounds: int):
         self._call("rala_b200_multi_set_rounds", C.c_uint32(rounds), C.c_uint32(final_rounds))
-        self.caps[3], self.caps[4] = rounds, final_rounds
+        if hasattr(self, "caps"):   # only reserve() keeps a copy here: plan() sizes the buffers inside the library
+            self.caps[3], self.caps[4] = rounds, final_rounds
         return self
 
     def export_handle(self, k: int = 0) -> bytes:

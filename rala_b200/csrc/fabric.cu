@@ -454,8 +454,13 @@ __device__ __forceinline__ bool resolve_owned(const Peers& P, const ArenaLayout&
 // news from the peers arrives while a sweep runs, and a rank never waits for a slower peer to finish its own sweep.
 // After every sweep block 0 tells the peers how many victims are still open here (tagged with the barrier epoch of the
 // pass, so a value of the previous pass is never mistaken for a current one); the pass ends on a rank when every
-// rank has reported zero.  Ordering: each thread fences (system scope) after its pushes and before the grid barrier,
-// so a peer that reads "0 open" from this rank already holds every state this rank owns.
+// rank has reported zero.  A rank that has used up its sweeps with victims still open reports kGaveUp instead; a peer
+// that sees it gives up too (after its current sweep, or its watching threads stop), and the pass ends on a rank when
+// every rank has reported zero or kGaveUp, with FE_ROUNDS set if any gave up.  So even a pass that runs out of sweeps
+// ends in step on every rank, after every push has landed: the replicas agree, the step is void but consistent, and no
+// rank waits out the barrier timeout for a peer that stopped (a dead fabric lets the ranks run out of step).
+// Ordering: each thread fences (system scope) after its pushes and before the grid barrier, so a peer that reads
+// "0 open" (or kGaveUp) from this rank already holds every state this rank owns.
 // The grid is sized to be co-resident (launch_fabric_resolve), which the software grid barrier needs.
 // ---------------------------------------------------------------------------------------------
 struct ResolveCtl {
@@ -463,7 +468,9 @@ struct ResolveCtl {
     uint32_t released;  // grid barrier: phases released so far
     uint32_t go;        // decision of block 0 after a sweep: 1 = sweep again, 0 = the pass is over
     uint32_t sweeps;
-    uint32_t settled, pad[3];  // poll phase: victims that have been settled by the thread that watches them
+    uint32_t settled;   // poll phase: victims whose watching thread is done with them
+    uint32_t stopped;   // poll phase: a watching thread stopped because a peer gave up, its victim still open
+    uint32_t pad[2];
     unsigned long long log[kSweepLog][2];   // diagnostics: (open victims at the start of the sweep, ns since the kernel started) per sweep
 };
 static_assert(sizeof(ResolveCtl) == kResolveCtlBytes, "fabric.cuh sizes the control block");
@@ -490,6 +497,8 @@ __device__ __forceinline__ void grid_barrier(ResolveCtl* ctl, uint32_t& phase, u
     }
     __syncthreads();
 }
+
+constexpr uint32_t kGaveUp = 0xFFFFFFFFu;   // progress word of a rank that ran out of sweeps with victims still open
 
 __device__ __forceinline__ void st_release_sys64(unsigned long long* p, unsigned long long v) {
     asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
@@ -541,7 +550,7 @@ __global__ void __launch_bounds__(256) k_fabric_resolve(Peers P, ArenaLayout A, 
                                                        uint32_t* __restrict__ n_work, uint32_t* __restrict__ wait_pile,
                                                        uint32_t* __restrict__ wait_time, ResolveCtl* __restrict__ ctl, int pass,
                                                        uint32_t max_sweeps, unsigned long long timeout_ns) {
-    __shared__ uint32_t s_state;   // tail loop of block 0: 0 sweep again, 1 done
+    __shared__ uint32_t s_word;   // block 0: what this rank reports after a sweep (open victims, or kGaveUp)
     FabricHdr* mine = hdr_of(P, P.rank);
     if (mine->skip_pass) {
         if (blockIdx.x == 0 && threadIdx.x == 0) mine->rounds_needed[pass] = 1u;
@@ -553,22 +562,31 @@ __global__ void __launch_bounds__(256) k_fabric_resolve(Peers P, ArenaLayout A, 
     const unsigned long long t_start = global_timer_ns();
     uint32_t phase = 0;
 
-    // block 0, thread 0, after a sweep that left `open` victims: decide.  Returns 0 = the pass is over, 1 = sweep again.
-    // (`open` was published to the peers by the lanes of warp 0, see publish_open)
-    auto after_sweep = [&](uint32_t sweep, uint32_t n_before, uint32_t open) -> uint32_t {
+    auto peer_gave_up = [&]() -> bool {
+        for (uint32_t q = 0; q < W; ++q)
+            if (ld_acquire_sys64(&mine->progress[q]) == (tag | kGaveUp)) return true;
+        return false;
+    };
+
+    // block 0, thread 0, after a sweep that left `word` (open victims, or kGaveUp): decide.  Returns 0 = the pass is over,
+    // 1 = sweep again.  (`word` was published to the peers by the lanes of warp 0, see publish_open)
+    auto after_sweep = [&](uint32_t sweep, uint32_t n_before, uint32_t word) -> uint32_t {
         uint32_t go = 1u;
         bool dead = ld_relaxed_sys(&mine->dead) != 0u || global_timer_ns() - t_start > timeout_ns;
-        if (open == 0u) {   // everything here is settled and pushed: wait until that is true everywhere
+        bool gave_up = word == kGaveUp;
+        if (word == 0u || gave_up) {   // everything here is settled (or given up) and pushed: wait until that is true everywhere
             while (!dead) {
                 bool all = true;
-                for (uint32_t q = 0; q < W; ++q) all = all && ld_acquire_sys64(&mine->progress[q]) == tag;
+                for (uint32_t q = 0; q < W; ++q) {
+                    const unsigned long long p = ld_acquire_sys64(&mine->progress[q]);
+                    gave_up = gave_up || p == (tag | kGaveUp);
+                    all = all && (p == tag || p == (tag | kGaveUp));
+                }
                 if (all) break;
                 __nanosleep(100);
                 dead = ld_relaxed_sys(&mine->dead) != 0u || global_timer_ns() - t_start > timeout_ns;
             }
-            go = 0u;
-        } else if (sweep + 1u >= max_sweeps) {
-            atomicOr(&mine->error, (uint32_t) FE_ROUNDS);
+            if (gave_up) atomicOr(&mine->error, (uint32_t) FE_ROUNDS);
             go = 0u;
         }
         if (dead) {
@@ -584,7 +602,7 @@ __global__ void __launch_bounds__(256) k_fabric_resolve(Peers P, ArenaLayout A, 
             ctl->log[sweep][0] = n_before;
             ctl->log[sweep][1] = global_timer_ns() - t_start;
         }
-        if (!go) mine->rounds_needed[pass] = (open == 0u && !dead) ? sweep + 1u : 0u;
+        if (!go) mine->rounds_needed[pass] = (!gave_up && !dead) ? sweep + 1u : 0u;
         return go;
     };
 
@@ -612,12 +630,16 @@ __global__ void __launch_bounds__(256) k_fabric_resolve(Peers P, ArenaLayout A, 
             // goes on the moment it moves: the rest of the pass costs the longest cross-rank dependency chain (a push over
             // NVLink + a few local hops per link) instead of one whole-grid sweep, two grid barriers and the longest local
             // chase of the sweep per link (8 - 12 sweeps of 30 - 80 us on 8 GPUs, profiles/r02n).
-            bool gave_up = false;
+            bool gave_up = false, stopped = false;
             if (gtid < open) {
                 const uint32_t v = out[gtid];
                 for (uint32_t it = 1;; ++it) {
                     if ((it & 255u) == 0u && (ld_relaxed_sys(&mine->dead) != 0u || global_timer_ns() - t_start > timeout_ns)) {
                         gave_up = true;
+                        break;
+                    }
+                    if ((it & 255u) == 128u && peer_gave_up()) {   // the foreign state this victim waits for may never move
+                        stopped = true;
                         break;
                     }
                     const uint32_t f = wait_pile[v];
@@ -634,23 +656,32 @@ __global__ void __launch_bounds__(256) k_fabric_resolve(Peers P, ArenaLayout A, 
                     if (done) break;
                 }
                 if (gave_up) atomicExch(&mine->dead, 1u);
+                if (stopped) {
+                    atomicExch(&ctl->stopped, 1u);
+                    __threadfence();   // before block 0 counts this victim as done
+                }
                 atomicAdd(&ctl->settled, 1u);
             }
         }
         if (blockIdx.x == 0) {
-            if (poll && threadIdx.x == 0) {   // all victims of this rank settled (or somebody gave up)?
-                uint32_t got;
-                do {
-                    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(got) : "l"(&ctl->settled) : "memory");
-                    if (got < open) __nanosleep(100);
-                } while (got < open);
-                s_state = 0u;
+            const uint32_t done_sweeps = poll ? sweep + 1u : sweep;
+            if (threadIdx.x == 0) {
+                if (poll) {   // all victims of this rank settled (or somebody gave up)?
+                    uint32_t got;
+                    do {
+                        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(got) : "l"(&ctl->settled) : "memory");
+                        if (got < open) __nanosleep(100);
+                    } while (got < open);
+                }
+                uint32_t word = poll ? (*(volatile uint32_t*) &ctl->stopped ? kGaveUp : 0u) : open;
+                // victims still open after the last sweep allowed, or a peer has given up: give up too (FE_ROUNDS)
+                if (word != 0u && word != kGaveUp && (done_sweeps + 1u >= max_sweeps || peer_gave_up())) word = kGaveUp;
+                s_word = word;
             }
             __syncthreads();
-            const uint32_t left = poll ? 0u : open;
-            if (threadIdx.x < 32) publish_open(left);
+            if (threadIdx.x < 32) publish_open(s_word);
             if (threadIdx.x == 0) {
-                ctl->go = after_sweep(poll ? sweep + 1u : sweep, poll ? open : n, left);
+                ctl->go = after_sweep(done_sweeps, poll ? open : n, s_word);
                 __threadfence();
             }
         }
