@@ -285,12 +285,34 @@ int rala_b200_graph_phase_marks(rala_b200_graph* g, const uint8_t* d_T, uint32_t
  *       run; synchronize; demand -> [max over ranks]: re-reserve with larger capacities if something did not fit.
  *
  * A device id may be listed more than once (several ranks share a GPU): that is how the parity tests cover
- * world > 1 on a one-GPU box.  Restrictions: frozen pile table (no hills, no host pile breaking between the
- * passes: the clean-data chain rala_b200_graph_run executes); read ids, coordinates and counts 32-bit as above.
+ * world > 1 on a one-GPU box.  rala_b200_multi_run is the frozen-pile chain (no hills, no host pile breaking between
+ * the passes: what rala_b200_graph_run executes).  Pile tables that change between the passes (hill counters, pile
+ * breaking, promoted internals) take the STAGED calls below, the same boundaries as the single session's:
+ *
+ *   set_piles, set_hills, set_overlaps(k, shard k) ...; plan (or reserve + handles)
+ *   classify                                  graph.cpp:443-518; hill counters summed over the ranks on the device
+ *   get_hill_coverage, [host: break_over_chimeric_hills], set_piles           :704-720
+ *   retrim                                    :722-736
+ *   loop { get_lists (connections), [host: pits], set_piles, retrim_promote(&changed) } until !changed   :738-829
+ *   finish                                    :831-877, 552-632, 1281-1318
+ *   synchronize, demand                       the capacities were planned from a frozen step: if the staged passes
+ *                                             needed more (fits = 0, or counts fails), the results are incomplete;
+ *                                             reserve with the reported capacities and construct again
+ *   get_lists, edge_runs, get_edges, get_marked, get_seq_to_node ...
+ *
+ * Every staged call is made by every process with the same arguments and synchronises with the host; the counts it
+ * needs from other ranks (hill totals, list counts, is_changed) arrive through the exchange arenas, so all processes
+ * see the same values without a host collective.  Promotions go to the END of the global `overlaps` (graph.cpp:818):
+ * with shards in rank order that list is segment-major (segment 0: every rank's entries of the first pass in rank
+ * order; segment k: what the k-th round that promoted anything promoted, in rank order), and a rank's edges are one run
+ * of global ids per segment.  Read ids, coordinates and counts 32-bit as above.
  * ---------------------------------------------------------------------------------------------- */
 typedef struct rala_b200_multi rala_b200_multi;
 
 #define RALA_B200_MAX_RANKS 16
+/* segments of the staged `overlaps` list: the first pass plus at most 63 pit rounds that promote something
+ * (rala_b200_multi_retrim_promote fails with RALA_B200_ERR_LIMIT beyond, and the session's lists are void) */
+#define RALA_B200_MAX_SEGMENTS 64
 /* capacities of the exchange buffers (identical on every rank) */
 enum { RALA_B200_CAP_EVENTS = 0,   /* containment events one rank sends to one owner */
        RALA_B200_CAP_EDGES,        /* edges one rank sends to one owner */
@@ -317,8 +339,12 @@ typedef struct {
 int rala_b200_multi_create(rala_b200_multi** out, const int* devices, int n_local, int first_rank, int world);
 void rala_b200_multi_destroy(rala_b200_multi* m);
 const char* rala_b200_multi_last_error(const rala_b200_multi* m);
-/* replicated pile table (every local rank gets a copy); as rala_b200_graph_set_piles */
+/* replicated pile table (every local rank gets a copy); as rala_b200_graph_set_piles: called after classify it replaces
+ * the table every later staged pass trims against */
 int rala_b200_multi_set_piles(rala_b200_multi* m, const rala_pile_t* piles, const uint8_t* flags, uint32_t n_piles);
+/* replicated hill rows, as rala_b200_graph_set_hills; only the staged classify counts them (rala_b200_multi_run ignores
+ * them).  More hills than the exchange arenas were reserved for: reserve again. */
+int rala_b200_multi_set_hills(rala_b200_multi* m, const rala_hill_t* hills, uint32_t n_hills);
 /* shard of local rank k: records [t0, t0 + n) of the file, in file order */
 int rala_b200_multi_set_overlaps(rala_b200_multi* m, int k, const rala_ovl_t* ovl, uint64_t n, uint64_t t0);
 int rala_b200_multi_set_overlaps_columns(rala_b200_multi* m, int k, const uint32_t* a_id, const uint32_t* b_id, const uint32_t* a_begin,
@@ -350,8 +376,25 @@ int rala_b200_multi_demand(rala_b200_multi* m, uint64_t* need /* RALA_B200_N_CAP
 /* all ranks in one process: reserve with the default capacities, run, grow what did not fit, until a step fits */
 int rala_b200_multi_plan(rala_b200_multi* m);
 int rala_b200_multi_counts(rala_b200_multi* m, rala_b200_multi_counts_t* out);
-/* results of local rank k: the edges it emitted are edge ids [*first_edge, *first_edge + *n) (rows in id order) */
+/* results of local rank k: the edges it emitted are edge ids [*first_edge, *first_edge + *n) (rows in id order).  After a
+ * staged construct whose promotions gave rank k more than one run of ids: RALA_B200_ERR_STATE (use edge_runs). */
 int rala_b200_multi_edge_range(rala_b200_multi* m, int k, uint64_t* first_edge, uint64_t* n);
+/* the global id runs of the rows get_edges(k) / get_marked(k) return, in that order: (first id, count) pairs, adjacent
+ * runs merged; first_and_count_out (nullable: count only) holds 2 x RALA_B200_MAX_SEGMENTS values */
+int rala_b200_multi_edge_runs(rala_b200_multi* m, int k, uint64_t* first_and_count_out, uint32_t* n_runs_out);
+
+/* staged construct (see above); each call runs on every local rank and returns when they are done */
+int rala_b200_multi_classify(rala_b200_multi* m);
+int rala_b200_multi_retrim(rala_b200_multi* m);
+/* *is_changed (nullable): did the retrim of `overlaps` drop an entry on any rank (graph.cpp:801-807), the same on every rank */
+int rala_b200_multi_retrim_promote(rala_b200_multi* m, int* is_changed);
+int rala_b200_multi_finish(rala_b200_multi* m);
+/* hill counters of the first pass summed over all ranks (n_hills), as local rank k holds them */
+int rala_b200_multi_get_hill_coverage(rala_b200_multi* m, int k, uint32_t* cov_out);
+/* local rank k's entries of `overlaps` / `internals` (nullable) with their positions in the global lists (nullable);
+ * counts[0], counts[1] = how many (always written).  After finish: the final lists of graph.cpp:867-877. */
+int rala_b200_multi_get_lists(rala_b200_multi* m, int k, rala_ovl_t* ovl_out, uint64_t* ovl_pos_out, rala_ovl_t* int_out,
+                              uint64_t* int_pos_out, uint64_t* counts);
 int rala_b200_multi_get_edges(rala_b200_multi* m, int k, rala_edge_t* out);
 int rala_b200_multi_get_marked(rala_b200_multi* m, int k, uint8_t* out);
 int rala_b200_multi_get_seq_to_node(rala_b200_multi* m, uint32_t* out /* n_piles */);

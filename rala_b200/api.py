@@ -70,7 +70,11 @@ EXPORTS = [
     "rala_b200_multi_get_seq_to_node", "rala_b200_multi_get_piles", "rala_b200_multi_event_record",
     "rala_b200_multi_event_elapsed_ms", "rala_b200_multi_launch_count", "rala_b200_multi_stage_ms",
     "rala_b200_multi_set_outputs", "rala_b200_multi_set_barrier_timeout_ms", "rala_b200_multi_set_rounds", "rala_b200_multi_barrier_log", "rala_b200_multi_sweep_log",
+    # multi-GPU staged construct (pile tables that change between the passes)
+    "rala_b200_multi_set_hills", "rala_b200_multi_classify", "rala_b200_multi_retrim", "rala_b200_multi_retrim_promote",
+    "rala_b200_multi_finish", "rala_b200_multi_get_hill_coverage", "rala_b200_multi_get_lists", "rala_b200_multi_edge_runs",
 ]
+MAX_SEGMENTS = 64
 
 _LIB = None
 
@@ -494,6 +498,13 @@ N_CAPS = 6
 CAP_NAMES = ("events_per_pair", "edges_per_pair", "slice_edges", "max_sweeps", "max_final_sweeps", "local_edges")
 
 
+def _by_position(parts):
+    """[(rows, global positions), ...] -> the rows in position order"""
+    rows = np.concatenate([r for r, _ in parts]) if parts else np.zeros((0, 7), np.uint32)
+    pos = np.concatenate([p for _, p in parts]) if parts else np.zeros(0, np.uint64)
+    return np.ascontiguousarray(rows[np.argsort(pos, kind="stable")])
+
+
 class MultiCounts(C.Structure):
     _fields_ = [("world", C.c_int), ("n_local", C.c_int), ("n_records", C.c_uint64), ("n_piles", C.c_uint32),
                 ("n_alive_piles", C.c_uint32), ("n_nodes", C.c_uint32), ("n_edges", C.c_uint64), ("n_local_edges", C.c_uint64),
@@ -509,7 +520,8 @@ class Multi:
     """The multi-GPU session (rala_b200_multi): ranks [first_rank, first_rank + len(devices)) of `world` live in this
     process, one per entry of `devices` (an id may repeat: several ranks on one GPU, which is how the parity tests
     cover world > 1 on a one-GPU box).  Graph::construct's hot half + remove_transitive_edges with the pile table
-    frozen, bit-identical to the single-GPU session on the concatenation of the shards."""
+    frozen (run), or changed by the host between the passes (the staged calls classify .. finish, construct),
+    bit-identical to the single-GPU session on the concatenation of the shards."""
 
     def __init__(self, devices, first_rank: int = 0, world: int | None = None, lib=None):
         self.lib = lib or load()
@@ -524,6 +536,7 @@ class Multi:
             raise RalaB200Error(f"rala_b200_multi_create(devices={self.devices}) failed with status {rc}: "
                                 "sm_100 (B200) devices are required, there is no CPU fallback")
         self.n_piles = 0
+        self.n_hills = 0
         self._keep = {}
         if len(set(self.devices)) < self.n_local:
             # ranks sharing a GPU wait for each other INSIDE kernels: every stream needs a hardware queue of its own
@@ -556,6 +569,14 @@ class Multi:
         self.n_piles = p.shape[0]
         self._keep["piles"] = (p, f)
         self._call("rala_b200_multi_set_piles", _ptr(p), _ptr(f), C.c_uint32(self.n_piles))
+        return self
+
+    def set_hills(self, hills):
+        """Replicated hill rows (grouped by ascending pile id); only the staged classify counts them."""
+        h = _np(np.zeros((0, 3)) if hills is None else hills, np.uint32, 3)
+        self.n_hills = h.shape[0]
+        self._keep["hills"] = h
+        self._call("rala_b200_multi_set_hills", _ptr(h), C.c_uint32(self.n_hills))
         return self
 
     def set_overlaps(self, k: int, records, t0: int):
@@ -661,14 +682,100 @@ class Multi:
         self._call("rala_b200_multi_counts", C.byref(c))
         return c.as_dict()
 
+    # ---- staged construct (pile tables that change between the passes) ---------------------------
+    def classify(self):
+        self._call("rala_b200_multi_classify")
+        return self
+
+    def retrim(self):
+        self._call("rala_b200_multi_retrim")
+        return self
+
+    def retrim_promote(self) -> bool:
+        changed = C.c_int(0)
+        self._call("rala_b200_multi_retrim_promote", C.byref(changed))
+        return bool(changed.value)
+
+    def finish(self):
+        """graph.cpp:831-877, 552-632 and 1281-1318 on the staged lists."""
+        self._call("rala_b200_multi_finish")
+        return self
+
+    def hill_coverage(self, k: int = 0):
+        """Hill counters of the first pass summed over all ranks, as local rank k holds them."""
+        out = np.zeros(self.n_hills, dtype=np.uint32)
+        self._call("rala_b200_multi_get_hill_coverage", C.c_int(k), _ptr(out))
+        return out
+
+    def local_lists(self, k: int):
+        """(overlaps, their global positions, internals, their global positions) of local rank k."""
+        n = np.zeros(2, dtype=np.uint64)
+        self._call("rala_b200_multi_get_lists", C.c_int(k), None, None, None, None, _ptr(n))
+        ovl, inl = np.zeros((int(n[0]), 7), np.uint32), np.zeros((int(n[1]), 7), np.uint32)
+        opos, ipos = np.zeros(int(n[0]), np.uint64), np.zeros(int(n[1]), np.uint64)
+        self._call("rala_b200_multi_get_lists", C.c_int(k), _ptr(ovl), _ptr(opos), _ptr(inl), _ptr(ipos), _ptr(n))
+        return ovl, opos, inl, ipos
+
+    def lists(self):
+        """`overlaps` and `internals` in the reference's order, rebuilt from every local rank's entries and global positions
+        (the whole lists when every rank is local)."""
+        parts = [self.local_lists(k) for k in range(self.n_local)]
+        return _by_position([(p[0], p[1]) for p in parts]), _by_position([(p[2], p[3]) for p in parts])
+
+    def connections(self):
+        """(a_id, b_id) of every entry of `overlaps` in list order: the input of the host's pit loop (graph.cpp:740-744)."""
+        return np.ascontiguousarray(self.lists()[0][:, :2])
+
+    def construct(self, records, piles, flags=None, hills=None, pile_ops=None):
+        """Graph::construct's hot half and remove_transitive_edges on all ranks, with the same `pile_ops` contract as
+        Graph.construct (pile_ops=None: the pile table is frozen, but the staged calls still run).  Every rank local: the
+        records are cut with set_shards and plan() sizes the exchange buffers first."""
+        self.set_piles(piles, flags).set_hills(hills).set_shards(records)
+        self.plan()
+        self.classify()
+        if pile_ops is not None:
+            upd = pile_ops.break_over_chimeric_hills(self.hill_coverage())
+            if upd is not None:
+                self.set_piles(*upd)
+        self.retrim()
+        while True:
+            if pile_ops is not None:
+                upd = pile_ops.break_over_chimeric_pits(self.connections())
+                if upd is not None:
+                    self.set_piles(*upd)
+            if not self.retrim_promote():
+                break
+        self.finish()
+        need, fits = self.demand()
+        if not fits:   # plan() sized the buffers from a frozen step; the staged passes may need more
+            raise RalaB200Error(f"construct: the staged passes did not fit the exchange buffers (need {need.tolist()}): "
+                                "reserve() with larger capacities and construct again")
+        c = self.counts()
+        self.n_nodes, self.n_edges = c["n_nodes"], c["n_edges"]
+        return self
+
     # ---- results -----------------------------------------------------------------------------------
     def edge_range(self, k: int):
         first, n = C.c_uint64(0), C.c_uint64(0)
         self._call("rala_b200_multi_edge_range", C.c_int(k), C.byref(first), C.byref(n))
         return int(first.value), int(n.value)
 
+    def edge_runs(self, k: int):
+        """(n, 2) array of (first global edge id, count): the ids of the rows edges(k) returns, in that order."""
+        out = np.zeros((MAX_SEGMENTS, 2), dtype=np.uint64)
+        n = C.c_uint32(0)
+        self._call("rala_b200_multi_edge_runs", C.c_int(k), _ptr(out), C.byref(n))
+        return out[:int(n.value)]
+
+    def edge_ids(self, k: int):
+        """Global id of every row edges(k) returns."""
+        runs = self.edge_runs(k)
+        if runs.shape[0] == 0:
+            return np.zeros(0, dtype=np.int64)
+        return np.concatenate([np.arange(int(f), int(f) + int(c), dtype=np.int64) for f, c in runs])
+
     def edges(self, k: int, out=None):
-        _, n = self.edge_range(k)
+        n = int(self.edge_runs(k)[:, 1].sum())
         if out is None:
             out = np.zeros((n, 3), dtype=np.uint32)
         if n:
@@ -676,7 +783,7 @@ class Multi:
         return out
 
     def marked(self, k: int, out=None):
-        _, n = self.edge_range(k)
+        n = int(self.edge_runs(k)[:, 1].sum())
         if out is None:
             out = np.zeros(n, dtype=np.uint8)
         if n:
@@ -685,9 +792,11 @@ class Multi:
 
     def all_edges(self):
         """Edge rows and marks of the local ranks in edge-id order (the whole graph when every rank is local)."""
-        e = [self.edges(k) for k in range(self.n_local)]
-        m = [self.marked(k) for k in range(self.n_local)]
-        return np.concatenate(e), np.concatenate(m)
+        ids = [self.edge_ids(k) for k in range(self.n_local)]
+        e = np.concatenate([self.edges(k) for k in range(self.n_local)])
+        m = np.concatenate([self.marked(k) for k in range(self.n_local)])
+        order = np.argsort(np.concatenate(ids), kind="stable")
+        return e[order], m[order]
 
     def seq_to_node(self):
         out = np.zeros(self.n_piles, dtype=np.uint32)

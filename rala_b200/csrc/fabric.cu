@@ -857,8 +857,10 @@ void launch_inbox_degree(Launch& L, Peers P, ArenaLayout A, const BuildMeta* met
 // scatter the received edges into the rows of this rank's slice of the replicated CSR (slot order inside a row is
 // arbitrary, as in k_fill_csr).  col_eid[pos] = GLOBAL edge id (the transitive kernels break ties between parallel
 // edges by it, graph.cpp:1291-1293, and address their result bytes with it); T[that id] is cleared on the way.
+// RUNS: the emitting rank's local ids fall into several runs of global ids (EdgeRuns, staged construct)
+template <bool RUNS>
 __global__ void __launch_bounds__(256) k_inbox_fill(Peers P, ArenaLayout A, const BuildMeta* __restrict__ meta, uint32_t* __restrict__ cursor,
-                                                   uint32_t* __restrict__ col_eid, uint8_t* __restrict__ T) {
+                                                   uint32_t* __restrict__ col_eid, uint8_t* __restrict__ T, const EdgeRuns* __restrict__ runs) {
     const FabricHdr* mine = hdr_of(P, P.rank);
     const uint32_t par = mine->epoch & 1u, from = blockIdx.y;
     const uint32_t n = min(mine->sent[par][from][P.rank], A.cap_edge);
@@ -871,16 +873,27 @@ __global__ void __launch_bounds__(256) k_inbox_fill(Peers P, ArenaLayout A, cons
         if (row >= owned) continue;
         const uint32_t p = atomicAdd(&cursor[row], 1u);
         if (p >= slice) continue;
-        const uint32_t e = id_base + blk[3 * (size_t) A.cap_edge + i];
+        uint32_t e = id_base + blk[3 * (size_t) A.cap_edge + i];
+        if (RUNS) {   // the last segment whose local run starts at or before the id holds it
+            const uint32_t x = blk[3 * (size_t) A.cap_edge + i], W = runs->world;
+            uint32_t lo = 0, hi = runs->n_seg;
+            while (hi - lo > 1u) {
+                const uint32_t mid = (lo + hi) >> 1;
+                if (runs->lb[mid * W + from] <= x) lo = mid; else hi = mid;
+            }
+            e = runs->gb[lo * W + from] + (x - runs->lb[lo * W + from]);
+        }
         col[off + p] = make_uint2(blk[(size_t) A.cap_edge + i], blk[2 * (size_t) A.cap_edge + i]);
         col_eid[off + p] = e;
         T[e] = 0;
     }
 }
 
-void launch_inbox_fill(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, uint32_t* cursor, uint32_t* col_eid, uint8_t* T) {
+void launch_inbox_fill(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, uint32_t* cursor, uint32_t* col_eid, uint8_t* T,
+                       const EdgeRuns* runs) {
     dim3 grid(grid_for(A.cap_edge, 256, blocks_per_source(P.world)), P.world);
-    k_inbox_fill<<<grid, 256, 0, L.stream>>>(P, A, meta, cursor, col_eid, T);
+    if (runs) k_inbox_fill<true><<<grid, 256, 0, L.stream>>>(P, A, meta, cursor, col_eid, T, runs);
+    else k_inbox_fill<false><<<grid, 256, 0, L.stream>>>(P, A, meta, cursor, col_eid, T, nullptr);
     L.count++;
 }
 
@@ -906,8 +919,9 @@ void launch_push_csr(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, c
 }
 
 // T(e) = 1 results of the owned candidate edges -> the rank that emitted e (its T_in byte array, indexed by local edge id)
+template <bool RUNS>
 __global__ void __launch_bounds__(256) k_route_marks(Peers P, ArenaLayout A, const BuildMeta* __restrict__ meta, const uint8_t* __restrict__ T,
-                                                    const uint32_t* __restrict__ col_eid) {
+                                                    const uint32_t* __restrict__ col_eid, const EdgeRuns* __restrict__ runs) {
     __shared__ uint32_t s_base[kMaxRanks + 1];
     if (threadIdx.x <= (uint32_t) P.world) s_base[threadIdx.x] = meta->eid_base[threadIdx.x];
     __syncthreads();
@@ -915,14 +929,28 @@ __global__ void __launch_bounds__(256) k_route_marks(Peers P, ArenaLayout A, con
     for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < slice; p += gridDim.x * blockDim.x) {
         const uint32_t e = col_eid[off + p];
         if (!T[e]) continue;
-        const uint32_t r = owner_of(s_base, (uint32_t) P.world, e);
-        const uint32_t local = e - s_base[r];
+        uint32_t r, local;
+        if (RUNS) {   // the last run starting at or before e holds it (empty runs start where the next one does)
+            const uint32_t W = runs->world;
+            uint32_t lo = 0, hi = runs->n_seg * W;
+            while (hi - lo > 1u) {
+                const uint32_t mid = (lo + hi) >> 1;
+                if (runs->gb[mid] <= e) lo = mid; else hi = mid;
+            }
+            r = lo % W;
+            local = runs->lb[lo] + (e - runs->gb[lo]);
+        } else {
+            r = owner_of(s_base, (uint32_t) P.world, e);
+            local = e - s_base[r];
+        }
         if (local < A.t_cap) section<uint8_t>(P, (int) r, A.T_in)[local] = 1;
     }
 }
 
-void launch_route_marks(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, const uint8_t* T, const uint32_t* col_eid) {
-    k_route_marks<<<grid_for(A.cap_slice, 256, kNumSMs * 4), 256, 0, L.stream>>>(P, A, meta, T, col_eid);
+void launch_route_marks(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, const uint8_t* T, const uint32_t* col_eid,
+                        const EdgeRuns* runs) {
+    if (runs) k_route_marks<true><<<grid_for(A.cap_slice, 256, kNumSMs * 4), 256, 0, L.stream>>>(P, A, meta, T, col_eid, runs);
+    else k_route_marks<false><<<grid_for(A.cap_slice, 256, kNumSMs * 4), 256, 0, L.stream>>>(P, A, meta, T, col_eid, nullptr);
     L.count++;
 }
 
@@ -946,6 +974,101 @@ void launch_demand(Launch& L, Peers P, const uint32_t* ev_cnt0, const uint32_t* 
     L.count++;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Staged construct: the host changes the pile table between the passes (hill breaking, the pit loop of graph.cpp:704-829).
+// Every list pass leaves per-segment counts that all ranks need (global positions, is_changed, edge ids): each rank counts
+// its own, pushes them into every peer's seg_mail section and a barrier publishes them.
+// ---------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_seg_count(List l, const uint32_t* __restrict__ lo, uint32_t n_seg, const uint2* __restrict__ piles,
+                                                  int mode, uint32_t* __restrict__ out) {
+    __shared__ uint32_t s_lo[kMaxSegs + 1], s_cnt[2 * kMaxSegs];
+    for (uint32_t s = threadIdx.x; s <= n_seg; s += blockDim.x) s_lo[s] = lo[s];
+    for (uint32_t s = threadIdx.x; s < 2 * n_seg; s += blockDim.x) s_cnt[s] = 0u;
+    __syncthreads();
+    const uint32_t n = s_lo[n_seg];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        uint32_t a = 0, b = n_seg;   // segment of entry i: the last one starting at or before it
+        while (b - a > 1u) {
+            const uint32_t mid = (a + b) >> 1;
+            if (s_lo[mid] <= i) a = mid; else b = mid;
+        }
+        Entry e = load_entry(l, i);
+        const Pile pa = load_pile(piles, e.a), pb = load_pile(piles, e.b);
+        if (!pa.alive() || !pb.alive()) continue;
+        if (mode == kSegRetrim) {   // k_list_pass<kRetrim>: trim() accepts
+            if (trim(e.c, e.ori, pa, pb)) atomicAdd(&s_cnt[a], 1u);
+        } else {                    // k_list_pass<kFinalOvl> keeps it; k_emit_edges makes two edges of it
+            const uint8_t tag = l.tag[i];
+            if (tag != kA && tag != kB) atomicAdd(&s_cnt[a], 1u);
+            const uint8_t t = classify(e.c, relative(e.c, e.ori, pa, pb));
+            if (t == kAB || t == kBA) atomicAdd(&s_cnt[n_seg + a], 1u);
+        }
+    }
+    __syncthreads();
+    for (uint32_t s = threadIdx.x; s < 2 * n_seg; s += blockDim.x)
+        if (s_cnt[s]) atomicAdd(&out[s], s_cnt[s]);
+}
+
+void launch_seg_count(Launch& L, List l, const uint32_t* lo, uint32_t n_seg, const uint2* piles, int mode, uint32_t* out) {
+    k_seg_count<<<kNumSMs * 4, 256, 0, L.stream>>>(l, lo, n_seg, piles, mode, out);
+    L.count++;
+}
+
+__global__ void __launch_bounds__(32) k_seg_push(Peers P, ArenaLayout A, const uint32_t* __restrict__ box, uint32_t n) {
+    const int q = threadIdx.x;
+    if (q >= P.world) return;
+    const uint32_t par = (hdr_of(P, P.rank)->epoch + 1u) & 1u;   // the barrier that follows on this stream
+    uint32_t* dst = section<uint32_t>(P, q, A.seg_mail) + ((size_t) par * kMaxRanks + (size_t) P.rank) * kSegMail;
+    for (uint32_t k = 0; k < n; ++k) st_sys(dst + k, box[k]);
+}
+
+void launch_seg_push(Launch& L, Peers P, ArenaLayout A, const uint32_t* box, uint32_t n) {
+    k_seg_push<<<1, 32, 0, L.stream>>>(P, A, box, n);
+    L.count++;
+}
+
+__global__ void k_decode_states(Peers P, ArenaLayout A) {
+    uint32_t* S = section<uint32_t>(P, P.rank, A.S);
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < A.n_piles; i += gridDim.x * blockDim.x) {
+        const uint32_t d = S[i] & kNever;
+        S[i] = d == kNever ? kInf : d;
+    }
+}
+
+void launch_decode_states(Launch& L, Peers P, ArenaLayout A) {
+    k_decode_states<<<grid_for(A.n_piles, 256, kNumSMs * 4), 256, 0, L.stream>>>(P, A);
+    L.count++;
+}
+
+__device__ __forceinline__ void red_add_sys(uint32_t* p, uint32_t v) {
+    asm volatile("red.relaxed.sys.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+__global__ void k_push_hills(Peers P, ArenaLayout A, const uint32_t* __restrict__ cov, uint32_t n_hills) {
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n_hills; k += gridDim.x * blockDim.x) {
+        const uint32_t c = cov[k];
+        if (!c) continue;
+        for (int q = 0; q < P.world; ++q) red_add_sys(section<uint32_t>(P, q, A.hills) + k, c);
+    }
+}
+
+void launch_push_hills(Launch& L, Peers P, ArenaLayout A, const uint32_t* cov, uint32_t n_hills) {
+    if (!n_hills) return;
+    k_push_hills<<<grid_for(n_hills, 256, kNumSMs), 256, 0, L.stream>>>(P, A, cov, n_hills);
+    L.count++;
+}
+
+__global__ void k_final_deaths(Peers P, ArenaLayout A, uint32_t* __restrict__ dst) {
+    const uint32_t* S = section<uint32_t>(P, P.rank, A.S);
+    const bool skipped = hdr_of(P, P.rank)->skip_pass != 0u;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < A.n_piles; i += gridDim.x * blockDim.x) dst[i] = skipped ? kInf : S[i];
+}
+
+void launch_final_deaths(Launch& L, Peers P, ArenaLayout A, uint32_t* dst) {
+    k_final_deaths<<<grid_for(A.n_piles, 256, kNumSMs * 4), 256, 0, L.stream>>>(P, A, dst);
+    L.count++;
+}
+
 // CUDA loads kernels lazily, at their first launch, and that load waits for the device to drain: fatal when the
 // first launch of a kernel happens while another rank's barrier kernel is spinning on the same device (ranks sharing
 // a GPU) — the barrier waits for this rank, this rank's kernel waits for the barrier.  rala_b200_create loads them all.
@@ -964,10 +1087,17 @@ void preload_fabric() {
     cudaFuncGetAttributes(&a, k_route_edges);
     cudaFuncGetAttributes(&a, k_edge_meta);
     cudaFuncGetAttributes(&a, k_inbox_degree);
-    cudaFuncGetAttributes(&a, k_inbox_fill);
+    cudaFuncGetAttributes(&a, k_inbox_fill<false>);
+    cudaFuncGetAttributes(&a, k_inbox_fill<true>);
     cudaFuncGetAttributes(&a, k_push_csr);
-    cudaFuncGetAttributes(&a, k_route_marks);
+    cudaFuncGetAttributes(&a, k_route_marks<false>);
+    cudaFuncGetAttributes(&a, k_route_marks<true>);
     cudaFuncGetAttributes(&a, k_fabric_demand);
+    cudaFuncGetAttributes(&a, k_seg_count);
+    cudaFuncGetAttributes(&a, k_seg_push);
+    cudaFuncGetAttributes(&a, k_decode_states);
+    cudaFuncGetAttributes(&a, k_push_hills);
+    cudaFuncGetAttributes(&a, k_final_deaths);
 }
 
 }  // namespace rb

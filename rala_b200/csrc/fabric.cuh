@@ -26,6 +26,11 @@ constexpr int kMailSlots = 8;
 constexpr int kBarrierLog = 128;
 constexpr int kSweepLog = 48;
 constexpr int kResolveCtlBytes = 32 + kSweepLog * 16;
+// Staged construct (pile table changed by the host between the passes): the promotions of a pit round are appended to the
+// end of the GLOBAL `overlaps`, so a rank's local list is a run of SEGMENTS (segment 0: its entries of the first pass,
+// segment k: what it promoted in the k-th round that promoted anything), at most kMaxSegs of them.
+constexpr int kMaxSegs = 64;
+constexpr int kSegMail = 2 * kMaxSegs + 4;   // words one rank sends every peer after a staged list pass
 
 // mail slots: small scalars a rank publishes to every peer inside a barrier
 enum Mail { M_UNSETTLED = 0, M_NOVL, M_NINL, M_NEDGES, M_SENT_TO_YOU, M_EMITTED, M_SPARE1, M_SPARE2 };
@@ -66,9 +71,11 @@ struct ArenaLayout {
     size_t T_in;          // t_cap bytes: transitive test results for the edges THIS rank emitted, written by their evaluators
     size_t row_ptr;       // n_nodes_max + 2 words: CSR row offsets of the whole graph
     size_t col;           // world * cap_slice x (dst, len): CSR of the whole graph, slices in rank order
+    size_t seg_mail;      // [2 epoch parities][kMaxRanks source ranks][kSegMail] words: per-segment list counts of a staged pass
+    size_t hills;         // n_hills words: hill counters summed over the ranks (remote reductions of the first pass)
     size_t total;
     uint32_t cap_ev, cap_edge, cap_slice, t_cap;
-    uint32_t n_piles, n_nodes_max;
+    uint32_t n_piles, n_nodes_max, n_hills;
     uint32_t ppr;         // piles per rank, rounded up to whole blocks of 32 (sizes the per-rank loops)
     uint32_t npr_max;     // upper bound of the nodes one rank owns (sizes the row scan)
 };
@@ -102,6 +109,13 @@ struct BuildMeta {
     uint32_t node_begin[kMaxRanks + 1]; // first node owned by rank p
 };
 
+// Global edge ids of a staged construct: the dovetails of run (segment s, rank r) are edges [gb[i], gb[i] + 2 x count) with
+// i = s * world + r, and rank r emitted them as its local edges [lb[i], ...).  Runs are in global id order (segment-major).
+struct EdgeRuns {
+    uint32_t n_seg, world;
+    uint32_t gb[kMaxSegs * kMaxRanks];
+    uint32_t lb[kMaxSegs * kMaxRanks];
+};
 
 // launchers (fabric.cu)
 void launch_fabric_barrier(Launch& L, Peers P, Publish pub);
@@ -127,9 +141,26 @@ void launch_route_edges(Launch& L, Peers P, ArenaLayout A, const uint32_t* src, 
                         const uint32_t* n_edges, uint32_t edge_cap, const BuildMeta* meta, uint32_t* out_cnt);
 void launch_edge_meta(Launch& L, Peers P, ArenaLayout A, BuildMeta* meta, uint32_t* counters);
 void launch_inbox_degree(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, uint32_t* degree);
-void launch_inbox_fill(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, uint32_t* cursor, uint32_t* col_eid, uint8_t* T);
+// runs: nullptr = one contiguous id range per emitting rank (meta->eid_base); otherwise the runs of a staged construct
+void launch_inbox_fill(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, uint32_t* cursor, uint32_t* col_eid, uint8_t* T,
+                       const EdgeRuns* runs);
 void launch_push_csr(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, const uint32_t* row_ptr_local);
-void launch_route_marks(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, const uint8_t* T, const uint32_t* col_eid);
+void launch_route_marks(Launch& L, Peers P, ArenaLayout A, const BuildMeta* meta, const uint8_t* T, const uint32_t* col_eid,
+                        const EdgeRuns* runs);
 void launch_demand(Launch& L, Peers P, const uint32_t* ev_cnt0, const uint32_t* ev_cnt1, const uint32_t* edge_cnt, const BuildMeta* meta);
+
+// staged construct
+enum SegCountMode { kSegRetrim = 0, kSegFinal = 1 };
+// per-segment counts of a local list whose segment s is entries [lo[s], lo[s + 1]): kSegRetrim -> out[s] = entries a retrim keeps;
+// kSegFinal -> out[s] = entries the final filter keeps, out[n_seg + s] = dovetails that become edges.  out must be zeroed.
+void launch_seg_count(Launch& L, List l, const uint32_t* lo, uint32_t n_seg, const uint2* piles, int mode, uint32_t* out);
+// box[0 .. n) -> seg_mail[parity of the next barrier][this rank] of every rank (the barrier that follows publishes it)
+void launch_seg_push(Launch& L, Peers P, ArenaLayout A, const uint32_t* box, uint32_t n);
+// the replica's settled pile states -> death times (kInf = never) in place, before the deaths are applied
+void launch_decode_states(Launch& L, Peers P, ArenaLayout A);
+// this rank's hill counters added into every rank's hills section (zeroed before the events barrier of the same pass)
+void launch_push_hills(Launch& L, Peers P, ArenaLayout A, const uint32_t* cov, uint32_t n_hills);
+// death times of the final pass -> dst (kInf everywhere when the pass was skipped for want of events)
+void launch_final_deaths(Launch& L, Peers P, ArenaLayout A, uint32_t* dst);
 
 }  // namespace rb

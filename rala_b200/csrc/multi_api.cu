@@ -20,6 +20,17 @@ using namespace rb;
 
 namespace {
 
+// word offsets in FabricRank::stage (staged construct)
+enum StageWords : size_t {
+    SW_LO = 0,                      // kMaxSegs + 1: local start of every segment of `overlaps`, then its end
+    SW_BOX = 128,                   // kSegMail: this rank's counts of a staged pass, pushed to every peer
+    SW_FIN_N = 384,                 // kMaxSegs: local entries of every segment (final containment events)
+    SW_FIN_BASE = 448,              // kMaxSegs: global time of the first of them
+    SW_ZERO = 512,                  // a word that stays 0
+    SW_WORDS = 520
+};
+constexpr size_t kStageRunsByte = 4096;   // EdgeRuns
+
 struct FabricRank {
     rala_b200_ctx* ctx = nullptr;
     rala_b200_graph* g = nullptr;
@@ -28,6 +39,8 @@ struct FabricRank {
     Peers P{};
     ArenaLayout A{};
     DevBuf meta, out_cnt, tmin, wait, col_eid, T;
+    DevBuf stage;                  // staged construct: segment bounds, outgoing counts, time bases, edge runs (StageWords)
+    std::vector<uint32_t> stage_host;   // host copy of the words uploaded to `stage` (kept alive for the async copies)
     void* ipc_mapped[kMaxRanks]{};
     cudaGraphExec_t exec[2] = {nullptr, nullptr};   // [0] repeated run, [1] first run after set_piles (phase_events copies the table the other way)
     uint64_t graph_launches[2] = {0, 0};
@@ -40,6 +53,8 @@ struct FabricRank {
     uint32_t* cnt_edges() const { return out_cnt.as<uint32_t>() + 2 * kMaxRanks; }
     uint32_t* ctl(int pass) const { return out_cnt.as<uint32_t>() + 3 * kMaxRanks + pass * (kResolveCtlBytes / 4); }
     FabricHdr* hdr() const { return arena.as<FabricHdr>(); }
+    uint32_t* stage_w(size_t word) const { return stage.as<uint32_t>() + word; }
+    EdgeRuns* runs_dev() const { return reinterpret_cast<EdgeRuns*>(stage.as<uint8_t>() + kStageRunsByte); }
     template <class T> T* sec(size_t off) const { return reinterpret_cast<T*>(arena.as<uint8_t>() + off); }
 };
 
@@ -55,6 +70,15 @@ struct rala_b200_multi {
     bool use_graph = true;
     uint32_t barrier_timeout_ms = 10000;
     int runs_seen[2] = {0, 0};   // per graph variant: 0 next run is eager, 1 next run is captured, 2 replay
+    uint32_t n_hills = 0;
+    // staged construct (rala_b200_multi_classify .. finish): what every rank's lists hold, replicated through seg_mail
+    int staged = 0;                  // 0 none, 2 classified (list passes may follow), 3 finished
+    bool staged_edges = false;       // the last edge list came from finish: ids in runs (EdgeRuns), not one range per rank
+    uint32_t n_seg = 0;
+    std::vector<uint32_t> seg;       // [kMaxSegs][world]: entries of segment s of `overlaps` on rank r
+    std::vector<uint32_t> inl;       // [world]: entries of `internals` on rank r (one rank-major segment: it only shrinks)
+    std::vector<uint32_t> dov;       // [kMaxSegs][world]: dovetails of the final `overlaps` (edges / 2)
+    EdgeRuns runs{};
 };
 
 static int mfail(rala_b200_multi* m, int code, const char* fmt, ...) {
@@ -175,7 +199,7 @@ extern "C" void rala_b200_multi_destroy(rala_b200_multi* m) {
         cudaSetDevice(fr.device);
         if (fr.ev[0]) cudaEventDestroy(fr.ev[0]);
         if (fr.ev[1]) cudaEventDestroy(fr.ev[1]);
-        DevBuf* bufs[] = {&fr.arena, &fr.meta, &fr.out_cnt, &fr.tmin, &fr.wait, &fr.col_eid, &fr.T};
+        DevBuf* bufs[] = {&fr.arena, &fr.meta, &fr.out_cnt, &fr.tmin, &fr.wait, &fr.col_eid, &fr.T, &fr.stage};
         for (DevBuf* b : bufs) b->release();
         if (fr.g) rala_b200_graph_destroy(fr.g);
         rala_b200_destroy(fr.ctx);
@@ -189,12 +213,19 @@ extern "C" int rala_b200_multi_set_piles(rala_b200_multi* m, const rala_pile_t* 
     if (!m) return RALA_B200_ERR_ARG;
     for (FabricRank& fr : m->ranks) {
         MRC(m, fr, rala_b200_graph_set_piles(fr.g, piles, flags, n_piles));
-        MRC(m, fr, rala_b200_graph_set_hills(fr.g, nullptr, 0));
     }
     if (n_piles != m->n_piles) {
         m->n_piles = n_piles;
         m->reserved = false;
     }
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_multi_set_hills(rala_b200_multi* m, const rala_hill_t* hills, uint32_t n_hills) {
+    if (!m || (n_hills && !hills)) return RALA_B200_ERR_ARG;
+    for (FabricRank& fr : m->ranks) MRC(m, fr, rala_b200_graph_set_hills(fr.g, hills, n_hills));
+    if (n_hills > (m->reserved ? m->ranks[0].A.n_hills : 0u)) m->reserved = false;   // the arena's hills section grows
+    m->n_hills = n_hills;
     return RALA_B200_OK;
 }
 
@@ -205,6 +236,8 @@ extern "C" int rala_b200_multi_set_overlaps(rala_b200_multi* m, int k, const ral
                                              (unsigned long long) t0, (unsigned long long) n);
     MRC(m, fr, rala_b200_graph_set_overlaps(fr.g, ovl, n));
     MRC(m, fr, rala_b200_graph_set_shard(fr.g, (uint32_t) t0, fr.rank, m->world));
+    m->staged = 0;
+    m->staged_edges = false;
     if (n != fr.n_rec) m->reserved = false;
     fr.n_rec = n;
     drop_graphs(m);
@@ -220,6 +253,8 @@ extern "C" int rala_b200_multi_set_overlaps_columns(rala_b200_multi* m, int k, c
     const bool same_shape = n == fr.n_rec && m->reserved;
     MRC(m, fr, rala_b200_graph_set_overlaps_columns(fr.g, a_id, b_id, a_begin, a_end, b_begin, b_end, n));
     MRC(m, fr, rala_b200_graph_set_shard(fr.g, (uint32_t) t0, fr.rank, m->world));
+    m->staged = 0;
+    m->staged_edges = false;
     if (!same_shape) {
         m->reserved = false;
         drop_graphs(m);
@@ -237,6 +272,8 @@ extern "C" int rala_b200_multi_set_overlaps_packed(rala_b200_multi* m, int k, co
     const bool same_shape = n == fr.n_rec && m->reserved;
     MRC(m, fr, rala_b200_graph_set_overlaps_packed(fr.g, query_id, group_end, n_groups, b_id, a_span, b_span, n));
     MRC(m, fr, rala_b200_graph_set_shard(fr.g, (uint32_t) t0, fr.rank, m->world));
+    m->staged = 0;
+    m->staged_edges = false;
     if (!same_shape) {
         m->reserved = false;
         drop_graphs(m);
@@ -292,6 +329,9 @@ static ArenaLayout make_layout(const rala_b200_multi* m, const uint64_t* caps) {
     A.T_in = off;       off += align_up((size_t) A.t_cap, 256);
     A.row_ptr = off;    off += align_up(((size_t) A.n_nodes_max + 8) * 4, 256);
     A.col = off;        off += align_up(W * (size_t) A.cap_slice * 8, 256);
+    A.seg_mail = off;   off += align_up((size_t) 2 * kMaxRanks * kSegMail * 4, 256);
+    A.n_hills = m->n_hills;
+    A.hills = off;      off += align_up((size_t) A.n_hills * 4 + 4, 256);
     A.total = off;
     return A;
 }
@@ -328,6 +368,7 @@ extern "C" int rala_b200_multi_reserve(rala_b200_multi* m, const uint64_t* caps)
         // result bytes of the transitive pass, indexed by GLOBAL edge id: an id is < world x the edges one rank can emit,
         // whatever happened to the exchange buffers (nothing clears the array: the row fill clears the bytes it needs)
         MCU(m, fr.T.reserve(align_up(W * (size_t) A.t_cap + 16, 256)));
+        MCU(m, fr.stage.reserve(kStageRunsByte + sizeof(EdgeRuns)));
         MRC(m, fr, reserve_events(fr.g, (uint32_t) (W * A.cap_ev)));
         // the owned rows are scanned over npr_max + 1 entries
         const size_t rows = (size_t) A.npr_max + 16;
@@ -437,7 +478,7 @@ static int route_and_meet(rala_b200_multi* m, FabricRank& fr, int pass) {
 }
 
 // graph.cpp:469-480 / 831-866 on the piles this rank owns
-static int resolve_owned_piles(rala_b200_multi* m, FabricRank& fr, int pass) {
+static int resolve_owned_piles(rala_b200_multi* m, FabricRank& fr, int pass, bool hills = false) {
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
     const ResolveBufs rb = resolve_bufs(g);
@@ -455,9 +496,19 @@ static int resolve_owned_piles(rala_b200_multi* m, FabricRank& fr, int pass) {
     launch_fabric_resolve(L, fr.P, fr.A, rb, fr.wait.as<uint32_t>(), fr.ctl(pass), pass, rounds, 1000000ull * m->barrier_timeout_ms,
                           fr.resolve_blocks);
     MCU(m, end_stage(g, ST_K1B_KERNEL));
+    // staged construct: the hill counters of the local records (pile.cpp:457-469) read the death times BEFORE the deaths are
+    // applied, then go into the replicated total (every rank's hills section, published by the survivors barrier)
+    if (hills) {
+        const uint32_t* h = g->hills.as<uint32_t>();
+        const uint32_t n = g->n_hills;
+        launch_decode_states(L, fr.P, fr.A);
+        launch_hill_coverage(L, g->recs.view, g->t0, g->piles.as<uint2>(), g->hill_rec.as<uint32_t>(), g->cap, h, h + n, h + 2 * (size_t) n,
+                             n, g->hills.as<uint32_t>() + 3 * (size_t) n, fr.sec<uint32_t>(fr.A.S), g->n_piles, g->cnt());
+        launch_push_hills(L, fr.P, fr.A, h + 3 * (size_t) n, n);
+    }
     // every replica now holds every pile's final state: piles with a finite death time die (graph.cpp:471,477,838,842)
     // (a skipped pass killed nobody: the table and the liveness bitmap stay as they are)
-    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->cnt(), g->alive_bits.as<uint32_t>(), true,
+    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->cnt(), g->alive_bits.as<uint32_t>(), !hills,
                         skip_flag(fr.P));
     MCU(m, cudaGetLastError());
     return RALA_B200_OK;
@@ -553,7 +604,8 @@ static int phase_g_csr(rala_b200_multi* m, FabricRank& fr) {
     uint32_t* ticket;
     scan_state(g, rows, &status, &ticket);
     launch_scan_u32(L, g->cursor.as<uint32_t>(), g->row_ptr.as<uint32_t>(), rows, status, ticket);
-    launch_inbox_fill(L, fr.P, fr.A, fr.meta_dev(), g->cursor.as<uint32_t>(), fr.col_eid.as<uint32_t>(), fr.T.as<uint8_t>());
+    launch_inbox_fill(L, fr.P, fr.A, fr.meta_dev(), g->cursor.as<uint32_t>(), fr.col_eid.as<uint32_t>(), fr.T.as<uint8_t>(),
+                      m->staged_edges ? fr.runs_dev() : nullptr);
     launch_push_csr(L, fr.P, fr.A, fr.meta_dev(), g->row_ptr.as<uint32_t>());
     launch_fabric_barrier(L, fr.P, no_mail(m));
     MCU(m, cudaGetLastError());
@@ -580,7 +632,7 @@ static int phase_h_transitive(rala_b200_multi* m, FabricRank& fr) {
     launch_transitive(L, ga, g->n_nodes_max, g->edge_cap, g->heavy_view(), g->work_counter.as<uint32_t>(), g->cnt(), 0u, 0xFFFFFFFFu,
                       fr.meta_dev()->node_begin + fr.rank);
     MCU(m, end_stage(g, ST_K3_KERNELS));
-    launch_route_marks(L, fr.P, fr.A, fr.meta_dev(), fr.T.as<uint8_t>(), fr.col_eid.as<uint32_t>());
+    launch_route_marks(L, fr.P, fr.A, fr.meta_dev(), fr.T.as<uint8_t>(), fr.col_eid.as<uint32_t>(), m->staged_edges ? fr.runs_dev() : nullptr);
     launch_fabric_barrier(L, fr.P, no_mail(m));
     return RALA_B200_OK;
 }
@@ -631,6 +683,8 @@ extern "C" int rala_b200_multi_run(rala_b200_multi* m) {
     if (!m->reserved || !m->connected) return mfail(m, RALA_B200_ERR_STATE, "run: reserve (and connect) the exchange arenas first");
     for (FabricRank& fr : m->ranks)
         if (fr.g->state < 1) return mfail(m, RALA_B200_ERR_STATE, "run: rank %d has no inputs", fr.rank);
+    m->staged = 0;
+    m->staged_edges = false;
     const int variant = m->ranks[0].g->piles_fresh ? 1 : 0;
     if (!m->use_graph || m->runs_seen[variant] == 0) {
         const int rc = enqueue_step(m);
@@ -745,6 +799,8 @@ extern "C" int rala_b200_multi_plan(rala_b200_multi* m) {
     if (rc) return rc;
     for (int attempt = 0; attempt < 6; ++attempt) {
         rc = rala_b200_multi_reserve(m, caps);
+        m->staged = 0;
+        m->staged_edges = false;
         if (!rc) rc = enqueue_step(m);
         if (!rc) rc = rala_b200_multi_synchronize(m);
         uint64_t need[RALA_B200_N_CAPS];
@@ -800,10 +856,54 @@ extern "C" int rala_b200_multi_counts(rala_b200_multi* m, rala_b200_multi_counts
     return RALA_B200_OK;
 }
 
+// global id runs of local rank k's edges, in local order, adjacent runs merged: out (nullable) holds 2 x RALA_B200_MAX_SEGMENTS
+static int edge_runs_of(rala_b200_multi* m, int k, uint64_t* out, uint32_t* n_out) {
+    FabricRank& fr = m->ranks[k];
+    if (fr.g->state < 4) return mfail(m, RALA_B200_ERR_STATE, "edge_runs: run (or finish) first");
+    std::vector<uint64_t> r;   // first, count, first, count, ...
+    auto add = [&](uint64_t first, uint64_t count) {
+        if (!count) return;
+        if (!r.empty() && r[r.size() - 2] + r.back() == first) r.back() += count;
+        else r.insert(r.end(), {first, count});
+    };
+    if (m->staged_edges) {
+        for (uint32_t s = 0; s < m->runs.n_seg; ++s) {
+            const size_t i = (size_t) s * m->world + fr.rank;
+            add(m->runs.gb[i], 2ull * m->dov[i]);
+        }
+    } else {
+        MCU(m, cudaSetDevice(fr.device));
+        MCU(m, cudaStreamSynchronize(fr.ctx->L.stream));
+        BuildMeta bm;
+        MCU(m, cudaMemcpy(&bm, fr.meta.p, sizeof(bm), cudaMemcpyDeviceToHost));
+        add(bm.eid_base[fr.rank], bm.eid_base[fr.rank + 1] - bm.eid_base[fr.rank]);
+    }
+    *n_out = (uint32_t) (r.size() / 2);
+    if (out && !r.empty()) memcpy(out, r.data(), r.size() * sizeof(uint64_t));
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_multi_edge_runs(rala_b200_multi* m, int k, uint64_t* first_and_count_out, uint32_t* n_runs_out) {
+    if (!m || k < 0 || k >= m->n_local || !n_runs_out) return RALA_B200_ERR_ARG;
+    return edge_runs_of(m, k, first_and_count_out, n_runs_out);
+}
+
 extern "C" int rala_b200_multi_edge_range(rala_b200_multi* m, int k, uint64_t* first_edge, uint64_t* n) {
     if (!m || k < 0 || k >= m->n_local || !first_edge || !n) return RALA_B200_ERR_ARG;
     FabricRank& fr = m->ranks[k];
     if (fr.g->state < 4) return mfail(m, RALA_B200_ERR_STATE, "edge_range: run first");
+    if (m->staged_edges) {
+        uint64_t r[2 * kMaxSegs];
+        uint32_t n_runs = 0;
+        int rc = edge_runs_of(m, k, r, &n_runs);
+        if (rc) return rc;
+        if (n_runs > 1)
+            return mfail(m, RALA_B200_ERR_STATE, "edge_range: rank %d's edges are %u runs of global ids (a staged construct promoted "
+                         "overlaps): use rala_b200_multi_edge_runs", fr.rank, n_runs);
+        *first_edge = n_runs ? r[0] : 0;
+        *n = n_runs ? r[1] : 0;
+        return RALA_B200_OK;
+    }
     MCU(m, cudaSetDevice(fr.device));
     MCU(m, cudaStreamSynchronize(fr.ctx->L.stream));
     BuildMeta bm;
@@ -910,5 +1010,336 @@ extern "C" int rala_b200_multi_stage_ms(rala_b200_multi* m, int k, float* ms_out
     if (!m || k < 0 || k >= m->n_local || !ms_out) return RALA_B200_ERR_ARG;
     FabricRank& fr = m->ranks[k];
     MRC(m, fr, rala_b200_graph_stage_ms(fr.g, ms_out));
+    return RALA_B200_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Staged construct: Graph::construct with a pile table the host changes between the passes (graph.cpp:443-829), then
+// 831-877, 552-632 and 1281-1318.  The reference appends what a pit round promotes to the END of the global `overlaps`
+// (:818), so with shards in rank order the global list is segment-major: segment 0 = every rank's entries of the first
+// pass in rank order, segment k = what the k-th promoting round promoted, in rank order.  Each rank's local list is its
+// part of every segment, in segment order.  Every list pass ends with a barrier that publishes the new per-(segment,
+// rank) counts (seg_mail); the host reads them from its own arena, so every process holds the same table and takes the
+// same decisions (is_changed, a new segment) without a host collective.
+// ---------------------------------------------------------------------------------------------
+static List sub_list(const List& l, uint32_t off) {
+    List s = l;
+    s.a += off; s.b += off; s.ab += off; s.ae += off; s.bb += off; s.be += off; s.tag += off;
+    return s;
+}
+
+static uint32_t& seg_at(rala_b200_multi* m, std::vector<uint32_t>& v, uint32_t s, int q) { return v[(size_t) s * m->world + q]; }
+
+// local start of every segment of rank `fr`'s `overlaps` (and its end) -> stage words SW_LO ..
+static int upload_segment_bounds(rala_b200_multi* m, FabricRank& fr) {
+    std::vector<uint32_t>& h = fr.stage_host;
+    h.assign(SW_WORDS, 0u);
+    uint32_t local = 0;
+    for (uint32_t s = 0; s < m->n_seg; ++s) {
+        h[SW_LO + s] = local;
+        local += seg_at(m, m->seg, s, fr.rank);
+    }
+    h[SW_LO + m->n_seg] = local;
+    MCU(m, cudaMemcpyAsync(fr.stage.p, h.data(), SW_WORDS * 4, cudaMemcpyHostToDevice, fr.ctx->L.stream));
+    return RALA_B200_OK;
+}
+
+// after a staged barrier: wait for every local rank, then the counts every rank published in it (words per rank)
+static int read_seg_mail(rala_b200_multi* m, std::vector<uint32_t>& mail) {
+    int rc = rala_b200_multi_synchronize(m);
+    if (rc) return rc;
+    for (FabricRank& fr : m->ranks) {
+        FabricHdr h;
+        rc = read_hdr(m, fr, &h);
+        if (rc) return rc;
+        if (h.error & FE_TIMEOUT)
+            return mfail(m, RALA_B200_ERR_CUDA, "rank %d: rank %u did not reach barrier %u within %u ms", fr.rank, h.dead_peer, h.dead_epoch,
+                         m->barrier_timeout_ms);
+    }
+    FabricRank& fr = m->ranks[0];
+    uint32_t epoch = 0;
+    MCU(m, cudaMemcpy(&epoch, &fr.hdr()->epoch, 4, cudaMemcpyDeviceToHost));
+    mail.resize((size_t) m->world * kSegMail);
+    const uint32_t* src = fr.sec<uint32_t>(fr.A.seg_mail) + (size_t) (epoch & 1u) * kMaxRanks * kSegMail;
+    MCU(m, cudaMemcpy(mail.data(), src, mail.size() * 4, cudaMemcpyDeviceToHost));
+    return RALA_B200_OK;
+}
+
+static int staged_ready(rala_b200_multi* m, const char* what) {
+    if (!m->reserved || !m->connected) return mfail(m, RALA_B200_ERR_STATE, "%s: reserve (and connect) the exchange arenas first", what);
+    for (FabricRank& fr : m->ranks)
+        if (fr.g->state < 1) return mfail(m, RALA_B200_ERR_STATE, "%s: rank %d has no inputs", what, fr.rank);
+    return RALA_B200_OK;
+}
+
+// graph.cpp:443-518 (phases a - c of a step) with the hill counters of the first pass summed over the ranks
+extern "C" int rala_b200_multi_classify(rala_b200_multi* m) {
+    if (!m) return RALA_B200_ERR_ARG;
+    int rc = staged_ready(m, "classify");
+    if (rc) return rc;
+    drop_graphs(m);
+    m->staged = 0;
+    m->staged_edges = false;
+    const bool hills = m->n_hills > 0;
+    for (FabricRank& fr : m->ranks) {
+        MCU(m, cudaSetDevice(fr.device));
+        if (hills) MCU(m, cudaMemsetAsync(fr.sec<uint32_t>(fr.A.hills), 0, (size_t) m->n_hills * 4, fr.ctx->L.stream));   // before the events barrier
+        rc = phase_a_events(m, fr);
+        if (rc) return rc;
+    }
+    for (FabricRank& fr : m->ranks) {
+        MCU(m, cudaSetDevice(fr.device));
+        rc = resolve_owned_piles(m, fr, 0, hills);
+        if (rc) return rc;
+    }
+    for (FabricRank& fr : m->ranks) {
+        rc = phase_c_survivors(m, fr);
+        if (rc) return rc;
+        if (hills)
+            MCU(m, cudaMemcpyAsync(fr.g->hills.as<uint32_t>() + 3 * (size_t) m->n_hills, fr.sec<uint32_t>(fr.A.hills), (size_t) m->n_hills * 4,
+                                   cudaMemcpyDeviceToDevice, fr.ctx->L.stream));
+    }
+    rc = rala_b200_multi_synchronize(m);
+    if (rc) return rc;
+    FabricRank& fr = m->ranks[0];
+    std::vector<unsigned char> raw(sizeof(FabricHdr));
+    MCU(m, cudaMemcpy(raw.data(), fr.arena.p, sizeof(FabricHdr), cudaMemcpyDeviceToHost));
+    const FabricHdr* h = reinterpret_cast<const FabricHdr*>(raw.data());
+    if (h->error & FE_TIMEOUT) return mfail(m, RALA_B200_ERR_CUDA, "classify: a barrier timed out (rank %u, barrier %u)", h->dead_peer, h->dead_epoch);
+    const uint32_t par = h->epoch & 1u;
+    m->n_seg = 1;
+    m->seg.assign((size_t) kMaxSegs * m->world, 0u);
+    m->dov.assign((size_t) kMaxSegs * m->world, 0u);
+    m->inl.assign((size_t) m->world, 0u);
+    for (int q = 0; q < m->world; ++q) {
+        seg_at(m, m->seg, 0, q) = h->mail[par][q][M_NOVL];
+        m->inl[q] = h->mail[par][q][M_NINL];
+    }
+    m->staged = 2;
+    return RALA_B200_OK;
+}
+
+// one list pass on every local rank (graph.cpp:722-736 / 801-824): count what every segment keeps, run the pass, publish
+static int staged_list_pass(rala_b200_multi* m, bool promote, int* is_changed) {
+    const char* what = promote ? "retrim_promote" : "retrim";
+    if (is_changed) *is_changed = 0;
+    if (m->staged != 2) return mfail(m, RALA_B200_ERR_STATE, "%s: classify (rala_b200_multi_classify) first", what);
+    // the single session's rule for a pass against an unchanged table (identity: skipped); the flags are the same on every
+    // rank and in every process, which all made the same calls
+    const rala_b200_graph* g0 = m->ranks[0].g;
+    if (!g0->piles_dirty && g0->skip_clean_retrim && (!promote || !g0->promote_pending)) return RALA_B200_OK;
+    const uint32_t S = m->n_seg;
+    for (FabricRank& fr : m->ranks) {
+        MCU(m, cudaSetDevice(fr.device));
+        rala_b200_graph* g = fr.g;
+        Launch& L = fr.ctx->L;
+        int rc = upload_segment_bounds(m, fr);
+        if (rc) return rc;
+        MCU(m, cudaMemsetAsync(fr.stage_w(SW_BOX), 0, kSegMail * 4, L.stream));
+        launch_seg_count(L, g->ovl[g->ovl_cur].view, fr.stage_w(SW_LO), S, g->piles.as<uint2>(), kSegRetrim, fr.stage_w(SW_BOX));
+        MRC(m, fr, promote ? rala_b200_graph_retrim_promote(g, nullptr) : rala_b200_graph_retrim(g));
+        MCU(m, cudaMemcpyAsync(fr.stage_w(SW_BOX + S), g->cnt() + g->slot_ovl, 4, cudaMemcpyDeviceToDevice, L.stream));
+        MCU(m, cudaMemcpyAsync(fr.stage_w(SW_BOX + S + 1), g->cnt() + g->slot_inl, 4, cudaMemcpyDeviceToDevice, L.stream));
+        launch_seg_push(L, fr.P, fr.A, fr.stage_w(SW_BOX), S + 2);
+        launch_fabric_barrier(L, fr.P, no_mail(m));
+        MCU(m, cudaGetLastError());
+    }
+    std::vector<uint32_t> mail;
+    int rc = read_seg_mail(m, mail);
+    if (rc) return rc;
+    bool changed = false, promoted = false;
+    for (int q = 0; q < m->world; ++q) {
+        const uint32_t* box = mail.data() + (size_t) q * kSegMail;
+        uint64_t kept = 0, before = 0;
+        for (uint32_t s = 0; s < S; ++s) {
+            kept += box[s];
+            before += seg_at(m, m->seg, s, q);
+        }
+        changed = changed || kept != before;
+        promoted = promoted || box[S] != kept;
+    }
+    if (promoted && S == (uint32_t) kMaxSegs) {
+        m->staged = 0;
+        return mfail(m, RALA_B200_ERR_LIMIT, "%s: a pit round promoted overlaps after %d rounds that did: at most %d segments of `overlaps` "
+                     "(RALA_B200_MAX_SEGMENTS); the session's lists are void", what, kMaxSegs - 1, kMaxSegs);
+    }
+    for (int q = 0; q < m->world; ++q) {
+        const uint32_t* box = mail.data() + (size_t) q * kSegMail;
+        uint32_t kept = 0;
+        for (uint32_t s = 0; s < S; ++s) {
+            seg_at(m, m->seg, s, q) = box[s];
+            kept += box[s];
+        }
+        if (promoted) seg_at(m, m->seg, S, q) = box[S] - kept;   // a new segment only in a round where some rank promoted
+        m->inl[q] = box[S + 1];
+    }
+    if (promoted) m->n_seg = S + 1;
+    if (is_changed) *is_changed = changed ? 1 : 0;
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_multi_retrim(rala_b200_multi* m) { return m ? staged_list_pass(m, false, nullptr) : RALA_B200_ERR_ARG; }
+
+extern "C" int rala_b200_multi_retrim_promote(rala_b200_multi* m, int* is_changed) {
+    return m ? staged_list_pass(m, true, is_changed) : RALA_B200_ERR_ARG;
+}
+
+// graph.cpp:831-848 on the staged lists: the time of an entry is its global position in overlaps ++ internals, one base per
+// segment of `overlaps` (classify_final on the segment's part of the local list) and one for `internals`
+static int phase_d_staged(rala_b200_multi* m, FabricRank& fr) {
+    MCU(m, cudaSetDevice(fr.device));
+    rala_b200_graph* g = fr.g;
+    Launch& L = fr.ctx->L;
+    if (g->state != 2) return mfail(m, RALA_B200_ERR_STATE, "finish: rank %d is not classified", fr.rank);
+    std::vector<uint32_t>& h = fr.stage_host;
+    h.assign(SW_WORDS, 0u);
+    uint64_t before = 0;
+    uint32_t local = 0;
+    for (uint32_t s = 0; s < m->n_seg; ++s) {
+        h[SW_LO + s] = local;
+        for (int q = 0; q < m->world; ++q) {
+            const uint32_t n = seg_at(m, m->seg, s, q);
+            if (q == fr.rank) {
+                h[SW_FIN_N + s] = n;
+                h[SW_FIN_BASE + s] = (uint32_t) before;
+                local += n;
+            }
+            before += n;
+        }
+    }
+    h[SW_LO + m->n_seg] = local;
+    for (int q = 0; q < fr.rank; ++q) before += m->inl[q];
+    if (before + m->inl[fr.rank] >= (1ull << 31)) return mfail(m, RALA_B200_ERR_LIMIT, "finish: list positions must stay below 2^31");
+    h[SW_ZERO + 1] = (uint32_t) before;   // time base of the local `internals`
+    MCU(m, cudaMemcpyAsync(fr.stage.p, h.data(), SW_WORDS * 4, cudaMemcpyHostToDevice, L.stream));
+    MCU(m, begin_stage(g, ST_FINALIZE));
+    MCU(m, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, L.stream));
+    MCU(m, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, L.stream));
+    MCU(m, zero_counter(g, C_EV));
+    MCU(m, clear_victim_histogram(g));
+    MCU(m, cudaMemcpyAsync(g->cnt() + C_TBASE_INL, fr.stage_w(SW_ZERO + 1), 4, cudaMemcpyDeviceToDevice, L.stream));
+    g->final_time_base_slot = C_TBASE_INL;
+    const List ovl = g->ovl[g->ovl_cur].view;
+    for (uint32_t s = 0; s < m->n_seg; ++s) {
+        if (s && !h[SW_FIN_N + s]) continue;   // (segment 0's launch also types `internals`)
+        launch_classify_final(L, sub_list(ovl, h[SW_LO + s]), fr.stage_w(SW_FIN_N + s), fr.stage_w(SW_FIN_BASE + s), g->inl[g->inl_cur].view,
+                              s ? fr.stage_w(SW_ZERO) : g->cnt() + g->slot_inl, g->cnt() + C_TBASE_INL, g->cap, g->piles.as<uint2>(),
+                              g->events_view(), g->ev_cap, resolve_bufs(g).vcursor, g->cnt());
+    }
+    MCU(m, cudaGetLastError());
+    return route_and_meet(m, fr, 1);
+}
+
+// graph.cpp:867-877: the final lists (what edge creation reads), their per-segment counts and dovetails, published
+static int phase_final_lists(rala_b200_multi* m, FabricRank& fr) {
+    MCU(m, cudaSetDevice(fr.device));
+    rala_b200_graph* g = fr.g;
+    Launch& L = fr.ctx->L;
+    const uint32_t S = m->n_seg;
+    MCU(m, cudaMemsetAsync(fr.stage_w(SW_BOX), 0, kSegMail * 4, L.stream));
+    launch_seg_count(L, g->ovl[g->ovl_cur].view, fr.stage_w(SW_LO), S, g->piles.as<uint2>(), kSegFinal, fr.stage_w(SW_BOX));
+    launch_final_deaths(L, fr.P, fr.A, g->dbuf.as<uint32_t>());   // the k_list_pass<kFinalInt> filter reads them (C_DSEL = 0 here)
+    MRC(m, fr, materialize_final_lists(g));
+    MCU(m, cudaMemcpyAsync(fr.stage_w(SW_BOX + 2 * S), g->cnt() + g->slot_inl, 4, cudaMemcpyDeviceToDevice, L.stream));
+    launch_seg_push(L, fr.P, fr.A, fr.stage_w(SW_BOX), 2 * S + 1);
+    launch_fabric_barrier(L, fr.P, no_mail(m));
+    MCU(m, cudaGetLastError());
+    return RALA_B200_OK;
+}
+
+// graph.cpp:831-877, 552-632 and 1281-1318 on the staged lists; edge ids are positions among the final dovetails in
+// global list order, so a rank's edges are one run of ids per segment (rala_b200_multi_edge_runs)
+extern "C" int rala_b200_multi_finish(rala_b200_multi* m) {
+    if (!m) return RALA_B200_ERR_ARG;
+    if (m->staged != 2) return mfail(m, RALA_B200_ERR_STATE, "finish: classify (rala_b200_multi_classify) first");
+    int rc = staged_ready(m, "finish");
+    if (rc) return rc;
+    for (FabricRank& fr : m->ranks)
+        if ((rc = phase_d_staged(m, fr))) return rc;
+    for (FabricRank& fr : m->ranks)
+        if ((rc = phase_e_final_resolve(m, fr))) return rc;
+    for (FabricRank& fr : m->ranks)
+        if ((rc = phase_final_lists(m, fr))) return rc;
+    std::vector<uint32_t> mail;
+    if ((rc = read_seg_mail(m, mail))) return rc;
+    const uint32_t S = m->n_seg;
+    const int W = m->world;
+    for (int q = 0; q < W; ++q) {
+        const uint32_t* box = mail.data() + (size_t) q * kSegMail;
+        for (uint32_t s = 0; s < S; ++s) {
+            seg_at(m, m->seg, s, q) = box[s];
+            seg_at(m, m->dov, s, q) = box[S + s];
+        }
+        m->inl[q] = box[2 * S];
+    }
+    EdgeRuns& R = m->runs;
+    R.n_seg = S;
+    R.world = (uint32_t) W;
+    uint64_t g_id = 0;
+    std::vector<uint64_t> l_id((size_t) W, 0);
+    for (uint32_t s = 0; s < S; ++s)
+        for (int q = 0; q < W; ++q) {
+            const size_t i = (size_t) s * W + q;
+            R.gb[i] = (uint32_t) g_id;
+            R.lb[i] = (uint32_t) l_id[q];
+            g_id += 2ull * m->dov[i];
+            l_id[q] += 2ull * m->dov[i];
+        }
+    if (g_id >= (1ull << 31)) return mfail(m, RALA_B200_ERR_LIMIT, "finish: %llu edges (ids must stay below 2^31)", (unsigned long long) g_id);
+    for (FabricRank& fr : m->ranks) {
+        MCU(m, cudaSetDevice(fr.device));
+        MCU(m, cudaMemcpyAsync(fr.runs_dev(), &m->runs, sizeof(EdgeRuns), cudaMemcpyHostToDevice, fr.ctx->L.stream));
+    }
+    m->staged_edges = true;
+    static const PhaseFn kBuild[] = {phase_f_edges, phase_g_csr, phase_h_transitive, phase_i_marks};
+    for (PhaseFn phase : kBuild)
+        for (FabricRank& fr : m->ranks)
+            if ((rc = phase(m, fr))) return rc;
+    m->staged = 3;
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_multi_get_hill_coverage(rala_b200_multi* m, int k, uint32_t* cov_out) {
+    if (!m || k < 0 || k >= m->n_local) return RALA_B200_ERR_ARG;
+    if (m->staged < 2) return mfail(m, RALA_B200_ERR_STATE, "get_hill_coverage: classify (rala_b200_multi_classify) first");
+    FabricRank& fr = m->ranks[k];
+    MRC(m, fr, rala_b200_graph_get_hill_coverage(fr.g, cov_out));
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_multi_get_lists(rala_b200_multi* m, int k, rala_ovl_t* ovl_out, uint64_t* ovl_pos_out, rala_ovl_t* int_out,
+                                         uint64_t* int_pos_out, uint64_t* counts) {
+    if (!m || k < 0 || k >= m->n_local || !counts) return RALA_B200_ERR_ARG;
+    if (m->staged < 2) return mfail(m, RALA_B200_ERR_STATE, "get_lists: classify (rala_b200_multi_classify) first");
+    FabricRank& fr = m->ranks[k];
+    const int me = fr.rank;
+    uint64_t n_ovl = 0;
+    for (uint32_t s = 0; s < m->n_seg; ++s) n_ovl += seg_at(m, m->seg, s, me);
+    counts[0] = n_ovl;
+    counts[1] = m->inl[me];
+    if (ovl_out || int_out) {
+        rala_b200_counts_t c;
+        MRC(m, fr, rala_b200_graph_counts(fr.g, &c));
+        if (c.n_overlaps != counts[0] || c.n_internals != counts[1])
+            return mfail(m, RALA_B200_ERR_STATE, "get_lists: rank %d holds %llu / %llu entries, the segment table says %llu / %llu", me,
+                         (unsigned long long) c.n_overlaps, (unsigned long long) c.n_internals, (unsigned long long) counts[0],
+                         (unsigned long long) counts[1]);
+        MRC(m, fr, rala_b200_graph_get_lists(fr.g, ovl_out, int_out));
+    }
+    if (ovl_pos_out) {
+        uint64_t global = 0, j = 0;
+        for (uint32_t s = 0; s < m->n_seg; ++s)
+            for (int q = 0; q < m->world; ++q) {
+                const uint32_t n = seg_at(m, m->seg, s, q);
+                if (q == me)
+                    for (uint32_t i = 0; i < n; ++i) ovl_pos_out[j++] = global + i;
+                global += n;
+            }
+    }
+    if (int_pos_out) {
+        uint64_t base = 0;
+        for (int q = 0; q < me; ++q) base += m->inl[q];
+        for (uint32_t i = 0; i < m->inl[me]; ++i) int_pos_out[i] = base + i;
+    }
     return RALA_B200_OK;
 }

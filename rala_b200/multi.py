@@ -148,7 +148,8 @@ def _slack(n: int) -> int:
 
 class DistributedGraph:
     """Drives one ShardSession per rank through the phases, with the collectives in between.
-    Like the product path it runs the frozen-pile chain only (no hills, no host pile breaking between the passes).
+    It runs the frozen-pile chain only (no hills, no host pile breaking between the passes): the staged construct for
+    pile tables that change between the passes needs the peer-memory fabric (rala_b200_multi_classify .. finish).
     A pass never reads a count back to the host, so its results are valid only if check() says so."""
 
     def __init__(self, session, rank: int, world: int, group=None):
@@ -307,8 +308,10 @@ class FabricGraph:
         self.caps = None
 
     # ---- inputs (local) ---------------------------------------------------------------------------------------
-    def set_inputs(self, records, piles, flags, t0: int):
+    def set_inputs(self, records, piles, flags, t0: int, hills=None):
         self.M.set_piles(piles, flags)
+        if hills is not None:   # only the staged construct counts them
+            self.M.set_hills(hills)
         self.M.set_overlaps(0, records, t0)
         return self
 
@@ -365,6 +368,46 @@ class FabricGraph:
     def check(self) -> dict:
         """Synchronises; raises when the last step did not fit its buffers or rounds, or a peer went missing."""
         return self.M.counts()
+
+    # ---- staged construct (collective: every rank makes the same calls) ----------------------------------------
+    def connections(self):
+        """(a_id, b_id) of the whole `overlaps` list in the reference's order: every rank's entries with their global
+        positions, all-gathered (the host's pit loop needs the whole list, graph.cpp:740-744)."""
+        ovl, pos, _, _ = self.M.local_lists(0)
+        mine = np.concatenate([pos.astype(np.int64)[:, None], ovl[:, :2].astype(np.int64)], 1)
+        parts = [None] * self.world
+        dist.all_gather_object(parts, mine, group=self.group)
+        rows = np.concatenate(parts)
+        return np.ascontiguousarray(rows[np.argsort(rows[:, 0], kind="stable"), 1:].astype(np.uint32))
+
+    def construct(self, pile_ops=None):
+        """Graph::construct's hot half and remove_transitive_edges with the same `pile_ops` contract as
+        api.Graph.construct; every rank passes pile ops that compute the same answers from the same inputs.  Hill
+        counters and is_changed come replicated from the library; the only host exchange added is the all-gather of
+        the connection list.  Raises when the staged passes outgrew the exchange buffers plan() sized from a frozen step
+        (the results are then incomplete): connect() again with the capacities demand() reports."""
+        if self.caps is None:
+            self.plan()
+        M = self.M
+        M.classify()
+        if pile_ops is not None:
+            upd = pile_ops.break_over_chimeric_hills(M.hill_coverage(0))
+            if upd is not None:
+                M.set_piles(*upd)
+        M.retrim()
+        while True:
+            if pile_ops is not None:
+                upd = pile_ops.break_over_chimeric_pits(self.connections())
+                if upd is not None:
+                    M.set_piles(*upd)
+            if not M.retrim_promote():
+                break
+        M.finish().synchronize()
+        need, fits = M.demand()
+        if self._max_over_ranks([0 if fits else 1])[0]:
+            raise api.RalaB200Error(f"construct: the staged passes did not fit the exchange buffers (rank {self.rank} needs "
+                                    f"{need.tolist()}, has {self.caps.tolist()}): connect() with larger capacities")
+        return self
 
     def edges(self):
         return self.M.edge_range(0), self.M.edges(0), self.M.marked(0)
