@@ -108,6 +108,37 @@ int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes, uint64_t n
 int rala_b200_filter_duplicates(rala_b200_ctx* ctx, const uint32_t* a_id, const uint32_t* b_id, const uint32_t* length,
                                 uint64_t n, uint8_t* valid_out, float* device_ms);
 
+/* PAF text on the device (SURVEY.md 8(f) row 2): bioparser's PafParser (overlap.cpp:22-31 builds the records) and the
+ * name -> id lookup of Overlap::transmute (overlap.cpp:36-82 against Graph::initialize's name_to_id_).
+ * Reads: names = the read names back to back, read i = names[name_end[i-1], name_end[i]) (name_end[-1] = 0), id = i;
+ * read_len[i] = its sequence length.  A name listed twice is refused (RALA_B200_ERR_ARG): which of the two name_to_id_
+ * keeps is not pinned, so the library does not guess.
+ * Text contract (anything else is refused with RALA_B200_ERR_ARG and a message naming the 1-based line and column; the
+ * smallest offending line is reported): lines end in '\n' (the last one may lack it), fields are separated by tabs, at
+ * least 12 of them; columns 2, 3, 4, 7, 8, 9, 11 are plain decimal numbers below 2^32 (leading zeros allowed); columns
+ * 1 and 6 are the names, byte for byte; orientation = first byte of column 5 != '+'; columns 10, 12 and every extra
+ * column (minimap2 tags, CIGARs) are never read, so a '\r' before '\n' needs no handling.  An empty line, fewer than 12
+ * fields, a non-digit or a value >= 2^32 in a parsed column is refused.  Overlap::length() = column 11.
+ * The text crosses PCIe in chunks of RALA_B200_PAF_CHUNK_BYTES cut behind their last '\n' (a longer line is refused with
+ * RALA_B200_ERR_LIMIT); caller memory that is page-locked is uploaded in place, other memory through a pinned staging
+ * pair, and the upload of one chunk overlaps the parse of the one before.  Text beyond 4 GiB is fine; records < 2^31. */
+#define RALA_B200_PAF_CHUNK_BYTES (32u << 20)
+typedef struct {
+    uint64_t n_records;              /* lines = records, file order */
+    uint64_t n_unresolved;           /* records with a name that is not among the reads (INVALID) */
+    uint64_t n_length_mismatch;      /* records whose resolved name has a PAF length (column 2 or 7) other than read_len */
+    uint64_t first_length_mismatch;  /* index of the first of them; UINT64_MAX when there is none */
+    uint64_t n_bytes;                /* text bytes */
+    uint64_t n_chunks;               /* upload chunks the text took */
+} rala_b200_paf_stats_t;
+/* Stateless form, like rala_b200_filter_duplicates: parse + lookup, no duplicate filter.  cols_out holds 7 columns of cap
+ * words: a_id | INVALID << 31, b_id | orientation << 31, a_begin, a_end, b_begin, b_end, length (column 11).  An unresolved
+ * name has id 0x7FFFFFFF and sets INVALID (bit 31 of a_id).  Length mismatches are only counted.  device_ms (nullable)
+ * receives the kernel time of the line scan and the parse (name table and uploads excluded). */
+int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads,
+                        const char* text, uint64_t n_bytes, uint32_t* cols_out, uint64_t cap, rala_b200_paf_stats_t* stats,
+                        float* device_ms);
+
 /* ------------------------------------------------------------------------------------------------
  * Graph session: the drop-in for Graph::construct's hot loops and Graph::remove_transitive_edges.
  * Call order (what the patched Graph::construct does, INTEGRATION.md):
@@ -166,6 +197,18 @@ int rala_b200_graph_set_overlaps_packed(rala_b200_graph* g, const uint32_t* quer
                                         const uint32_t* b_id, const uint32_t* a_span, const uint32_t* b_span, uint64_t n);
 int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* piles, const uint8_t* flags /* nullable */,
                               uint32_t n_piles);
+/* The read names and lengths the PAF text is resolved against (name_to_id_ of Graph::initialize, graph.cpp:253-271, and
+ * the sequence lengths transmute checks, overlap.cpp:54-59, 73-78); once per session.  Layout and refusals as
+ * rala_b200_parse_paf.  The name table stays on the device. */
+int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads);
+/* PAF text in FILE ORDER -> the session's records, replacing the host parse and transmute of graph.cpp:443-451 and the
+ * records set_overlaps* would receive: the text is parsed as rala_b200_parse_paf does, the duplicate filter of
+ * Graph::initialize (graph.cpp:273-303, :340-361) runs on the parsed columns, and a record leaves INVALID when a name did
+ * not resolve or the filter drops it.  A record that stays valid while its PAF read length (column 2 or 7) differs from
+ * set_reads' length is refused (RALA_B200_ERR_ARG, naming its line): the reference exits on such a record when transmute
+ * reaches it (overlap.cpp:54-59, 73-78); the library is stricter and also refuses one whose pile is already dead.  After
+ * a refused call the session holds no records (classify needs a new set_overlaps*).  stats: nullable. */
+int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats);
 /* Optional: have build / transitive / run write their results STRAIGHT into caller memory the GPU can address
  * (cudaHostAlloc / cudaHostRegister'ed host memory, or device memory): the rala_edge_t rows (graph.cpp:576-632)
  * leave as soon as the edge list exists, on a forked stream beside the CSR build and the transitive pass, and the

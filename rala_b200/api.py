@@ -41,10 +41,51 @@ class Counts(C.Structure):
         return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
+class PafStats(C.Structure):
+    _fields_ = [("n_records", C.c_uint64), ("n_unresolved", C.c_uint64), ("n_length_mismatch", C.c_uint64),
+                ("first_length_mismatch", C.c_uint64), ("n_bytes", C.c_uint64), ("n_chunks", C.c_uint64)]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
+PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES
+
+
+def _text(text):
+    """PAF text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
+    if isinstance(text, (bytes, bytearray, memoryview)):
+        text = np.frombuffer(text, np.uint8)
+    if hasattr(text, "data_ptr"):
+        if not text.is_contiguous() or text.device.type != "cpu" or text.element_size() != 1:
+            raise RalaB200Error("PAF text must be a contiguous uint8 CPU tensor")
+        return text, int(text.numel())
+    text = np.ascontiguousarray(text, dtype=np.uint8).reshape(-1)
+    return text, int(text.shape[0])
+
+
+def _names(names, read_len):
+    """Read names as a list of bytes, or as (blob, name_end) -> (blob uint8, name_end uint64, read_len uint32)."""
+    if isinstance(names, tuple):
+        blob, ends = names
+        blob = np.frombuffer(bytes(blob), np.uint8) if isinstance(blob, (bytes, bytearray)) else np.ascontiguousarray(blob, np.uint8)
+        ends = np.ascontiguousarray(ends, np.uint64)
+    else:
+        blob = np.frombuffer(b"".join(names), np.uint8)
+        ends = np.cumsum(np.fromiter((len(n) for n in names), np.uint64, len(names)), dtype=np.uint64)
+    rl = np.ascontiguousarray(read_len, np.uint32)
+    if rl.shape[0] != ends.shape[0]:
+        raise RalaB200Error("one read length per read name")
+    if blob.size == 0:
+        blob = np.zeros(1, np.uint8)
+    return blob, ends, rl
+
+
 EXPORTS = [
     "rala_b200_abi_version", "rala_b200_create", "rala_b200_destroy", "rala_b200_last_error",
     "rala_b200_launch_count", "rala_b200_event_record", "rala_b200_event_elapsed_ms", "rala_b200_synchronize",
     "rala_b200_trim_classify", "rala_b200_transitive_reduce", "rala_b200_filter_duplicates",
+    "rala_b200_parse_paf", "rala_b200_graph_set_reads", "rala_b200_graph_set_overlaps_paf",
     "rala_b200_graph_create", "rala_b200_graph_destroy", "rala_b200_graph_set_overlaps",
     "rala_b200_graph_set_piles", "rala_b200_graph_set_hills", "rala_b200_graph_classify",
     "rala_b200_graph_retrim", "rala_b200_graph_retrim_promote", "rala_b200_graph_finalize",
@@ -263,6 +304,20 @@ class Context:
                                                         _ptr(valid), C.byref(ms)), "filter_duplicates")
         return (valid, float(ms.value)) if with_time else valid
 
+    def parse_paf(self, text, names, read_len, with_time: bool = False):
+        """PAF text -> (columns (7, n) uint32: a_id | invalid << 31, b_id | orientation << 31, a_begin, a_end, b_begin,
+        b_end, length (column 11); stats dict) with the reads' names resolved on the device (no duplicate filter)."""
+        buf, n_bytes = _text(text)
+        blob, ends, rl = _names(names, read_len)
+        cap = n_bytes // 19 + 2
+        cols = np.zeros((7, cap), dtype=np.uint32)
+        st, ms = PafStats(), C.c_float(0.0)
+        self.check(self.lib.rala_b200_parse_paf(self.handle, _ptr(blob), _ptr(ends), _ptr(rl), C.c_uint32(ends.shape[0]), _ptr(buf),
+                                                C.c_uint64(n_bytes), _ptr(cols), C.c_uint64(cap), C.byref(st), C.byref(ms)), "parse_paf")
+        stats = st.as_dict()
+        out = np.ascontiguousarray(cols[:, :stats["n_records"]])
+        return (out, stats, float(ms.value)) if with_time else (out, stats)
+
 
 class Graph:
     """Host-side mirror of rala::Graph for the hot path (graph.hpp:37-60).
@@ -325,6 +380,20 @@ class Graph:
         self._call("rala_b200_graph_set_overlaps_packed", _ptr(p.query_id), _ptr(p.group_end), C.c_uint32(int(p.query_id.shape[0])),
                    _ptr(p.b_id), _ptr(p.a_span), _ptr(p.b_span), C.c_uint64(p.n))
         return self
+
+    def set_reads(self, names, read_len):
+        """Read names (list of bytes, or (blob, name_end)) and sequence lengths the PAF text is resolved against."""
+        blob, ends, rl = _names(names, read_len)
+        self._call("rala_b200_graph_set_reads", _ptr(blob), _ptr(ends), _ptr(rl), C.c_uint32(ends.shape[0]))
+        return self
+
+    def set_overlaps_paf(self, text) -> dict:
+        """PAF text in file order -> the session's records (parse, name lookup, duplicate filter on the device); returns
+        the stats (records, unresolved names, read-length mismatches, bytes, upload chunks)."""
+        buf, n_bytes = _text(text)
+        st = PafStats()
+        self._call("rala_b200_graph_set_overlaps_paf", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
+        return st.as_dict()
 
     def set_outputs(self, edges_out=None, marked_out=None):
         """Pinned host (or device-visible) buffers the run writes its edge rows and marks into directly."""

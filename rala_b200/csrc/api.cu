@@ -37,6 +37,7 @@ extern "C" int rala_b200_create(rala_b200_ctx** out, int device) {
     preload_transitive();
     preload_fabric();
     preload_frontend();
+    preload_paf();
     cudaGetLastError();
     cudaEventCreate(&ctx->ev[0]);
     cudaEventCreate(&ctx->ev[1]);
@@ -178,6 +179,7 @@ extern "C" void rala_b200_graph_destroy(rala_b200_graph* g) {
     cudaSetDevice(g->ctx->device);
     cudaStreamSynchronize(g->ctx->L.stream);
     drop_run_graphs(g);
+    destroy_paf_reader(g->paf);
     DevBuf* bufs[] = {&g->rec, &g->recs.buf, &g->alive_bits, &g->piles, &g->piles_raw, &g->pile_flags_raw, &g->piles_initial, &g->hills, &g->ovl[0].buf,
                       &g->ovl[1].buf, &g->inl[0].buf, &g->inl[1].buf, &g->events, &g->hill_rec, &g->dbuf, &g->flags, &g->segs, &g->tiles,
                       &g->counters, &g->scan_pool, &g->seq_to_node, &g->edges, &g->row_ptr, &g->cursor, &g->col,
@@ -228,7 +230,7 @@ static int reserve_scan_pool(rala_b200_graph* g) {
 
 // device lists sized for n records (worst case every record survives; the scratch lists of the survivors pass are
 // indexed by record position)
-static int reserve_for_records(rala_b200_graph* g, uint64_t n) {
+int reserve_for_records(rala_b200_graph* g, uint64_t n) {
     rala_b200_ctx* ctx = g->ctx;
     g->n_rec = (uint32_t) n;
     CU(ctx, g->recs.reserve((uint32_t) ((n + 3) / 4 * 4 + 4)));

@@ -1,0 +1,551 @@
+// paf.cu — PAF text in host memory -> the graph session's device-resident records (SURVEY.md 8(f) row 2): the parse of
+// bioparser's PafParser (graph.cpp:443-451 runs it once more for every construct pass) and the name -> id lookup of
+// Overlap::transmute (overlap.cpp:36-82) on the device, followed by the front end's duplicate filter (frontend.cu).
+//
+//   names once per session:  k_paf_names        open-addressing table of the read names (64-bit hash; a hit is confirmed
+//                                                against the name bytes, so a hash collision never resolves to a wrong id)
+//   per upload chunk:        k_paf_line_ends    '\n' per tile (16-byte loads), decoupled look-back, one line end per record
+//                            k_paf_parse        one warp per line: tab positions by ballot, lane f parses field f
+//   per call (session):      k_filter_duplicates, k_paf_fold   is_valid_overlap_ folded into the INVALID bit
+//
+// Input contract (the library refuses what it cannot map onto the reference's reading without guessing): tab-separated,
+// at least 12 fields; columns 2, 3, 4, 7, 8, 9, 11 plain decimal below 2^32; orientation = first byte of column 5 != '+';
+// names are the exact bytes of columns 1 and 6; columns 10, 12 and every extra column are never read.
+#include <cstring>
+
+#include "kernels.h"
+#include "session.h"
+
+namespace rb {
+
+constexpr uint32_t kPafChunk = RALA_B200_PAF_CHUNK_BYTES;
+constexpr int kScanItems = 4;                                          // 16-byte loads per thread and tile
+constexpr uint32_t kScanTile = kTileThreads * 16u * kScanItems;        // 16 KiB of text per tile
+constexpr uint32_t kPafPad = kScanTile + 256;                          // readable bytes behind a chunk (whole tiles, line words)
+constexpr uint32_t kUnknownId = 0x7FFFFFFFu;                           // a name that is not in the table
+constexpr uint32_t kMinLine = 19;                                      // 11 tabs + 7 digits + '\n': no valid line is shorter
+enum : uint32_t { kErrFields = 1, kErrEmpty = 2, kErrDigit = 3, kErrOverflow = 4 };
+// device words of one call: the first four start at ~0 (minima), the rest at 0; line bases of the chunks follow
+enum { W_ERR = 0, W_DUP, W_FIRST_MISMATCH, W_FIRST_BAD, W_UNRESOLVED, W_MISMATCH, W_BASES = 8 };
+
+struct NameTable {
+    const uint8_t* blob;
+    const unsigned long long* end;   // name i = blob[end[i-1], end[i])
+    const uint32_t* read_len;
+    unsigned long long* slots;       // hash >> 32 << 32 | id, ~0 = empty
+    uint32_t mask;
+};
+
+struct PafCols {
+    uint32_t *a, *b, *ab, *ae, *bb, *be, *len;
+    uint8_t* mismatch;
+};
+
+__device__ __forceinline__ unsigned long long name_hash(const uint8_t* p, uint32_t n) {
+    unsigned long long h = 0xcbf29ce484222325ull;   // FNV-1a, then the murmur3 finaliser for the slot bits
+    for (uint32_t i = 0; i < n; ++i) h = (h ^ p[i]) * 0x100000001b3ull;
+    h ^= h >> 33; h *= 0xff51afd7ed558ccdull;
+    h ^= h >> 33; h *= 0xc4ceb9fe1a85ec53ull;
+    return h ^ (h >> 33);
+}
+
+__device__ __forceinline__ bool same_bytes(const uint8_t* a, const uint8_t* b, uint32_t n) {
+    for (uint32_t i = 0; i < n; ++i)
+        if (a[i] != b[i]) return false;
+    return true;
+}
+
+__device__ __forceinline__ uint32_t name_lookup(const NameTable& t, const uint8_t* p, uint32_t n) {
+    const unsigned long long h = name_hash(p, n);
+    const uint32_t tag = (uint32_t) (h >> 32);
+    for (uint32_t s = (uint32_t) h & t.mask;; s = (s + 1) & t.mask) {   // the table is at most half full
+        const unsigned long long e = __ldg(t.slots + s);
+        if (e == ~0ull) return kUnknownId;
+        if ((uint32_t) (e >> 32) == tag) {
+            const uint32_t id = (uint32_t) e;
+            const unsigned long long b0 = id ? __ldg(t.end + id - 1) : 0ull, b1 = __ldg(t.end + id);
+            if (b1 - b0 == n && same_bytes(t.blob + b0, p, n)) return id;
+        }
+    }
+}
+
+// One thread per read name.  Two equal names take the same probe sequence, so whichever claims a slot first is seen by
+// the other: every duplicate is found, and the smallest (later id, earlier id) pair is reported.
+__global__ void __launch_bounds__(256) k_paf_names(NameTable t, uint32_t n, unsigned long long* __restrict__ dup) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const unsigned long long b0 = i ? t.end[i - 1] : 0ull;
+        const uint32_t len = (uint32_t) (t.end[i] - b0);
+        const unsigned long long h = name_hash(t.blob + b0, len);
+        const unsigned long long mine = (h >> 32 << 32) | i;
+        for (uint32_t s = (uint32_t) h & t.mask;; s = (s + 1) & t.mask) {
+            const unsigned long long old = atomicCAS(t.slots + s, ~0ull, mine);
+            if (old == ~0ull) break;
+            if ((old >> 32) != (h >> 32)) continue;
+            const uint32_t id = (uint32_t) old;
+            const unsigned long long c0 = id ? t.end[id - 1] : 0ull;
+            if (t.end[id] - c0 == len && same_bytes(t.blob + c0, t.blob + b0, len)) {
+                atomicMin(dup, (unsigned long long) max(i, id) << 32 | min(i, id));
+                break;
+            }
+        }
+    }
+}
+
+// '\n' positions of one chunk in order.  Item r of thread t covers bytes [r * 4096 + t * 16, +16) of the tile (a warp
+// reads 512 contiguous bytes per load); the 32 (item, warp) counts are scanned by one warp, the tile prefix comes from
+// the decoupled look-back of common.cuh.  The last tile writes the running line count behind this chunk.
+__global__ void __launch_bounds__(kTileThreads) k_paf_line_ends(const uint8_t* __restrict__ text, uint32_t len,
+                                                               uint32_t* __restrict__ line_end, unsigned long long* __restrict__ status,
+                                                               uint32_t* __restrict__ ticket, unsigned long long* __restrict__ bases,
+                                                               uint32_t chunk) {
+    static_assert(kScanItems * kTileWarps == 32, "one warp scans the partial counts");
+    __shared__ uint32_t s_cnt[kScanItems * kTileWarps];
+    __shared__ uint32_t s_tile;
+    const uint32_t tid = threadIdx.x, lane = lane_id(), warp = warp_id();
+    const uint32_t num_tiles = (len + kScanTile - 1) / kScanTile;
+    while (true) {
+        if (tid == 0) s_tile = atomicAdd(ticket, 1u);
+        __syncthreads();
+        const uint32_t tile = s_tile;
+        if (tile >= num_tiles) break;
+        uint32_t nl[kScanItems], pre[kScanItems];
+#pragma unroll
+        for (int r = 0; r < kScanItems; ++r) {
+            const uint32_t off = tile * kScanTile + r * (kTileThreads * 16u) + tid * 16u;
+            const uint4 q = *reinterpret_cast<const uint4*>(text + off);
+            const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+            uint32_t m = 0;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const uint32_t x = w[j] ^ 0x0A0A0A0Au;   // zero byte <=> '\n' (exact per byte: no borrow between bytes)
+                const uint32_t z = ~(((x & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | x) & 0x80808080u;
+                m |= (((z >> 7) & 1u) | ((z >> 14) & 2u) | ((z >> 21) & 4u) | ((z >> 28) & 8u)) << (4 * j);
+            }
+            if (off + 16u > len) m &= off < len ? (1u << (len - off)) - 1u : 0u;
+            nl[r] = m;
+            const uint32_t c = __popc(m), inc = warp_inclusive_scan(c);
+            pre[r] = inc - c;
+            if (lane == 31) s_cnt[r * kTileWarps + warp] = inc;
+        }
+        __syncthreads();
+        if (warp == 0) {
+            const uint32_t c = s_cnt[lane], inc = warp_inclusive_scan(c);
+            const uint32_t total = __shfl_sync(0xFFFFFFFFu, inc, 31);
+            const unsigned long long excl = lookback_exclusive(status, tile, total);
+            s_cnt[lane] = (uint32_t) excl + inc - c;
+            if (tile == num_tiles - 1 && lane == 0) bases[chunk + 1] = bases[chunk] + excl + total;
+        }
+        __syncthreads();
+#pragma unroll
+        for (int r = 0; r < kScanItems; ++r) {
+            const uint32_t off = tile * kScanTile + r * (kTileThreads * 16u) + tid * 16u;
+            uint32_t pos = s_cnt[r * kTileWarps + warp] + pre[r], m = nl[r];
+            while (m) {
+                line_end[pos++] = off + (uint32_t) (__ffs(m) - 1);
+                m &= m - 1;
+            }
+        }
+        __syncthreads();
+    }
+}
+
+// One warp per line.  128 bytes per step (a 4-byte word per lane), tabs found by ballot and ranked by a warp scan; the
+// walk stops at the 11th tab, so tags behind column 12 (CIGARs of tens of KB) are never read.  Then lane f parses field f.
+// Record index = global line index (file order).  A refused line lowers the error word: (line << 8) | kind << 4 | column.
+__global__ void __launch_bounds__(256) k_paf_parse(const uint8_t* __restrict__ text, const uint32_t* __restrict__ line_end,
+                                                   const unsigned long long* __restrict__ bases, uint32_t chunk, NameTable t,
+                                                   PafCols out, unsigned long long rec_cap, unsigned long long* __restrict__ words) {
+    __shared__ uint32_t s_tab[kTileWarps][11];
+    const unsigned long long base = bases[chunk];
+    const uint32_t n_lines = (uint32_t) (bases[chunk + 1] - base);
+    const uint32_t lane = lane_id(), warp = warp_id();
+    for (uint32_t line = blockIdx.x * kTileWarps + warp; line < n_lines; line += gridDim.x * kTileWarps) {
+        const uint32_t s = line ? line_end[line - 1] + 1u : 0u, e = line_end[line];
+        uint32_t ntab = 0;
+        __syncwarp();
+        for (uint32_t w = s & ~3u; w < e && ntab < 11u; w += 128u) {
+            const uint32_t p0 = w + 4u * lane;
+            const uint32_t word = *reinterpret_cast<const uint32_t*>(text + p0);
+            uint32_t m = 0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                m |= ((((word >> (8 * k)) & 0xFFu) == '\t') & (p0 + k >= s) & (p0 + k < e) ? 1u : 0u) << k;
+            const uint32_t c = __popc(m), inc = warp_inclusive_scan(c);
+            for (uint32_t r = ntab + inc - c; m && r < 11u; ++r, m &= m - 1) s_tab[warp][r] = p0 + (uint32_t) (__ffs(m) - 1);
+            ntab += __shfl_sync(0xFFFFFFFFu, inc, 31);
+        }
+        __syncwarp();
+        uint32_t err = 0, val = 0;
+        if (e == s) {
+            err = kErrEmpty << 4 | 1u;
+        } else if (ntab < 11u) {
+            err = kErrFields << 4 | (ntab + 1u);   // fields found
+        } else if (lane < 11u) {
+            const uint32_t fb = lane ? s_tab[warp][lane - 1] + 1u : s, fe = s_tab[warp][lane];
+            if (lane == 0 || lane == 5) {
+                val = name_lookup(t, text + fb, fe - fb);
+            } else if (lane == 4) {
+                val = text[fb] != '+';   // fb == fe: the tab itself
+            } else if (lane != 9) {
+                unsigned long long v = 0;
+                if (fb == fe) err = kErrDigit << 4 | (lane + 1u);
+                for (uint32_t p = fb; p < fe; ++p) {
+                    const uint32_t d = (uint32_t) text[p] - '0';
+                    if (d > 9u) { err = kErrDigit << 4 | (lane + 1u); break; }
+                    v = v * 10u + d;
+                    if (v > 0xFFFFFFFFull) { err = kErrOverflow << 4 | (lane + 1u); break; }
+                }
+                val = (uint32_t) v;
+            }
+        }
+        const unsigned long long gline = base + line;
+        const uint32_t bad = __ballot_sync(0xFFFFFFFFu, err != 0u);
+        if (bad) {
+            const uint32_t code = __shfl_sync(0xFFFFFFFFu, err, __ffs(bad) - 1);
+            if (lane == 0) atomicMin(words + W_ERR, gline << 8 | code);
+            continue;
+        }
+        const uint32_t a = __shfl_sync(0xFFFFFFFFu, val, 0), a_len = __shfl_sync(0xFFFFFFFFu, val, 1);
+        const uint32_t ab = __shfl_sync(0xFFFFFFFFu, val, 2), ae = __shfl_sync(0xFFFFFFFFu, val, 3);
+        const uint32_t ori = __shfl_sync(0xFFFFFFFFu, val, 4), b = __shfl_sync(0xFFFFFFFFu, val, 5);
+        const uint32_t b_len = __shfl_sync(0xFFFFFFFFu, val, 6), bb = __shfl_sync(0xFFFFFFFFu, val, 7);
+        const uint32_t be = __shfl_sync(0xFFFFFFFFu, val, 8), length = __shfl_sync(0xFFFFFFFFu, val, 10);
+        if (lane == 0) {
+            const bool ka = a != kUnknownId, kb = b != kUnknownId;
+            const bool mism = (ka && a_len != __ldg(t.read_len + a)) || (kb && b_len != __ldg(t.read_len + b));
+            if (!(ka && kb)) atomicAdd(words + W_UNRESOLVED, 1ull);
+            if (mism) {
+                atomicAdd(words + W_MISMATCH, 1ull);
+                atomicMin(words + W_FIRST_MISMATCH, gline);
+            }
+            if (gline < rec_cap) {
+                out.a[gline] = a | (ka && kb ? 0u : kInvalidBit);
+                out.b[gline] = b | ori << 31;
+                out.ab[gline] = ab;
+                out.ae[gline] = ae;
+                out.bb[gline] = bb;
+                out.be[gline] = be;
+                out.len[gline] = length;
+                out.mismatch[gline] = mism ? 1 : 0;
+            }
+        }
+    }
+}
+
+// is_valid_overlap_ into the INVALID bit while the parsed columns move to the session's records; a record that stays
+// valid with a read length the caller's reads contradict lowers W_FIRST_BAD (transmute would exit on it)
+__global__ void __launch_bounds__(256) k_paf_fold(PafCols in, const uint8_t* __restrict__ valid, uint32_t n, List recs,
+                                                  unsigned long long* __restrict__ words) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const bool v = valid[i] != 0;
+        recs.a[i] = in.a[i] | (v ? 0u : kInvalidBit);
+        recs.b[i] = in.b[i];
+        recs.ab[i] = in.ab[i];
+        recs.ae[i] = in.ae[i];
+        recs.bb[i] = in.bb[i];
+        recs.be[i] = in.be[i];
+        if (v && in.mismatch[i]) atomicMin(words + W_FIRST_BAD, (unsigned long long) i);
+    }
+}
+
+void preload_paf() {
+    cudaFuncAttributes a;
+    cudaFuncGetAttributes(&a, k_paf_names);
+    cudaFuncGetAttributes(&a, k_paf_line_ends);
+    cudaFuncGetAttributes(&a, k_paf_parse);
+    cudaFuncGetAttributes(&a, k_paf_fold);
+}
+
+}  // namespace rb
+
+// ---------------------------------------------------------------------------------------------
+// host side: the name table, the chunked upload and the call's bookkeeping
+// ---------------------------------------------------------------------------------------------
+struct PafReader {
+    DevBuf names;                 // blob | ends | read lengths | table slots
+    NameTable table{};
+    uint32_t n_reads = 0;
+    bool have_names = false;
+    DevBuf text[2];               // device side of the staging pair
+    DevBuf line_end, status, words, cols, valid;
+    char* pinned[2] = {nullptr, nullptr};
+    cudaStream_t copy = nullptr;  // uploads: chunk k + 1 crosses PCIe while chunk k is parsed
+    cudaEvent_t copied[2]{}, parsed[2]{};
+    std::vector<cudaEvent_t> timing;   // (start, stop) around the kernels of every chunk
+    unsigned long long rec_cap = 0;
+    std::vector<unsigned long long> w;   // the words of the last call, read back
+
+    PafCols view() const {
+        const size_t col = align_up((size_t) rec_cap * 4, 256);
+        char* b = cols.as<char>();
+        return PafCols{(uint32_t*) b, (uint32_t*) (b + col), (uint32_t*) (b + 2 * col), (uint32_t*) (b + 3 * col),
+                       (uint32_t*) (b + 4 * col), (uint32_t*) (b + 5 * col), (uint32_t*) (b + 6 * col), (uint8_t*) (b + 7 * col)};
+    }
+    ~PafReader() {
+        if (copy) cudaStreamSynchronize(copy);
+        DevBuf* bufs[] = {&names, &text[0], &text[1], &line_end, &status, &words, &cols, &valid};
+        for (DevBuf* b : bufs) b->release();
+        for (int k = 0; k < 2; ++k) {
+            if (pinned[k]) cudaFreeHost(pinned[k]);
+            if (copied[k]) cudaEventDestroy(copied[k]);
+            if (parsed[k]) cudaEventDestroy(parsed[k]);
+        }
+        for (cudaEvent_t e : timing) cudaEventDestroy(e);
+        if (copy) cudaStreamDestroy(copy);
+    }
+};
+
+void destroy_paf_reader(PafReader* r) { delete r; }
+
+static int paf_set_names(rala_b200_ctx* ctx, PafReader& R, const char* names, const uint64_t* name_end, const uint32_t* read_len,
+                         uint32_t n_reads) {
+    R.have_names = false;
+    if (n_reads && (!name_end || !read_len)) return fail(ctx, RALA_B200_ERR_ARG, "set_reads: name ends and read lengths are needed");
+    if (n_reads >= (1u << 31)) return fail(ctx, RALA_B200_ERR_LIMIT, "too many reads (%u >= 2^31)", n_reads);
+    uint64_t prev = 0;
+    for (uint32_t i = 0; i < n_reads; ++i) {
+        if (name_end[i] < prev || name_end[i] - prev >= (1ull << 32))
+            return fail(ctx, RALA_B200_ERR_ARG, "set_reads: name %u ends at %llu, before its start %llu (or is 4 GiB long)", i,
+                        (unsigned long long) name_end[i], (unsigned long long) prev);
+        prev = name_end[i];
+    }
+    const uint64_t blob = n_reads ? name_end[n_reads - 1] : 0;
+    if (blob && !names) return fail(ctx, RALA_B200_ERR_ARG, "set_reads: names are missing");
+    uint32_t slots = 1024;
+    while (slots < 2ull * n_reads) slots <<= 1;
+    const size_t o_end = align_up(blob + 1, 256), o_len = o_end + align_up((size_t) n_reads * 8 + 8, 256),
+                 o_slots = o_len + align_up((size_t) n_reads * 4 + 4, 256), bytes = o_slots + (size_t) slots * 8;
+    CU(ctx, cudaSetDevice(ctx->device));
+    CU(ctx, R.names.reserve(bytes));
+    CU(ctx, R.words.reserve(256));
+    char* b = R.names.as<char>();
+    cudaStream_t s = ctx->L.stream;
+    if (blob) CU(ctx, cudaMemcpyAsync(b, names, blob, cudaMemcpyHostToDevice, s));
+    if (n_reads) {
+        CU(ctx, cudaMemcpyAsync(b + o_end, name_end, (size_t) n_reads * 8, cudaMemcpyHostToDevice, s));
+        CU(ctx, cudaMemcpyAsync(b + o_len, read_len, (size_t) n_reads * 4, cudaMemcpyHostToDevice, s));
+    }
+    CU(ctx, cudaMemsetAsync(b + o_slots, 0xFF, (size_t) slots * 8, s));
+    CU(ctx, cudaMemsetAsync(R.words.p, 0xFF, 8 * (W_DUP + 1), s));
+    R.table = NameTable{(const uint8_t*) b, (const unsigned long long*) (b + o_end), (const uint32_t*) (b + o_len),
+                        (unsigned long long*) (b + o_slots), slots - 1};
+    if (n_reads) {
+        k_paf_names<<<grid_for(n_reads, 256, kNumSMs * 8), 256, 0, s>>>(R.table, n_reads, R.words.as<unsigned long long>() + W_DUP);
+        ctx->L.count++;
+        CU(ctx, cudaGetLastError());
+    }
+    unsigned long long dup = ~0ull;
+    CU(ctx, cudaMemcpyAsync(&dup, R.words.as<unsigned long long>() + W_DUP, 8, cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaStreamSynchronize(s));
+    if (dup != ~0ull)
+        return fail(ctx, RALA_B200_ERR_ARG, "set_reads: reads %u and %u have the same name (which one name_to_id_ keeps is not pinned)",
+                    (unsigned) dup, (unsigned) (dup >> 32));
+    R.n_reads = n_reads;
+    R.have_names = true;
+    return RALA_B200_OK;
+}
+
+static const char* paf_error_text(uint32_t kind) {
+    switch (kind) {
+        case kErrFields: return "has fewer than 12 tab-separated fields (fields found: column number)";
+        case kErrEmpty: return "is empty";
+        case kErrDigit: return "is not a plain decimal number";
+        default: return "does not fit 32 bits";
+    }
+}
+
+// Parses the whole text into R.cols (record index = line index, file order).  *n_out = records; kernel_ms (nullable) = device
+// time of the chunks' kernels (line scan + parse), uploads excluded.
+static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* st,
+                            float* kernel_ms, uint64_t* n_out) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->L.stream;
+    // no valid line is shorter than kMinLine bytes (the last one may lack its '\n'): more lines than that means a refusal
+    R.rec_cap = (n_bytes + 1) / kMinLine + 1;
+    if (R.rec_cap > (1ull << 31)) R.rec_cap = 1ull << 31;
+    const size_t col = align_up((size_t) R.rec_cap * 4, 256);
+    CU(ctx, R.cols.reserve(7 * col + align_up((size_t) R.rec_cap, 256)));
+    const uint64_t max_chunks = n_bytes ? 2 * (n_bytes / kPafChunk) + 2 : 0;   // two consecutive chunks span >= one chunk size
+    CU(ctx, R.words.reserve((W_BASES + max_chunks + 2) * 8));
+    CU(ctx, R.line_end.reserve(((size_t) kPafChunk + 2) * 4));
+    const size_t status_words = tiles_of((uint64_t) kPafChunk + 1) + 1;
+    CU(ctx, R.status.reserve(status_words * 8));
+    for (int k = 0; k < 2; ++k) {
+        CU(ctx, R.text[k].reserve((size_t) kPafChunk + 1 + kPafPad));
+        if (!R.copied[k]) CU(ctx, cudaEventCreateWithFlags(&R.copied[k], cudaEventDisableTiming));
+        if (!R.parsed[k]) CU(ctx, cudaEventCreateWithFlags(&R.parsed[k], cudaEventDisableTiming));
+    }
+    if (!R.copy) CU(ctx, cudaStreamCreateWithFlags(&R.copy, cudaStreamNonBlocking));
+    while (R.timing.size() < 2 * max_chunks) {
+        cudaEvent_t e;
+        CU(ctx, cudaEventCreate(&e));
+        R.timing.push_back(e);
+    }
+    // caller memory that is page-locked is uploaded in place; anything else goes through the pinned staging pair
+    bool direct = false;
+    if (n_bytes) {
+        cudaPointerAttributes attr;
+        if (cudaPointerGetAttributes(&attr, text) == cudaSuccess) direct = attr.type == cudaMemoryTypeHost;
+        cudaGetLastError();
+    }
+    for (int k = 0; !direct && n_bytes && k < 2; ++k)
+        if (!R.pinned[k]) CU(ctx, cudaHostAlloc((void**) &R.pinned[k], kPafChunk + 1, cudaHostAllocDefault));
+    unsigned long long* words = R.words.as<unsigned long long>();
+    CU(ctx, cudaMemsetAsync(words, 0xFF, 8 * W_UNRESOLVED, s));
+    CU(ctx, cudaMemsetAsync(words + W_UNRESOLVED, 0, 8 * (W_BASES + 1 - W_UNRESOLVED), s));
+    CU(ctx, cudaStreamSynchronize(s));   // the copy stream starts from settled words and buffers
+    const PafCols out = R.view();
+    uint64_t pos = 0;
+    uint32_t k = 0;
+    for (; pos < n_bytes; ++k) {
+        if (k >= max_chunks) return fail(ctx, RALA_B200_ERR_LIMIT, "PAF text: more upload chunks than planned");
+        uint64_t len = n_bytes - pos < kPafChunk ? n_bytes - pos : kPafChunk;
+        const bool last = pos + len == n_bytes;
+        if (!last) {   // cut behind the last '\n' of the window; the tail goes with the next chunk
+            const void* nl = memrchr(text + pos, '\n', len);
+            if (!nl) {
+                unsigned long long lines = 0;
+                CU(ctx, cudaStreamSynchronize(R.copy));
+                CU(ctx, cudaMemcpyAsync(&lines, words + W_BASES + k, 8, cudaMemcpyDeviceToHost, s));
+                CU(ctx, cudaStreamSynchronize(s));
+                return fail(ctx, RALA_B200_ERR_LIMIT, "PAF line %llu is longer than the upload chunk (%u bytes)", lines + 1, kPafChunk);
+            }
+            len = (uint64_t) ((const char*) nl - (text + pos)) + 1;
+        }
+        const int slot = k & 1;
+        const char* src = text + pos;
+        if (!direct) {
+            if (k >= 2) CU(ctx, cudaEventSynchronize(R.copied[slot]));   // the upload of chunk k - 2 has left the buffer
+            memcpy(R.pinned[slot], src, len);
+            src = R.pinned[slot];
+        }
+        if (k >= 2) CU(ctx, cudaStreamWaitEvent(R.copy, R.parsed[slot], 0));   // chunk k - 2 is parsed: its device buffer is free
+        char* dtext = R.text[slot].as<char>();
+        CU(ctx, cudaMemcpyAsync(dtext, src, len, cudaMemcpyHostToDevice, R.copy));
+        uint32_t scan_len = (uint32_t) len;
+        if (last && text[n_bytes - 1] != '\n') {   // the final line without its '\n'
+            CU(ctx, cudaMemsetAsync(dtext + len, '\n', 1, R.copy));
+            ++scan_len;
+        }
+        CU(ctx, cudaEventRecord(R.copied[slot], R.copy));
+        CU(ctx, cudaStreamWaitEvent(s, R.copied[slot], 0));
+        CU(ctx, cudaEventRecord(R.timing[2 * k], s));
+        CU(ctx, cudaMemsetAsync(R.status.p, 0, status_words * 8, s));
+        unsigned long long* st_words = R.status.as<unsigned long long>();
+        k_paf_line_ends<<<grid_for(scan_len, kScanTile, kNumSMs * 8), kTileThreads, 0, s>>>(
+            (const uint8_t*) dtext, scan_len, R.line_end.as<uint32_t>(), st_words + 1, (uint32_t*) st_words, words + W_BASES, k);
+        ctx->L.count++;
+        k_paf_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
+            (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table, out, R.rec_cap, words);
+        ctx->L.count++;
+        CU(ctx, cudaGetLastError());
+        CU(ctx, cudaEventRecord(R.timing[2 * k + 1], s));
+        CU(ctx, cudaEventRecord(R.parsed[slot], s));
+        pos += len;
+    }
+    R.w.assign(W_BASES + k + 1, 0ull);
+    CU(ctx, cudaMemcpyAsync(R.w.data(), words, R.w.size() * 8, cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaStreamSynchronize(s));
+    if (kernel_ms) {
+        *kernel_ms = 0.f;
+        for (uint32_t c = 0; c < k; ++c) {
+            float ms = 0.f;
+            CU(ctx, cudaEventElapsedTime(&ms, R.timing[2 * c], R.timing[2 * c + 1]));
+            *kernel_ms += ms;
+        }
+    }
+    if (R.w[W_ERR] != ~0ull) {
+        const uint32_t code = (uint32_t) (R.w[W_ERR] & 0xFF), kind = code >> 4, column = code & 15;
+        const unsigned long long line = (R.w[W_ERR] >> 8) + 1;
+        if (kind == kErrFields) return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu has %u tab-separated fields, at least 12 are needed", line, column);
+        if (kind == kErrEmpty) return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu, column 1: the line is empty", line);
+        return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu, column %u: %s", line, column, paf_error_text(kind));
+    }
+    const unsigned long long n = R.w[W_BASES + k];
+    if (n >= (1ull << 31)) return fail(ctx, RALA_B200_ERR_LIMIT, "too many overlap records (%llu >= 2^31)", n);
+    st->n_records = n;
+    st->n_unresolved = R.w[W_UNRESOLVED];
+    st->n_length_mismatch = R.w[W_MISMATCH];
+    st->first_length_mismatch = R.w[W_FIRST_MISMATCH];
+    st->n_bytes = n_bytes;
+    st->n_chunks = k;
+    *n_out = n;
+    return RALA_B200_OK;
+}
+
+// A refused call returns with no upload in flight: the caller may free its text at once.
+static int paf_parse(rala_b200_ctx* ctx, PafReader& R, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* st, float* kernel_ms,
+                     uint64_t* n_out) {
+    const int rc = paf_parse_chunks(ctx, R, text, n_bytes, st, kernel_ms, n_out);
+    if (rc) {
+        if (R.copy) cudaStreamSynchronize(R.copy);
+        cudaStreamSynchronize(ctx->L.stream);
+    }
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint64_t* name_end, const uint32_t* read_len,
+                                         uint32_t n_reads) {
+    if (!g) return RALA_B200_ERR_ARG;
+    if (!g->paf) g->paf = new PafReader();
+    return paf_set_names(g->ctx, *g->paf, names, name_end, read_len, n_reads);
+}
+
+extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats) {
+    if (!g || (n_bytes && !text)) return RALA_B200_ERR_ARG;
+    rala_b200_ctx* ctx = g->ctx;
+    if (!g->paf || !g->paf->have_names) return fail(ctx, RALA_B200_ERR_STATE, "set_overlaps_paf: set_reads first");
+    PafReader& R = *g->paf;
+    // the session's records are void until this call has succeeded
+    g->n_rec = 0;
+    g->state = 0;
+    rala_b200_paf_stats_t st{};
+    uint64_t n = 0;
+    int rc = paf_parse(ctx, R, text, n_bytes, &st, nullptr, &n);
+    if (rc) return rc;
+    rc = reserve_for_records(g, n);
+    if (rc) return rc;
+    if (n) {
+        const PafCols c = R.view();
+        CU(ctx, R.valid.reserve(align_up((size_t) n, 256)));
+        launch_filter_duplicates(ctx->L, c.a, c.b, c.len, (uint32_t) n, R.valid.as<uint8_t>());
+        k_paf_fold<<<grid_for(n, 256, kNumSMs * 8), 256, 0, ctx->L.stream>>>(c, R.valid.as<uint8_t>(), (uint32_t) n, g->recs.view,
+                                                                             R.words.as<unsigned long long>());
+        ctx->L.count++;
+        CU(ctx, cudaGetLastError());
+    }
+    unsigned long long bad = ~0ull;
+    CU(ctx, cudaMemcpyAsync(&bad, R.words.as<unsigned long long>() + W_FIRST_BAD, 8, cudaMemcpyDeviceToHost, ctx->L.stream));
+    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
+    if (stats) *stats = st;
+    if (bad != ~0ull) {
+        g->n_rec = 0;
+        g->state = 0;
+        return fail(ctx, RALA_B200_ERR_ARG,
+                    "PAF line %llu: a read length (column 2 or 7) differs from the length given to set_reads, and the record is "
+                    "valid after the duplicate filter (the reference's transmute exits on it)", bad + 1);
+    }
+    return RALA_B200_OK;
+}
+
+extern "C" int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads,
+                                   const char* text, uint64_t n_bytes, uint32_t* cols_out, uint64_t cap, rala_b200_paf_stats_t* stats,
+                                   float* device_ms) {
+    if (!ctx || !stats || (n_bytes && !text)) return RALA_B200_ERR_ARG;
+    if (device_ms) *device_ms = 0.f;
+    PafReader R;
+    int rc = paf_set_names(ctx, R, names, name_end, read_len, n_reads);
+    if (rc) return rc;
+    uint64_t n = 0;
+    rc = paf_parse(ctx, R, text, n_bytes, stats, device_ms, &n);
+    if (rc) return rc;
+    if (n > cap || (n && !cols_out))
+        return fail(ctx, RALA_B200_ERR_ARG, "parse_paf: the text has %llu records, the output holds %llu", (unsigned long long) n,
+                    (unsigned long long) cap);
+    const PafCols c = R.view();
+    const uint32_t* src[7] = {c.a, c.b, c.ab, c.ae, c.bb, c.be, c.len};
+    for (int k = 0; k < 7 && n; ++k)
+        CU(ctx, cudaMemcpyAsync(cols_out + (size_t) k * cap, src[k], (size_t) n * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
+    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
+    return RALA_B200_OK;
+}

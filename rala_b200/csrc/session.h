@@ -139,6 +139,7 @@ struct rala_b200_graph {
     // rala_b200_graph_run as a replayed CUDA graph (see run_key / RunGraph below)
     bool use_cuda_graph = true, capturing = false;
     struct RunGraph* run_graphs = nullptr;   // two cached instances: first run after set_piles / repeated run
+    struct PafReader* paf = nullptr;         // read-name table and PAF upload buffers (paf.cu), from the first set_reads
 
     uint32_t* cnt() const { return counters.as<uint32_t>(); }
     Events events_view() const {
@@ -201,3 +202,7 @@ int phase_survivors(rala_b200_graph* g);
 int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base, const uint32_t* inl_base);
 int read_counters(rala_b200_graph* g, uint32_t* h);
 int materialize_final_lists(rala_b200_graph* g);
+int reserve_for_records(rala_b200_graph* g, uint64_t n);
+
+// ---- paf.cu ----------------------------------------------------------------------------------------------------
+void destroy_paf_reader(PafReader* r);
