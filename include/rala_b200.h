@@ -104,7 +104,7 @@ int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes, uint64_t n
  * ignored; length[i] = Overlap::length() as parsed (PAF column 11, MHAP: the longer span).  valid_out[i] = what
  * is_valid_overlap_[i] holds after the pass: 0 for unresolved records, self overlaps and every record of a query group but
  * the last longest one per target.  device_ms (nullable) receives the kernel time.  SURVEY.md 8(f) row 1, first half; the
- * coverage accumulation of the same pass (:305-321, pile.cpp:274-297) stays host code. */
+ * coverage accumulation of the same pass (:305-321, pile.cpp:274-297) is rala_b200_build_piles. */
 int rala_b200_filter_duplicates(rala_b200_ctx* ctx, const uint32_t* a_id, const uint32_t* b_id, const uint32_t* length,
                                 uint64_t n, uint8_t* valid_out, float* device_ms);
 
@@ -138,6 +138,38 @@ typedef struct {
 int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads,
                         const char* text, uint64_t n_bytes, uint32_t* cols_out, uint64_t cap, rala_b200_paf_stats_t* stats,
                         float* device_ms);
+
+/* The pile table from the overlap records (SURVEY.md 8(f) row 1, second half): the coverage half of Graph::initialize
+ * (store_overlap_bounds + Pile::add_layers, graph.cpp:305-321, pile.cpp:274-297), the valid region and pile liveness
+ * (Pile::find_valid_region, pile.cpp:307, 329) and the median (Pile::find_median).  The rule, as restated from the
+ * reference's goldens (begin, end and median of every pile of tests/golden/g_*):
+ *   - every record whose two names resolved counts, also those the duplicate filter drops;
+ *   - it adds [a_begin + 15, a_end - 15) to read a and [b_begin + 15, b_end - 15) to read b (forward-strand coordinates as
+ *     parsed, orientation ignored); coverage[x] = number of intervals containing x, x in [0, read_len);
+ *   - the valid region is the longest maximal run of positions with coverage >= 4; the pile is dead (end == 0) when there
+ *     is none or it is shorter than 1 260;
+ *   - the median of a live pile is element size / 2 (0-based) of the sorted coverage over [begin, end) (nth_element).
+ * Restated, NOT pinned (no golden has such a case), so decided here and counted in the stats:
+ *   - ties between equally long runs: the first one wins (strict > of a left-to-right scan);
+ *   - a run of exactly 1 260 lives.
+ * Refused rather than guessed (RALA_B200_ERR_ARG; the message names the smallest offending record, 0-based, or its 1-based
+ * PAF line in the session form): a self overlap, an interval that is empty or inverted after the shrink
+ * (begin + 15 >= end - 15), an end beyond the read's length, a read id >= n_reads.  Coverage >= 65 536 (Pile keeps it in
+ * 16 bits) is refused with RALA_B200_ERR_LIMIT.  Records < 2^29, read lengths < 2^30. */
+typedef struct {
+    uint64_t n_counted;      /* records that added coverage (both names resolved) */
+    uint64_t n_runs;         /* constant-coverage runs over all reads (rala_b200_graph_get_coverage_runs) */
+    uint32_t max_coverage;
+    uint32_t n_live;         /* piles with a valid region */
+    uint32_t n_tied;         /* live piles whose longest region is not unique: the first-wins rule decided them */
+    uint32_t n_exact_min;    /* live piles whose region is exactly 1 260 long: the >= 1 260 rule decided them */
+} rala_b200_pile_stats_t;
+/* Stateless form on HOST columns in the rala_b200_graph_set_overlaps_columns layout: bit 31 of a_id marks an unresolved
+ * record (it adds nothing), bit 31 of b_id is ignored.  piles_out: n_reads rows, dead = {0, 0}; medians_out (nullable):
+ * n_reads values, 0 for a dead pile; stats (nullable); device_ms (nullable) = kernel time, uploads excluded. */
+int rala_b200_build_piles(rala_b200_ctx* ctx, const uint32_t* a_id, const uint32_t* b_id, const uint32_t* a_begin, const uint32_t* a_end,
+                          const uint32_t* b_begin, const uint32_t* b_end, uint64_t n, const uint32_t* read_len, uint32_t n_reads,
+                          rala_pile_t* piles_out, uint16_t* medians_out, rala_b200_pile_stats_t* stats, float* device_ms);
 
 /* ------------------------------------------------------------------------------------------------
  * Graph session: the drop-in for Graph::construct's hot loops and Graph::remove_transitive_edges.
@@ -209,6 +241,22 @@ int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint6
  * reaches it (overlap.cpp:54-59, 73-78); the library is stricter and also refuses one whose pile is already dead.  After
  * a refused call the session holds no records (classify needs a new set_overlaps*).  stats: nullable. */
 int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats);
+/* The pile table of the reads given to set_reads, built on the device (rule and refusals as rala_b200_build_piles) from
+ * the records of the last successful set_overlaps_paf, counted as parsed: before the duplicate filter.  It is installed as
+ * set_piles(piles, NULL, n_reads) would (flags 0; the hills are left as they are) and the next classify / run uses it.
+ * RALA_B200_ERR_STATE after set_overlaps / _columns / _packed (their records have the filter folded in) or set_reads.
+ * A refused call changes nothing in the session.  stats: nullable. */
+int rala_b200_graph_build_piles(rala_b200_graph* g, rala_b200_pile_stats_t* stats);
+/* After build_piles: the median of every pile it built (n_reads values of set_reads, 0 = dead pile), what Pile::find_median
+ * leaves.  The medians and runs below belong to the last successful build_piles, whatever set_piles did since. */
+int rala_b200_graph_get_medians(rala_b200_graph* g, uint16_t* out);
+/* After build_piles: the constant-coverage runs of every read over [0, read_len), for the host's chimeric pit and hill
+ * detection (Pile::find_chimeric_pits / find_chimeric_hills expand them into Pile::data_).  Runs are maximal (the coverage
+ * changes at every run start); read r has the runs [run_off[r], run_off[r + 1]), run k covers [run_begin[k], run_begin[k + 1])
+ * or up to read_len for the read's last one, with coverage run_cov[k].  run_off (n_reads + 1 words) is always written;
+ * run_begin and run_cov are written when both are given and cap >= run_off[n_piles] (RALA_B200_ERR_ARG when cap is smaller),
+ * so a first call with NULL buffers asks for the size. */
+int rala_b200_graph_get_coverage_runs(rala_b200_graph* g, uint32_t* run_off, uint32_t* run_begin, uint16_t* run_cov, uint64_t cap);
 /* Optional: have build / transitive / run write their results STRAIGHT into caller memory the GPU can address
  * (cudaHostAlloc / cudaHostRegister'ed host memory, or device memory): the rala_edge_t rows (graph.cpp:576-632)
  * leave as soon as the edge list exists, on a forked stream beside the CSR build and the transitive pass, and the

@@ -52,6 +52,14 @@ class PafStats(C.Structure):
 PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES
 
 
+class PileStats(C.Structure):
+    _fields_ = [("n_counted", C.c_uint64), ("n_runs", C.c_uint64), ("max_coverage", C.c_uint32), ("n_live", C.c_uint32),
+                ("n_tied", C.c_uint32), ("n_exact_min", C.c_uint32)]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
 def _text(text):
     """PAF text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
     if isinstance(text, (bytes, bytearray, memoryview)):
@@ -86,6 +94,7 @@ EXPORTS = [
     "rala_b200_launch_count", "rala_b200_event_record", "rala_b200_event_elapsed_ms", "rala_b200_synchronize",
     "rala_b200_trim_classify", "rala_b200_transitive_reduce", "rala_b200_filter_duplicates",
     "rala_b200_parse_paf", "rala_b200_graph_set_reads", "rala_b200_graph_set_overlaps_paf",
+    "rala_b200_build_piles", "rala_b200_graph_build_piles", "rala_b200_graph_get_medians", "rala_b200_graph_get_coverage_runs",
     "rala_b200_graph_create", "rala_b200_graph_destroy", "rala_b200_graph_set_overlaps",
     "rala_b200_graph_set_piles", "rala_b200_graph_set_hills", "rala_b200_graph_classify",
     "rala_b200_graph_retrim", "rala_b200_graph_retrim_promote", "rala_b200_graph_finalize",
@@ -318,6 +327,22 @@ class Context:
         out = np.ascontiguousarray(cols[:, :stats["n_records"]])
         return (out, stats, float(ms.value)) if with_time else (out, stats)
 
+    def build_piles(self, columns, read_len, with_time: bool = False):
+        """Graph::initialize's coverage half on the device: six host columns in the set_overlaps_columns layout (bit 31 of
+        a_id = unresolved record; records the duplicate filter drops still count) + the read lengths -> (piles (n_reads, 2)
+        uint32, dead = 0 0; medians (n_reads,) uint16, 0 = dead; stats dict)."""
+        cols = [_np(c, np.uint32) for c in columns]
+        n = cols[0].shape[0]
+        if len(cols) != 6 or any(c.shape[0] != n for c in cols):
+            raise RalaB200Error("build_piles needs six columns of equal length")
+        rl = _np(read_len, np.uint32)
+        piles = np.zeros((rl.shape[0], 2), dtype=np.uint32)
+        med = np.zeros(rl.shape[0], dtype=np.uint16)
+        st, ms = PileStats(), C.c_float(0.0)
+        self.check(self.lib.rala_b200_build_piles(self.handle, *[_ptr(c) for c in cols], C.c_uint64(n), _ptr(rl), C.c_uint32(rl.shape[0]),
+                                                  _ptr(piles), _ptr(med), C.byref(st), C.byref(ms)), "build_piles")
+        return (piles, med, st.as_dict(), float(ms.value)) if with_time else (piles, med, st.as_dict())
+
 
 class Graph:
     """Host-side mirror of rala::Graph for the hot path (graph.hpp:37-60).
@@ -385,6 +410,7 @@ class Graph:
         """Read names (list of bytes, or (blob, name_end)) and sequence lengths the PAF text is resolved against."""
         blob, ends, rl = _names(names, read_len)
         self._call("rala_b200_graph_set_reads", _ptr(blob), _ptr(ends), _ptr(rl), C.c_uint32(ends.shape[0]))
+        self._n_reads = int(ends.shape[0])
         return self
 
     def set_overlaps_paf(self, text) -> dict:
@@ -394,6 +420,31 @@ class Graph:
         st = PafStats()
         self._call("rala_b200_graph_set_overlaps_paf", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
         return st.as_dict()
+
+    def build_piles(self) -> dict:
+        """The pile table from the records of the last set_overlaps_paf, built on the device and installed as
+        set_piles(piles) would (flags 0, hills untouched); returns the stats."""
+        st = PileStats()
+        self._call("rala_b200_graph_build_piles", C.byref(st))
+        self.n_piles = self._built_piles = self._n_reads
+        return st.as_dict()
+
+    def medians(self):
+        """After build_piles: Pile::find_median of every pile (uint16, 0 = dead)."""
+        out = np.zeros(getattr(self, "_built_piles", 0), dtype=np.uint16)
+        self._call("rala_b200_graph_get_medians", _ptr(out))
+        return out
+
+    def coverage_runs(self):
+        """After build_piles: (run_off (n_piles + 1), run_begin, run_cov uint16) — the maximal constant-coverage runs of
+        every read over [0, read_len); read r's runs are [run_off[r], run_off[r + 1])."""
+        off = np.zeros(getattr(self, "_built_piles", 0) + 1, dtype=np.uint32)
+        self._call("rala_b200_graph_get_coverage_runs", _ptr(off), None, None, C.c_uint64(0))
+        total = int(off[-1])
+        begin = np.zeros(max(total, 1), dtype=np.uint32)
+        cov = np.zeros(max(total, 1), dtype=np.uint16)
+        self._call("rala_b200_graph_get_coverage_runs", _ptr(off), _ptr(begin), _ptr(cov), C.c_uint64(total))
+        return off, begin[:total], cov[:total]
 
     def set_outputs(self, edges_out=None, marked_out=None):
         """Pinned host (or device-visible) buffers the run writes its edge rows and marks into directly."""

@@ -38,6 +38,7 @@ extern "C" int rala_b200_create(rala_b200_ctx** out, int device) {
     preload_fabric();
     preload_frontend();
     preload_paf();
+    preload_piles();
     cudaGetLastError();
     cudaEventCreate(&ctx->ev[0]);
     cudaEventCreate(&ctx->ev[1]);
@@ -180,6 +181,7 @@ extern "C" void rala_b200_graph_destroy(rala_b200_graph* g) {
     cudaStreamSynchronize(g->ctx->L.stream);
     drop_run_graphs(g);
     destroy_paf_reader(g->paf);
+    destroy_pile_builder(g->pile_builder);
     DevBuf* bufs[] = {&g->rec, &g->recs.buf, &g->alive_bits, &g->piles, &g->piles_raw, &g->pile_flags_raw, &g->piles_initial, &g->hills, &g->ovl[0].buf,
                       &g->ovl[1].buf, &g->inl[0].buf, &g->inl[1].buf, &g->events, &g->hill_rec, &g->dbuf, &g->flags, &g->segs, &g->tiles,
                       &g->counters, &g->scan_pool, &g->seq_to_node, &g->edges, &g->row_ptr, &g->cursor, &g->col,
@@ -233,6 +235,7 @@ static int reserve_scan_pool(rala_b200_graph* g) {
 int reserve_for_records(rala_b200_graph* g, uint64_t n) {
     rala_b200_ctx* ctx = g->ctx;
     g->n_rec = (uint32_t) n;
+    g->paf_records = false;   // set_overlaps_paf sets it again once its records are in place
     CU(ctx, g->recs.reserve((uint32_t) ((n + 3) / 4 * 4 + 4)));
     uint32_t cap = (uint32_t) align_up((size_t) n, 128);
     if (cap < 1024) cap = 1024;

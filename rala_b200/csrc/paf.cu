@@ -264,7 +264,7 @@ void preload_paf() {
 struct PafReader {
     DevBuf names;                 // blob | ends | read lengths | table slots
     NameTable table{};
-    uint32_t n_reads = 0;
+    uint32_t n_reads = 0, max_len = 0;
     bool have_names = false;
     DevBuf text[2];               // device side of the staging pair
     DevBuf line_end, status, words, cols, valid;
@@ -341,6 +341,8 @@ static int paf_set_names(rala_b200_ctx* ctx, PafReader& R, const char* names, co
         return fail(ctx, RALA_B200_ERR_ARG, "set_reads: reads %u and %u have the same name (which one name_to_id_ keeps is not pinned)",
                     (unsigned) dup, (unsigned) (dup >> 32));
     R.n_reads = n_reads;
+    R.max_len = 0;
+    for (uint32_t i = 0; i < n_reads; ++i) R.max_len = read_len[i] > R.max_len ? read_len[i] : R.max_len;
     R.have_names = true;
     return RALA_B200_OK;
 }
@@ -488,6 +490,7 @@ extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, 
                                          uint32_t n_reads) {
     if (!g) return RALA_B200_ERR_ARG;
     if (!g->paf) g->paf = new PafReader();
+    g->paf_records = false;   // the records' ids refer to the reads they were parsed against
     return paf_set_names(g->ctx, *g->paf, names, name_end, read_len, n_reads);
 }
 
@@ -499,6 +502,7 @@ extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* 
     // the session's records are void until this call has succeeded
     g->n_rec = 0;
     g->state = 0;
+    g->paf_records = false;
     rala_b200_paf_stats_t st{};
     uint64_t n = 0;
     int rc = paf_parse(ctx, R, text, n_bytes, &st, nullptr, &n);
@@ -525,7 +529,18 @@ extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* 
                     "PAF line %llu: a read length (column 2 or 7) differs from the length given to set_reads, and the record is "
                     "valid after the duplicate filter (the reference's transmute exits on it)", bad + 1);
     }
+    g->paf_records = true;
     return RALA_B200_OK;
+}
+
+bool paf_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len) {
+    if (!g->paf_records || !g->paf || !g->paf->have_names) return false;
+    const PafCols c = g->paf->view();
+    *cols = PileCols{c.a, c.b, c.ab, c.ae, c.bb, c.be};
+    *read_len = g->paf->table.read_len;
+    *n_reads = g->paf->n_reads;
+    *max_len = g->paf->max_len;
+    return true;
 }
 
 extern "C" int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads,

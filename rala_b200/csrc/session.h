@@ -140,6 +140,8 @@ struct rala_b200_graph {
     bool use_cuda_graph = true, capturing = false;
     struct RunGraph* run_graphs = nullptr;   // two cached instances: first run after set_piles / repeated run
     struct PafReader* paf = nullptr;         // read-name table and PAF upload buffers (paf.cu), from the first set_reads
+    bool paf_records = false;                // the records came from set_overlaps_paf: its parsed columns are still there
+    struct PileBuilder* pile_builder = nullptr;   // event, sort and run buffers of build_piles (piles.cu)
 
     uint32_t* cnt() const { return counters.as<uint32_t>(); }
     Events events_view() const {
@@ -206,3 +208,12 @@ int reserve_for_records(rala_b200_graph* g, uint64_t n);
 
 // ---- paf.cu ----------------------------------------------------------------------------------------------------
 void destroy_paf_reader(PafReader* r);
+// the overlap columns build_piles counts: the parsed records of the last successful set_overlaps_paf, before the duplicate
+// filter was folded in (bit 31 of a = unresolved name), and the reads' lengths (device); false when there are none
+struct PileCols {
+    const uint32_t *a, *b, *ab, *ae, *bb, *be;
+};
+bool paf_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len);
+
+// ---- piles.cu --------------------------------------------------------------------------------------------------
+void destroy_pile_builder(PileBuilder* p);
