@@ -185,7 +185,7 @@ extern "C" void rala_b200_graph_destroy(rala_b200_graph* g) {
     DevBuf* bufs[] = {&g->rec, &g->recs.buf, &g->alive_bits, &g->piles, &g->piles_raw, &g->pile_flags_raw, &g->piles_initial, &g->hills, &g->ovl[0].buf,
                       &g->ovl[1].buf, &g->inl[0].buf, &g->inl[1].buf, &g->events, &g->hill_rec, &g->dbuf, &g->flags, &g->segs, &g->tiles,
                       &g->counters, &g->scan_pool, &g->seq_to_node, &g->edges, &g->row_ptr, &g->cursor, &g->col,
-                      &g->col_eid, &g->T, &g->marked, &g->heavy, &g->work_counter, &g->edges_aos};
+                      &g->col_eid, &g->T, &g->marked, &g->heavy, &g->work_counter, &g->edges_aos, &g->slot_degree, &g->tile_dov};
     for (DevBuf* b : bufs) b->release();
     for (int i = 0; i < RALA_B200_N_STAGES; ++i) {
         cudaEventDestroy(g->ev_start[i]);
@@ -211,7 +211,6 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
     CU(ctx, g->edges.reserve(align_up((size_t) edge_cap * 4, 256) * 3));
     CU(ctx, g->col.reserve((size_t) edge_cap * 8));
     CU(ctx, g->col_eid.reserve((size_t) edge_cap * 4));
-    CU(ctx, g->edge_rank.reserve((size_t) edge_cap * 4));
     CU(ctx, g->T.reserve(align_up(edge_cap, 256)));
     CU(ctx, g->marked.reserve(align_up(edge_cap, 256)));
     g->heavy_cap = edge_cap / 16 + 4096;
@@ -220,7 +219,7 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
 }
 
 static int reserve_scan_pool(rala_b200_graph* g) {
-    // worst stage: classify = runs scan + two containment scans over the piles; build = piles + list + node degrees;
+    // worst stage: classify = runs scan + two containment scans over the piles; build = one scan over the piles;
     // the multi-GPU session adds scans over its exchange capacities (<= 2 x the record count): 16 x leaves room
     size_t words = 16 * (tiles_of(g->n_rec) + tiles_of(2ull * g->n_piles + 8) + 8);
     if (words > g->scan_pool_words) {
@@ -245,6 +244,7 @@ int reserve_for_records(rala_b200_graph* g, uint64_t n) {
             CU(ctx, g->inl[i].reserve(cap));
         }
         CU(ctx, g->hill_rec.reserve((size_t) cap * 4));
+        CU(ctx, g->tile_dov.reserve((emit_tiles(cap) + 8) * 4));
         g->cap = cap;
         int rc2 = reserve_events(g, cap);
         if (!rc2) rc2 = reserve_edges(g, 2 * cap);
@@ -387,6 +387,7 @@ extern "C" int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* 
         CU(ctx, g->seq_to_node.reserve((size_t) n_piles * 4 + 16));
         CU(ctx, g->row_ptr.reserve(((size_t) g->n_nodes_max + 8) * 4));
         CU(ctx, g->cursor.reserve(((size_t) g->n_nodes_max + 8) * 4));
+        CU(ctx, g->slot_degree.reserve(((size_t) g->n_nodes_max + 8) * 4));
         int rc = reserve_scan_pool(g);
         if (rc) return rc;
     }
@@ -681,21 +682,24 @@ extern "C" int rala_b200_graph_finalize(rala_b200_graph* g) {
     return rc;
 }
 
-// node ids + the edges of the overlaps in list order (graph.cpp:552-632).  In a multi-GPU phase the list is the local
-// shard's and the node ids are global: the pile table is replicated.
-static int emit_edges(rala_b200_graph* g) {
+// node ids + the edges of the overlaps in list order (graph.cpp:552-632), and with `csr` their CSR rows.  In a multi-GPU
+// phase the list is the local shard's and the node ids are global: the pile table is replicated.
+static int emit_edges(rala_b200_graph* g, bool csr) {
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_BUILD));
     CU(ctx, zero_counter(g, C_NODES, 4));   // C_NODES, C_ALIVE, C_DOVETAILS, C_EDGES
-    CU(ctx, cudaMemsetAsync(g->cursor.p, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
+    GraphArrays ga = g->graph_view();
+    if (csr) CU(ctx, cudaMemsetAsync(ga.slot_degree, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
+    else ga.cursor = nullptr;
     unsigned long long* status;
     uint32_t* ticket;
     scan_state(g, g->n_piles, &status, &ticket);
-    launch_node_ids(ctx->L, g->piles.as<uint2>(), g->n_piles, g->seq_to_node.as<uint32_t>(), g->cnt(), status, ticket);
-    scan_state(g, emit_scan_span(g->cap), &status, &ticket);
-    launch_emit_edges(ctx->L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), g->graph_view(),
-                      g->edge_cap, g->cnt(), status, ticket);
+    const List ovl = g->ovl[g->ovl_cur].view;
+    const uint32_t* n_ovl = g->cnt() + g->slot_ovl;
+    launch_count_scan(ctx->L, ovl, n_ovl, g->cap, g->piles.as<uint2>(), g->n_piles, ga, g->edge_cap, g->tile_dov.as<uint32_t>(), g->cnt(),
+                      status, ticket);
+    launch_emit_edges(ctx->L, ovl, n_ovl, g->cap, g->piles.as<uint2>(), ga, g->edge_cap, g->tile_dov.as<uint32_t>());
     return RALA_B200_OK;
 }
 
@@ -704,19 +708,15 @@ extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "build: finalize first");
-    int rc = emit_edges(g);
+    int rc = emit_edges(g, true);
     if (rc) return rc;
-    unsigned long long* status;
-    uint32_t* ticket;
-    // the edge list is final: rows into the caller's buffer on a forked stream, beside the CSR build and (inside a
-    // whole run) the transitive pass; edges beyond the caller's capacity are not written (n_edges tells)
+    // the edge list is final: rows into the caller's buffer on a forked stream, beside (inside a whole run) the
+    // transitive pass; edges beyond the caller's capacity are not written (n_edges tells)
     if (g->out_edges && g->out_edges_cap && fork_side(ctx->L, 0)) {
         launch_pack_edges(ctx->L, ctx->L.side[0], g->graph_view(), g->edge_cap < g->out_edges_cap ? g->edge_cap : g->out_edges_cap,
                           g->cnt() + C_EDGES, g->out_edges);
         g->download_pending = true;
     }
-    scan_state(g, (uint64_t) g->n_nodes_max + 1, &status, &ticket);
-    launch_build_csr(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->cnt(), status, ticket, true);
     if (g->download_pending && !g->in_run) {
         join_side(ctx->L, 0);
         g->download_pending = false;
@@ -1001,7 +1001,7 @@ extern "C" int rala_b200_graph_set_kept_overlaps(rala_b200_graph* g, const rala_
     DevBuf tmp;
     CU(ctx, tmp.reserve((size_t) n * 28 + 16));
     if (n) CU(ctx, cudaMemcpyAsync(tmp.p, kept, (size_t) n * 28, cudaMemcpyHostToDevice, ctx->L.stream));
-    launch_aos_to_list(ctx->L, tmp.as<uint32_t>(), (uint32_t) n, g->ovl[g->ovl_cur].view);
+    launch_aos_to_list(ctx->L, tmp.as<uint32_t>(), (uint32_t) n, g->piles.as<uint2>(), g->n_piles, g->ovl[g->ovl_cur].view);
     const uint32_t n32 = (uint32_t) n;
     CU(ctx, cudaMemcpyAsync(g->cnt() + g->slot_ovl, &n32, 4, cudaMemcpyHostToDevice, ctx->L.stream));
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
@@ -1233,7 +1233,7 @@ extern "C" int rala_b200_graph_phase_emit_edges(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "emit_edges: finalize first");
-    int rc = emit_edges(g);
+    int rc = emit_edges(g, false);   // the CSR is built over the edges of all ranks (phase_csr)
     if (rc) return rc;
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;

@@ -666,13 +666,19 @@ __global__ void k_list_to_aos(List l, const uint32_t* __restrict__ n_ptr, uint32
     }
 }
 
-// rala_ovl_t rows -> SoA list (upload of a host-filtered `overlaps`, C ABI rala_b200_graph_set_kept_overlaps)
-__global__ void k_aos_to_list(const uint32_t* __restrict__ aos, uint32_t n, List l) {
+// rala_ovl_t rows -> SoA list (upload of a host-filtered `overlaps`, C ABI rala_b200_graph_set_kept_overlaps).  Each entry
+// is typed against the pile table as it stands, as edge creation does (graph.cpp:594, no trim): the build trusts the tag.
+__global__ void k_aos_to_list(const uint32_t* __restrict__ aos, uint32_t n, const uint2* __restrict__ piles, uint32_t n_piles, List l) {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const uint32_t* q = aos + (size_t) i * 7;
         Entry e;
         e.a = q[0]; e.b = q[1] & 0x7FFFFFFFu; e.c.ab = q[2]; e.c.ae = q[3]; e.c.bb = q[4]; e.c.be = q[5]; e.ori = q[6] & 1u;
-        store_entry(l, i, e, kRejected);   // the type is recomputed by whoever needs it (edge creation, graph.cpp:594)
+        uint8_t t = kRejected;
+        if (e.a < n_piles && e.b < n_piles) {
+            const Pile pa = load_pile(piles, e.a), pb = load_pile(piles, e.b);
+            if (pa.alive() && pb.alive()) t = classify(e.c, relative(e.c, e.ori, pa, pb));
+        }
+        store_entry(l, i, e, t);
     }
 }
 
@@ -793,9 +799,9 @@ void launch_list_to_aos(Launch& L, List l, const uint32_t* n_ptr, uint32_t cap, 
     L.count++;
 }
 
-void launch_aos_to_list(Launch& L, const uint32_t* aos, uint32_t n, List l) {
+void launch_aos_to_list(Launch& L, const uint32_t* aos, uint32_t n, const uint2* piles, uint32_t n_piles, List l) {
     if (n == 0) return;
-    k_aos_to_list<<<grid_for(n, 256, kNumSMs * 8), 256, 0, L.stream>>>(aos, n, l);
+    k_aos_to_list<<<grid_for(n, 256, kNumSMs * 8), 256, 0, L.stream>>>(aos, n, piles, n_piles, l);
     L.count++;
 }
 

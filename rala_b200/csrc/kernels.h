@@ -92,7 +92,7 @@ void launch_trim_classify_aos(Launch& L, uint32_t* rec, uint32_t n, const uint2*
 void launch_pack_piles(Launch& L, const uint2* in, const uint8_t* flags, uint2* out, uint32_t n);
 void launch_unpack_piles(Launch& L, const uint2* in, uint2* out, uint32_t n);
 void launch_list_to_aos(Launch& L, List l, const uint32_t* n_ptr, uint32_t cap, uint32_t* out);
-void launch_aos_to_list(Launch& L, const uint32_t* aos, uint32_t n, List l);
+void launch_aos_to_list(Launch& L, const uint32_t* aos, uint32_t n, const uint2* piles, uint32_t n_piles, List l);
 void launch_list_connections(Launch& L, List l, const uint32_t* n_ptr, uint32_t cap, uint32_t* out);
 
 // containment.cu
@@ -121,21 +121,28 @@ struct GraphArrays {
     uint32_t* seq_to_node;   // n_piles
     uint32_t *src, *dst, *len;   // edge id order
     uint32_t* row_ptr;       // n_nodes_max + 1
-    uint32_t* cursor;        // n_nodes_max + 1 (degree histogram, then fill cursor)
+    uint32_t* cursor;        // n_nodes_max + 1: fill cursor (the degree histogram first, on the paths that fill with k_fill_csr)
+    uint32_t* slot_degree;   // 2 per pile: out-degree of slot 2x + s = node 2 rank(x) + s (k_count_edges -> k_scan_piles)
     uint2* col;              // CSR (dst, len)
     uint32_t* col_eid;       // CSR edge id
-    uint32_t* rank;          // per edge: its position inside its source row, as handed out by the degree count in k_emit_edges
     uint8_t* T;              // per edge: transitive test passed
     uint8_t* marked;         // per edge: removed
 };
-void launch_node_ids(Launch& L, const uint2* piles, uint32_t n_piles, uint32_t* seq_to_node, uint32_t* counters,
-                     unsigned long long* status, uint32_t* ticket);
-// entries per thread of k_emit_edges (its tiles are 256 x this); its look-back scan needs one status word per tile.
-// 2 and 1 (more, smaller tiles: a longer look-back chain) measured no faster than 4 (profiles/r02aa_ab.json).
-constexpr int kEmitItems = 4;
-inline uint64_t emit_scan_span(uint64_t cap) { return cap * (4 / kEmitItems); }   // in units of the common 1024-entry tile
-void launch_emit_edges(Launch& L, List ovl, const uint32_t* n_ptr, uint32_t cap, const uint2* piles, GraphArrays g,
-                       uint32_t edge_cap, uint32_t* counters, unsigned long long* status, uint32_t* ticket);
+// Edges of the final `overlaps` (graph.cpp:552-632) in two launches, with node ids and, when g.cursor is set, the CSR rows:
+//   launch_count_scan  slot degrees and per-tile dovetail counts (k_count_edges), then one look-back over the piles for
+//                      seq_to_node, C_NODES / C_ALIVE, row_ptr + cursor, and the edge-id bases of the list tiles with
+//                      C_DOVETAILS / C_EDGES / C_OVERFLOW (k_scan_piles).  slot_degree must be zero on entry.
+//   launch_emit_edges  the edge columns, and with g.cursor set the CSR slots and T cleared (k_emit_edges)
+// g.cursor == nullptr switches the CSR outputs off (multi-GPU: the edges are routed to the owners of their source nodes).
+// tile_dov holds emit_tiles(cap) words.  The look-back needs the scan state of n_piles.
+// list entries per thread of k_count_edges / k_emit_edges (their tiles are 256 x this).  4 entries (64 registers, 4 blocks per
+// SM, a small spill) measured +17 us per step and 1 entry (8 blocks per SM) +11 us against 2 at 5 blocks (profiles/r02am_*)
+constexpr int kEmitItems = 2;
+inline uint64_t emit_tiles(uint64_t cap) { return (cap + 256 * kEmitItems - 1) / (256 * kEmitItems); }
+void launch_count_scan(Launch& L, List ovl, const uint32_t* n_ptr, uint32_t cap, const uint2* piles, uint32_t n_piles, GraphArrays g,
+                       uint32_t edge_cap, uint32_t* tile_dov, uint32_t* counters, unsigned long long* status, uint32_t* ticket);
+void launch_emit_edges(Launch& L, List ovl, const uint32_t* n_ptr, uint32_t cap, const uint2* piles, GraphArrays g, uint32_t edge_cap,
+                       const uint32_t* tile_base);
 void launch_pack_edges(Launch& L, cudaStream_t stream, GraphArrays g, uint32_t edge_cap, const uint32_t* n_edges_ptr, uint32_t* out);
 // degree histogram for an edge list that did not come from emit_edges (stateless transitive stage)
 void launch_degree_hist(Launch& L, const uint32_t* src, const uint32_t* n_edges_ptr, uint32_t edge_cap, uint32_t* cursor);
@@ -148,8 +155,9 @@ void launch_time_bases(Launch& L, const uint32_t* counts, uint32_t rank, uint32_
 void launch_adjacency_view(Launch& L, const uint32_t* key, const uint8_t* marked, const uint32_t* n_edges_ptr, uint32_t edge_cap,
                            uint32_t n_nodes, uint32_t* degree_cursor, uint32_t* row_ptr, uint32_t* ids_tmp, uint32_t* ids_sorted,
                            unsigned long long* status, uint32_t* ticket);
+// CSR of an edge list that did not come from emit_edges: g.cursor holds its degree histogram (launch_degree_hist)
 void launch_build_csr(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t edge_cap, uint32_t* counters,
-                      unsigned long long* status, uint32_t* ticket, bool ranked = false);
+                      unsigned long long* status, uint32_t* ticket);
 
 // transitive.cu
 struct HeavyItems {

@@ -569,12 +569,13 @@ static int phase_f_edges(rala_b200_multi* m, FabricRank& fr) {
     unsigned long long* status;
     uint32_t* ticket;
     scan_state(g, g->n_piles, &status, &ticket);
-    launch_node_ids(L, g->piles.as<uint2>(), g->n_piles, g->seq_to_node.as<uint32_t>(), g->cnt(), status, ticket);
-    launch_node_bounds(L, fr.P, fr.A, g->cnt() + C_NODES, fr.meta_dev());
-    scan_state(g, emit_scan_span(g->cap), &status, &ticket);
     GraphArrays ga = g->graph_view();
-    ga.cursor = nullptr;   // no local degree histogram: the owners count what they receive
-    launch_emit_edges(L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), ga, g->edge_cap, g->cnt(), status, ticket);
+    ga.cursor = nullptr;   // no local CSR: the owners build theirs from what they receive
+    const List ovl = g->ovl[g->ovl_cur].view;
+    launch_count_scan(L, ovl, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), g->n_piles, ga, g->edge_cap, g->tile_dov.as<uint32_t>(),
+                      g->cnt(), status, ticket);
+    launch_node_bounds(L, fr.P, fr.A, g->cnt() + C_NODES, fr.meta_dev());
+    launch_emit_edges(L, ovl, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), ga, g->edge_cap, g->tile_dov.as<uint32_t>());
     if (g->out_edges && g->out_edges_cap && fork_side(L, 0)) {   // rows of the local edges straight into the caller's memory
         launch_pack_edges(L, L.side[0], g->graph_view(), g->edge_cap < g->out_edges_cap ? g->edge_cap : g->out_edges_cap,
                           g->cnt() + C_EDGES, g->out_edges);

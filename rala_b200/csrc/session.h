@@ -116,7 +116,8 @@ struct rala_b200_graph {
     // graph
     DevBuf edges_aos;
     DevBuf seq_to_node, edges, row_ptr, cursor, col, col_eid, T, marked, heavy, work_counter;
-    DevBuf edge_rank;   // row slot of every edge (k_emit_edges -> k_fill_csr)
+    DevBuf slot_degree;   // 2 per pile: out-degrees of the node slots (k_count_edges -> k_scan_piles)
+    DevBuf tile_dov;      // per tile of the list: dovetails, then the tile's edge-id base (k_count_edges -> k_scan_piles -> k_emit_edges)
     uint32_t edge_cap = 0, heavy_cap = 0, n_nodes_max = 0;
     // results written straight into the caller's memory by the run (rala_b200_graph_set_outputs)
     uint32_t* out_edges = nullptr;   // device-visible address of the caller's rala_edge_t rows
@@ -164,7 +165,7 @@ struct rala_b200_graph {
         g.cursor = cursor.as<uint32_t>();
         g.col = col.as<uint2>();
         g.col_eid = col_eid.as<uint32_t>();
-        g.rank = edge_rank.as<uint32_t>();
+        g.slot_degree = slot_degree.as<uint32_t>();
         g.T = T.as<uint8_t>();
         g.marked = marked.as<uint8_t>();
         return g;
