@@ -18,7 +18,10 @@
  *   - there is NO CPU fallback: without a CUDA device rala_b200_create() fails.
  *
  * Limits: ids, coordinates and counts are 32-bit (SURVEY.md appendix D); read lengths < 2^30;
- * overlap records per context < 2^31.
+ * overlap records per context < 2^31.  Transitive reduction: a node with more than 1024 out-edges is
+ * split by destination into ceil(degree / 768) hash chunks of at most 2048 distinct destinations each
+ * (destination d goes to chunk ((d * 0x85EBCA6B mod 2^32) >> 12) mod chunks); more, or more than 2^32
+ * block work items in one pass, is refused with RALA_B200_ERR_LIMIT.  Random ids put ~768 in a chunk.
  */
 #ifndef RALA_B200_H
 #define RALA_B200_H
@@ -94,7 +97,8 @@ int rala_b200_trim_classify(rala_b200_ctx* ctx, rala_ovl_t* ovl, uint64_t n,
                             const rala_pile_t* piles, uint32_t n_piles, uint8_t* type_out);
 
 /* Graph::remove_transitive_edges (graph.cpp:1281-1318) on an arbitrary edge list:
- * marked_out[e] = 1 for every edge the reference removes; *n_pairs = its return value. */
+ * marked_out[e] = 1 for every edge the reference removes; *n_pairs = its return value.
+ * RALA_B200_ERR_LIMIT: the hash-chunk limit above. */
 int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes, uint64_t n_edges,
                                 const rala_edge_t* edges, uint8_t* marked_out, uint64_t* n_pairs);
 

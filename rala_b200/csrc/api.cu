@@ -213,8 +213,6 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
     CU(ctx, g->col_eid.reserve((size_t) edge_cap * 4));
     CU(ctx, g->T.reserve(align_up(edge_cap, 256)));
     CU(ctx, g->marked.reserve(align_up(edge_cap, 256)));
-    g->heavy_cap = edge_cap / 16 + 4096;
-    CU(ctx, g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 3));
     return RALA_B200_OK;
 }
 
@@ -388,6 +386,8 @@ extern "C" int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* 
         CU(ctx, g->row_ptr.reserve(((size_t) g->n_nodes_max + 8) * 4));
         CU(ctx, g->cursor.reserve(((size_t) g->n_nodes_max + 8) * 4));
         CU(ctx, g->slot_degree.reserve(((size_t) g->n_nodes_max + 8) * 4));
+        g->heavy_cap = g->n_nodes_max;   // one entry per node (HeavyItems)
+        CU(ctx, g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 2));
         int rc = reserve_scan_pool(g);
         if (rc) return rc;
     }
@@ -729,8 +729,7 @@ extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
 
 static int run_transitive(rala_b200_graph* g) {
     rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, zero_counter(g, C_PAIRS, 2));   // C_PAIRS, C_HEAVY
-    CU(ctx, zero_counter(g, C_HOP_LO, 2));
+    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
     CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 64, ctx->L.stream));
     CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));
     launch_transitive(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->heavy_view(), g->work_counter.as<uint32_t>(),
@@ -780,7 +779,7 @@ static int run_eager(rala_b200_graph* g) {
 // operations (27 kernels, memsets, small copies) are identical from run to run: the second run with a key is
 // captured into a CUDA graph and later runs replay it with one launch.
 struct RunKey {
-    const void *rec, *recs, *piles, *piles_initial, *events, *segs, *dbuf, *edges, *col, *scan_pool, *tiles, *ovl0, *inl0, *hills;
+    const void *rec, *recs, *piles, *piles_initial, *events, *segs, *dbuf, *edges, *col, *scan_pool, *tiles, *ovl0, *inl0, *hills, *heavy;
     const void *out_edges, *out_marked;
     uint32_t n_rec, n_piles, n_hills, cap, ev_cap, edge_cap, heavy_cap, t0, out_edges_cap, out_marked_cap;
     int world, rank, coop_blocks;
@@ -809,6 +808,7 @@ static RunKey run_key(const rala_b200_graph* g) {
     k.rec = g->rec.p; k.recs = g->recs.buf.p; k.piles = g->piles.p; k.piles_initial = g->piles_initial.p;
     k.events = g->events.p; k.segs = g->segs.p; k.dbuf = g->dbuf.p; k.edges = g->edges.p; k.col = g->col.p;
     k.scan_pool = g->scan_pool.p; k.tiles = g->tiles.p; k.ovl0 = g->ovl[0].buf.p; k.inl0 = g->inl[0].buf.p; k.hills = g->hills.p;
+    k.heavy = g->heavy.p;   // sized from n_piles, which can shrink and grow back without a new allocation
     k.n_rec = g->n_rec; k.n_piles = g->n_piles; k.n_hills = g->n_hills; k.cap = g->cap; k.ev_cap = g->ev_cap;
     k.edge_cap = g->edge_cap; k.heavy_cap = g->heavy_cap; k.t0 = g->t0;
     k.out_edges = g->out_edges; k.out_marked = g->out_marked; k.out_edges_cap = g->out_edges_cap; k.out_marked_cap = g->out_marked_cap;
@@ -896,9 +896,9 @@ int read_counters(rala_b200_graph* g, uint32_t* h) {
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
     if (g->scan_pool_exhausted)
         return fail(ctx, RALA_B200_ERR_LIMIT, "the look-back status pool was exhausted inside a stage (%zu words): the results are void", g->scan_pool_words);
-    if (h[C_OVERFLOW] || (g->state >= 2 && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap || h[C_HILL] > g->cap || h[C_HEAVY] > g->heavy_cap)
-        return fail(ctx, RALA_B200_ERR_LIMIT, "a device list overflowed its capacity (cap=%u events=%u hills=%u heavy=%u/%u)",
-                    g->cap, h[C_EV], h[C_HILL], h[C_HEAVY], g->heavy_cap);
+    if (h[C_OVERFLOW] || (g->state >= 2 && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap || h[C_HILL] > g->cap)
+        return fail(ctx, RALA_B200_ERR_LIMIT, "a device list overflowed its capacity (cap=%u events=%u hills=%u heavy items=%u)",
+                    g->cap, h[C_EV], h[C_HILL], h[C_HEAVY]);
     return RALA_B200_OK;
 }
 
@@ -1141,7 +1141,7 @@ extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes,
     g->n_piles = (n_nodes + 1) / 2;
     g->n_nodes_max = n_nodes;
     g->edge_cap = (uint32_t) n_edges;
-    g->heavy_cap = g->edge_cap / 16 + 4096;
+    g->heavy_cap = n_nodes;
     DevBuf rows;
     cudaError_t e = rows.reserve((size_t) n_edges * 12);
     if (e == cudaSuccess) e = g->edges.reserve(align_up((size_t) g->edge_cap * 4, 256) * 3);
@@ -1149,7 +1149,7 @@ extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes,
     if (e == cudaSuccess) e = g->col_eid.reserve((size_t) g->edge_cap * 4);
     if (e == cudaSuccess) e = g->T.reserve(align_up(g->edge_cap, 256));
     if (e == cudaSuccess) e = g->marked.reserve(align_up(g->edge_cap, 256));
-    if (e == cudaSuccess) e = g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 3);
+    if (e == cudaSuccess) e = g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 2);
     if (e == cudaSuccess) e = g->row_ptr.reserve(((size_t) n_nodes + 8) * 4);
     if (e == cudaSuccess) e = g->cursor.reserve(((size_t) n_nodes + 8) * 4);
     g->scan_pool_words = 4 * (tiles_of((uint64_t) n_nodes + 1) + 8);
@@ -1194,7 +1194,9 @@ extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes,
     CUX(cudaMemcpyAsync(h, g->counters.p, sizeof(h), cudaMemcpyDeviceToHost, s));
     CUX(cudaStreamSynchronize(s));
 #undef CUX
-    if (h[C_OVERFLOW] || h[C_HEAVY] > g->heavy_cap) return cleanup(fail(ctx, RALA_B200_ERR_LIMIT, "heavy work list overflow"));
+    if (h[C_OVERFLOW])
+        return cleanup(fail(ctx, RALA_B200_ERR_LIMIT, "transitive_reduce: more than 2048 destinations of one node in one hash chunk, "
+                                                      "or more than 2^32 heavy work items"));
     if (n_pairs) *n_pairs = h[C_PAIRS];
     return cleanup(RALA_B200_OK);
 }
@@ -1326,8 +1328,7 @@ extern "C" int rala_b200_graph_phase_transitive(rala_b200_graph* g) {
     if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "transitive: build first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_TRANSITIVE));
-    CU(ctx, zero_counter(g, C_PAIRS, 2));
-    CU(ctx, zero_counter(g, C_HOP_LO, 2));
+    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
     CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 64, ctx->L.stream));
     launch_node_range(ctx->L, g->graph_view(), g->cnt(), (uint32_t) g->rank, (uint32_t) g->world, g->work_counter.as<uint32_t>() + 4);
     CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));

@@ -21,14 +21,15 @@ enum Counter {
     C_DOVETAILS,    // dovetail overlaps = edges / 2
     C_EDGES,        // edges_.size()
     C_PAIRS,        // marked pairs
-    C_HEAVY,        // heavy work items of the transitive pass
-    C_OVERFLOW,     // some list hit its capacity
+    C_HEAVY_NODES, C_HEAVY,   // nodes handed to k_transitive_heavy and their work items (one 64-bit word, see heavy_append)
     C_HOP_LO, C_HOP_HI,   // two-hop visits (64-bit)
     C_TBASE_OVL, C_TBASE_INL,     // multi-GPU: global time bases of the local lists in the final pass
     C_EV_FIRST, C_ROUNDS_FIRST,   // events / rounds of the first-pass resolution (C_EV / C_ROUNDS are reused by the final pass)
+    C_OVERFLOW,     // some list hit its capacity
     C_LIST0,        // 16 rotating list-count slots follow
     C_COUNT = C_LIST0 + 16
 };
+static_assert(C_HEAVY_NODES % 2 == 0 && C_HOP_LO % 2 == 0, "64-bit counters sit on 8-byte boundaries");
 
 struct Launch {
     cudaStream_t stream;
@@ -160,8 +161,10 @@ void launch_build_csr(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t e
                       unsigned long long* status, uint32_t* ticket);
 
 // transitive.cu
+// nodes of the transitive pass that one block per work item takes (k_transitive_heavy): one entry per node, so a list
+// of n_nodes_max entries never overflows; unit_base[i] = work items of the entries before i (ascending in i)
 struct HeavyItems {
-    uint32_t *node, *hash_chunk, *nbr_chunk;
+    uint32_t *node, *unit_base;
     uint32_t cap;
 };
 void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t edge_cap, HeavyItems heavy,

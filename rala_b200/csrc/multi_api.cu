@@ -621,8 +621,7 @@ static int phase_h_transitive(rala_b200_multi* m, FabricRank& fr) {
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
     MCU(m, begin_stage(g, ST_TRANSITIVE));
-    MCU(m, zero_counter(g, C_PAIRS, 2));
-    MCU(m, zero_counter(g, C_HOP_LO, 2));
+    MCU(m, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
     MCU(m, cudaMemsetAsync(g->work_counter.p, 0, 64, L.stream));
     GraphArrays ga = g->graph_view();
     ga.row_ptr = fr.sec<uint32_t>(fr.A.row_ptr);
@@ -849,7 +848,6 @@ extern "C" int rala_b200_multi_counts(rala_b200_multi* m, rala_b200_multi_counts
         out->n_two_hop += (uint64_t) c[C_HOP_LO] | ((uint64_t) c[C_HOP_HI] << 32);
         out->n_transitive_pairs += c[C_PAIRS];
         out->n_heavy_items += c[C_HEAVY];
-        if (c[C_HEAVY] > fr.g->heavy_cap) out->fabric_error |= (uint32_t) FE_INBOX;
     }
     if (out->fabric_error)
         return mfail(m, RALA_B200_ERR_LIMIT, "the last step did not fit its exchange buffers or rounds (fabric error bits %u): plan again",

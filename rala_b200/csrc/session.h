@@ -174,8 +174,7 @@ struct rala_b200_graph {
         HeavyItems h;
         size_t colb = align_up((size_t) heavy_cap * 4, 256);
         h.node = (uint32_t*) heavy.as<char>();
-        h.hash_chunk = (uint32_t*) (heavy.as<char>() + colb);
-        h.nbr_chunk = (uint32_t*) (heavy.as<char>() + 2 * colb);
+        h.unit_base = (uint32_t*) (heavy.as<char>() + colb);
         h.cap = heavy_cap;
         return h;
     }

@@ -14,7 +14,8 @@
 //                node of an overlap graph, mean out-degree ~9; a full warp per such node leaves 3/4 of
 //                the lanes idle during set-up and pays the per-node overhead four times as often)
 //   light path : one warp per node      (16 < deg <= 64 and <= 32768 two-hop visits)
-//   heavy path : one block per (node, hash chunk of 1024 neighbours, stream chunk of 256 neighbours)
+//   heavy path : one block per (node, hash chunk of 1024 neighbours, stream chunk of 256 neighbours); the two kernels
+//                above hand it NODES, and its blocks map onto the work items of each node through a prefix
 // Measured alternatives that lost (profiles/README.md): one thread per edge with a linear or (rows sorted)
 // binary-search membership test, and the group path streaming one row N+(b) at a time: both expose the
 // latency of dependent L2 gathers; the flattened stream keeps 4 independent gathers in flight per lane.
@@ -80,7 +81,8 @@ __device__ __forceinline__ bool table_insert_bounded(uint32_t* keys, unsigned lo
     return false;
 }
 
-// returns the slot of key or kEmpty
+// returns the slot of key or kEmpty.  The light path's table has at least 2d slots for its d keys: it is at most half
+// full, so the probe always meets an empty slot.
 __device__ __forceinline__ uint32_t table_find(const uint32_t* keys, uint32_t mask, uint32_t log2cap, uint32_t key) {
     uint32_t s = hash_slot(key, log2cap);
     while (true) {
@@ -89,6 +91,49 @@ __device__ __forceinline__ uint32_t table_find(const uint32_t* keys, uint32_t ma
         if (k == kEmpty) return kEmpty;
         s = (s + 1u) & mask;
     }
+}
+
+// same, but gives up (returns kEmpty: the key is absent) after probing the whole table.  A hash chunk of the heavy path
+// can hold exactly kHeavyCap keys, which leaves no empty slot to stop at.
+__device__ __forceinline__ uint32_t table_find_bounded(const uint32_t* keys, uint32_t mask, uint32_t log2cap, uint32_t key) {
+    uint32_t s = hash_slot(key, log2cap);
+    for (uint32_t probes = 0; probes <= mask; ++probes) {
+        const uint32_t k = keys[s];
+        if (k == key) return s;
+        if (k == kEmpty) return kEmpty;
+        s = (s + 1u) & mask;
+    }
+    return kEmpty;
+}
+
+// Hands node a to k_transitive_heavy as `units` work items.  The node count (low word) and the item count (high word)
+// move in ONE 64-bit atomic, so entry i's unit base is the sum of the items of entries 0 .. i-1: the bases ascend with
+// the entry index, and k_transitive_heavy finds the entry of an item by search.  A node is handed over at most once,
+// so the node count stays below heavy.cap (= n_nodes_max); more than 2^32 items in all is an overflow.
+__device__ __forceinline__ void heavy_append(HeavyItems heavy, uint32_t* counters, uint32_t a, unsigned long long units) {
+    const unsigned long long old =
+        atomicAdd(reinterpret_cast<unsigned long long*>(counters + C_HEAVY_NODES), (units << 32) | 1ull);
+    const uint32_t i = (uint32_t) old;
+    if (i < heavy.cap && (old >> 32) + units <= 0xFFFFFFFFull) {
+        heavy.node[i] = a;
+        heavy.unit_base[i] = (uint32_t) (old >> 32);
+    } else {
+        counters[C_OVERFLOW] = 1u;
+    }
+}
+
+// largest i < n with base[i] <= u (base[0] == 0 <= u, base ascending): a 32-ary search, one probe per lane and
+// ceil(log32 n) dependent loads; every lane of the warp returns the same i
+__device__ __forceinline__ uint32_t heavy_entry(const uint32_t* __restrict__ base, uint32_t n, uint32_t u, uint32_t lane) {
+    uint32_t lo = 0, hi = n;   // base[lo] <= u, and hi == n or base[hi] > u
+    while (hi - lo > 1) {
+        const uint32_t step = (hi - lo + 31) / 32;
+        const uint32_t p = lo + lane * step;
+        const uint32_t le = __ballot_sync(0xFFFFFFFFu, p < hi && base[p] <= u);   // lanes 0 .. k, lane 0 always
+        lo += (31 - __clz(le)) * step;
+        hi = min(hi, lo + step);
+    }
+    return lo;
 }
 
 
@@ -190,16 +235,7 @@ __global__ void __launch_bounds__(kLightWarps * 32, kGroupMinBlocks) k_transitiv
             }
             __syncwarp();
             if (act && W > kGroupMaxVisits) {   // short row, very long rows behind it: give the node to a block
-                if (gl == 0) {
-                    const uint32_t hb = atomicAdd(&counters[C_HEAVY], 1u);
-                    if (hb < heavy.cap) {
-                        heavy.node[hb] = a;
-                        heavy.hash_chunk[hb] = 0;
-                        heavy.nbr_chunk[hb] = 0;
-                    } else {
-                        counters[C_OVERFLOW] = 1u;
-                    }
-                }
+                if (gl == 0) heavy_append(heavy, counters, a, 1ull);
                 act = false;
             }
             // ---- rank sort by (destination, edge id): composites are distinct, pads (~0) sort behind every edge ----
@@ -311,20 +347,9 @@ __global__ void __launch_bounds__(kLightWarps * 32) k_transitive_light(
             const uint32_t a = base + l;
             const uint32_t ra0 = __shfl_sync(0xFFFFFFFFu, r0, l);
             const uint32_t d = __shfl_sync(0xFFFFFFFFu, deg, l);
-            if (d > (uint32_t) kLightMaxDeg) {
-                const uint32_t nca = num_hash_chunks(d), ncb = (d + kHeavyNbrChunk - 1) / kHeavyNbrChunk;
-                uint32_t hb = 0;
-                if (lane == 0) hb = atomicAdd(&counters[C_HEAVY], nca * ncb);
-                hb = __shfl_sync(0xFFFFFFFFu, hb, 0);
-                for (uint32_t i = lane; i < nca * ncb; i += 32) {
-                    if (hb + i < heavy.cap) {
-                        heavy.node[hb + i] = a;
-                        heavy.hash_chunk[hb + i] = i / ncb;
-                        heavy.nbr_chunk[hb + i] = i % ncb;
-                    } else {
-                        counters[C_OVERFLOW] = 1u;
-                    }
-                }
+            if (d > (uint32_t) kLightMaxDeg) {   // one work item per (hash chunk, stream chunk)
+                if (lane == 0)
+                    heavy_append(heavy, counters, a, (unsigned long long) num_hash_chunks(d) * ((d + kHeavyNbrChunk - 1) / kHeavyNbrChunk));
                 continue;
             }
             // table capacity: power of two >= 2d, at least 16
@@ -357,20 +382,8 @@ __global__ void __launch_bounds__(kLightWarps * 32) k_transitive_light(
             const uint32_t W = carry;
             if (lane == 0) S.noff[d] = W;
             __syncwarp();
-            if (W > kLightMaxVisits) {   // few neighbours but very long rows behind them: give it to a block
-                const uint32_t ncb = (d + kHeavyNbrChunk - 1) / kHeavyNbrChunk;   // == 1
-                uint32_t hb = 0;
-                if (lane == 0) hb = atomicAdd(&counters[C_HEAVY], ncb);
-                hb = __shfl_sync(0xFFFFFFFFu, hb, 0);
-                if (lane < ncb) {
-                    if (hb + lane < heavy.cap) {
-                        heavy.node[hb + lane] = a;
-                        heavy.hash_chunk[hb + lane] = 0;
-                        heavy.nbr_chunk[hb + lane] = lane;
-                    } else {
-                        counters[C_OVERFLOW] = 1u;
-                    }
-                }
+            if (W > kLightMaxVisits) {   // few neighbours but very long rows behind them: give it to a block (one item)
+                if (lane == 0) heavy_append(heavy, counters, a, 1ull);
                 __syncwarp();
                 continue;
             }
@@ -428,12 +441,17 @@ __global__ void __launch_bounds__(kHeavyThreads) k_transitive_heavy(
     uint8_t* __restrict__ T, HeavyItems heavy, uint32_t* __restrict__ counters) {
     __shared__ HeavySmem S;
     const uint32_t tid = threadIdx.x, lane = lane_id(), warp = warp_id();
-    const uint32_t n_items = min(counters[C_HEAVY], heavy.cap);
+    const uint32_t n_nodes = min(counters[C_HEAVY_NODES], heavy.cap);
+    const uint32_t n_items = n_nodes ? counters[C_HEAVY] : 0u;
     unsigned long long visits = 0;
     for (uint32_t item = blockIdx.x; item < n_items; item += gridDim.x) {
-        const uint32_t a = heavy.node[item], ca = heavy.hash_chunk[item], cb = heavy.nbr_chunk[item];
+        // node a's items: hash chunk ca (slow) x stream chunk cb (fast)
+        const uint32_t k = heavy_entry(heavy.unit_base, n_nodes, item, lane);
+        const uint32_t a = heavy.node[k], local = item - heavy.unit_base[k];
         const uint32_t ra0 = row_ptr[a], d = row_ptr[a + 1] - ra0;
-        const uint32_t nca = num_hash_chunks(d);
+        const uint32_t nca = num_hash_chunks(d), ncb = (d + kHeavyNbrChunk - 1) / kHeavyNbrChunk;
+        const uint32_t ca = local / ncb, cb = local % ncb;
+        if (ca >= nca) continue;   // only behind an overflow (the result is refused): the block agrees, no barrier is skipped
         const uint32_t k0 = cb * kHeavyNbrChunk, k1 = min(d, k0 + kHeavyNbrChunk), nb = k1 - k0;
         uint32_t log2cap = 4;
         while ((1u << log2cap) < 2u * min(d, (uint32_t) kHeavyHashChunk)) ++log2cap;
@@ -448,7 +466,7 @@ __global__ void __launch_bounds__(kHeavyThreads) k_transitive_heavy(
             const uint2 e = col[ra0 + i];
             if (hash_chunk_of(e.x, nca) != ca) continue;
             if (!table_insert_bounded(S.keys, S.vals, mask, log2cap, e.x, ((unsigned long long) col_eid[ra0 + i] << 32) | e.y))
-                counters[C_OVERFLOW] = 1u;   // > 2048 distinct destinations hashed into one chunk: reported as an error
+                counters[C_OVERFLOW] = 1u;   // > kHeavyCap distinct destinations hashed into one chunk: reported as an error
         }
         uint32_t dg = 0;
         if (tid < nb) {
@@ -490,7 +508,7 @@ __global__ void __launch_bounds__(kHeavyThreads) k_transitive_heavy(
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 if (ok[u]) {
-                    const uint32_t s = table_find(S.keys, mask, log2cap, e[u].x);
+                    const uint32_t s = table_find_bounded(S.keys, mask, log2cap, e[u].x);
                     if (s != kEmpty && !S.hit[s]) {
                         if (comparable(lab[u] + e[u].y, (uint32_t) S.vals[s])) S.hit[s] = 1;
                     }
