@@ -301,6 +301,11 @@ int rala_b200_graph_set_kept_overlaps(rala_b200_graph* g, const rala_ovl_t* kept
 int rala_b200_graph_get_seq_to_node(rala_b200_graph* g, uint32_t* out /* n_piles; 0xFFFFFFFF = dead */);
 int rala_b200_graph_get_edges(rala_b200_graph* g, rala_edge_t* out /* n_edges */);
 int rala_b200_graph_get_marked(rala_b200_graph* g, uint8_t* out /* n_edges */);
+/* The CSR adjacency build writes for the transitive pass (read-only there, so the same after transitive): node v's out-edges
+ * are slots row_ptr_out[v] .. row_ptr_out[v + 1] of col_out (pairs {destination node, length}) and col_eid_out (their edge
+ * ids), in no particular order inside a row.  row_ptr_out: n_nodes + 1 words, col_out: 2 x n_edges, col_eid_out: n_edges.
+ * After build (RALA_B200_ERR_STATE before); synchronises the session's stream. */
+int rala_b200_graph_get_csr(rala_b200_graph* g, uint32_t* row_ptr_out, uint32_t* col_out, uint32_t* col_eid_out);
 /* Adjacency VIEW, built on the device: off_out[v] .. off_out[v + 1] delimit, in ids_out, the ids of node v's out-edges (which = 0:
  * suffix_edges_, graph.cpp:603 / 625) or in-edges (which = 1: prefix_edges_, :605-606 / 622-624) in ascending edge id, as the
  * reference keeps them; with skip_marked != 0 (after transitive) without the removed edges: the adjacency

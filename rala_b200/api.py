@@ -104,6 +104,7 @@ EXPORTS = [
     "rala_b200_graph_get_marked", "rala_b200_graph_stage_ms", "rala_b200_graph_set_kept_overlaps",
     "rala_b200_graph_use_cuda_graph", "rala_b200_graph_set_overlaps_columns", "rala_b200_graph_set_outputs",
     "rala_b200_graph_set_overlaps_packed", "rala_b200_multi_set_overlaps_packed", "rala_b200_graph_get_adjacency",
+    "rala_b200_graph_get_csr",
     # multi-GPU phases
     "rala_b200_create_on_stream", "rala_b200_graph_set_shard", "rala_b200_graph_phase_events",
     "rala_b200_graph_phase_resolve", "rala_b200_graph_phase_survivors", "rala_b200_graph_phase_emit_edges",
@@ -567,6 +568,16 @@ class Graph:
         n = C.c_uint64(0)
         self._call("rala_b200_graph_get_adjacency", C.c_int(which), C.c_int(1 if skip_marked else 0), _ptr(off), _ptr(ids), C.byref(n))
         return off, ids[:int(n.value)]
+
+    def csr(self):
+        """(row_ptr (n_nodes + 1), col (n_edges, 2) = (destination, length), col_eid (n_edges)): the CSR rows build wrote
+        for the transitive pass; slot order inside a row is arbitrary."""
+        c = self.counts()
+        row_ptr = np.zeros(c["n_nodes"] + 1, dtype=np.uint32)
+        col = np.zeros((max(c["n_edges"], 1), 2), dtype=np.uint32)
+        col_eid = np.zeros(max(c["n_edges"], 1), dtype=np.uint32)
+        self._call("rala_b200_graph_get_csr", _ptr(row_ptr), _ptr(col), _ptr(col_eid))
+        return row_ptr, col[:c["n_edges"]], col_eid[:c["n_edges"]]
 
     def stage_ms(self) -> dict:
         ms = (C.c_float * N_STAGES)()

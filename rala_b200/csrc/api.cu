@@ -1019,6 +1019,24 @@ extern "C" int rala_b200_graph_get_seq_to_node(rala_b200_graph* g, uint32_t* out
     return RALA_B200_OK;
 }
 
+// the CSR adjacency build wrote for the transitive pass (k_scan_piles / k_emit_edges); the transitive pass only reads it
+extern "C" int rala_b200_graph_get_csr(rala_b200_graph* g, uint32_t* row_ptr_out, uint32_t* col_out, uint32_t* col_eid_out) {
+    if (!g || !row_ptr_out || !col_out || !col_eid_out) return RALA_B200_ERR_ARG;
+    rala_b200_ctx* ctx = g->ctx;
+    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "get_csr: build first");
+    uint32_t h[C_COUNT];
+    int rc = read_counters(g, h);
+    if (rc) return rc;
+    const uint32_t n_nodes = h[C_NODES], n_edges = h[C_EDGES];
+    CU(ctx, cudaMemcpyAsync(row_ptr_out, g->row_ptr.p, ((size_t) n_nodes + 1) * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
+    if (n_edges) {
+        CU(ctx, cudaMemcpyAsync(col_out, g->col.p, (size_t) n_edges * 8, cudaMemcpyDeviceToHost, ctx->L.stream));
+        CU(ctx, cudaMemcpyAsync(col_eid_out, g->col_eid.p, (size_t) n_edges * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
+    }
+    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
+    return RALA_B200_OK;
+}
+
 extern "C" int rala_b200_graph_get_edges(rala_b200_graph* g, rala_edge_t* out) {
     if (!g || !out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
