@@ -143,6 +143,43 @@ int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* n
                         const char* text, uint64_t n_bytes, uint32_t* cols_out, uint64_t cap, rala_b200_paf_stats_t* stats,
                         float* device_ms);
 
+/* MHAP text on the device (SURVEY.md 8(f) row 2): bioparser's MhapParser and the reference's MHAP Overlap constructor
+ * (overlap.cpp:12-20, SURVEY.md 8(a) row a1).  Reads: read_len[i] = the sequence length of read i, in the order given to set_reads; MHAP
+ * names reads by number, so no name table is built.
+ * Text contract (anything else is refused with RALA_B200_ERR_ARG and a message naming the 1-based line and field; the
+ * smallest offending line is reported and, within it, the smallest field):
+ *   - lines end in '\n' (the last one may lack it); an empty line is refused;
+ *   - fields are separated by single spaces (0x20), at least 12 of them; fields after the 12th are never read;
+ *   - a '\r' that ends field 12 at the end of the line is dropped (CRLF files); anywhere else it is an ordinary byte;
+ *   - fields 3 (error) and 4 (shared minmers) are never read and may be empty;
+ *   - fields 1 and 2 are read ids, plain decimal with 1 <= id <= n_reads: a_id = field 1 - 1, b_id = field 2 - 1.  Id 0 or
+ *     an id above n_reads is refused as "not a read id" (the reference indexes its sequences with it), so an MHAP
+ *     record is never unresolved;
+ *   - fields 5 (a_rc) and 9 (b_rc) are exactly "0" or "1", anything else is refused; orientation = a_rc != b_rc;
+ *   - fields 6, 7, 10, 11 (a_begin, a_end, b_begin, b_end) and 8, 12 (the read lengths) are plain decimal below 2^32,
+ *     leading zeros allowed; a non-digit or a value >= 2^32 is refused as in the PAF contract;
+ *   - coordinates are stored as given, on either strand (no flip when a_rc = 1).  Restated from SURVEY a1, NOT pinned by
+ *     a golden: n_query_rc counts the records this rule decided;
+ *   - Overlap::length() = max(a_end - a_begin, b_end - b_begin), each difference mod 2^32 (the constructor's uint32_t
+ *     arithmetic); the duplicate filter reads it;
+ *   - fields 8 and 12 are checked against read_len as PAF columns 2 and 7 are.
+ * Upload as for PAF: chunks of RALA_B200_PAF_CHUNK_BYTES cut behind their last '\n' (a longer line: RALA_B200_ERR_LIMIT),
+ * page-locked caller memory in place.  No valid line is shorter than 22 bytes (ten one-byte fields, two empty ones,
+ * eleven spaces, '\n'), which sizes the record buffers. */
+typedef struct {
+    uint64_t n_records;              /* lines = records, file order */
+    uint64_t n_length_mismatch;      /* records whose field 8 or 12 differs from read_len */
+    uint64_t first_length_mismatch;  /* index of the first of them; UINT64_MAX when there is none */
+    uint64_t n_query_rc;             /* records with a_rc = 1: their coordinates were taken as given */
+    uint64_t n_bytes;                /* text bytes */
+    uint64_t n_chunks;               /* upload chunks the text took */
+} rala_b200_mhap_stats_t;
+/* Stateless form: parse only, no duplicate filter.  cols_out holds 7 columns of cap words: a_id (INVALID never set),
+ * b_id | orientation << 31, a_begin, a_end, b_begin, b_end, length.  Length mismatches are only counted.  device_ms
+ * (nullable) receives the kernel time of the line scan and the parse (uploads excluded). */
+int rala_b200_parse_mhap(rala_b200_ctx* ctx, const uint32_t* read_len, uint32_t n_reads, const char* text, uint64_t n_bytes,
+                         uint32_t* cols_out, uint64_t cap, rala_b200_mhap_stats_t* stats, float* device_ms);
+
 /* The pile table from the overlap records (SURVEY.md 8(f) row 1, second half): the coverage half of Graph::initialize
  * (store_overlap_bounds + Pile::add_layers, graph.cpp:305-321, pile.cpp:274-297), the valid region and pile liveness
  * (Pile::find_valid_region, pile.cpp:307, 329) and the median (Pile::find_median).  The rule, as restated from the
@@ -235,7 +272,7 @@ int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* piles, cons
                               uint32_t n_piles);
 /* The read names and lengths the PAF text is resolved against (name_to_id_ of Graph::initialize, graph.cpp:253-271, and
  * the sequence lengths transmute checks, overlap.cpp:54-59, 73-78); once per session.  Layout and refusals as
- * rala_b200_parse_paf.  The name table stays on the device. */
+ * rala_b200_parse_paf.  The name table stays on the device.  MHAP text uses only the lengths and their order. */
 int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads);
 /* PAF text in FILE ORDER -> the session's records, replacing the host parse and transmute of graph.cpp:443-451 and the
  * records set_overlaps* would receive: the text is parsed as rala_b200_parse_paf does, the duplicate filter of
@@ -245,8 +282,14 @@ int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint6
  * reaches it (overlap.cpp:54-59, 73-78); the library is stricter and also refuses one whose pile is already dead.  After
  * a refused call the session holds no records (classify needs a new set_overlaps*).  stats: nullable. */
 int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats);
+/* MHAP text in FILE ORDER -> the session's records, as set_overlaps_paf does for PAF: parsed as rala_b200_parse_mhap,
+ * then the duplicate filter, whose drops leave INVALID.  Needs set_reads first; only its lengths and count are used (ids
+ * are numbers).  A record that stays valid while field 8 or 12 differs from set_reads' length is refused, naming its line.
+ * After a refused call the session holds no records.  stats: nullable. */
+int rala_b200_graph_set_overlaps_mhap(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_mhap_stats_t* stats);
 /* The pile table of the reads given to set_reads, built on the device (rule and refusals as rala_b200_build_piles) from
- * the records of the last successful set_overlaps_paf, counted as parsed: before the duplicate filter.  It is installed as
+ * the records of the last successful set_overlaps_paf or set_overlaps_mhap, counted as parsed: before the duplicate
+ * filter.  A refused record is named by its line in that text ("PAF line N" / "MHAP line N").  It is installed as
  * set_piles(piles, NULL, n_reads) would (flags 0; the hills are left as they are) and the next classify / run uses it.
  * RALA_B200_ERR_STATE after set_overlaps / _columns / _packed (their records have the filter folded in) or set_reads.
  * A refused call changes nothing in the session.  stats: nullable. */

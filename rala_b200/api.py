@@ -49,7 +49,15 @@ class PafStats(C.Structure):
         return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
-PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES
+class MhapStats(C.Structure):
+    _fields_ = [("n_records", C.c_uint64), ("n_length_mismatch", C.c_uint64), ("first_length_mismatch", C.c_uint64),
+                ("n_query_rc", C.c_uint64), ("n_bytes", C.c_uint64), ("n_chunks", C.c_uint64)]
+
+    def as_dict(self):
+        return {k: int(getattr(self, k)) for k, _ in self._fields_}
+
+
+PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES (the MHAP reader uses the same chunks)
 
 
 class PileStats(C.Structure):
@@ -61,12 +69,12 @@ class PileStats(C.Structure):
 
 
 def _text(text):
-    """PAF text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
+    """PAF / MHAP text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
     if isinstance(text, (bytes, bytearray, memoryview)):
         text = np.frombuffer(text, np.uint8)
     if hasattr(text, "data_ptr"):
         if not text.is_contiguous() or text.device.type != "cpu" or text.element_size() != 1:
-            raise RalaB200Error("PAF text must be a contiguous uint8 CPU tensor")
+            raise RalaB200Error("overlap text must be a contiguous uint8 CPU tensor")
         return text, int(text.numel())
     text = np.ascontiguousarray(text, dtype=np.uint8).reshape(-1)
     return text, int(text.shape[0])
@@ -94,6 +102,7 @@ EXPORTS = [
     "rala_b200_launch_count", "rala_b200_event_record", "rala_b200_event_elapsed_ms", "rala_b200_synchronize",
     "rala_b200_trim_classify", "rala_b200_transitive_reduce", "rala_b200_filter_duplicates",
     "rala_b200_parse_paf", "rala_b200_graph_set_reads", "rala_b200_graph_set_overlaps_paf",
+    "rala_b200_parse_mhap", "rala_b200_graph_set_overlaps_mhap",
     "rala_b200_build_piles", "rala_b200_graph_build_piles", "rala_b200_graph_get_medians", "rala_b200_graph_get_coverage_runs",
     "rala_b200_graph_create", "rala_b200_graph_destroy", "rala_b200_graph_set_overlaps",
     "rala_b200_graph_set_piles", "rala_b200_graph_set_hills", "rala_b200_graph_classify",
@@ -328,6 +337,20 @@ class Context:
         out = np.ascontiguousarray(cols[:, :stats["n_records"]])
         return (out, stats, float(ms.value)) if with_time else (out, stats)
 
+    def parse_mhap(self, text, read_len, with_time: bool = False):
+        """MHAP text -> (columns (7, n) uint32: a_id, b_id | orientation << 31, a_begin, a_end, b_begin, b_end, length
+        (the longer span); stats dict).  Ids are 1-based in the text, checked against len(read_len); no duplicate filter."""
+        buf, n_bytes = _text(text)
+        rl = _np(read_len, np.uint32)
+        cap = n_bytes // 22 + 2
+        cols = np.zeros((7, cap), dtype=np.uint32)
+        st, ms = MhapStats(), C.c_float(0.0)
+        self.check(self.lib.rala_b200_parse_mhap(self.handle, _ptr(rl), C.c_uint32(rl.shape[0]), _ptr(buf), C.c_uint64(n_bytes),
+                                                 _ptr(cols), C.c_uint64(cap), C.byref(st), C.byref(ms)), "parse_mhap")
+        stats = st.as_dict()
+        out = np.ascontiguousarray(cols[:, :stats["n_records"]])
+        return (out, stats, float(ms.value)) if with_time else (out, stats)
+
     def build_piles(self, columns, read_len, with_time: bool = False):
         """Graph::initialize's coverage half on the device: six host columns in the set_overlaps_columns layout (bit 31 of
         a_id = unresolved record; records the duplicate filter drops still count) + the read lengths -> (piles (n_reads, 2)
@@ -408,7 +431,8 @@ class Graph:
         return self
 
     def set_reads(self, names, read_len):
-        """Read names (list of bytes, or (blob, name_end)) and sequence lengths the PAF text is resolved against."""
+        """Read names (list of bytes, or (blob, name_end)) and sequence lengths the PAF text is resolved against; MHAP text
+        uses the lengths and their order (id k + 1 = read k)."""
         blob, ends, rl = _names(names, read_len)
         self._call("rala_b200_graph_set_reads", _ptr(blob), _ptr(ends), _ptr(rl), C.c_uint32(ends.shape[0]))
         self._n_reads = int(ends.shape[0])
@@ -422,8 +446,16 @@ class Graph:
         self._call("rala_b200_graph_set_overlaps_paf", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
         return st.as_dict()
 
+    def set_overlaps_mhap(self, text) -> dict:
+        """MHAP text in file order -> the session's records (parse, id check, duplicate filter on the device); returns the
+        stats (records, read-length mismatches, records with a_rc = 1, bytes, upload chunks)."""
+        buf, n_bytes = _text(text)
+        st = MhapStats()
+        self._call("rala_b200_graph_set_overlaps_mhap", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
+        return st.as_dict()
+
     def build_piles(self) -> dict:
-        """The pile table from the records of the last set_overlaps_paf, built on the device and installed as
+        """The pile table from the records of the last set_overlaps_paf / _mhap, built on the device and installed as
         set_piles(piles) would (flags 0, hills untouched); returns the stats."""
         st = PileStats()
         self._call("rala_b200_graph_build_piles", C.byref(st))

@@ -232,7 +232,7 @@ static int reserve_scan_pool(rala_b200_graph* g) {
 int reserve_for_records(rala_b200_graph* g, uint64_t n) {
     rala_b200_ctx* ctx = g->ctx;
     g->n_rec = (uint32_t) n;
-    g->paf_records = false;   // set_overlaps_paf sets it again once its records are in place
+    g->text_records = kTextNone;   // set_overlaps_paf / _mhap set it again once their records are in place
     CU(ctx, g->recs.reserve((uint32_t) ((n + 3) / 4 * 4 + 4)));
     uint32_t cap = (uint32_t) align_up((size_t) n, 128);
     if (cap < 1024) cap = 1024;

@@ -1,16 +1,20 @@
-// paf.cu — PAF text in host memory -> the graph session's device-resident records (SURVEY.md 8(f) row 2): the parse of
-// bioparser's PafParser (graph.cpp:443-451 runs it once more for every construct pass) and the name -> id lookup of
-// Overlap::transmute (overlap.cpp:36-82) on the device, followed by the front end's duplicate filter (frontend.cu).
+// paf.cu — PAF or MHAP text in host memory -> the graph session's device-resident records (SURVEY.md 8(f) row 2): the
+// parse of bioparser's PafParser / MhapParser (graph.cpp:443-451 runs it once more for every construct pass) and, for PAF,
+// the name -> id lookup of Overlap::transmute (overlap.cpp:36-82) on the device, followed by the front end's duplicate
+// filter (frontend.cu).
 //
 //   names once per session:  k_paf_names        open-addressing table of the read names (64-bit hash; a hit is confirmed
 //                                                against the name bytes, so a hash collision never resolves to a wrong id)
 //   per upload chunk:        k_paf_line_ends    '\n' per tile (16-byte loads), decoupled look-back, one line end per record
 //                            k_paf_parse        one warp per line: tab positions by ballot, lane f parses field f
+//                         or k_mhap_parse       the same for MHAP: spaces, numeric ids checked against the read count
 //   per call (session):      k_filter_duplicates, k_paf_fold   is_valid_overlap_ folded into the INVALID bit
 //
-// Input contract (the library refuses what it cannot map onto the reference's reading without guessing): tab-separated,
-// at least 12 fields; columns 2, 3, 4, 7, 8, 9, 11 plain decimal below 2^32; orientation = first byte of column 5 != '+';
-// names are the exact bytes of columns 1 and 6; columns 10, 12 and every extra column are never read.
+// Input contracts (the library refuses what it cannot map onto the reference's reading without guessing; the full text
+// is in include/rala_b200.h).  PAF: tab-separated, at least 12 fields; columns 2, 3, 4, 7, 8, 9, 11 plain decimal below
+// 2^32; orientation = first byte of column 5 != '+'; names are the exact bytes of columns 1 and 6; columns 10, 12 and
+// every extra column are never read.  MHAP: space-separated, at least 12 fields; ids 1..n_reads; strands 0 or 1; fields
+// 3, 4 and every extra field are never read.
 #include <cstring>
 
 #include "kernels.h"
@@ -23,10 +27,11 @@ constexpr int kScanItems = 4;                                          // 16-byt
 constexpr uint32_t kScanTile = kTileThreads * 16u * kScanItems;        // 16 KiB of text per tile
 constexpr uint32_t kPafPad = kScanTile + 256;                          // readable bytes behind a chunk (whole tiles, line words)
 constexpr uint32_t kUnknownId = 0x7FFFFFFFu;                           // a name that is not in the table
-constexpr uint32_t kMinLine = 19;                                      // 11 tabs + 7 digits + '\n': no valid line is shorter
-enum : uint32_t { kErrFields = 1, kErrEmpty = 2, kErrDigit = 3, kErrOverflow = 4 };
+constexpr uint32_t kMinPafLine = 19;                                   // 11 tabs + 7 digits + '\n': no valid line is shorter
+constexpr uint32_t kMinMhapLine = 22;                                  // 11 spaces + 10 digits + '\n' (fields 3, 4 empty)
+enum : uint32_t { kErrFields = 1, kErrEmpty = 2, kErrDigit = 3, kErrOverflow = 4, kErrReadId = 5, kErrStrand = 6 };
 // device words of one call: the first four start at ~0 (minima), the rest at 0; line bases of the chunks follow
-enum { W_ERR = 0, W_DUP, W_FIRST_MISMATCH, W_FIRST_BAD, W_UNRESOLVED, W_MISMATCH, W_BASES = 8 };
+enum { W_ERR = 0, W_DUP, W_FIRST_MISMATCH, W_FIRST_BAD, W_UNRESOLVED, W_MISMATCH, W_QUERY_RC, W_BASES = 8 };
 
 struct NameTable {
     const uint8_t* blob;
@@ -149,8 +154,42 @@ __global__ void __launch_bounds__(kTileThreads) k_paf_line_ends(const uint8_t* _
     }
 }
 
-// One warp per line.  128 bytes per step (a 4-byte word per lane), tabs found by ballot and ranked by a warp scan; the
-// walk stops at the 11th tab, so tags behind column 12 (CIGARs of tens of KB) are never read.  Then lane f parses field f.
+// The first `kWant` separators of line [s, e) into pos[] by one warp, 128 bytes per step (a 4-byte word per lane): found
+// by ballot, ranked by a warp scan.  Returns how many there are, at most kWant; the walk stops once it has them, so bytes
+// behind them (PAF tags, CIGARs of tens of KB; MHAP extra fields) are never read.
+template <uint32_t kSep, uint32_t kWant>
+__device__ __forceinline__ uint32_t warp_separators(const uint8_t* __restrict__ text, uint32_t s, uint32_t e, uint32_t* pos,
+                                                    uint32_t lane) {
+    uint32_t n = 0;
+    for (uint32_t w = s & ~3u; w < e && n < kWant; w += 128u) {
+        const uint32_t p0 = w + 4u * lane;
+        const uint32_t word = *reinterpret_cast<const uint32_t*>(text + p0);
+        uint32_t m = 0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+            m |= ((((word >> (8 * k)) & 0xFFu) == kSep) & (p0 + k >= s) & (p0 + k < e) ? 1u : 0u) << k;
+        const uint32_t c = __popc(m), inc = warp_inclusive_scan(c);
+        for (uint32_t r = n + inc - c; m && r < kWant; ++r, m &= m - 1) pos[r] = p0 + (uint32_t) (__ffs(m) - 1);
+        n += __shfl_sync(0xFFFFFFFFu, inc, 31);
+    }
+    return n < kWant ? n : kWant;
+}
+
+// Plain decimal [fb, fe) below 2^32 (leading zeros allowed).  A refusal sets err = kind << 4 | field: an empty field or a
+// non-digit (kErrDigit), or the 33rd bit (kErrOverflow), whichever comes first from the left.
+__device__ __forceinline__ uint32_t parse_u32(const uint8_t* __restrict__ text, uint32_t fb, uint32_t fe, uint32_t field, uint32_t& err) {
+    unsigned long long v = 0;
+    if (fb == fe) err = kErrDigit << 4 | field;
+    for (uint32_t p = fb; p < fe; ++p) {
+        const uint32_t d = (uint32_t) text[p] - '0';
+        if (d > 9u) { err = kErrDigit << 4 | field; break; }
+        v = v * 10u + d;
+        if (v > 0xFFFFFFFFull) { err = kErrOverflow << 4 | field; break; }
+    }
+    return (uint32_t) v;
+}
+
+// One warp per line: tab positions by warp_separators, stopping at the 11th tab, then lane f parses field f.
 // Record index = global line index (file order).  A refused line lowers the error word: (line << 8) | kind << 4 | column.
 __global__ void __launch_bounds__(256) k_paf_parse(const uint8_t* __restrict__ text, const uint32_t* __restrict__ line_end,
                                                    const unsigned long long* __restrict__ bases, uint32_t chunk, NameTable t,
@@ -161,19 +200,8 @@ __global__ void __launch_bounds__(256) k_paf_parse(const uint8_t* __restrict__ t
     const uint32_t lane = lane_id(), warp = warp_id();
     for (uint32_t line = blockIdx.x * kTileWarps + warp; line < n_lines; line += gridDim.x * kTileWarps) {
         const uint32_t s = line ? line_end[line - 1] + 1u : 0u, e = line_end[line];
-        uint32_t ntab = 0;
         __syncwarp();
-        for (uint32_t w = s & ~3u; w < e && ntab < 11u; w += 128u) {
-            const uint32_t p0 = w + 4u * lane;
-            const uint32_t word = *reinterpret_cast<const uint32_t*>(text + p0);
-            uint32_t m = 0;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-                m |= ((((word >> (8 * k)) & 0xFFu) == '\t') & (p0 + k >= s) & (p0 + k < e) ? 1u : 0u) << k;
-            const uint32_t c = __popc(m), inc = warp_inclusive_scan(c);
-            for (uint32_t r = ntab + inc - c; m && r < 11u; ++r, m &= m - 1) s_tab[warp][r] = p0 + (uint32_t) (__ffs(m) - 1);
-            ntab += __shfl_sync(0xFFFFFFFFu, inc, 31);
-        }
+        const uint32_t ntab = warp_separators<'\t', 11>(text, s, e, s_tab[warp], lane);
         __syncwarp();
         uint32_t err = 0, val = 0;
         if (e == s) {
@@ -187,15 +215,7 @@ __global__ void __launch_bounds__(256) k_paf_parse(const uint8_t* __restrict__ t
             } else if (lane == 4) {
                 val = text[fb] != '+';   // fb == fe: the tab itself
             } else if (lane != 9) {
-                unsigned long long v = 0;
-                if (fb == fe) err = kErrDigit << 4 | (lane + 1u);
-                for (uint32_t p = fb; p < fe; ++p) {
-                    const uint32_t d = (uint32_t) text[p] - '0';
-                    if (d > 9u) { err = kErrDigit << 4 | (lane + 1u); break; }
-                    v = v * 10u + d;
-                    if (v > 0xFFFFFFFFull) { err = kErrOverflow << 4 | (lane + 1u); break; }
-                }
-                val = (uint32_t) v;
+                val = parse_u32(text, fb, fe, lane + 1u, err);
             }
         }
         const unsigned long long gline = base + line;
@@ -232,6 +252,77 @@ __global__ void __launch_bounds__(256) k_paf_parse(const uint8_t* __restrict__ t
     }
 }
 
+// MHAP: one warp per line, spaces by warp_separators up to the 12th, then lane f parses field f + 1 (lanes 2 and 3, the
+// error and the shared minmers, stay idle).  Ids are 1-based, checked against [1, n_reads]; strands are exactly '0' or '1';
+// orientation = a_rc != b_rc; Overlap::length() = max(a_end - a_begin, b_end - b_begin) in uint32_t arithmetic, as the
+// reference's MHAP constructor computes it.  A '\r' that ends field 12 at the line's end is dropped (CRLF files).
+__global__ void __launch_bounds__(256) k_mhap_parse(const uint8_t* __restrict__ text, const uint32_t* __restrict__ line_end,
+                                                    const unsigned long long* __restrict__ bases, uint32_t chunk,
+                                                    const uint32_t* __restrict__ read_len, uint32_t n_reads, PafCols out,
+                                                    unsigned long long rec_cap, unsigned long long* __restrict__ words) {
+    __shared__ uint32_t s_sep[kTileWarps][12];
+    const unsigned long long base = bases[chunk];
+    const uint32_t n_lines = (uint32_t) (bases[chunk + 1] - base);
+    const uint32_t lane = lane_id(), warp = warp_id();
+    for (uint32_t line = blockIdx.x * kTileWarps + warp; line < n_lines; line += gridDim.x * kTileWarps) {
+        const uint32_t s = line ? line_end[line - 1] + 1u : 0u, e = line_end[line];
+        __syncwarp();
+        const uint32_t nsep = warp_separators<' ', 12>(text, s, e, s_sep[warp], lane);
+        __syncwarp();
+        uint32_t err = 0, val = 0;
+        if (e == s) {
+            err = kErrEmpty << 4 | 1u;
+        } else if (nsep < 11u) {
+            err = kErrFields << 4 | (nsep + 1u);   // fields found
+        } else if (lane < 12u && (lane < 2u || lane > 3u)) {
+            const uint32_t fb = lane ? s_sep[warp][lane - 1] + 1u : s;
+            uint32_t fe = lane < nsep ? s_sep[warp][lane] : e;
+            if (lane == 11u && nsep == 11u && fe > fb && text[fe - 1] == '\r') --fe;
+            if (lane == 4u || lane == 8u) {
+                const uint32_t d = (uint32_t) text[fb] - '0';   // fb == fe: the separator itself
+                if (fe - fb != 1u || d > 1u) err = kErrStrand << 4 | (lane + 1u);
+                val = d;
+            } else {
+                val = parse_u32(text, fb, fe, lane + 1u, err);
+                if (lane < 2u && !err) {
+                    if (val == 0u || val > n_reads) err = kErrReadId << 4 | (lane + 1u);
+                    val -= 1u;
+                }
+            }
+        }
+        const unsigned long long gline = base + line;
+        const uint32_t bad = __ballot_sync(0xFFFFFFFFu, err != 0u);
+        if (bad) {
+            const uint32_t code = __shfl_sync(0xFFFFFFFFu, err, __ffs(bad) - 1);
+            if (lane == 0) atomicMin(words + W_ERR, gline << 8 | code);
+            continue;
+        }
+        const uint32_t a = __shfl_sync(0xFFFFFFFFu, val, 0), b = __shfl_sync(0xFFFFFFFFu, val, 1);
+        const uint32_t a_rc = __shfl_sync(0xFFFFFFFFu, val, 4), ab = __shfl_sync(0xFFFFFFFFu, val, 5);
+        const uint32_t ae = __shfl_sync(0xFFFFFFFFu, val, 6), a_len = __shfl_sync(0xFFFFFFFFu, val, 7);
+        const uint32_t b_rc = __shfl_sync(0xFFFFFFFFu, val, 8), bb = __shfl_sync(0xFFFFFFFFu, val, 9);
+        const uint32_t be = __shfl_sync(0xFFFFFFFFu, val, 10), b_len = __shfl_sync(0xFFFFFFFFu, val, 11);
+        if (lane == 0) {
+            const bool mism = a_len != __ldg(read_len + a) || b_len != __ldg(read_len + b);
+            if (a_rc) atomicAdd(words + W_QUERY_RC, 1ull);
+            if (mism) {
+                atomicAdd(words + W_MISMATCH, 1ull);
+                atomicMin(words + W_FIRST_MISMATCH, gline);
+            }
+            if (gline < rec_cap) {
+                out.a[gline] = a;
+                out.b[gline] = b | (a_rc ^ b_rc) << 31;
+                out.ab[gline] = ab;
+                out.ae[gline] = ae;
+                out.bb[gline] = bb;
+                out.be[gline] = be;
+                out.len[gline] = max(ae - ab, be - bb);
+                out.mismatch[gline] = mism ? 1 : 0;
+            }
+        }
+    }
+}
+
 // is_valid_overlap_ into the INVALID bit while the parsed columns move to the session's records; a record that stays
 // valid with a read length the caller's reads contradict lowers W_FIRST_BAD (transmute would exit on it)
 __global__ void __launch_bounds__(256) k_paf_fold(PafCols in, const uint8_t* __restrict__ valid, uint32_t n, List recs,
@@ -253,6 +344,7 @@ void preload_paf() {
     cudaFuncGetAttributes(&a, k_paf_names);
     cudaFuncGetAttributes(&a, k_paf_line_ends);
     cudaFuncGetAttributes(&a, k_paf_parse);
+    cudaFuncGetAttributes(&a, k_mhap_parse);
     cudaFuncGetAttributes(&a, k_paf_fold);
 }
 
@@ -347,23 +439,32 @@ static int paf_set_names(rala_b200_ctx* ctx, PafReader& R, const char* names, co
     return RALA_B200_OK;
 }
 
-static const char* paf_error_text(uint32_t kind) {
+static const char* text_error_text(uint32_t kind) {
     switch (kind) {
-        case kErrFields: return "has fewer than 12 tab-separated fields (fields found: column number)";
-        case kErrEmpty: return "is empty";
         case kErrDigit: return "is not a plain decimal number";
-        default: return "does not fit 32 bits";
+        case kErrOverflow: return "does not fit 32 bits";
+        case kErrReadId: return "is not a read id (1 to the number of reads given to set_reads)";
+        default: return "is not a strand (exactly 0 or 1)";
     }
 }
 
+// What one call of either reader counted (the union of the PAF and the MHAP stats).
+struct TextStats {
+    uint64_t n_records, n_unresolved, n_length_mismatch, first_length_mismatch, n_query_rc, n_bytes, n_chunks;
+};
+
 // Parses the whole text into R.cols (record index = line index, file order).  *n_out = records; kernel_ms (nullable) = device
-// time of the chunks' kernels (line scan + parse), uploads excluded.
-static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* st,
+// time of the chunks' kernels (line scan + parse), uploads excluded.  The format decides the parse kernel, the shortest
+// valid line and the wording of refusals; upload, line scan and the call's words are the same for both.
+static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
                             float* kernel_ms, uint64_t* n_out) {
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->L.stream;
-    // no valid line is shorter than kMinLine bytes (the last one may lack its '\n'): more lines than that means a refusal
-    R.rec_cap = (n_bytes + 1) / kMinLine + 1;
+    const bool mhap = fmt == kTextMhap;
+    const char* label = mhap ? "MHAP" : "PAF";
+    const char* field = mhap ? "field" : "column";
+    // no valid line is shorter than the format's minimum (the last one may lack its '\n'): more lines than that means a refusal
+    R.rec_cap = (n_bytes + 1) / (mhap ? kMinMhapLine : kMinPafLine) + 1;
     if (R.rec_cap > (1ull << 31)) R.rec_cap = 1ull << 31;
     const size_t col = align_up((size_t) R.rec_cap * 4, 256);
     CU(ctx, R.cols.reserve(7 * col + align_up((size_t) R.rec_cap, 256)));
@@ -400,7 +501,7 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
     uint64_t pos = 0;
     uint32_t k = 0;
     for (; pos < n_bytes; ++k) {
-        if (k >= max_chunks) return fail(ctx, RALA_B200_ERR_LIMIT, "PAF text: more upload chunks than planned");
+        if (k >= max_chunks) return fail(ctx, RALA_B200_ERR_LIMIT, "%s text: more upload chunks than planned", label);
         uint64_t len = n_bytes - pos < kPafChunk ? n_bytes - pos : kPafChunk;
         const bool last = pos + len == n_bytes;
         if (!last) {   // cut behind the last '\n' of the window; the tail goes with the next chunk
@@ -410,7 +511,7 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
                 CU(ctx, cudaStreamSynchronize(R.copy));
                 CU(ctx, cudaMemcpyAsync(&lines, words + W_BASES + k, 8, cudaMemcpyDeviceToHost, s));
                 CU(ctx, cudaStreamSynchronize(s));
-                return fail(ctx, RALA_B200_ERR_LIMIT, "PAF line %llu is longer than the upload chunk (%u bytes)", lines + 1, kPafChunk);
+                return fail(ctx, RALA_B200_ERR_LIMIT, "%s line %llu is longer than the upload chunk (%u bytes)", label, lines + 1, kPafChunk);
             }
             len = (uint64_t) ((const char*) nl - (text + pos)) + 1;
         }
@@ -437,8 +538,12 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
         k_paf_line_ends<<<grid_for(scan_len, kScanTile, kNumSMs * 8), kTileThreads, 0, s>>>(
             (const uint8_t*) dtext, scan_len, R.line_end.as<uint32_t>(), st_words + 1, (uint32_t*) st_words, words + W_BASES, k);
         ctx->L.count++;
-        k_paf_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
-            (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table, out, R.rec_cap, words);
+        if (mhap)
+            k_mhap_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
+                (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table.read_len, R.n_reads, out, R.rec_cap, words);
+        else
+            k_paf_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
+                (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table, out, R.rec_cap, words);
         ctx->L.count++;
         CU(ctx, cudaGetLastError());
         CU(ctx, cudaEventRecord(R.timing[2 * k + 1], s));
@@ -459,9 +564,11 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
     if (R.w[W_ERR] != ~0ull) {
         const uint32_t code = (uint32_t) (R.w[W_ERR] & 0xFF), kind = code >> 4, column = code & 15;
         const unsigned long long line = (R.w[W_ERR] >> 8) + 1;
-        if (kind == kErrFields) return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu has %u tab-separated fields, at least 12 are needed", line, column);
-        if (kind == kErrEmpty) return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu, column 1: the line is empty", line);
-        return fail(ctx, RALA_B200_ERR_ARG, "PAF line %llu, column %u: %s", line, column, paf_error_text(kind));
+        if (kind == kErrFields)
+            return fail(ctx, RALA_B200_ERR_ARG, "%s line %llu has %u %s-separated fields, at least 12 are needed", label, line, column,
+                        mhap ? "space" : "tab");
+        if (kind == kErrEmpty) return fail(ctx, RALA_B200_ERR_ARG, "%s line %llu, %s 1: the line is empty", label, line, field);
+        return fail(ctx, RALA_B200_ERR_ARG, "%s line %llu, %s %u: %s", label, line, field, column, text_error_text(kind));
     }
     const unsigned long long n = R.w[W_BASES + k];
     if (n >= (1ull << 31)) return fail(ctx, RALA_B200_ERR_LIMIT, "too many overlap records (%llu >= 2^31)", n);
@@ -469,6 +576,7 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
     st->n_unresolved = R.w[W_UNRESOLVED];
     st->n_length_mismatch = R.w[W_MISMATCH];
     st->first_length_mismatch = R.w[W_FIRST_MISMATCH];
+    st->n_query_rc = R.w[W_QUERY_RC];
     st->n_bytes = n_bytes;
     st->n_chunks = k;
     *n_out = n;
@@ -476,9 +584,9 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, const char* text, 
 }
 
 // A refused call returns with no upload in flight: the caller may free its text at once.
-static int paf_parse(rala_b200_ctx* ctx, PafReader& R, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* st, float* kernel_ms,
-                     uint64_t* n_out) {
-    const int rc = paf_parse_chunks(ctx, R, text, n_bytes, st, kernel_ms, n_out);
+static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
+                      float* kernel_ms, uint64_t* n_out) {
+    const int rc = paf_parse_chunks(ctx, R, fmt, text, n_bytes, st, kernel_ms, n_out);
     if (rc) {
         if (R.copy) cudaStreamSynchronize(R.copy);
         cudaStreamSynchronize(ctx->L.stream);
@@ -490,22 +598,25 @@ extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, 
                                          uint32_t n_reads) {
     if (!g) return RALA_B200_ERR_ARG;
     if (!g->paf) g->paf = new PafReader();
-    g->paf_records = false;   // the records' ids refer to the reads they were parsed against
+    g->text_records = kTextNone;   // the records' ids refer to the reads they were parsed against
     return paf_set_names(g->ctx, *g->paf, names, name_end, read_len, n_reads);
 }
 
-extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats) {
+// Text in file order -> the session's records: parse, duplicate filter, INVALID bit folded in.  *counted = *st holds the
+// call's counts (also when a read-length refusal follows).
+static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st, bool* counted) {
     if (!g || (n_bytes && !text)) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (!g->paf || !g->paf->have_names) return fail(ctx, RALA_B200_ERR_STATE, "set_overlaps_paf: set_reads first");
+    const bool mhap = fmt == kTextMhap;
+    if (!g->paf || !g->paf->have_names)
+        return fail(ctx, RALA_B200_ERR_STATE, "set_overlaps_%s: set_reads first", mhap ? "mhap" : "paf");
     PafReader& R = *g->paf;
     // the session's records are void until this call has succeeded
     g->n_rec = 0;
     g->state = 0;
-    g->paf_records = false;
-    rala_b200_paf_stats_t st{};
+    g->text_records = kTextNone;
     uint64_t n = 0;
-    int rc = paf_parse(ctx, R, text, n_bytes, &st, nullptr, &n);
+    int rc = text_parse(ctx, R, fmt, text, n_bytes, st, nullptr, &n);
     if (rc) return rc;
     rc = reserve_for_records(g, n);
     if (rc) return rc;
@@ -521,26 +632,64 @@ extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* 
     unsigned long long bad = ~0ull;
     CU(ctx, cudaMemcpyAsync(&bad, R.words.as<unsigned long long>() + W_FIRST_BAD, 8, cudaMemcpyDeviceToHost, ctx->L.stream));
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
-    if (stats) *stats = st;
+    *counted = true;
     if (bad != ~0ull) {
         g->n_rec = 0;
         g->state = 0;
         return fail(ctx, RALA_B200_ERR_ARG,
-                    "PAF line %llu: a read length (column 2 or 7) differs from the length given to set_reads, and the record is "
-                    "valid after the duplicate filter (the reference's transmute exits on it)", bad + 1);
+                    "%s line %llu: a read length (%s) differs from the length given to set_reads, and the record is "
+                    "valid after the duplicate filter (the reference's transmute exits on it)", mhap ? "MHAP" : "PAF", bad + 1,
+                    mhap ? "field 8 or 12" : "column 2 or 7");
     }
-    g->paf_records = true;
+    g->text_records = fmt;
     return RALA_B200_OK;
 }
 
-bool paf_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len) {
-    if (!g->paf_records || !g->paf || !g->paf->have_names) return false;
+static void paf_stats_of(const TextStats& t, rala_b200_paf_stats_t* st) {
+    *st = rala_b200_paf_stats_t{t.n_records, t.n_unresolved, t.n_length_mismatch, t.first_length_mismatch, t.n_bytes, t.n_chunks};
+}
+
+static void mhap_stats_of(const TextStats& t, rala_b200_mhap_stats_t* st) {
+    *st = rala_b200_mhap_stats_t{t.n_records, t.n_length_mismatch, t.first_length_mismatch, t.n_query_rc, t.n_bytes, t.n_chunks};
+}
+
+extern "C" int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_paf_stats_t* stats) {
+    TextStats st{};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextPaf, text, n_bytes, &st, &counted);
+    if (stats && counted) paf_stats_of(st, stats);
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_overlaps_mhap(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_mhap_stats_t* stats) {
+    TextStats st{};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextMhap, text, n_bytes, &st, &counted);
+    if (stats && counted) mhap_stats_of(st, stats);
+    return rc;
+}
+
+TextFormat text_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len) {
+    if (g->text_records == kTextNone || !g->paf || !g->paf->have_names) return kTextNone;
     const PafCols c = g->paf->view();
     *cols = PileCols{c.a, c.b, c.ab, c.ae, c.bb, c.be};
     *read_len = g->paf->table.read_len;
     *n_reads = g->paf->n_reads;
     *max_len = g->paf->max_len;
-    return true;
+    return g->text_records;
+}
+
+// The parsed columns of R (n records) into 7 x cap host words.
+static int download_columns(rala_b200_ctx* ctx, const PafReader& R, const char* what, uint64_t n, uint32_t* cols_out, uint64_t cap) {
+    if (n > cap || (n && !cols_out))
+        return fail(ctx, RALA_B200_ERR_ARG, "%s: the text has %llu records, the output holds %llu", what, (unsigned long long) n,
+                    (unsigned long long) cap);
+    const PafCols c = R.view();
+    const uint32_t* src[7] = {c.a, c.b, c.ab, c.ae, c.bb, c.be, c.len};
+    for (int k = 0; k < 7 && n; ++k)
+        CU(ctx, cudaMemcpyAsync(cols_out + (size_t) k * cap, src[k], (size_t) n * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
+    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
+    return RALA_B200_OK;
 }
 
 extern "C" int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads,
@@ -552,15 +701,28 @@ extern "C" int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const 
     int rc = paf_set_names(ctx, R, names, name_end, read_len, n_reads);
     if (rc) return rc;
     uint64_t n = 0;
-    rc = paf_parse(ctx, R, text, n_bytes, stats, device_ms, &n);
+    TextStats st{};
+    rc = text_parse(ctx, R, kTextPaf, text, n_bytes, &st, device_ms, &n);
     if (rc) return rc;
-    if (n > cap || (n && !cols_out))
-        return fail(ctx, RALA_B200_ERR_ARG, "parse_paf: the text has %llu records, the output holds %llu", (unsigned long long) n,
-                    (unsigned long long) cap);
-    const PafCols c = R.view();
-    const uint32_t* src[7] = {c.a, c.b, c.ab, c.ae, c.bb, c.be, c.len};
-    for (int k = 0; k < 7 && n; ++k)
-        CU(ctx, cudaMemcpyAsync(cols_out + (size_t) k * cap, src[k], (size_t) n * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
-    CU(ctx, cudaStreamSynchronize(ctx->L.stream));
-    return RALA_B200_OK;
+    paf_stats_of(st, stats);
+    return download_columns(ctx, R, "parse_paf", n, cols_out, cap);
+}
+
+extern "C" int rala_b200_parse_mhap(rala_b200_ctx* ctx, const uint32_t* read_len, uint32_t n_reads, const char* text, uint64_t n_bytes,
+                                    uint32_t* cols_out, uint64_t cap, rala_b200_mhap_stats_t* stats, float* device_ms) {
+    if (!ctx || !stats || (n_bytes && !text) || (n_reads && !read_len)) return RALA_B200_ERR_ARG;
+    if (device_ms) *device_ms = 0.f;
+    if (n_reads >= (1u << 31)) return fail(ctx, RALA_B200_ERR_LIMIT, "too many reads (%u >= 2^31)", n_reads);
+    CU(ctx, cudaSetDevice(ctx->device));
+    PafReader R;   // no name table: only the lengths, which the parse checks fields 8 and 12 against
+    CU(ctx, R.names.reserve((size_t) n_reads * 4 + 16));
+    if (n_reads) CU(ctx, cudaMemcpyAsync(R.names.p, read_len, (size_t) n_reads * 4, cudaMemcpyHostToDevice, ctx->L.stream));
+    R.table.read_len = R.names.as<uint32_t>();
+    R.n_reads = n_reads;
+    uint64_t n = 0;
+    TextStats st{};
+    int rc = text_parse(ctx, R, kTextMhap, text, n_bytes, &st, device_ms, &n);
+    if (rc) return rc;
+    mhap_stats_of(st, stats);
+    return download_columns(ctx, R, "parse_mhap", n, cols_out, cap);
 }

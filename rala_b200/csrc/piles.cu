@@ -313,9 +313,9 @@ static const char* pile_error_text(uint32_t kind) {
 }
 
 // in: device columns of n records; read_len: device, n_reads words.  Leaves P.piles / P.medians / the runs filled.
-// paf_lines: name a refused record by its 1-based PAF line instead of its 0-based index.
+// line_label ("PAF", "MHAP"; nullable): name a refused record by its 1-based line of that text instead of its 0-based index.
 static int build_piles_device(rala_b200_ctx* ctx, PileBuilder& P, PileCols in, uint64_t n, const uint32_t* read_len, uint32_t n_reads,
-                              uint32_t max_len, bool paf_lines, rala_b200_pile_stats_t* st, float* device_ms) {
+                              uint32_t max_len, const char* line_label, rala_b200_pile_stats_t* st, float* device_ms) {
     P.ready = false;
     if (n >= (1ull << 29)) return fail(ctx, RALA_B200_ERR_LIMIT, "build_piles: too many overlap records (%llu >= 2^29: 4 events each)", (unsigned long long) n);
     if (n_reads >= (1u << 31)) return fail(ctx, RALA_B200_ERR_LIMIT, "build_piles: too many reads (%u >= 2^31)", n_reads);
@@ -383,7 +383,7 @@ static int build_piles_device(rala_b200_ctx* ctx, PileBuilder& P, PileCols in, u
     if (w[PW_ERR] != ~0ull) {
         const unsigned long long rec = w[PW_ERR] >> 8;
         const uint32_t kind = (uint32_t) (w[PW_ERR] & 0xFF);
-        if (paf_lines) return fail(ctx, RALA_B200_ERR_ARG, "build_piles: PAF line %llu %s", rec + 1, pile_error_text(kind));
+        if (line_label) return fail(ctx, RALA_B200_ERR_ARG, "build_piles: %s line %llu %s", line_label, rec + 1, pile_error_text(kind));
         return fail(ctx, RALA_B200_ERR_ARG, "build_piles: record %llu (0-based) %s", rec, pile_error_text(kind));
     }
     if (w[PW_MAXCOV] >= 65536)
@@ -425,7 +425,7 @@ extern "C" int rala_b200_build_piles(rala_b200_ctx* ctx, const uint32_t* a_id, c
     if (n_reads) CU(ctx, cudaMemcpyAsync(P.rlen.p, read_len, (size_t) n_reads * 4, cudaMemcpyHostToDevice, s));
     const PileCols in{(const uint32_t*) b, (const uint32_t*) (b + col), (const uint32_t*) (b + 2 * col), (const uint32_t*) (b + 3 * col),
                       (const uint32_t*) (b + 4 * col), (const uint32_t*) (b + 5 * col)};
-    int rc = build_piles_device(ctx, P, in, n, P.rlen.as<uint32_t>(), n_reads, max_len, false, stats, device_ms);
+    int rc = build_piles_device(ctx, P, in, n, P.rlen.as<uint32_t>(), n_reads, max_len, nullptr, stats, device_ms);
     if (rc) return rc;
     if (n_reads) CU(ctx, cudaMemcpyAsync(piles_out, P.piles.p, (size_t) n_reads * 8, cudaMemcpyDeviceToHost, s));
     if (n_reads && medians_out) CU(ctx, cudaMemcpyAsync(medians_out, P.medians.p, (size_t) n_reads * 2, cudaMemcpyDeviceToHost, s));
@@ -439,12 +439,13 @@ extern "C" int rala_b200_graph_build_piles(rala_b200_graph* g, rala_b200_pile_st
     PileCols in;
     const uint32_t* read_len = nullptr;
     uint32_t n_reads = 0, max_len = 0;
-    if (!paf_records_view(g, &in, &read_len, &n_reads, &max_len))
-        return fail(ctx, RALA_B200_ERR_STATE, "build_piles: needs the records of a successful set_overlaps_paf (records given to "
-                    "set_overlaps* have the duplicate filter folded in, and coverage counts the records it drops)");
+    const TextFormat fmt = text_records_view(g, &in, &read_len, &n_reads, &max_len);
+    if (fmt == kTextNone)
+        return fail(ctx, RALA_B200_ERR_STATE, "build_piles: needs the records of a successful set_overlaps_paf or _mhap (records "
+                    "given to set_overlaps* have the duplicate filter folded in, and coverage counts the records it drops)");
     if (!g->pile_builder) g->pile_builder = new PileBuilder();
     PileBuilder& P = *g->pile_builder;
-    int rc = build_piles_device(ctx, P, in, g->n_rec, read_len, n_reads, max_len, true, stats, nullptr);
+    int rc = build_piles_device(ctx, P, in, g->n_rec, read_len, n_reads, max_len, fmt == kTextMhap ? "MHAP" : "PAF", stats, nullptr);
     if (rc) return rc;
     std::vector<rala_pile_t> piles(n_reads);
     if (n_reads) CU(ctx, cudaMemcpyAsync(piles.data(), P.piles.p, (size_t) n_reads * 8, cudaMemcpyDeviceToHost, ctx->L.stream));

@@ -86,6 +86,9 @@ struct ListBuf {
     }
 };
 
+// the overlap text a session's records were parsed from (paf.cu); build_piles names refused records by its lines
+enum TextFormat : uint8_t { kTextNone = 0, kTextPaf, kTextMhap };
+
 enum Stage { ST_CLASSIFY = 0, ST_RETRIM, ST_FINALIZE, ST_BUILD, ST_TRANSITIVE, ST_K1_KERNEL, ST_K1B_KERNEL, ST_K3_KERNELS, ST_K1S_KERNEL };
 
 struct rala_b200_graph {
@@ -140,8 +143,8 @@ struct rala_b200_graph {
     // rala_b200_graph_run as a replayed CUDA graph (see run_key / RunGraph below)
     bool use_cuda_graph = true, capturing = false;
     struct RunGraph* run_graphs = nullptr;   // two cached instances: first run after set_piles / repeated run
-    struct PafReader* paf = nullptr;         // read-name table and PAF upload buffers (paf.cu), from the first set_reads
-    bool paf_records = false;                // the records came from set_overlaps_paf: its parsed columns are still there
+    struct PafReader* paf = nullptr;         // read-name table and text upload buffers (paf.cu), from the first set_reads
+    TextFormat text_records = kTextNone;     // the records came from set_overlaps_paf / _mhap: its parsed columns are still there
     struct PileBuilder* pile_builder = nullptr;   // event, sort and run buffers of build_piles (piles.cu)
 
     uint32_t* cnt() const { return counters.as<uint32_t>(); }
@@ -208,12 +211,13 @@ int reserve_for_records(rala_b200_graph* g, uint64_t n);
 
 // ---- paf.cu ----------------------------------------------------------------------------------------------------
 void destroy_paf_reader(PafReader* r);
-// the overlap columns build_piles counts: the parsed records of the last successful set_overlaps_paf, before the duplicate
-// filter was folded in (bit 31 of a = unresolved name), and the reads' lengths (device); false when there are none
+// the overlap columns build_piles counts: the parsed records of the last successful set_overlaps_paf / _mhap, before the
+// duplicate filter was folded in (bit 31 of a = unresolved name), and the reads' lengths (device); returns the text format
+// they came from, kTextNone when there are none
 struct PileCols {
     const uint32_t *a, *b, *ab, *ae, *bb, *be;
 };
-bool paf_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len);
+TextFormat text_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len);
 
 // ---- piles.cu --------------------------------------------------------------------------------------------------
 void destroy_pile_builder(PileBuilder* p);

@@ -73,6 +73,25 @@ class Dataset:
                 ]
                 f.write("".join(lines))
 
+    def write_mhap(self, path: str) -> None:
+        """The same records as MHAP: "a+1 b+1 0.0 <span> 0 ab ae la ori bb be lb" (1-based ids, a_rc = 0, b_rc = orientation;
+        the shared-minmers field carries the span, which no reader uses)."""
+        r = self.records
+        ln = self.read_len
+        with open(path, "w") as f:
+            chunk = 1 << 18
+            for s in range(0, r.shape[0], chunk):
+                q = r[s:s + chunk]
+                a, b = q[:, 0], q[:, 1]
+                span = np.maximum(q[:, 3] - q[:, 2], q[:, 5] - q[:, 4])
+                lines = [
+                    "%d %d 0.0 %d 0 %d %d %d %d %d %d %d\n" % (a_ + 1, b_ + 1, sp, ab, ae, la, fl & 1, bb, be, lb)
+                    for a_, b_, sp, ab, ae, la, fl, bb, be, lb in zip(
+                        a.tolist(), b.tolist(), span.tolist(), q[:, 2].tolist(), q[:, 3].tolist(), ln[a].tolist(),
+                        q[:, 6].tolist(), q[:, 4].tolist(), q[:, 5].tolist(), ln[b].tolist())
+                ]
+                f.write("".join(lines))
+
 
 def _pairs_sorted(g0: np.ndarray, g1: np.ndarray, min_ovl: int):
     """All (i, j), i < j in g0-sorted order, whose genome intervals share >= min_ovl bases."""
