@@ -200,7 +200,7 @@ int reserve_events(rala_b200_graph* g, uint32_t ev_cap) {
     // growing re-allocates: contents are not preserved (callers grow before they fill)
     g->ev_cap = ev_cap;
     CU(ctx, g->events.reserve(align_up((size_t) ev_cap * 4, 256) * 3));
-    CU(ctx, g->segs.reserve(align_up((size_t) ev_cap * 4, 256) * 2));
+    CU(ctx, g->segs.reserve(align_up((size_t) ev_cap * 8, 256) + (size_t) ev_cap * 16));
     return RALA_B200_OK;
 }
 
@@ -380,7 +380,7 @@ extern "C" int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* 
     if (n_piles != g->n_piles) {
         g->n_piles = n_piles;
         g->n_nodes_max = 2 * n_piles;
-        CU(ctx, g->dbuf.reserve(align_up((size_t) n_piles + 64, 64) * 4 * 5));
+        CU(ctx, g->dbuf.reserve(align_up((size_t) n_piles + 64, 64) * 4 * 8));
         CU(ctx, g->alive_bits.reserve(((size_t) n_piles / 32 + 2) * 4));
         CU(ctx, g->seq_to_node.reserve((size_t) n_piles * 4 + 16));
         CU(ctx, g->row_ptr.reserve(((size_t) g->n_nodes_max + 8) * 4));
@@ -426,15 +426,19 @@ ResolveBufs resolve_bufs(const rala_b200_graph* g) {
     r.vstart = b + 2 * stride;
     r.work0 = b + 3 * stride;
     r.work1 = b + 4 * stride;
+    r.hidx = b + 5 * stride;
+    r.first = reinterpret_cast<unsigned long long*>(b + 6 * stride);   // two strides
     r.n_work = g->flags.as<uint32_t>();
+    r.seg = g->segs.as<unsigned long long>();
+    r.hev = reinterpret_cast<uint4*>(g->segs.as<char>() + align_up((size_t) g->ev_cap * 8, 256));
     r.seg_c = g->segs.as<uint32_t>();
     r.seg_t = (uint32_t*) (g->segs.as<char>() + align_up((size_t) g->ev_cap * 4, 256));
     return r;
 }
 
-// the classify kernels bump the per-victim histogram while they emit events: clear it first
-cudaError_t clear_victim_histogram(rala_b200_graph* g) {
-    return cudaMemsetAsync(resolve_bufs(g).vcursor, 0, ((size_t) g->n_piles + 64) * 4, g->ctx->L.stream);
+// the classify kernels keep every victim's earliest event while they emit events: clear it to "none" (all ones) first
+cudaError_t clear_earliest_events(rala_b200_graph* g) {
+    return cudaMemsetAsync(resolve_bufs(g).first, 0xFF, ((size_t) g->n_piles + 64) * 8, g->ctx->L.stream);
 }
 
 static int resolve_containment(rala_b200_graph* g, bool decode, bool skip_if_empty) {
@@ -463,10 +467,10 @@ int phase_events(rala_b200_graph* g) {
     CU(ctx, begin_stage(g, ST_CLASSIFY));
     CU(ctx, cudaMemsetAsync(g->counters.p, 0, C_COUNT * 4, ctx->L.stream));
     if (g->n_hills) CU(ctx, cudaMemsetAsync(g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills, 0, (size_t) g->n_hills * 4, ctx->L.stream));
-    CU(ctx, clear_victim_histogram(g));
+    CU(ctx, clear_earliest_events(g));
     CU(ctx, stage_event(g, g->ev_start[ST_K1_KERNEL]));
     launch_classify_events(ctx->L, g->recs.view, g->n_rec, g->t0, g->piles.as<uint2>(), g->n_piles, g->events_view(),
-                           g->ev_cap, resolve_bufs(g).vcursor, g->hill_rec.as<uint32_t>(), g->cap, g->cnt());
+                           g->ev_cap, resolve_bufs(g).first, g->hill_rec.as<uint32_t>(), g->cap, g->cnt());
     CU(ctx, end_stage(g, ST_K1_KERNEL));
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;
@@ -653,10 +657,10 @@ int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base /* device, n
     CU(ctx, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     CU(ctx, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     CU(ctx, zero_counter(g, C_EV));
-    CU(ctx, clear_victim_histogram(g));
+    CU(ctx, clear_earliest_events(g));
     launch_classify_final(ctx->L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, ovl_base, g->inl[g->inl_cur].view,
                           g->cnt() + g->slot_inl, inl_base, g->cap, g->piles.as<uint2>(), g->events_view(), g->ev_cap,
-                          resolve_bufs(g).vcursor, g->cnt());
+                          resolve_bufs(g).first, g->cnt());
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;
 }
@@ -1285,8 +1289,8 @@ extern "C" int rala_b200_graph_import_gathered(rala_b200_graph* g, int kind, con
         if (rc) return rc;
         Events ev = g->events_view();
         launch_import_gathered(ctx->L, d_gathered, cap, (uint32_t) world, ev.v, ev.c, ev.t, g->ev_cap, g->cnt() + C_EV, g->cnt() + C_OVERFLOW);
-        CU(ctx, clear_victim_histogram(g));
-        launch_events_hist(ctx->L, g->events_view(), g->cnt() + C_EV, g->ev_cap, resolve_bufs(g).vcursor);
+        CU(ctx, clear_earliest_events(g));
+        launch_events_first(ctx->L, g->events_view(), g->cnt() + C_EV, g->ev_cap, resolve_bufs(g).first);
     } else {
         int rc = reserve_edges(g, (uint32_t) total_cap);     // the local edges were exported before
         if (rc) return rc;

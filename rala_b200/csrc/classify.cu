@@ -112,7 +112,7 @@ constexpr int kEvStage = 96;   // per-warp staging of events before one aggregat
 template <int MINB, int R>
 __global__ void __launch_bounds__(kTileThreads, MINB) k_classify_events(
     List recs, uint32_t n, uint32_t t0, const uint2* __restrict__ piles, uint32_t n_piles,
-    Events ev, uint32_t ev_cap, uint32_t* __restrict__ vcount, uint32_t* __restrict__ hill_rec, uint32_t hill_cap,
+    Events ev, uint32_t ev_cap, unsigned long long* __restrict__ first, uint32_t* __restrict__ hill_rec, uint32_t hill_cap,
     uint32_t* __restrict__ counters) {
     __shared__ uint32_t s_ev[kTileWarps][3][kEvStage];
     const uint32_t lane = lane_id(), warp = warp_id();
@@ -176,11 +176,12 @@ __global__ void __launch_bounds__(kTileThreads, MINB) k_classify_events(
             const uint32_t m = __ballot_sync(0xFFFFFFFFu, is_ev);
             if (m) {
                 if (is_ev) {
-                    atomicAdd(&vcount[evv], 1u);   // per-victim histogram for the resolution's counting sort
+                    const uint32_t t = t0 + (uint32_t) R * q + r;
+                    atomicMin(&first[evv], ((unsigned long long) t << 32) | evc);   // the victim's earliest event (containment.cu)
                     const uint32_t p = staged + __popc(m & ((1u << lane) - 1u));
                     s_ev[warp][0][p] = evv;
                     s_ev[warp][1][p] = evc;
-                    s_ev[warp][2][p] = t0 + (uint32_t) R * q + r;
+                    s_ev[warp][2][p] = t;
                 }
                 staged += __popc(m);
                 __syncwarp();
@@ -587,7 +588,7 @@ __global__ void __launch_bounds__(kTileThreads) k_list_pass(
 __global__ void k_classify_final(List lst0, const uint32_t* __restrict__ n_ptr0, const uint32_t* __restrict__ time_base_ptr0,
                                  List lst1, const uint32_t* __restrict__ n_ptr1, const uint32_t* __restrict__ time_base_ptr1,
                                  uint32_t cap, const uint2* __restrict__ piles, Events ev,
-                                 uint32_t ev_cap, uint32_t* __restrict__ vcount, uint32_t* __restrict__ counters) {
+                                 uint32_t ev_cap, unsigned long long* __restrict__ first, uint32_t* __restrict__ counters) {
     const List lst = blockIdx.y ? lst1 : lst0;
     const uint32_t* n_ptr = blockIdx.y ? n_ptr1 : n_ptr0;
     const uint32_t* time_base_ptr = blockIdx.y ? time_base_ptr1 : time_base_ptr0;
@@ -608,12 +609,13 @@ __global__ void k_classify_final(List lst0, const uint32_t* __restrict__ n_ptr0,
                 if (lane_id() == leader) gbase = atomicAdd(&counters[C_EV], (uint32_t) __popc(m));
                 gbase = __shfl_sync(m, gbase, leader);
                 uint32_t p = gbase + rank;
+                const uint32_t v = t == kA ? e.b : e.a, c = t == kA ? e.a : e.b;
                 if (p < ev_cap) {
-                    ev.v[p] = t == kA ? e.b : e.a;
-                    ev.c[p] = t == kA ? e.a : e.b;
+                    ev.v[p] = v;
+                    ev.c[p] = c;
                     ev.t[p] = time_base + i;
                 }
-                atomicAdd(&vcount[t == kA ? e.b : e.a], 1u);
+                atomicMin(&first[v], ((unsigned long long) (time_base + i) << 32) | c);
             }
         }
         lst.tag[i] = t;
@@ -707,10 +709,10 @@ void launch_unpack_records(Launch& L, const uint32_t* query_id, const uint32_t* 
 }
 
 void launch_classify_events(Launch& L, List recs, uint32_t n, uint32_t t0, const uint2* piles, uint32_t n_piles,
-                            Events ev, uint32_t ev_cap, uint32_t* vcount, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters) {
+                            Events ev, uint32_t ev_cap, unsigned long long* first, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters) {
     if (n == 0) return;
     // 3 blocks / SM at 80 registers: 4 and 5 blocks (64 / 48 registers) lost 15 and 25 us per step (profiles/r02a_ab.json)
-    k_classify_events<kEventsMinBlocks, kEventsItems><<<grid_for(n, kTileThreads * kEventsItems, kNumSMs * kEventsMinBlocks), kTileThreads, 0, L.stream>>>(recs, n, t0, piles, n_piles, ev, ev_cap, vcount,
+    k_classify_events<kEventsMinBlocks, kEventsItems><<<grid_for(n, kTileThreads * kEventsItems, kNumSMs * kEventsMinBlocks), kTileThreads, 0, L.stream>>>(recs, n, t0, piles, n_piles, ev, ev_cap, first,
                                                                                         hill_rec, hill_cap, counters);
     L.count++;
 }
@@ -770,9 +772,9 @@ void launch_list_pass(Launch& L, int mode, List in, const uint32_t* n_in, uint32
 
 void launch_classify_final(Launch& L, List ovl, const uint32_t* n_ovl, const uint32_t* ovl_time_base, List inl,
                            const uint32_t* n_inl, const uint32_t* inl_time_base, uint32_t cap, const uint2* piles, Events ev,
-                           uint32_t ev_cap, uint32_t* vcount, uint32_t* counters) {
+                           uint32_t ev_cap, unsigned long long* first, uint32_t* counters) {
     k_classify_final<<<dim3(grid_for(cap, 256, kNumSMs * 4), 2), 256, 0, L.stream>>>(ovl, n_ovl, ovl_time_base, inl, n_inl, inl_time_base,
-                                                                                     cap, piles, ev, ev_cap, vcount, counters);
+                                                                                     cap, piles, ev, ev_cap, first, counters);
     L.count++;
 }
 

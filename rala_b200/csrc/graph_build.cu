@@ -592,8 +592,8 @@ void launch_time_bases(Launch& L, const uint32_t* counts, uint32_t rank, uint32_
 
 // exclusive scan of n values: exclusive_out[i] and values_inout[i] both receive the prefix
 void launch_scan_u32(Launch& L, uint32_t* values_inout, uint32_t* exclusive_out, uint32_t n, unsigned long long* status,
-                     uint32_t* ticket, const uint32_t* skip, const uint32_t* run_if) {
-    k_scan_degrees<<<grid_for(n, kTile, kNumSMs * 8), kTileThreads, 0, L.stream>>>(values_inout, exclusive_out, n, status, ticket, skip, run_if, nullptr);
+                     uint32_t* ticket, const uint32_t* skip, const uint32_t* run_if, const uint32_t* live) {
+    k_scan_degrees<<<grid_for(n, kTile, kNumSMs * 8), kTileThreads, 0, L.stream>>>(values_inout, exclusive_out, n, status, ticket, skip, run_if, live);
     L.count++;
 }
 

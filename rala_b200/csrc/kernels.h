@@ -65,7 +65,7 @@ void launch_records_to_soa(Launch& L, const uint32_t* aos, uint32_t n, List recs
 void launch_unpack_records(Launch& L, const uint32_t* query_id, const uint32_t* group_end, uint32_t n_groups, const uint32_t* a_span,
                            const uint32_t* b_span, uint32_t n, List recs);
 void launch_classify_events(Launch& L, List recs, uint32_t n, uint32_t t0, const uint2* piles, uint32_t n_piles,
-                            Events ev, uint32_t ev_cap, uint32_t* vcount, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters);
+                            Events ev, uint32_t ev_cap, unsigned long long* first, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters);
 // runs of the survivors pass (128 records each): packed counts (overlaps | internals << 16) and the scanned offsets
 struct RunBufs {
     uint32_t *cnt, *off_a, *off_b;   // num_runs each
@@ -88,7 +88,7 @@ void launch_list_pass(Launch& L, int mode, List in, const uint32_t* n_in, uint32
                       unsigned long long* status, uint32_t* ticket);
 void launch_classify_final(Launch& L, List ovl, const uint32_t* n_ovl, const uint32_t* ovl_time_base, List inl,
                            const uint32_t* n_inl, const uint32_t* inl_time_base, uint32_t cap, const uint2* piles, Events ev,
-                           uint32_t ev_cap, uint32_t* vcount, uint32_t* counters);
+                           uint32_t ev_cap, unsigned long long* first, uint32_t* counters);
 void launch_trim_classify_aos(Launch& L, uint32_t* rec, uint32_t n, const uint2* piles, uint32_t n_piles, uint8_t* type_out);
 void launch_pack_piles(Launch& L, const uint2* in, const uint8_t* flags, uint2* out, uint32_t n);
 void launch_unpack_piles(Launch& L, const uint2* in, uint2* out, uint32_t n);
@@ -97,17 +97,24 @@ void launch_aos_to_list(Launch& L, const uint32_t* aos, uint32_t n, const uint2*
 void launch_list_connections(Launch& L, List l, const uint32_t* n_ptr, uint32_t cap, uint32_t* out);
 
 // containment.cu
+// The classify kernels (and launch_events_first) keep every victim's earliest event in `first` (an atomicMin of
+// t << 32 | container; all ones = no event: clear to all ones before).  launch_resolve settles the victims that event
+// settles alone and groups the events of the others ("hard" victims, dense indices 0 .. n_work[0] - 1) by victim.
 struct ResolveBufs {
     uint32_t* S;         // n_piles: state during the resolution, death times (kInf = never) afterwards
-    uint32_t* vcursor;   // n_piles + 1: per-victim event histogram on entry, scatter cursor inside
-    uint32_t* vstart;    // n_piles + 1
+    unsigned long long* first;   // n_piles: earliest event per pile; after k_resolve_fast, the hard victims' segment bounds
+                                 // by pile (uint2 {begin, end}) for k_resolve
+    uint32_t* hidx;      // n_piles: dense index of a hard victim (the event filter's segment)
+    uint32_t* vcursor;   // n_piles + 1: events per segment (hard victim; multi-GPU fabric: pile), then a copy of vstart
+    uint32_t* vstart;    // n_piles + 1: segment offsets
     uint32_t *work0, *work1;   // n_piles each
-    uint32_t* n_work;    // 4 words
-    uint32_t *seg_c, *seg_t;   // event capacity each
+    uint32_t* n_work;    // 4 words: [0..2] rotating worklist counters (the first = hard victims), [3] events of hard victims
+    unsigned long long* seg;   // event capacity: events of the hard victims by segment, t << 32 | container
+    uint4* hev;          // event capacity: events of the hard victims before the scatter {dense index, rank in segment, t, c}
+    uint32_t *seg_c, *seg_t;   // multi-GPU fabric: per-pile segments, container and time columns (in seg's memory)
 };
 int resolve_max_blocks();
-// per-victim histogram of an imported event list (the classify kernels build it on the fly otherwise)
-void launch_events_hist(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_cap, uint32_t* vcount);
+void launch_events_first(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_cap, unsigned long long* first);
 // decode = false leaves the resolution's state encoding in rb.S: the following launch_apply_deaths(decode = true) turns
 // it into death times while it applies them (one launch less when nothing reads the death times in between)
 // skip_if_empty: with no events at all every kernel returns at once (nobody dies; rb.S is left as it is)
@@ -116,8 +123,9 @@ void launch_resolve(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_
                     bool skip_if_empty = false);
 
 // graph_build.cu
+// live: optional device count, only the first *live + 1 values are scanned
 void launch_scan_u32(Launch& L, uint32_t* values_inout, uint32_t* exclusive_out, uint32_t n, unsigned long long* status,
-                     uint32_t* ticket, const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr);
+                     uint32_t* ticket, const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr, const uint32_t* live = nullptr);
 struct GraphArrays {
     uint32_t* seq_to_node;   // n_piles
     uint32_t *src, *dst, *len;   // edge id order

@@ -463,8 +463,7 @@ static int route_and_meet(rala_b200_multi* m, FabricRank& fr, int pass) {
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
     // States of FOREIGN piles are only ever written by their owners' pushes, which start after the barrier below: the
-    // replica is cleared here, together with everything else the resolution of this pass starts from (the classify kernel
-    // before this call was the last user of the victim histogram).
+    // replica is cleared here, together with everything else the resolution of this pass starts from.
     launch_pass_reset(L, fr.P, fr.A, resolve_bufs(g), fr.tmin.as<uint32_t>(), fr.wait.as<uint32_t>(), fr.ctl(pass));
     launch_route_events(L, fr.P, fr.A, g->events_view(), g->cnt() + C_EV, g->ev_cap, fr.cnt_ev(pass));
     Publish pub = no_mail(m);
@@ -1215,7 +1214,7 @@ static int phase_d_staged(rala_b200_multi* m, FabricRank& fr) {
     MCU(m, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, L.stream));
     MCU(m, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, L.stream));
     MCU(m, zero_counter(g, C_EV));
-    MCU(m, clear_victim_histogram(g));
+    MCU(m, clear_earliest_events(g));
     MCU(m, cudaMemcpyAsync(g->cnt() + C_TBASE_INL, fr.stage_w(SW_ZERO + 1), 4, cudaMemcpyDeviceToDevice, L.stream));
     g->final_time_base_slot = C_TBASE_INL;
     const List ovl = g->ovl[g->ovl_cur].view;
@@ -1223,7 +1222,7 @@ static int phase_d_staged(rala_b200_multi* m, FabricRank& fr) {
         if (s && !h[SW_FIN_N + s]) continue;   // (segment 0's launch also types `internals`)
         launch_classify_final(L, sub_list(ovl, h[SW_LO + s]), fr.stage_w(SW_FIN_N + s), fr.stage_w(SW_FIN_BASE + s), g->inl[g->inl_cur].view,
                               s ? fr.stage_w(SW_ZERO) : g->cnt() + g->slot_inl, g->cnt() + C_TBASE_INL, g->cap, g->piles.as<uint2>(),
-                              g->events_view(), g->ev_cap, resolve_bufs(g).vcursor, g->cnt());
+                              g->events_view(), g->ev_cap, resolve_bufs(g).first, g->cnt());
     }
     MCU(m, cudaGetLastError());
     return route_and_meet(m, fr, 1);

@@ -112,7 +112,7 @@ struct rala_b200_graph {
     int ovl_cur = 0, inl_cur = 0;
     int slot_ovl = C_LIST0, slot_inl = C_LIST0 + 1, next_slot = C_LIST0 + 2;
     DevBuf events, hill_rec;
-    DevBuf dbuf, flags, segs, tiles;   // dbuf: S | vcursor | vstart | work0 | work1 ; segs: seg_c | seg_t ; tiles: info | off
+    DevBuf dbuf, flags, segs, tiles;   // dbuf: S | vcursor | vstart | work0 | work1 | hidx | first (2 strides) ; segs: seg | hev ; tiles: info | off
     DevBuf counters;
     DevBuf scan_pool;
     size_t scan_pool_words = 0, scan_used = 0;
@@ -199,7 +199,7 @@ cudaError_t begin_stage(rala_b200_graph* g, int stage);
 cudaError_t end_stage(rala_b200_graph* g, int stage);
 cudaError_t zero_counter(rala_b200_graph* g, int slot, int n = 1);
 ResolveBufs resolve_bufs(const rala_b200_graph* g);
-cudaError_t clear_victim_histogram(rala_b200_graph* g);
+cudaError_t clear_earliest_events(rala_b200_graph* g);
 int reserve_events(rala_b200_graph* g, uint32_t ev_cap);
 int reserve_edges(rala_b200_graph* g, uint32_t edge_cap);
 int phase_events(rala_b200_graph* g);
