@@ -393,6 +393,9 @@ int rala_b200_graph_stage_ms(rala_b200_graph* g, float* ms_out /* RALA_B200_N_ST
  * ---------------------------------------------------------------------------------------------- */
 /* a context that enqueues on the caller's CUDA stream (cudaStream_t), e.g. torch's current stream */
 int rala_b200_create_on_stream(rala_b200_ctx** out, int device, void* cuda_stream);
+/* After set_shard with world > 1 the session holds one rank's share of a step: rala_b200_graph_build, _transitive and
+ * _run return RALA_B200_ERR_STATE (they would give a partial edge list or marks); use the phase calls below, or the
+ * multi-GPU session.  set_shard(g, 0, 0, 1) makes it a whole session again. */
 int rala_b200_graph_set_shard(rala_b200_graph* g, uint32_t t0, int rank, int world);
 int rala_b200_graph_phase_events(rala_b200_graph* g);
 int rala_b200_graph_phase_resolve(rala_b200_graph* g, int first_pass);

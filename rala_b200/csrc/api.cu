@@ -217,14 +217,27 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
 }
 
 static int reserve_scan_pool(rala_b200_graph* g) {
-    // worst stage: classify = runs scan + two containment scans over the piles; build = one scan over the piles;
-    // the multi-GPU session adds scans over its exchange capacities (<= 2 x the record count): 16 x leaves room
-    size_t words = 16 * (tiles_of(g->n_rec) + tiles_of(2ull * g->n_piles + 8) + 8);
+    // worst stage: classify = runs scan + two containment scans over the piles; build = one scan over the piles or the
+    // nodes (2 per pile); the multi-GPU session adds scans over its exchange capacities (<= 2 x the record count): 16 x
+    // leaves room
+    size_t words = 16 * (tiles_of(g->n_rec) + tiles_of((uint64_t) g->n_nodes_max + 8) + 8);
     if (words > g->scan_pool_words) {
         CU(g->ctx, g->scan_pool.reserve(words * 8));
         g->scan_pool_words = words;
     }
     return RALA_B200_OK;
+}
+
+// node arrays of the graph: CSR rows, fill cursor, slot degrees and the heavy work list
+static int reserve_nodes(rala_b200_graph* g, uint32_t n_nodes) {
+    rala_b200_ctx* ctx = g->ctx;
+    g->n_nodes_max = n_nodes;
+    CU(ctx, g->row_ptr.reserve(((size_t) n_nodes + 8) * 4));
+    CU(ctx, g->cursor.reserve(((size_t) n_nodes + 8) * 4));
+    CU(ctx, g->slot_degree.reserve(((size_t) n_nodes + 8) * 4));
+    g->heavy_cap = n_nodes;   // one entry per node (HeavyItems)
+    CU(ctx, g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 2));
+    return reserve_scan_pool(g);
 }
 
 // device lists sized for n records (worst case every record survives; the scratch lists of the survivors pass are
@@ -251,8 +264,8 @@ int reserve_for_records(rala_b200_graph* g, uint64_t n) {
     CU(ctx, g->tiles.reserve(align_up((size_t) classify_num_runs((uint32_t) n) + 8, 64) * 4 * 3));
     int rc = reserve_scan_pool(g);
     if (rc) return rc;
-    if (g->state < 1 && g->n_piles) g->state = 1;
-    if (g->state > 1) g->state = 1;
+    if (g->state == SS_EMPTY && g->n_piles) g->state = SS_INPUTS;
+    if (g->state > SS_INPUTS) g->state = SS_INPUTS;
     return RALA_B200_OK;
 }
 
@@ -379,22 +392,16 @@ extern "C" int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* 
                       g->piles.as<uint2>(), n_piles);
     if (n_piles != g->n_piles) {
         g->n_piles = n_piles;
-        g->n_nodes_max = 2 * n_piles;
         CU(ctx, g->dbuf.reserve(align_up((size_t) n_piles + 64, 64) * 4 * 8));
         CU(ctx, g->alive_bits.reserve(((size_t) n_piles / 32 + 2) * 4));
         CU(ctx, g->seq_to_node.reserve((size_t) n_piles * 4 + 16));
-        CU(ctx, g->row_ptr.reserve(((size_t) g->n_nodes_max + 8) * 4));
-        CU(ctx, g->cursor.reserve(((size_t) g->n_nodes_max + 8) * 4));
-        CU(ctx, g->slot_degree.reserve(((size_t) g->n_nodes_max + 8) * 4));
-        g->heavy_cap = g->n_nodes_max;   // one entry per node (HeavyItems)
-        CU(ctx, g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 2));
-        int rc = reserve_scan_pool(g);
+        int rc = reserve_nodes(g, 2 * n_piles);
         if (rc) return rc;
     }
     g->piles_dirty = true;
     g->promote_pending = true;
     g->piles_fresh = true;
-    if (g->state < 1 && g->n_rec) g->state = 1;
+    if (g->state == SS_EMPTY && g->n_rec) g->state = SS_INPUTS;
     return RALA_B200_OK;
 }
 
@@ -455,7 +462,7 @@ static int resolve_containment(rala_b200_graph* g, bool decode, bool skip_if_emp
 // ---- graph.cpp:443-518 in three phases (the multi-GPU path exchanges events between them) ----------------
 int phase_events(rala_b200_graph* g) {
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 1) return fail(ctx, RALA_B200_ERR_STATE, "classify: set_overlaps and set_piles first");
+    if (g->state < SS_INPUTS) return fail(ctx, RALA_B200_ERR_STATE, "classify: set_overlaps and set_piles first");
     CU(ctx, cudaSetDevice(ctx->device));
     // classify kills piles in the working table: keep the table it started from, so that calling classify
     // again without a new set_piles re-runs on the same input (bench loops, retries)
@@ -493,9 +500,9 @@ static int phase_resolve(rala_b200_graph* g, bool first_pass) {
         const uint32_t* h = g->hills.as<uint32_t>();
         launch_hill_coverage(ctx->L, g->recs.view, g->t0, g->piles.as<uint2>(), g->hill_rec.as<uint32_t>(), g->cap, h,
                              h + g->n_hills, h + 2 * (size_t) g->n_hills, g->n_hills,
-                             g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills, g->dbuf.as<uint32_t>(), g->n_piles, g->cnt());
+                             g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills, g->dbuf.as<uint32_t>(), g->cnt());
     }
-    launch_apply_deaths(ctx->L, g->piles.as<uint2>(), g->dbuf.as<uint32_t>(), g->n_piles, g->cnt(), g->alive_bits.as<uint32_t>(), fused_decode,
+    launch_apply_deaths(ctx->L, g->piles.as<uint2>(), g->dbuf.as<uint32_t>(), g->n_piles, g->alive_bits.as<uint32_t>(), fused_decode,
                         nullptr, skip_if_empty ? g->cnt() + C_EV : nullptr);
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;
@@ -526,7 +533,7 @@ int phase_survivors(rala_b200_graph* g) {
     CU(ctx, end_stage(g, ST_CLASSIFY));
     g->piles_dirty = false;   // lists are trimmed against the table as it stands (only liveness changed, and the split filtered on it)
     g->promote_pending = false;   // and every internal was typed against it
-    g->state = 2;
+    g->state = SS_CLASSIFIED;
     g->final_lists_ready = true;
     g->retrim_passes = 0;
     return RALA_B200_OK;
@@ -549,7 +556,7 @@ static int retrim_list(rala_b200_graph* g, ListBuf* bufs, int* cur, int* slot) {
     CU(ctx, zero_counter(g, out_slot));
     List none{};
     launch_list_pass(ctx->L, 1 /*kRetrim*/, bufs[*cur].view, g->cnt() + *slot, g->cap, g->piles.as<uint2>(), bufs[*cur ^ 1].view,
-                     g->cnt() + out_slot, none, nullptr, nullptr, g->cap, nullptr, g->n_piles, nullptr, g->cnt(), status, ticket);
+                     g->cnt() + out_slot, none, nullptr, nullptr, g->cap, nullptr, nullptr, status, ticket);
     *cur ^= 1;
     *slot = out_slot;
     return RALA_B200_OK;
@@ -559,7 +566,7 @@ static int retrim_list(rala_b200_graph* g, ListBuf* bufs, int* cur, int* slot) {
 extern "C" int rala_b200_graph_retrim(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 2) return fail(ctx, RALA_B200_ERR_STATE, "retrim: classify first");
+    if (g->state != SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "retrim: classify first");
     if (!g->piles_dirty && g->skip_clean_retrim) return RALA_B200_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_RETRIM));
@@ -577,7 +584,7 @@ extern "C" int rala_b200_graph_retrim(rala_b200_graph* g) {
 extern "C" int rala_b200_graph_retrim_promote(rala_b200_graph* g, int* is_changed) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 2) return fail(ctx, RALA_B200_ERR_STATE, "retrim_promote: classify first");
+    if (g->state != SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "retrim_promote: classify first");
     if (is_changed) *is_changed = 0;
     // Against a pile table the internals were already trimmed AND typed with, trim() is the identity and they keep their
     // (non-dovetail) type.  retrim() trims them but does not re-type them: after set_piles -> retrim the promotion of
@@ -598,7 +605,7 @@ extern "C" int rala_b200_graph_retrim_promote(rala_b200_graph* g, int* is_change
     CU(ctx, cudaMemcpyAsync(g->cnt() + ovl_out, g->cnt() + after_slot, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     launch_list_pass(ctx->L, 2 /*kPromote*/, g->inl[g->inl_cur].view, g->cnt() + g->slot_inl, g->cap, g->piles.as<uint2>(),
                      g->inl[g->inl_cur ^ 1].view, g->cnt() + inl_out, g->ovl[g->ovl_cur].view, g->cnt() + ovl_out,
-                     g->cnt() + after_slot, g->cap, nullptr, g->n_piles, nullptr, g->cnt(), status, ticket);
+                     g->cnt() + after_slot, g->cap, nullptr, nullptr, status, ticket);
     g->inl_cur ^= 1;
     g->slot_inl = inl_out;
     g->slot_ovl = ovl_out;
@@ -619,7 +626,7 @@ extern "C" int rala_b200_graph_retrim_promote(rala_b200_graph* g, int* is_change
 // graph.cpp:849-877 on demand: the final `internals` (alive at their own time, not kA/kB) and `overlaps`
 // (both piles alive at the end, not kA/kB)
 int materialize_final_lists(rala_b200_graph* g) {
-    if (g->final_lists_ready || g->state < 3) return RALA_B200_OK;
+    if (g->final_lists_ready || g->state < SS_FINALIZED) return RALA_B200_OK;
     rala_b200_ctx* ctx = g->ctx;
     unsigned long long* status;
     uint32_t* ticket;
@@ -631,15 +638,14 @@ int materialize_final_lists(rala_b200_graph* g) {
     CU(ctx, zero_counter(g, inl_out));
     launch_list_pass(ctx->L, 4 /*kFinalInt*/, g->inl[g->inl_cur].view, g->cnt() + g->slot_inl, g->cap, g->piles.as<uint2>(),
                      g->inl[g->inl_cur ^ 1].view, g->cnt() + inl_out, none, nullptr, nullptr, g->cap, g->dbuf.as<uint32_t>(),
-                     g->n_piles, g->cnt() + g->final_time_base_slot, g->cnt(), status, ticket);
+                     g->cnt() + g->final_time_base_slot, status, ticket);
     g->inl_cur ^= 1;
     g->slot_inl = inl_out;
     scan_state(g, g->cap, &status, &ticket);
     int ovl_out = g->new_slot();
     CU(ctx, zero_counter(g, ovl_out));
     launch_list_pass(ctx->L, 3 /*kFinalOvl*/, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(),
-                     g->ovl[g->ovl_cur ^ 1].view, g->cnt() + ovl_out, none, nullptr, nullptr, g->cap, nullptr, g->n_piles,
-                     nullptr, g->cnt(), status, ticket);
+                     g->ovl[g->ovl_cur ^ 1].view, g->cnt() + ovl_out, none, nullptr, nullptr, g->cap, nullptr, nullptr, status, ticket);
     g->ovl_cur ^= 1;
     g->slot_ovl = ovl_out;
     CU(ctx, cudaGetLastError());
@@ -648,47 +654,55 @@ int materialize_final_lists(rala_b200_graph* g) {
 }
 
 // ---- graph.cpp:831-877 in two phases ---------------------------------------------------------------------
-int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base /* device, nullable */,
-                              const uint32_t* inl_base /* device */) {
+int begin_final_pass(rala_b200_graph* g, int time_base_slot) {
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 2) return fail(ctx, RALA_B200_ERR_STATE, "finalize: classify first");
+    if (g->state != SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "finalize: classify first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_FINALIZE));
     CU(ctx, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     CU(ctx, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     CU(ctx, zero_counter(g, C_EV));
     CU(ctx, clear_earliest_events(g));
+    g->final_time_base_slot = time_base_slot;
+    return RALA_B200_OK;
+}
+
+int end_final_pass(rala_b200_graph* g) {
+    // The filtered `overlaps` / `internals` vectors of graph.cpp:867-877 are NOT materialised here: edge creation
+    // (build) applies the same filter on the fly (both piles alive, type kAB/kBA), and nothing else on the path
+    // reads them.  get_lists / counts materialise them on demand (materialize_final_lists).
+    g->final_lists_ready = false;
+    CU(g->ctx, end_stage(g, ST_FINALIZE));
+    g->state = SS_FINALIZED;
+    return RALA_B200_OK;
+}
+
+int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base, int inl_base_slot) {
+    rala_b200_ctx* ctx = g->ctx;
+    int rc = begin_final_pass(g, inl_base_slot);
+    if (rc) return rc;
     launch_classify_final(ctx->L, g->ovl[g->ovl_cur].view, g->cnt() + g->slot_ovl, ovl_base, g->inl[g->inl_cur].view,
-                          g->cnt() + g->slot_inl, inl_base, g->cap, g->piles.as<uint2>(), g->events_view(), g->ev_cap,
+                          g->cnt() + g->slot_inl, g->cnt() + inl_base_slot, g->cap, g->piles.as<uint2>(), g->events_view(), g->ev_cap,
                           resolve_bufs(g).first, g->cnt());
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;
 }
 
 static int phase_final_resolve(rala_b200_graph* g) {
-    rala_b200_ctx* ctx = g->ctx;
     int rc = phase_resolve(g, false);
-    if (rc) return rc;
-    // The filtered `overlaps` / `internals` vectors of graph.cpp:867-877 are NOT materialised here: edge creation
-    // (build) applies the same filter on the fly (both piles alive, type kAB/kBA), and nothing else on the path
-    // reads them.  get_lists / counts materialise them on demand (materialize_final_lists).
-    g->final_lists_ready = false;
-    CU(ctx, end_stage(g, ST_FINALIZE));
-    g->state = 3;
-    return RALA_B200_OK;
+    return rc ? rc : end_final_pass(g);
 }
 
 extern "C" int rala_b200_graph_finalize(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
-    g->final_time_base_slot = g->slot_ovl;   // internals are timed after every entry of `overlaps`
-    int rc = phase_final_events(g, nullptr, g->cnt() + g->slot_ovl);
+    int rc = phase_final_events(g, nullptr, g->slot_ovl);   // internals are timed after every entry of `overlaps`
     if (!rc) rc = phase_final_resolve(g);
     return rc;
 }
 
 // node ids + the edges of the overlaps in list order (graph.cpp:552-632), and with `csr` their CSR rows.  In a multi-GPU
 // phase the list is the local shard's and the node ids are global: the pile table is replicated.
-static int emit_edges(rala_b200_graph* g, bool csr) {
+int emit_edges(rala_b200_graph* g, bool csr) {
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_BUILD));
@@ -707,44 +721,82 @@ static int emit_edges(rala_b200_graph* g, bool csr) {
     return RALA_B200_OK;
 }
 
+// the edge list is final: rows into the caller's buffer on a forked stream, beside (inside a whole run) the transitive
+// pass; edges beyond the caller's capacity are not written (n_edges tells)
+void fork_edge_download(rala_b200_graph* g) {
+    Launch& L = g->ctx->L;
+    if (!g->out_edges || !g->out_edges_cap || !fork_side(L, 0)) return;
+    launch_pack_edges(L, L.side[0], g->graph_view(), g->edge_cap < g->out_edges_cap ? g->edge_cap : g->out_edges_cap, g->cnt() + C_EDGES,
+                      g->out_edges);
+    g->download_pending = true;
+}
+
+// CSR over an edge list whose columns and counts are in place (the NCCL phases' gathered edges, transitive_reduce)
+int csr_from_edge_list(rala_b200_graph* g) {
+    rala_b200_ctx* ctx = g->ctx;
+    CU(ctx, cudaMemsetAsync(g->cursor.p, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
+    GraphArrays ga = g->graph_view();
+    launch_degree_hist(ctx->L, ga.src, g->cnt() + C_EDGES, g->edge_cap, ga.cursor);
+    unsigned long long* status;
+    uint32_t* ticket;
+    scan_state(g, (uint64_t) g->n_nodes_max + 1, &status, &ticket);
+    launch_build_csr(ctx->L, ga, g->n_nodes_max, g->edge_cap, g->cnt(), status, ticket);
+    CU(ctx, cudaGetLastError());
+    return RALA_B200_OK;
+}
+
+int end_build(rala_b200_graph* g) {
+    CU(g->ctx, cudaGetLastError());
+    CU(g->ctx, end_stage(g, ST_BUILD));
+    g->state = SS_BUILT;
+    return RALA_B200_OK;
+}
+
+// build, transitive and run take every source node; a shard of a multi-GPU step takes part only through the phase calls
+static int refuse_shard(rala_b200_graph* g, const char* what) {
+    return fail(g->ctx, RALA_B200_ERR_STATE, "%s: the session is rank %d of %d (rala_b200_graph_set_shard): use the phase calls "
+                "(rala_b200_graph_phase_*) or the multi-GPU session", what, g->rank, g->world);
+}
+
 // graph.cpp:552-632
 extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "build: finalize first");
+    if (g->world > 1) return refuse_shard(g, "build");
+    if (g->state != SS_FINALIZED) return fail(ctx, RALA_B200_ERR_STATE, "build: finalize first");
     int rc = emit_edges(g, true);
     if (rc) return rc;
-    // the edge list is final: rows into the caller's buffer on a forked stream, beside (inside a whole run) the
-    // transitive pass; edges beyond the caller's capacity are not written (n_edges tells)
-    if (g->out_edges && g->out_edges_cap && fork_side(ctx->L, 0)) {
-        launch_pack_edges(ctx->L, ctx->L.side[0], g->graph_view(), g->edge_cap < g->out_edges_cap ? g->edge_cap : g->out_edges_cap,
-                          g->cnt() + C_EDGES, g->out_edges);
-        g->download_pending = true;
-    }
+    fork_edge_download(g);
     if (g->download_pending && !g->in_run) {
         join_side(ctx->L, 0);
         g->download_pending = false;
     }
+    return end_build(g);
+}
+
+int transitive_stage(rala_b200_graph* g, const GraphArrays& ga, const uint32_t* node_range) {
+    rala_b200_ctx* ctx = g->ctx;
+    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
+    // the two node counters of K3 (a node range of the NCCL phase sits behind them, in words 4 and 5)
+    CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 8, ctx->L.stream));
+    CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));
+    launch_transitive(ctx->L, ga, g->n_nodes_max, g->heavy_view(), g->work_counter.as<uint32_t>(), g->cnt(), node_range);
+    CU(ctx, end_stage(g, ST_K3_KERNELS));
     CU(ctx, cudaGetLastError());
-    CU(ctx, end_stage(g, ST_BUILD));
-    g->state = 4;
     return RALA_B200_OK;
 }
 
-static int run_transitive(rala_b200_graph* g) {
+// marked(e) = T(e) | T(e ^ 1) (copied into `copy` too when given); closes ST_TRANSITIVE
+int marks_stage(rala_b200_graph* g, const GraphArrays& ga, uint8_t* copy, uint32_t copy_cap) {
     rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
-    CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 64, ctx->L.stream));
-    CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));
-    launch_transitive(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->heavy_view(), g->work_counter.as<uint32_t>(),
-                      g->cnt(), 0u, 0xFFFFFFFFu, g->world > 1 ? g->work_counter.as<uint32_t>() + 4 : nullptr);
-    CU(ctx, end_stage(g, ST_K3_KERNELS));
-    launch_finalize_marks(ctx->L, g->graph_view(), g->edge_cap, g->cnt(), g->out_marked, g->out_marked_cap);
+    launch_finalize_marks(ctx->L, ga, g->edge_cap, g->cnt(), copy, copy_cap);
     if (g->download_pending) {
         join_side(ctx->L, 0);
         g->download_pending = false;
     }
     CU(ctx, cudaGetLastError());
+    CU(ctx, end_stage(g, ST_TRANSITIVE));
+    g->state = SS_REDUCED;
     return RALA_B200_OK;
 }
 
@@ -752,14 +804,13 @@ static int run_transitive(rala_b200_graph* g) {
 extern "C" int rala_b200_graph_transitive(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "transitive: build first");
+    if (g->world > 1) return refuse_shard(g, "transitive");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "transitive: build first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_TRANSITIVE));
-    int rc = run_transitive(g);
-    if (rc) return rc;
-    CU(ctx, end_stage(g, ST_TRANSITIVE));
-    g->state = 5;
-    return RALA_B200_OK;
+    const GraphArrays ga = g->graph_view();
+    int rc = transitive_stage(g, ga, nullptr);
+    return rc ? rc : marks_stage(g, ga, g->out_marked, g->out_marked_cap);
 }
 
 static int run_eager(rala_b200_graph* g) {
@@ -792,7 +843,8 @@ struct RunKey {
 
 // host-side bookkeeping a run leaves behind (restored after a replay)
 struct RunHostState {
-    int ovl_cur, inl_cur, slot_ovl, slot_inl, next_slot, final_time_base_slot, state;
+    int ovl_cur, inl_cur, slot_ovl, slot_inl, next_slot, final_time_base_slot;
+    SessionState state;
     bool final_lists_ready, piles_dirty, piles_fresh, promote_pending;
     uint32_t retrim_passes;
     size_t scan_used;
@@ -843,8 +895,9 @@ extern "C" int rala_b200_graph_use_cuda_graph(rala_b200_graph* g, int enabled) {
 extern "C" int rala_b200_graph_run(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
+    if (g->world > 1) return refuse_shard(g, "run");
     if (!g->use_cuda_graph) return run_eager(g);
-    if (g->state < 1) return fail(ctx, RALA_B200_ERR_STATE, "run: set_overlaps and set_piles first");
+    if (g->state < SS_INPUTS) return fail(ctx, RALA_B200_ERR_STATE, "run: set_overlaps and set_piles first");
     CU(ctx, cudaSetDevice(ctx->device));
     if (!g->run_graphs) g->run_graphs = new RunGraph[2];
     const RunKey key = run_key(g);
@@ -900,7 +953,7 @@ int read_counters(rala_b200_graph* g, uint32_t* h) {
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
     if (g->scan_pool_exhausted)
         return fail(ctx, RALA_B200_ERR_LIMIT, "the look-back status pool was exhausted inside a stage (%zu words): the results are void", g->scan_pool_words);
-    if (h[C_OVERFLOW] || (g->state >= 2 && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap || h[C_HILL] > g->cap)
+    if (h[C_OVERFLOW] || (g->state >= SS_CLASSIFIED && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap || h[C_HILL] > g->cap)
         return fail(ctx, RALA_B200_ERR_LIMIT, "a device list overflowed its capacity (cap=%u events=%u hills=%u heavy items=%u)",
                     g->cap, h[C_EV], h[C_HILL], h[C_HEAVY]);
     return RALA_B200_OK;
@@ -914,12 +967,12 @@ extern "C" int rala_b200_graph_counts(rala_b200_graph* g, rala_b200_counts_t* ou
     if (rc) return rc;
     memset(out, 0, sizeof(*out));
     out->n_records = g->n_rec;
-    out->n_overlaps = g->state >= 2 ? h[g->slot_ovl] : 0;
-    out->n_internals = g->state >= 2 ? h[g->slot_inl] : 0;
-    out->n_candidates = g->state >= 3 ? h[C_EV_FIRST] : h[C_EV];
-    out->n_rounds = g->state >= 3 ? h[C_ROUNDS_FIRST] : h[C_ROUNDS];
-    out->n_final_candidates = g->state >= 3 ? h[C_EV] : 0;
-    out->n_final_rounds = g->state >= 3 ? h[C_ROUNDS] : 0;
+    out->n_overlaps = g->state >= SS_CLASSIFIED ? h[g->slot_ovl] : 0;
+    out->n_internals = g->state >= SS_CLASSIFIED ? h[g->slot_inl] : 0;
+    out->n_candidates = g->state >= SS_FINALIZED ? h[C_EV_FIRST] : h[C_EV];
+    out->n_rounds = g->state >= SS_FINALIZED ? h[C_ROUNDS_FIRST] : h[C_ROUNDS];
+    out->n_final_candidates = g->state >= SS_FINALIZED ? h[C_EV] : 0;
+    out->n_final_rounds = g->state >= SS_FINALIZED ? h[C_ROUNDS] : 0;
     out->n_piles = g->n_piles;
     out->n_alive_piles = h[C_ALIVE];
     out->n_nodes = h[C_NODES];
@@ -954,7 +1007,7 @@ extern "C" int rala_b200_graph_get_piles(rala_b200_graph* g, rala_pile_t* piles_
 extern "C" int rala_b200_graph_get_connections(rala_b200_graph* g, uint32_t* ab_out) {
     if (!g || !ab_out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 2) return fail(ctx, RALA_B200_ERR_STATE, "get_connections: classify first");
+    if (g->state < SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "get_connections: classify first");
     uint32_t h[C_COUNT];
     int rc = read_counters(g, h);
     if (rc) return rc;
@@ -972,7 +1025,7 @@ extern "C" int rala_b200_graph_get_connections(rala_b200_graph* g, uint32_t* ab_
 extern "C" int rala_b200_graph_get_lists(rala_b200_graph* g, rala_ovl_t* overlaps_out, rala_ovl_t* internals_out) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 2) return fail(ctx, RALA_B200_ERR_STATE, "get_lists: classify first");
+    if (g->state < SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "get_lists: classify first");
     uint32_t h[C_COUNT];
     int rc = materialize_final_lists(g);
     if (!rc) rc = read_counters(g, h);
@@ -997,7 +1050,7 @@ extern "C" int rala_b200_graph_get_lists(rala_b200_graph* g, rala_ovl_t* overlap
 extern "C" int rala_b200_graph_set_kept_overlaps(rala_b200_graph* g, const rala_ovl_t* kept, uint64_t n) {
     if (!g || (n && !kept)) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "set_kept_overlaps: finalize first");
+    if (g->state != SS_FINALIZED) return fail(ctx, RALA_B200_ERR_STATE, "set_kept_overlaps: finalize first");
     if (n > g->cap) return fail(ctx, RALA_B200_ERR_LIMIT, "set_kept_overlaps: %llu entries exceed the list capacity %u", (unsigned long long) n, g->cap);
     CU(ctx, cudaSetDevice(ctx->device));
     int rc = materialize_final_lists(g);   // `internals` keeps its final form
@@ -1016,7 +1069,7 @@ extern "C" int rala_b200_graph_set_kept_overlaps(rala_b200_graph* g, const rala_
 extern "C" int rala_b200_graph_get_seq_to_node(rala_b200_graph* g, uint32_t* out) {
     if (!g || !out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "get_seq_to_node: build first");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "get_seq_to_node: build first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaMemcpyAsync(out, g->seq_to_node.p, (size_t) g->n_piles * 4, cudaMemcpyDeviceToHost, ctx->L.stream));
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
@@ -1027,7 +1080,7 @@ extern "C" int rala_b200_graph_get_seq_to_node(rala_b200_graph* g, uint32_t* out
 extern "C" int rala_b200_graph_get_csr(rala_b200_graph* g, uint32_t* row_ptr_out, uint32_t* col_out, uint32_t* col_eid_out) {
     if (!g || !row_ptr_out || !col_out || !col_eid_out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "get_csr: build first");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "get_csr: build first");
     uint32_t h[C_COUNT];
     int rc = read_counters(g, h);
     if (rc) return rc;
@@ -1044,7 +1097,7 @@ extern "C" int rala_b200_graph_get_csr(rala_b200_graph* g, uint32_t* row_ptr_out
 extern "C" int rala_b200_graph_get_edges(rala_b200_graph* g, rala_edge_t* out) {
     if (!g || !out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "get_edges: build first");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "get_edges: build first");
     uint32_t h[C_COUNT];
     int rc = read_counters(g, h);
     if (rc) return rc;
@@ -1061,7 +1114,7 @@ extern "C" int rala_b200_graph_get_edges(rala_b200_graph* g, rala_edge_t* out) {
 extern "C" int rala_b200_graph_get_marked(rala_b200_graph* g, uint8_t* out) {
     if (!g || !out) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 5) return fail(ctx, RALA_B200_ERR_STATE, "get_marked: transitive first");
+    if (g->state < SS_REDUCED) return fail(ctx, RALA_B200_ERR_STATE, "get_marked: transitive first");
     uint32_t h[C_COUNT];
     int rc = read_counters(g, h);
     if (rc) return rc;
@@ -1076,8 +1129,8 @@ extern "C" int rala_b200_graph_get_adjacency(rala_b200_graph* g, int which, int 
                                              uint64_t* n_ids_out) {
     if (!g || !off_out || !ids_out || !n_ids_out || which < 0 || which > 1) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "get_adjacency: build first");
-    if (skip_marked && g->state < 5) return fail(ctx, RALA_B200_ERR_STATE, "get_adjacency: transitive first (or pass skip_marked = 0)");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "get_adjacency: build first");
+    if (skip_marked && g->state < SS_REDUCED) return fail(ctx, RALA_B200_ERR_STATE, "get_adjacency: transitive first (or pass skip_marked = 0)");
     uint32_t h[C_COUNT];
     int rc = read_counters(g, h);
     if (rc) return rc;
@@ -1146,6 +1199,40 @@ extern "C" int rala_b200_trim_classify(rala_b200_ctx* ctx, rala_ovl_t* ovl, uint
     return RALA_B200_OK;
 }
 
+// the stateless reduction on a throw-away session: its node and edge arrays hold the caller's graph
+static int transitive_reduce_on(rala_b200_graph* g, uint32_t n_nodes, uint32_t n_edges, const rala_edge_t* edges, uint8_t* marked_out,
+                                uint64_t* n_pairs) {
+    rala_b200_ctx* ctx = g->ctx;
+    cudaStream_t s = ctx->L.stream;
+    int rc = reserve_nodes(g, n_nodes);
+    if (!rc) rc = reserve_edges(g, n_edges);
+    if (rc) return rc;
+    CU(ctx, g->edges_aos.reserve((size_t) n_edges * 12));
+    const GraphArrays ga = g->graph_view();
+    CU(ctx, cudaMemcpyAsync(g->edges_aos.p, edges, (size_t) n_edges * 12, cudaMemcpyHostToDevice, s));
+    CU(ctx, cudaMemcpy2DAsync(ga.src, 4, g->edges_aos.as<char>(), 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
+    CU(ctx, cudaMemcpy2DAsync(ga.dst, 4, g->edges_aos.as<char>() + 4, 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
+    CU(ctx, cudaMemcpy2DAsync(ga.len, 4, g->edges_aos.as<char>() + 8, 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
+    uint32_t h[C_COUNT];
+    memset(h, 0, sizeof(h));
+    h[C_NODES] = n_nodes;
+    h[C_EDGES] = n_edges;
+    CU(ctx, cudaMemcpyAsync(g->counters.p, h, sizeof(h), cudaMemcpyHostToDevice, s));
+    CU(ctx, begin_stage(g, ST_TRANSITIVE));
+    rc = csr_from_edge_list(g);
+    if (!rc) rc = transitive_stage(g, ga, nullptr);
+    if (!rc) rc = marks_stage(g, ga, nullptr, 0u);
+    if (rc) return rc;
+    CU(ctx, cudaMemcpyAsync(marked_out, g->marked.p, n_edges, cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaMemcpyAsync(h, g->counters.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaStreamSynchronize(s));
+    if (h[C_OVERFLOW])
+        return fail(ctx, RALA_B200_ERR_LIMIT, "transitive_reduce: more than 2048 destinations of one node in one hash chunk, "
+                                              "or more than 2^32 heavy work items");
+    if (n_pairs) *n_pairs = h[C_PAIRS];
+    return RALA_B200_OK;
+}
+
 extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes, uint64_t n_edges, const rala_edge_t* edges,
                                            uint8_t* marked_out, uint64_t* n_pairs) {
     if (!ctx || (n_edges && (!edges || !marked_out))) return RALA_B200_ERR_ARG;
@@ -1156,71 +1243,12 @@ extern "C" int rala_b200_transitive_reduce(rala_b200_ctx* ctx, uint32_t n_nodes,
         if (edges[i].src >= n_nodes || edges[i].dst >= n_nodes) return fail(ctx, RALA_B200_ERR_ARG, "edge %llu references a node >= n_nodes", (unsigned long long) i);
     }
     CU(ctx, cudaSetDevice(ctx->device));
-    // a throw-away session provides the buffers
     rala_b200_graph* g = nullptr;
     int rc = rala_b200_graph_create(ctx, &g);
     if (rc) return rc;
-    g->n_piles = (n_nodes + 1) / 2;
-    g->n_nodes_max = n_nodes;
-    g->edge_cap = (uint32_t) n_edges;
-    g->heavy_cap = n_nodes;
-    DevBuf rows;
-    cudaError_t e = rows.reserve((size_t) n_edges * 12);
-    if (e == cudaSuccess) e = g->edges.reserve(align_up((size_t) g->edge_cap * 4, 256) * 3);
-    if (e == cudaSuccess) e = g->col.reserve((size_t) g->edge_cap * 8);
-    if (e == cudaSuccess) e = g->col_eid.reserve((size_t) g->edge_cap * 4);
-    if (e == cudaSuccess) e = g->T.reserve(align_up(g->edge_cap, 256));
-    if (e == cudaSuccess) e = g->marked.reserve(align_up(g->edge_cap, 256));
-    if (e == cudaSuccess) e = g->heavy.reserve(align_up((size_t) g->heavy_cap * 4, 256) * 2);
-    if (e == cudaSuccess) e = g->row_ptr.reserve(((size_t) n_nodes + 8) * 4);
-    if (e == cudaSuccess) e = g->cursor.reserve(((size_t) n_nodes + 8) * 4);
-    g->scan_pool_words = 4 * (tiles_of((uint64_t) n_nodes + 1) + 8);
-    if (e == cudaSuccess) e = g->scan_pool.reserve(g->scan_pool_words * 8);
-    if (e != cudaSuccess) {
-        rows.release();
-        rala_b200_graph_destroy(g);
-        return fail(ctx, RALA_B200_ERR_CUDA, "transitive_reduce: %s", cudaGetErrorString(e));
-    }
-    auto cleanup = [&](int code) {
-        rows.release();
-        rala_b200_graph_destroy(g);
-        return code;
-    };
-    GraphArrays ga = g->graph_view();
-    cudaStream_t s = ctx->L.stream;
-#define CUX(call)                                                                                      \
-    do {                                                                                               \
-        cudaError_t err__ = (call);                                                                    \
-        if (err__ != cudaSuccess) return cleanup(fail(ctx, RALA_B200_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(err__))); \
-    } while (0)
-    CUX(cudaMemcpyAsync(rows.p, edges, (size_t) n_edges * 12, cudaMemcpyHostToDevice, s));
-    CUX(cudaMemcpy2DAsync(ga.src, 4, rows.as<char>(), 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
-    CUX(cudaMemcpy2DAsync(ga.dst, 4, rows.as<char>() + 4, 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
-    CUX(cudaMemcpy2DAsync(ga.len, 4, rows.as<char>() + 8, 12, 4, n_edges, cudaMemcpyDeviceToDevice, s));
-    uint32_t hc[C_COUNT];
-    memset(hc, 0, sizeof(hc));
-    hc[C_NODES] = n_nodes;
-    hc[C_EDGES] = (uint32_t) n_edges;
-    CUX(cudaMemcpyAsync(g->counters.p, hc, sizeof(hc), cudaMemcpyHostToDevice, s));
-    CUX(cudaMemsetAsync(g->cursor.p, 0, ((size_t) n_nodes + 8) * 4, s));
-    CUX(cudaMemsetAsync(g->scan_pool.p, 0, g->scan_pool_words * 8, s));
-    launch_degree_hist(ctx->L, ga.src, g->cnt() + C_EDGES, g->edge_cap, ga.cursor);
-    unsigned long long* status;
-    uint32_t* ticket;
-    scan_state(g, (uint64_t) n_nodes + 1, &status, &ticket);
-    launch_build_csr(ctx->L, ga, n_nodes, g->edge_cap, g->cnt(), status, ticket);
-    rc = run_transitive(g);
-    if (rc) return cleanup(rc);
-    uint32_t h[C_COUNT];
-    CUX(cudaMemcpyAsync(marked_out, g->marked.p, n_edges, cudaMemcpyDeviceToHost, s));
-    CUX(cudaMemcpyAsync(h, g->counters.p, sizeof(h), cudaMemcpyDeviceToHost, s));
-    CUX(cudaStreamSynchronize(s));
-#undef CUX
-    if (h[C_OVERFLOW])
-        return cleanup(fail(ctx, RALA_B200_ERR_LIMIT, "transitive_reduce: more than 2048 destinations of one node in one hash chunk, "
-                                                      "or more than 2^32 heavy work items"));
-    if (n_pairs) *n_pairs = h[C_PAIRS];
-    return cleanup(RALA_B200_OK);
+    rc = transitive_reduce_on(g, n_nodes, (uint32_t) n_edges, edges, marked_out, n_pairs);
+    rala_b200_graph_destroy(g);
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1256,7 +1284,7 @@ extern "C" int rala_b200_graph_phase_survivors(rala_b200_graph* g) { return g ? 
 extern "C" int rala_b200_graph_phase_emit_edges(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state != 3) return fail(ctx, RALA_B200_ERR_STATE, "emit_edges: finalize first");
+    if (g->state != SS_FINALIZED) return fail(ctx, RALA_B200_ERR_STATE, "emit_edges: finalize first");
     int rc = emit_edges(g, false);   // the CSR is built over the edges of all ranks (phase_csr)
     if (rc) return rc;
     CU(ctx, cudaGetLastError());
@@ -1309,7 +1337,7 @@ extern "C" uint64_t rala_b200_exchange_block_words(int kind, uint32_t cap) {
 extern "C" int rala_b200_graph_export_list_counts(rala_b200_graph* g, uint32_t* d_pair) {
     if (!g || !d_pair) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 2) return fail(ctx, RALA_B200_ERR_STATE, "export_list_counts: classify first");
+    if (g->state < SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "export_list_counts: classify first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, cudaMemcpyAsync(d_pair, g->cnt() + g->slot_ovl, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
     CU(ctx, cudaMemcpyAsync(d_pair + 1, g->cnt() + g->slot_inl, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
@@ -1321,8 +1349,7 @@ extern "C" int rala_b200_graph_phase_final_events_gathered(rala_b200_graph* g, c
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     launch_time_bases(ctx->L, d_counts, (uint32_t) g->rank, (uint32_t) world, g->cnt() + C_TBASE_OVL);
-    g->final_time_base_slot = C_TBASE_INL;
-    return phase_final_events(g, g->cnt() + C_TBASE_OVL, g->cnt() + C_TBASE_INL);
+    return phase_final_events(g, g->cnt() + C_TBASE_OVL, C_TBASE_INL);
 }
 
 // CSR over ALL edges (replicated on every rank)
@@ -1330,35 +1357,21 @@ extern "C" int rala_b200_graph_phase_csr(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, cudaMemsetAsync(g->cursor.p, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
-    GraphArrays ga = g->graph_view();
-    launch_degree_hist(ctx->L, ga.src, g->cnt() + C_EDGES, g->edge_cap, ga.cursor);
-    unsigned long long* status;
-    uint32_t* ticket;
-    scan_state(g, (uint64_t) g->n_nodes_max + 1, &status, &ticket);
-    launch_build_csr(ctx->L, ga, g->n_nodes_max, g->edge_cap, g->cnt(), status, ticket);
-    CU(ctx, cudaGetLastError());
-    CU(ctx, end_stage(g, ST_BUILD));
-    g->state = 4;
-    return RALA_B200_OK;
+    int rc = csr_from_edge_list(g);
+    return rc ? rc : end_build(g);
 }
 
 // T(e) for the candidate edges whose source node this rank owns
 extern "C" int rala_b200_graph_phase_transitive(rala_b200_graph* g) {
     if (!g) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
-    if (g->state < 4) return fail(ctx, RALA_B200_ERR_STATE, "transitive: build first");
+    if (g->state < SS_BUILT) return fail(ctx, RALA_B200_ERR_STATE, "transitive: build first");
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_TRANSITIVE));
-    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
-    CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 64, ctx->L.stream));
-    launch_node_range(ctx->L, g->graph_view(), g->cnt(), (uint32_t) g->rank, (uint32_t) g->world, g->work_counter.as<uint32_t>() + 4);
-    CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));
-    launch_transitive(ctx->L, g->graph_view(), g->n_nodes_max, g->edge_cap, g->heavy_view(), g->work_counter.as<uint32_t>(),
-                      g->cnt(), 0u, 0xFFFFFFFFu, g->work_counter.as<uint32_t>() + 4);
-    CU(ctx, end_stage(g, ST_K3_KERNELS));
-    CU(ctx, cudaGetLastError());
-    return RALA_B200_OK;
+    const GraphArrays ga = g->graph_view();
+    uint32_t* node_range = g->work_counter.as<uint32_t>() + 4;
+    launch_node_range(ctx->L, ga, g->cnt(), (uint32_t) g->rank, (uint32_t) g->world, node_range);
+    return transitive_stage(g, ga, node_range);
 }
 
 extern "C" int rala_b200_graph_export_marks(rala_b200_graph* g, uint8_t* d_T, uint32_t n) {
@@ -1375,9 +1388,5 @@ extern "C" int rala_b200_graph_phase_marks(rala_b200_graph* g, const uint8_t* d_
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     if (n) CU(ctx, cudaMemcpyAsync(g->T.p, d_T, n, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    launch_finalize_marks(ctx->L, g->graph_view(), g->edge_cap, g->cnt(), nullptr, 0u);
-    CU(ctx, cudaGetLastError());
-    CU(ctx, end_stage(g, ST_TRANSITIVE));
-    g->state = 5;
-    return RALA_B200_OK;
+    return marks_stage(g, g->graph_view(), nullptr, 0u);
 }

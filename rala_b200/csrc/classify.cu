@@ -440,9 +440,8 @@ __global__ void k_hill_coverage(List recs, uint32_t t0, const uint2* __restrict_
                                 const uint32_t* __restrict__ hill_rec, uint32_t hill_cap,
                                 const uint32_t* __restrict__ hill_pile, const uint32_t* __restrict__ hill_begin,
                                 const uint32_t* __restrict__ hill_end, uint32_t n_hills, uint32_t* __restrict__ hill_cov,
-                                const uint32_t* __restrict__ dbuf, uint32_t n_piles, const uint32_t* __restrict__ counters) {
+                                const uint32_t* __restrict__ D, const uint32_t* __restrict__ counters) {
     const uint32_t n = min(counters[C_HILL], hill_cap);
-    const uint32_t* D = dbuf + (size_t) counters[C_DSEL] * n_piles;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const uint32_t idx = hill_rec[i];
         Entry e = load_entry(recs, idx);   // the record passed the static gates: the invalid bit of column a is clear
@@ -477,11 +476,9 @@ __global__ void k_hill_coverage(List recs, uint32_t t0, const uint2* __restrict_
 // DECODE: dbuf still holds the resolution's state words (containment.cu: settled bit | death time, 0x7FFFFFFF = never);
 // they are turned into death times (kInf = never) on the way, which saves the separate k_decode_state launch.
 template <bool DECODE>
-__global__ void k_apply_deaths(uint2* __restrict__ piles, uint32_t* __restrict__ dbuf, uint32_t n_piles,
-                               const uint32_t* __restrict__ counters, uint32_t* __restrict__ alive_bits, const uint32_t* __restrict__ skip,
-                               const uint32_t* __restrict__ run_if) {
+__global__ void k_apply_deaths(uint2* __restrict__ piles, uint32_t* __restrict__ D, uint32_t n_piles, uint32_t* __restrict__ alive_bits,
+                               const uint32_t* __restrict__ skip, const uint32_t* __restrict__ run_if) {
     if ((skip && *skip) || (run_if && *run_if == 0u)) return;
-    uint32_t* D = dbuf + (size_t) counters[C_DSEL] * n_piles;
     for (uint32_t base = blockIdx.x * blockDim.x; base < n_piles; base += gridDim.x * blockDim.x) {
         const uint32_t i = base + threadIdx.x;
         bool alive = false;
@@ -502,27 +499,26 @@ __global__ void k_apply_deaths(uint2* __restrict__ piles, uint32_t* __restrict__
 
 // =============================================================================================
 // Ordered list passes.  MODE selects what happens to an entry:
-//   kSplitAlive   P -> overlaps (tag != kX) / internals (tag == kX), both piles alive   graph.cpp:493-515
 //   kRetrim       list -> list, dropping entries trim() rejects                          :722-736, 801-807
 //   kPromote      internals -> internals / appended to overlaps when now a dovetail      :809-824
 //   kFinalOvl     overlaps -> overlaps, keeping entries with both piles alive and not kA/kB  :831-848, 869-877
 //   kFinalInt     internals -> internals (alive at their own time, not kA/kB)            :849-867
 // =============================================================================================
-enum ListMode { kSplitAlive = 0, kRetrim = 1, kPromote = 2, kFinalOvl = 3, kFinalInt = 4 };
+enum ListMode { kRetrim = 1, kPromote = 2, kFinalOvl = 3, kFinalInt = 4 };
 
+// 4 blocks per SM (64 registers): unbounded, ptxas gives kFinalInt 79 registers and kRetrim / kFinalOvl a small spill
 template <int MODE>
-__global__ void __launch_bounds__(kTileThreads) k_list_pass(
+__global__ void __launch_bounds__(kTileThreads, 4) k_list_pass(
     List in, const uint32_t* __restrict__ n_in_ptr, uint32_t in_cap, const uint2* __restrict__ piles,
     List out_a, uint32_t* __restrict__ n_out_a, List out_b, uint32_t* __restrict__ n_out_b,
-    const uint32_t* __restrict__ b_base_ptr, uint32_t cap, const uint32_t* __restrict__ dbuf, uint32_t n_piles, const uint32_t* __restrict__ time_base_ptr,
-    const uint32_t* __restrict__ counters, unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket) {
+    const uint32_t* __restrict__ b_base_ptr, uint32_t cap, const uint32_t* __restrict__ D, const uint32_t* __restrict__ time_base_ptr,
+    unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket) {
     __shared__ TileShared sh;
     const uint32_t tid = threadIdx.x;
     const uint32_t n = min(*n_in_ptr, in_cap);
     const uint32_t num_tiles = (n + kTile - 1) / kTile;
     // kPromote appends behind the current end of `overlaps` (count in a slot this kernel never writes)
     const uint32_t b_off = b_base_ptr ? *b_base_ptr : 0u;
-    const uint32_t* D = dbuf ? dbuf + (size_t) counters[C_DSEL] * n_piles : nullptr;
     const uint32_t time_base = time_base_ptr ? *time_base_ptr : 0u;
     __syncthreads();
 
@@ -545,9 +541,7 @@ __global__ void __launch_bounds__(kTileThreads) k_list_pass(
                 e[r] = load_entry(in, idx);
                 tag[r] = in.tag[idx];
                 const Pile pa = load_pile(piles, e[r].a), pb = load_pile(piles, e[r].b);
-                if (MODE == kSplitAlive) {
-                    if (pa.alive() && pb.alive()) dest[r] = tag[r] == kX ? 2 : 1;
-                } else if (MODE == kRetrim) {
+                if (MODE == kRetrim) {
                     if (pa.alive() && pb.alive() && trim(e[r].c, e[r].ori, pa, pb)) dest[r] = 1;
                 } else if (MODE == kPromote) {
                     if (pa.alive() && pb.alive() && trim(e[r].c, e[r].ori, pa, pb)) {
@@ -738,29 +732,27 @@ uint32_t classify_num_runs(uint32_t n) { return (n + kRunRecords - 1) / kRunReco
 void launch_hill_coverage(Launch& L, List recs, uint32_t t0, const uint2* piles, const uint32_t* hill_rec,
                           uint32_t hill_cap, const uint32_t* hill_pile, const uint32_t* hill_begin,
                           const uint32_t* hill_end, uint32_t n_hills, uint32_t* hill_cov, const uint32_t* dbuf,
-                          uint32_t n_piles, const uint32_t* counters) {
+                          const uint32_t* counters) {
     k_hill_coverage<<<kNumSMs * 2, 256, 0, L.stream>>>(recs, t0, piles, hill_rec, hill_cap, hill_pile, hill_begin, hill_end,
-                                                       n_hills, hill_cov, dbuf, n_piles, counters);
+                                                       n_hills, hill_cov, dbuf, counters);
     L.count++;
 }
 
-void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, const uint32_t* counters,
-                         uint32_t* alive_bits, bool decode, const uint32_t* skip, const uint32_t* run_if) {
+void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, uint32_t* alive_bits, bool decode,
+                         const uint32_t* skip, const uint32_t* run_if) {
     if (n_piles == 0) return;
-    if (decode) k_apply_deaths<true><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, counters, alive_bits, skip, run_if);
-    else k_apply_deaths<false><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, counters, alive_bits, skip, run_if);
+    if (decode) k_apply_deaths<true><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if);
+    else k_apply_deaths<false><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if);
     L.count++;
 }
 
 void launch_list_pass(Launch& L, int mode, List in, const uint32_t* n_in, uint32_t in_cap, const uint2* piles, List out_a,
                       uint32_t* n_out_a, List out_b, uint32_t* n_out_b, const uint32_t* b_base, uint32_t cap, const uint32_t* dbuf,
-                      uint32_t n_piles, const uint32_t* time_base, const uint32_t* counters, unsigned long long* status,
-                      uint32_t* ticket) {
+                      const uint32_t* time_base, unsigned long long* status, uint32_t* ticket) {
     int grid = grid_for(in_cap, kTile, kNumSMs * 8);
 #define RB_LP(M) k_list_pass<M><<<grid, kTileThreads, 0, L.stream>>>(in, n_in, in_cap, piles, out_a, n_out_a, out_b, \
-        n_out_b, b_base, cap, dbuf, n_piles, time_base, counters, status, ticket)
+        n_out_b, b_base, cap, dbuf, time_base, status, ticket)
     switch (mode) {
-        case kSplitAlive: RB_LP(kSplitAlive); break;
         case kRetrim: RB_LP(kRetrim); break;
         case kPromote: RB_LP(kPromote); break;
         case kFinalOvl: RB_LP(kFinalOvl); break;
@@ -826,7 +818,6 @@ void preload_classify() {
     cudaFuncGetAttributes(&a, k_hill_coverage);
     cudaFuncGetAttributes(&a, k_apply_deaths<true>);
     cudaFuncGetAttributes(&a, k_apply_deaths<false>);
-    cudaFuncGetAttributes(&a, k_list_pass<kSplitAlive>);
     cudaFuncGetAttributes(&a, k_list_pass<kRetrim>);
     cudaFuncGetAttributes(&a, k_list_pass<kPromote>);
     cudaFuncGetAttributes(&a, k_list_pass<kFinalOvl>);

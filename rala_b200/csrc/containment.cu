@@ -291,10 +291,7 @@ __global__ void __launch_bounds__(256) k_resolve(const uint2* __restrict__ seg_r
         out = const_cast<uint32_t*>(tmp);
         ++round;
     }
-    if (threadIdx.x == 0) {
-        counters[C_ROUNDS] = round;
-        counters[C_DSEL] = 0u;
-    }
+    if (threadIdx.x == 0) counters[C_ROUNDS] = round;
 }
 
 void launch_events_first(Launch& L, Events ev, const uint32_t* n_events, uint32_t ev_cap, unsigned long long* first) {

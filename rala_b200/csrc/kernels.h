@@ -11,11 +11,9 @@ namespace rb {
 
 // slots of the device-side counter block (uint32 each)
 enum Counter {
-    C_P = 0,        // (unused)
-    C_EV,           // containment events of the current resolution
+    C_EV = 0,       // containment events of the current resolution
     C_HILL,         // records touching a pile with hills
     C_ROUNDS,       // fixed-point rounds
-    C_DSEL,         // which of the four death-time buffers holds the result
     C_NODES,        // nodes_.size()
     C_ALIVE,        // alive piles
     C_DOVETAILS,    // dovetail overlaps = edges / 2
@@ -77,15 +75,14 @@ uint32_t classify_num_runs(uint32_t n);
 void launch_hill_coverage(Launch& L, List recs, uint32_t t0, const uint2* piles, const uint32_t* hill_rec,
                           uint32_t hill_cap, const uint32_t* hill_pile, const uint32_t* hill_begin,
                           const uint32_t* hill_end, uint32_t n_hills, uint32_t* hill_cov, const uint32_t* dbuf,
-                          uint32_t n_piles, const uint32_t* counters);
+                          const uint32_t* counters);
 // skip: optional device flag, non-zero = do nothing (multi-GPU: a containment pass without events); run_if: optional device
 // count, zero = do nothing (single GPU: the final containment pass when it has no events)
-void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, const uint32_t* counters,
-                         uint32_t* alive_bits, bool decode, const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr);
+void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, uint32_t* alive_bits, bool decode,
+                         const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr);
 void launch_list_pass(Launch& L, int mode, List in, const uint32_t* n_in, uint32_t in_cap, const uint2* piles, List out_a,
                       uint32_t* n_out_a, List out_b, uint32_t* n_out_b, const uint32_t* b_base, uint32_t cap,
-                      const uint32_t* dbuf, uint32_t n_piles, const uint32_t* time_base, const uint32_t* counters,
-                      unsigned long long* status, uint32_t* ticket);
+                      const uint32_t* dbuf, const uint32_t* time_base, unsigned long long* status, uint32_t* ticket);
 void launch_classify_final(Launch& L, List ovl, const uint32_t* n_ovl, const uint32_t* ovl_time_base, List inl,
                            const uint32_t* n_inl, const uint32_t* inl_time_base, uint32_t cap, const uint2* piles, Events ev,
                            uint32_t ev_cap, unsigned long long* first, uint32_t* counters);
@@ -175,9 +172,9 @@ struct HeavyItems {
     uint32_t *node, *unit_base;
     uint32_t cap;
 };
-void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t edge_cap, HeavyItems heavy,
-                       uint32_t* work_counter, uint32_t* counters, uint32_t node_begin, uint32_t node_end,
-                       const uint32_t* node_range /* device {begin, end}, nullable */);
+// node_range: device {begin, end} of the source nodes to evaluate; nullptr = all of them
+void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, HeavyItems heavy, uint32_t* work_counter, uint32_t* counters,
+                       const uint32_t* node_range);
 void launch_node_range(Launch& L, GraphArrays g, const uint32_t* counters, uint32_t rank, uint32_t world, uint32_t* out);
 void launch_finalize_marks(Launch& L, GraphArrays g, uint32_t edge_cap, uint32_t* counters, uint8_t* marked_copy /* nullable */,
                            uint32_t copy_cap);

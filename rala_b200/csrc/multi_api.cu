@@ -502,13 +502,12 @@ static int resolve_owned_piles(rala_b200_multi* m, FabricRank& fr, int pass, boo
         const uint32_t n = g->n_hills;
         launch_decode_states(L, fr.P, fr.A);
         launch_hill_coverage(L, g->recs.view, g->t0, g->piles.as<uint2>(), g->hill_rec.as<uint32_t>(), g->cap, h, h + n, h + 2 * (size_t) n,
-                             n, g->hills.as<uint32_t>() + 3 * (size_t) n, fr.sec<uint32_t>(fr.A.S), g->n_piles, g->cnt());
+                             n, g->hills.as<uint32_t>() + 3 * (size_t) n, fr.sec<uint32_t>(fr.A.S), g->cnt());
         launch_push_hills(L, fr.P, fr.A, h + 3 * (size_t) n, n);
     }
     // every replica now holds every pile's final state: piles with a finite death time die (graph.cpp:471,477,838,842)
     // (a skipped pass killed nobody: the table and the liveness bitmap stay as they are)
-    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->cnt(), g->alive_bits.as<uint32_t>(), !hills,
-                        skip_flag(fr.P));
+    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->alive_bits.as<uint32_t>(), !hills, skip_flag(fr.P));
     MCU(m, cudaGetLastError());
     return RALA_B200_OK;
 }
@@ -542,8 +541,7 @@ static int phase_d_final_events(rala_b200_multi* m, FabricRank& fr) {
     MCU(m, cudaSetDevice(fr.device));
     rala_b200_graph* g = fr.g;
     launch_time_bases_mail(fr.ctx->L, fr.P, g->cnt() + C_TBASE_OVL);
-    g->final_time_base_slot = C_TBASE_INL;
-    MRC(m, fr, phase_final_events(g, g->cnt() + C_TBASE_OVL, g->cnt() + C_TBASE_INL));   // graph.cpp:831-848 on the local lists
+    MRC(m, fr, phase_final_events(g, g->cnt() + C_TBASE_OVL, C_TBASE_INL));   // graph.cpp:831-848 on the local lists
     return route_and_meet(m, fr, 1);
 }
 
@@ -551,35 +549,18 @@ static int phase_e_final_resolve(rala_b200_multi* m, FabricRank& fr) {
     MCU(m, cudaSetDevice(fr.device));
     int rc = resolve_owned_piles(m, fr, 1);
     if (rc) return rc;
-    rala_b200_graph* g = fr.g;
-    g->final_lists_ready = false;
-    MCU(m, end_stage(g, ST_FINALIZE));
-    g->state = 3;
+    MRC(m, fr, end_final_pass(fr.g));
     return RALA_B200_OK;
 }
 
 // graph.cpp:552-632: node ids (replicated), the edges of the local dovetails, routed to the owners of their sources
 static int phase_f_edges(rala_b200_multi* m, FabricRank& fr) {
-    MCU(m, cudaSetDevice(fr.device));
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
-    MCU(m, begin_stage(g, ST_BUILD));
-    MCU(m, zero_counter(g, C_NODES, 4));
-    unsigned long long* status;
-    uint32_t* ticket;
-    scan_state(g, g->n_piles, &status, &ticket);
-    GraphArrays ga = g->graph_view();
-    ga.cursor = nullptr;   // no local CSR: the owners build theirs from what they receive
-    const List ovl = g->ovl[g->ovl_cur].view;
-    launch_count_scan(L, ovl, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), g->n_piles, ga, g->edge_cap, g->tile_dov.as<uint32_t>(),
-                      g->cnt(), status, ticket);
+    MRC(m, fr, emit_edges(g, false));   // no local CSR: the owners build theirs from what they receive
+    fork_edge_download(g);
     launch_node_bounds(L, fr.P, fr.A, g->cnt() + C_NODES, fr.meta_dev());
-    launch_emit_edges(L, ovl, g->cnt() + g->slot_ovl, g->cap, g->piles.as<uint2>(), ga, g->edge_cap, g->tile_dov.as<uint32_t>());
-    if (g->out_edges && g->out_edges_cap && fork_side(L, 0)) {   // rows of the local edges straight into the caller's memory
-        launch_pack_edges(L, L.side[0], g->graph_view(), g->edge_cap < g->out_edges_cap ? g->edge_cap : g->out_edges_cap,
-                          g->cnt() + C_EDGES, g->out_edges);
-        g->download_pending = true;
-    }
+    const GraphArrays ga = g->graph_view();
     // result bytes of the local edges: cleared now, written by the evaluating ranks after two more barriers
     launch_clear_bytes16(L, fr.sec<uint8_t>(fr.A.T_in), g->cnt() + C_EDGES, fr.A.t_cap);
     launch_route_edges(L, fr.P, fr.A, ga.src, ga.dst, ga.len, g->cnt() + C_EDGES, g->edge_cap, fr.meta_dev(), fr.cnt_edges());
@@ -608,9 +589,7 @@ static int phase_g_csr(rala_b200_multi* m, FabricRank& fr) {
                       m->staged_edges ? fr.runs_dev() : nullptr);
     launch_push_csr(L, fr.P, fr.A, fr.meta_dev(), g->row_ptr.as<uint32_t>());
     launch_fabric_barrier(L, fr.P, no_mail(m));
-    MCU(m, cudaGetLastError());
-    MCU(m, end_stage(g, ST_BUILD));
-    g->state = 4;
+    MRC(m, fr, end_build(g));
     return RALA_B200_OK;
 }
 
@@ -620,17 +599,12 @@ static int phase_h_transitive(rala_b200_multi* m, FabricRank& fr) {
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
     MCU(m, begin_stage(g, ST_TRANSITIVE));
-    MCU(m, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
-    MCU(m, cudaMemsetAsync(g->work_counter.p, 0, 64, L.stream));
     GraphArrays ga = g->graph_view();
     ga.row_ptr = fr.sec<uint32_t>(fr.A.row_ptr);
     ga.col = fr.sec<uint2>(fr.A.col);
     ga.col_eid = fr.col_eid.as<uint32_t>();
     ga.T = fr.T.as<uint8_t>();
-    MCU(m, stage_event(g, g->ev_start[ST_K3_KERNELS]));
-    launch_transitive(L, ga, g->n_nodes_max, g->edge_cap, g->heavy_view(), g->work_counter.as<uint32_t>(), g->cnt(), 0u, 0xFFFFFFFFu,
-                      fr.meta_dev()->node_begin + fr.rank);
-    MCU(m, end_stage(g, ST_K3_KERNELS));
+    MRC(m, fr, transitive_stage(g, ga, fr.meta_dev()->node_begin + fr.rank));
     launch_route_marks(L, fr.P, fr.A, fr.meta_dev(), fr.T.as<uint8_t>(), fr.col_eid.as<uint32_t>(), m->staged_edges ? fr.runs_dev() : nullptr);
     launch_fabric_barrier(L, fr.P, no_mail(m));
     return RALA_B200_OK;
@@ -643,15 +617,9 @@ static int phase_i_marks(rala_b200_multi* m, FabricRank& fr) {
     Launch& L = fr.ctx->L;
     GraphArrays ga = g->graph_view();
     ga.T = fr.sec<uint8_t>(fr.A.T_in);
-    launch_finalize_marks(L, ga, g->edge_cap, g->cnt(), g->out_marked, g->out_marked_cap);
+    MRC(m, fr, marks_stage(g, ga, g->out_marked, g->out_marked_cap));
     launch_demand(L, fr.P, fr.cnt_ev(0), fr.cnt_ev(1), fr.cnt_edges(), fr.meta_dev());
-    if (g->download_pending) {
-        join_side(L, 0);
-        g->download_pending = false;
-    }
     MCU(m, cudaGetLastError());
-    MCU(m, end_stage(g, ST_TRANSITIVE));
-    g->state = 5;
     return RALA_B200_OK;
 }
 
@@ -681,7 +649,7 @@ extern "C" int rala_b200_multi_run(rala_b200_multi* m) {
     if (!m) return RALA_B200_ERR_ARG;
     if (!m->reserved || !m->connected) return mfail(m, RALA_B200_ERR_STATE, "run: reserve (and connect) the exchange arenas first");
     for (FabricRank& fr : m->ranks)
-        if (fr.g->state < 1) return mfail(m, RALA_B200_ERR_STATE, "run: rank %d has no inputs", fr.rank);
+        if (fr.g->state < SS_INPUTS) return mfail(m, RALA_B200_ERR_STATE, "run: rank %d has no inputs", fr.rank);
     m->staged = 0;
     m->staged_edges = false;
     const int variant = m->ranks[0].g->piles_fresh ? 1 : 0;
@@ -857,7 +825,7 @@ extern "C" int rala_b200_multi_counts(rala_b200_multi* m, rala_b200_multi_counts
 // global id runs of local rank k's edges, in local order, adjacent runs merged: out (nullable) holds 2 x RALA_B200_MAX_SEGMENTS
 static int edge_runs_of(rala_b200_multi* m, int k, uint64_t* out, uint32_t* n_out) {
     FabricRank& fr = m->ranks[k];
-    if (fr.g->state < 4) return mfail(m, RALA_B200_ERR_STATE, "edge_runs: run (or finish) first");
+    if (fr.g->state < SS_BUILT) return mfail(m, RALA_B200_ERR_STATE, "edge_runs: run (or finish) first");
     std::vector<uint64_t> r;   // first, count, first, count, ...
     auto add = [&](uint64_t first, uint64_t count) {
         if (!count) return;
@@ -889,7 +857,7 @@ extern "C" int rala_b200_multi_edge_runs(rala_b200_multi* m, int k, uint64_t* fi
 extern "C" int rala_b200_multi_edge_range(rala_b200_multi* m, int k, uint64_t* first_edge, uint64_t* n) {
     if (!m || k < 0 || k >= m->n_local || !first_edge || !n) return RALA_B200_ERR_ARG;
     FabricRank& fr = m->ranks[k];
-    if (fr.g->state < 4) return mfail(m, RALA_B200_ERR_STATE, "edge_range: run first");
+    if (fr.g->state < SS_BUILT) return mfail(m, RALA_B200_ERR_STATE, "edge_range: run first");
     if (m->staged_edges) {
         uint64_t r[2 * kMaxSegs];
         uint32_t n_runs = 0;
@@ -1066,7 +1034,7 @@ static int read_seg_mail(rala_b200_multi* m, std::vector<uint32_t>& mail) {
 static int staged_ready(rala_b200_multi* m, const char* what) {
     if (!m->reserved || !m->connected) return mfail(m, RALA_B200_ERR_STATE, "%s: reserve (and connect) the exchange arenas first", what);
     for (FabricRank& fr : m->ranks)
-        if (fr.g->state < 1) return mfail(m, RALA_B200_ERR_STATE, "%s: rank %d has no inputs", what, fr.rank);
+        if (fr.g->state < SS_INPUTS) return mfail(m, RALA_B200_ERR_STATE, "%s: rank %d has no inputs", what, fr.rank);
     return RALA_B200_OK;
 }
 
@@ -1188,7 +1156,6 @@ static int phase_d_staged(rala_b200_multi* m, FabricRank& fr) {
     MCU(m, cudaSetDevice(fr.device));
     rala_b200_graph* g = fr.g;
     Launch& L = fr.ctx->L;
-    if (g->state != 2) return mfail(m, RALA_B200_ERR_STATE, "finish: rank %d is not classified", fr.rank);
     std::vector<uint32_t>& h = fr.stage_host;
     h.assign(SW_WORDS, 0u);
     uint64_t before = 0;
@@ -1210,13 +1177,8 @@ static int phase_d_staged(rala_b200_multi* m, FabricRank& fr) {
     if (before + m->inl[fr.rank] >= (1ull << 31)) return mfail(m, RALA_B200_ERR_LIMIT, "finish: list positions must stay below 2^31");
     h[SW_ZERO + 1] = (uint32_t) before;   // time base of the local `internals`
     MCU(m, cudaMemcpyAsync(fr.stage.p, h.data(), SW_WORDS * 4, cudaMemcpyHostToDevice, L.stream));
-    MCU(m, begin_stage(g, ST_FINALIZE));
-    MCU(m, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, L.stream));
-    MCU(m, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, L.stream));
-    MCU(m, zero_counter(g, C_EV));
-    MCU(m, clear_earliest_events(g));
+    MRC(m, fr, begin_final_pass(g, C_TBASE_INL));
     MCU(m, cudaMemcpyAsync(g->cnt() + C_TBASE_INL, fr.stage_w(SW_ZERO + 1), 4, cudaMemcpyDeviceToDevice, L.stream));
-    g->final_time_base_slot = C_TBASE_INL;
     const List ovl = g->ovl[g->ovl_cur].view;
     for (uint32_t s = 0; s < m->n_seg; ++s) {
         if (s && !h[SW_FIN_N + s]) continue;   // (segment 0's launch also types `internals`)
@@ -1236,7 +1198,7 @@ static int phase_final_lists(rala_b200_multi* m, FabricRank& fr) {
     const uint32_t S = m->n_seg;
     MCU(m, cudaMemsetAsync(fr.stage_w(SW_BOX), 0, kSegMail * 4, L.stream));
     launch_seg_count(L, g->ovl[g->ovl_cur].view, fr.stage_w(SW_LO), S, g->piles.as<uint2>(), kSegFinal, fr.stage_w(SW_BOX));
-    launch_final_deaths(L, fr.P, fr.A, g->dbuf.as<uint32_t>());   // the k_list_pass<kFinalInt> filter reads them (C_DSEL = 0 here)
+    launch_final_deaths(L, fr.P, fr.A, g->dbuf.as<uint32_t>());   // the k_list_pass<kFinalInt> filter reads them
     MRC(m, fr, materialize_final_lists(g));
     MCU(m, cudaMemcpyAsync(fr.stage_w(SW_BOX + 2 * S), g->cnt() + g->slot_inl, 4, cudaMemcpyDeviceToDevice, L.stream));
     launch_seg_push(L, fr.P, fr.A, fr.stage_w(SW_BOX), 2 * S + 1);

@@ -613,7 +613,7 @@ static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* tex
     PafReader& R = *g->paf;
     // the session's records are void until this call has succeeded
     g->n_rec = 0;
-    g->state = 0;
+    g->state = SS_EMPTY;
     g->text_records = kTextNone;
     uint64_t n = 0;
     int rc = text_parse(ctx, R, fmt, text, n_bytes, st, nullptr, &n);
@@ -635,7 +635,7 @@ static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* tex
     *counted = true;
     if (bad != ~0ull) {
         g->n_rec = 0;
-        g->state = 0;
+        g->state = SS_EMPTY;
         return fail(ctx, RALA_B200_ERR_ARG,
                     "%s line %llu: a read length (%s) differs from the length given to set_reads, and the record is "
                     "valid after the duplicate filter (the reference's transmute exits on it)", mhap ? "MHAP" : "PAF", bad + 1,

@@ -89,6 +89,9 @@ struct ListBuf {
 // the overlap text a session's records were parsed from (paf.cu); build_piles names refused records by its lines
 enum TextFormat : uint8_t { kTextNone = 0, kTextPaf, kTextMhap };
 
+// how far the session's stages got on the current inputs
+enum SessionState { SS_EMPTY = 0, SS_INPUTS, SS_CLASSIFIED, SS_FINALIZED, SS_BUILT, SS_REDUCED };
+
 enum Stage { ST_CLASSIFY = 0, ST_RETRIM, ST_FINALIZE, ST_BUILD, ST_TRANSITIVE, ST_K1_KERNEL, ST_K1B_KERNEL, ST_K3_KERNELS, ST_K1S_KERNEL };
 
 struct rala_b200_graph {
@@ -136,7 +139,7 @@ struct rala_b200_graph {
     bool promote_pending = true;    // the table changed since the internals were last TYPED against it (retrim() trims but does not
                                     // re-type them): the next retrim_promote must run even if retrim() already cleared piles_dirty
     bool scan_pool_exhausted = false;   // a look-back kernel asked for more status words than the pool holds: the run is void
-    int state = 0;                  // 0 empty, 1 inputs set, 2 classified, 3 finalized, 4 built, 5 reduced
+    SessionState state = SS_EMPTY;
     uint32_t retrim_passes = 0;
     cudaEvent_t ev_start[RALA_B200_N_STAGES]{}, ev_stop[RALA_B200_N_STAGES]{};
     bool ev_valid[RALA_B200_N_STAGES]{};
@@ -202,12 +205,28 @@ ResolveBufs resolve_bufs(const rala_b200_graph* g);
 cudaError_t clear_earliest_events(rala_b200_graph* g);
 int reserve_events(rala_b200_graph* g, uint32_t ev_cap);
 int reserve_edges(rala_b200_graph* g, uint32_t edge_cap);
-int phase_events(rala_b200_graph* g);
-int phase_survivors(rala_b200_graph* g);
-int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base, const uint32_t* inl_base);
 int read_counters(rala_b200_graph* g, uint32_t* h);
 int materialize_final_lists(rala_b200_graph* g);
 int reserve_for_records(rala_b200_graph* g, uint64_t n);
+
+// ---- the per-rank stages every driver runs (single session, NCCL phase calls, fabric ranks, stateless reduce) -----------
+int phase_events(rala_b200_graph* g);
+int phase_survivors(rala_b200_graph* g);
+// final containment pass (graph.cpp:831-877): begin keeps the first pass's event / round counts and clears the events;
+// `internals` are timed from counter slot time_base_slot.  end closes the stage: the session is finalized.
+int begin_final_pass(rala_b200_graph* g, int time_base_slot);
+int end_final_pass(rala_b200_graph* g);
+int phase_final_events(rala_b200_graph* g, const uint32_t* ovl_base /* device, nullable */, int inl_base_slot);
+// node ids and the edges of the final `overlaps`, with csr their CSR rows (opens ST_BUILD); then, when the caller gave an
+// edge buffer (rala_b200_graph_set_outputs), their rows into it on side stream 0, joined by marks_stage
+int emit_edges(rala_b200_graph* g, bool csr);
+void fork_edge_download(rala_b200_graph* g);
+// CSR rows of an edge list that did not come from emit_edges (C_NODES / C_EDGES set, n_nodes_max rows)
+int csr_from_edge_list(rala_b200_graph* g);
+int end_build(rala_b200_graph* g);
+// K3 on the CSR in `ga` for the source nodes in node_range (device {begin, end}; nullptr = all), then marked(e) from ga.T
+int transitive_stage(rala_b200_graph* g, const GraphArrays& ga, const uint32_t* node_range);
+int marks_stage(rala_b200_graph* g, const GraphArrays& ga, uint8_t* copy /* nullable */, uint32_t copy_cap);
 
 // ---- paf.cu ----------------------------------------------------------------------------------------------------
 void destroy_paf_reader(PafReader* r);

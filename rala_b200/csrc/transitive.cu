@@ -170,18 +170,14 @@ struct GroupSmem {
 constexpr int kGroupMinBlocks = 6;
 __global__ void __launch_bounds__(kLightWarps * 32, kGroupMinBlocks) k_transitive_group(
     const uint32_t* __restrict__ row_ptr, const uint2* __restrict__ col, const uint32_t* __restrict__ col_eid,
-    uint8_t* __restrict__ T, uint32_t node_begin, uint32_t node_end, const uint32_t* __restrict__ node_range,
-    const uint32_t* __restrict__ n_nodes_ptr, uint32_t* __restrict__ work_counter, HeavyItems heavy,
-    uint32_t* __restrict__ counters) {
+    uint8_t* __restrict__ T, const uint32_t* __restrict__ node_range, const uint32_t* __restrict__ n_nodes_ptr,
+    uint32_t* __restrict__ work_counter, HeavyItems heavy, uint32_t* __restrict__ counters) {
     static_assert(kGroupMaxDeg == 16 && kGroupLanes == 8, "the search below is written for 16 keys, two per lane");
     __shared__ GroupSmem smem[kLightWarps][kGroupsPerWarp];
     const uint32_t lane = lane_id(), gl = lane & (kGroupLanes - 1), grp = lane / kGroupLanes;
     GroupSmem& S = smem[warp_id()][grp];
-    if (node_range) {
-        node_begin = node_range[0];
-        node_end = node_range[1];
-    }
-    const uint32_t n_end = min(node_end, *n_nodes_ptr);
+    const uint32_t node_begin = node_range ? node_range[0] : 0u;
+    const uint32_t n_end = node_range ? min(node_range[1], *n_nodes_ptr) : *n_nodes_ptr;
     unsigned long long visits = 0;
 
     while (true) {
@@ -316,17 +312,14 @@ struct LightSmem {
 
 __global__ void __launch_bounds__(kLightWarps * 32) k_transitive_light(
     const uint32_t* __restrict__ row_ptr, const uint2* __restrict__ col, const uint32_t* __restrict__ col_eid,
-    uint8_t* __restrict__ T, uint32_t node_begin, uint32_t node_end, const uint32_t* __restrict__ node_range,
-    const uint32_t* __restrict__ n_nodes_ptr, uint32_t* __restrict__ work_counter, HeavyItems heavy,
-    uint32_t* __restrict__ counters) {
+    uint8_t* __restrict__ T, const uint32_t* __restrict__ node_range, const uint32_t* __restrict__ n_nodes_ptr,
+    uint32_t* __restrict__ work_counter, HeavyItems heavy, uint32_t* __restrict__ counters) {
     __shared__ LightSmem smem[kLightWarps];
     LightSmem& S = smem[warp_id()];
     const uint32_t lane = lane_id();
-    if (node_range) {   // multi-GPU: this rank's share of the source nodes, computed on the device
-        node_begin = node_range[0];
-        node_end = node_range[1];
-    }
-    const uint32_t n_end = min(node_end, *n_nodes_ptr);
+    // multi-GPU: this rank's share of the source nodes, computed on the device
+    const uint32_t node_begin = node_range ? node_range[0] : 0u;
+    const uint32_t n_end = node_range ? min(node_range[1], *n_nodes_ptr) : *n_nodes_ptr;
     unsigned long long visits = 0;
 
     while (true) {
@@ -588,23 +581,17 @@ void launch_node_range(Launch& L, GraphArrays g, const uint32_t* counters, uint3
     L.count++;
 }
 
-void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, uint32_t edge_cap, HeavyItems heavy,
-                       uint32_t* work_counter, uint32_t* counters, uint32_t node_begin, uint32_t node_end,
+void launch_transitive(Launch& L, GraphArrays g, uint32_t n_nodes_max, HeavyItems heavy, uint32_t* work_counter, uint32_t* counters,
                        const uint32_t* node_range) {
-    (void) edge_cap;
-    uint64_t span = node_end > node_begin ? node_end - node_begin : 0;
-    if (span > n_nodes_max) span = n_nodes_max;
-    uint64_t blocks = (span + 32 * kLightWarps - 1) / (32 * kLightWarps);
-    if (blocks < 1) blocks = 1;
-    if (blocks > (uint64_t) kNumSMs * 8) blocks = kNumSMs * 8;
+    const int blocks = grid_for(n_nodes_max, 32 * kLightWarps, kNumSMs * 8);
     // the group and the light kernel take disjoint sets of nodes (by out-degree) and only meet in atomics (heavy work
     // list, visit counter): the light one (14 us, mostly idle SMs) runs beside the group one on a forked stream
     const bool forked = fork_side(L, 1);
-    k_transitive_group<<<(int) blocks, kLightWarps * 32, 0, L.stream>>>(g.row_ptr, g.col, g.col_eid, g.T, node_begin, node_end,
-                                                                       node_range, counters + C_NODES, work_counter + 1, heavy, counters);
+    k_transitive_group<<<blocks, kLightWarps * 32, 0, L.stream>>>(g.row_ptr, g.col, g.col_eid, g.T, node_range, counters + C_NODES,
+                                                                 work_counter + 1, heavy, counters);
     L.count++;
-    k_transitive_light<<<(int) blocks, kLightWarps * 32, 0, forked ? L.side[1] : L.stream>>>(
-        g.row_ptr, g.col, g.col_eid, g.T, node_begin, node_end, node_range, counters + C_NODES, work_counter, heavy, counters);
+    k_transitive_light<<<blocks, kLightWarps * 32, 0, forked ? L.side[1] : L.stream>>>(
+        g.row_ptr, g.col, g.col_eid, g.T, node_range, counters + C_NODES, work_counter, heavy, counters);
     L.count++;
     if (forked) join_side(L, 1);
     k_transitive_heavy<<<kNumSMs * 4, kHeavyThreads, 0, L.stream>>>(g.row_ptr, g.col, g.col_eid, g.T, heavy, counters);

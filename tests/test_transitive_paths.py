@@ -11,6 +11,8 @@ the selection restated below in numpy: a graph that drifts off its boundary fail
 Graphs follow the pair(e) = e ^ 1 convention of synth.hub_graph.  Forward edges join even nodes; every twin edge
 b^1 -> a^1 has the length TWIN, so a triangle among twins compares 2 TWIN with TWIN and never passes: the marks come
 from the forward triangles, whose lengths the tests choose (the twins still run through the kernels, as negatives)."""
+import ctypes as C
+
 import numpy as np
 import pytest
 
@@ -476,3 +478,25 @@ def test_large_hub_through_the_session_and_two_ranks(ctx):
     assert_same(m, P.marked, "marks (2 ranks)")
     assert M.counts()["n_transitive_pairs"] == P.n_pairs
     M.close()
+
+
+@pytest.mark.gpu
+def test_a_shard_refuses_the_whole_session_stages(ctx):
+    """After set_shard(world > 1) the session holds one rank's records: build, transitive and run refuse (status -3,
+    RALA_B200_ERR_STATE) instead of giving a partial CSR or no marks; back at world 1 the same session runs."""
+    ds = star_records(2_000)
+    piles = ds.flat_piles()
+    P = O.Pipeline(ds.records, piles).run()
+    G = api.Graph(ctx)
+    G.set_piles(piles).set_hills(None).set_overlaps(ds.records)
+    G._call("rala_b200_graph_set_shard", C.c_uint32(0), C.c_int(1), C.c_int(2))
+    G.classify()
+    G.finalize()
+    for stage in (G.build, G.transitive, G.run):
+        with pytest.raises(api.RalaB200Error, match=r"status -3: .*rank 1 of 2.*phase calls"):
+            stage()
+    G._call("rala_b200_graph_set_shard", C.c_uint32(0), C.c_int(0), C.c_int(1))
+    G.run()
+    assert_same(G.edges(), P.edges, "edges")
+    assert_same(G.marked(), P.marked, "marks")
+    G.close()
