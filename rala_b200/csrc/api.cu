@@ -102,21 +102,29 @@ extern "C" uint64_t rala_b200_launch_count(const rala_b200_ctx* ctx) { return ct
 
 size_t tiles_of(uint64_t n) { return (size_t) ((n + kTile - 1) / kTile) + 1; }
 
-// a fresh, zeroed (status words, ticket) pair from the pool for one look-back kernel
-bool scan_state(rala_b200_graph* g, uint64_t n_max, unsigned long long** status, uint32_t** ticket) {
-    size_t words = tiles_of(n_max) + 1;
-    if (g->scan_used + words > g->scan_pool_words) {
-        // Handing out words an earlier look-back kernel of the same stage already wrote would give wrong prefixes (or spin).
-        // The pool is sized for every stage (reserve_scan_pool); should a new caller break that, the run is declared
-        // void (read_counters reports it) and the words are recycled only so that the kernel arguments stay valid.
-        g->scan_pool_exhausted = true;
+// a fresh, zeroed (status words, ticket) pair from the pool for one look-back kernel with `tiles` tiles
+static bool scan_words(rala_b200_graph* g, uint64_t tiles, unsigned long long** status, uint32_t** ticket) {
+    const size_t words = (size_t) tiles + 1;
+    if (!g->scan_zeroed || g->scan_used + words > g->scan_pool_words) {
+        // The step prologue zeroes the pool, which is sized for a step (reserve_scan_pool).  Calls outside a step, and
+        // steps with more list passes (retrim rounds), clear it again: the clear is ordered behind every look-back kernel
+        // already enqueued.  Handing out words a look-back kernel already wrote would give wrong prefixes (or spin): a
+        // single kernel that asks for more than the whole pool declares the run void (read_counters reports it), and the
+        // words are recycled only so that the kernel arguments stay valid.
+        if (words > g->scan_pool_words || cudaMemsetAsync(g->scan_pool.p, 0, g->scan_pool_words * 8, g->ctx->L.stream) != cudaSuccess)
+            g->scan_pool_exhausted = true;
         g->scan_used = 0;
+        g->scan_zeroed = true;
     }
     unsigned long long* base = g->scan_pool.as<unsigned long long>() + g->scan_used;
     *ticket = reinterpret_cast<uint32_t*>(base);
     *status = base + 1;
-    g->scan_used += words;
+    g->scan_used = words > g->scan_pool_words ? 0 : g->scan_used + words;
     return !g->scan_pool_exhausted;
+}
+
+bool scan_state(rala_b200_graph* g, uint64_t n_max, unsigned long long** status, uint32_t** ticket) {
+    return scan_words(g, tiles_of(n_max), status, ticket);
 }
 
 // stage timers: plain event records, left out of a stream capture (an event recorded inside a capture cannot be timed)
@@ -136,12 +144,7 @@ cudaError_t stage_event(rala_b200_graph* g, cudaEvent_t ev) {
     return stream_capturing(g) ? cudaSuccess : cudaEventRecord(ev, g->ctx->L.stream);
 }
 
-cudaError_t begin_stage(rala_b200_graph* g, int stage) {
-    g->scan_used = 0;
-    cudaError_t e = cudaMemsetAsync(g->scan_pool.p, 0, g->scan_pool_words * 8, g->ctx->L.stream);
-    if (e != cudaSuccess) return e;
-    return stage_event(g, g->ev_start[stage]);
-}
+cudaError_t begin_stage(rala_b200_graph* g, int stage) { return stage_event(g, g->ev_start[stage]); }
 
 cudaError_t end_stage(rala_b200_graph* g, int stage) {
     g->ev_valid[stage] = !stream_capturing(g);
@@ -183,7 +186,7 @@ extern "C" void rala_b200_graph_destroy(rala_b200_graph* g) {
     destroy_paf_reader(g->paf);
     destroy_pile_builder(g->pile_builder);
     DevBuf* bufs[] = {&g->rec, &g->recs.buf, &g->alive_bits, &g->piles, &g->piles_raw, &g->pile_flags_raw, &g->piles_initial, &g->hills, &g->ovl[0].buf,
-                      &g->ovl[1].buf, &g->inl[0].buf, &g->inl[1].buf, &g->events, &g->hill_rec, &g->dbuf, &g->flags, &g->segs, &g->tiles,
+                      &g->ovl[1].buf, &g->inl[0].buf, &g->inl[1].buf, &g->events, &g->hill_rec, &g->dbuf, &g->flags, &g->segs,
                       &g->counters, &g->scan_pool, &g->seq_to_node, &g->edges, &g->row_ptr, &g->cursor, &g->col,
                       &g->col_eid, &g->T, &g->marked, &g->heavy, &g->work_counter, &g->edges_aos, &g->slot_degree, &g->tile_dov};
     for (DevBuf* b : bufs) b->release();
@@ -217,13 +220,16 @@ int reserve_edges(rala_b200_graph* g, uint32_t edge_cap) {
 }
 
 static int reserve_scan_pool(rala_b200_graph* g) {
-    // worst stage: classify = runs scan + two containment scans over the piles; build = one scan over the piles or the
-    // nodes (2 per pile); the multi-GPU session adds scans over its exchange capacities (<= 2 x the record count): 16 x
-    // leaves room
-    size_t words = 16 * (tiles_of(g->n_rec) + tiles_of((uint64_t) g->n_nodes_max + 8) + 8);
+    // one step: the survivors pass (a word per run), two containment resolutions over the piles and their scans (the
+    // fabric ranks), the pile scan of build or the CSR scan over the nodes of the multi-GPU paths, one retrim + promote
+    // round (three list passes) and, after the step, the two final list passes of get_lists / counts
+    const size_t piles = tiles_of((uint64_t) g->n_piles + 1) + 1, nodes = tiles_of((uint64_t) g->n_nodes_max + 8) + 1,
+                 lists = tiles_of(g->cap) + 1;
+    const size_t words = classify_num_runs(g->n_rec) + 1 + 4 * piles + 2 * nodes + 5 * lists + 64;
     if (words > g->scan_pool_words) {
         CU(g->ctx, g->scan_pool.reserve(words * 8));
         g->scan_pool_words = words;
+        g->scan_zeroed = false;
     }
     return RALA_B200_OK;
 }
@@ -240,8 +246,7 @@ static int reserve_nodes(rala_b200_graph* g, uint32_t n_nodes) {
     return reserve_scan_pool(g);
 }
 
-// device lists sized for n records (worst case every record survives; the scratch lists of the survivors pass are
-// indexed by record position)
+// device lists sized for n records (worst case every record survives)
 int reserve_for_records(rala_b200_graph* g, uint64_t n) {
     rala_b200_ctx* ctx = g->ctx;
     g->n_rec = (uint32_t) n;
@@ -261,7 +266,6 @@ int reserve_for_records(rala_b200_graph* g, uint64_t n) {
         if (!rc2) rc2 = reserve_edges(g, 2 * cap);
         if (rc2) return rc2;
     }
-    CU(ctx, g->tiles.reserve(align_up((size_t) classify_num_runs((uint32_t) n) + 8, 64) * 4 * 3));
     int rc = reserve_scan_pool(g);
     if (rc) return rc;
     if (g->state == SS_EMPTY && g->n_piles) g->state = SS_INPUTS;
@@ -448,6 +452,14 @@ cudaError_t clear_earliest_events(rala_b200_graph* g) {
     return cudaMemsetAsync(resolve_bufs(g).first, 0xFF, ((size_t) g->n_piles + 64) * 8, g->ctx->L.stream);
 }
 
+FinalPassReset final_pass_reset(const rala_b200_graph* g) {
+    FinalPassReset r;
+    r.first = resolve_bufs(g).first;
+    r.n_first = r.first ? g->n_piles + 64 : 0u;
+    r.counters = g->cnt();
+    return r;
+}
+
 static int resolve_containment(rala_b200_graph* g, bool decode, bool skip_if_empty) {
     rala_b200_ctx* ctx = g->ctx;
     unsigned long long* status;
@@ -464,17 +476,30 @@ int phase_events(rala_b200_graph* g) {
     rala_b200_ctx* ctx = g->ctx;
     if (g->state < SS_INPUTS) return fail(ctx, RALA_B200_ERR_STATE, "classify: set_overlaps and set_piles first");
     CU(ctx, cudaSetDevice(ctx->device));
-    // classify kills piles in the working table: keep the table it started from, so that calling classify
-    // again without a new set_piles re-runs on the same input (bench loops, retries)
-    if (g->piles_fresh)
-        CU(ctx, cudaMemcpyAsync(g->piles_initial.p, g->piles.p, (size_t) g->n_piles * 8, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    else
-        CU(ctx, cudaMemcpyAsync(g->piles.p, g->piles_initial.p, (size_t) g->n_piles * 8, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    g->piles_fresh = false;
     CU(ctx, begin_stage(g, ST_CLASSIFY));
-    CU(ctx, cudaMemsetAsync(g->counters.p, 0, C_COUNT * 4, ctx->L.stream));
-    if (g->n_hills) CU(ctx, cudaMemsetAsync(g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills, 0, (size_t) g->n_hills * 4, ctx->L.stream));
-    CU(ctx, clear_earliest_events(g));
+    // classify kills piles in the working table: keep the table it started from, so that calling classify
+    // again without a new set_piles re-runs on the same input (bench loops, retries).  One launch also clears what the
+    // step's stages count into: the counters, the hill coverage, the look-back pool, the earliest events of the first
+    // pass, the slot degrees of build and the node counters of the transitive pass.
+    StepPrologue pro{};
+    pro.piles = g->piles.as<uint2>();
+    pro.piles_initial = g->piles_initial.as<uint2>();
+    pro.n_piles = g->n_piles;
+    pro.snapshot = g->piles_fresh;
+    pro.first = resolve_bufs(g).first;
+    pro.n_first = pro.first ? g->n_piles + 64 : 0u;
+    uint32_t* zero[StepPrologue::kZero] = {g->cnt(), g->n_hills ? g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills : nullptr,
+                                           g->scan_pool.as<uint32_t>(), g->slot_degree.as<uint32_t>(), g->work_counter.as<uint32_t>()};
+    const size_t words[StepPrologue::kZero] = {C_COUNT, g->n_hills, 2 * g->scan_pool_words, (size_t) g->n_nodes_max + 8, 2};
+    for (int k = 0; k < StepPrologue::kZero; ++k) {
+        pro.zero[k] = zero[k];
+        pro.zero_words[k] = words[k];
+    }
+    launch_step_prologue(ctx->L, pro);
+    g->piles_fresh = false;
+    g->scan_used = 0;
+    g->scan_zeroed = true;
+    g->step_cleared = kStepBuild | kStepTransitive;
     CU(ctx, stage_event(g, g->ev_start[ST_K1_KERNEL]));
     launch_classify_events(ctx->L, g->recs.view, g->n_rec, g->t0, g->piles.as<uint2>(), g->n_piles, g->events_view(),
                            g->ev_cap, resolve_bufs(g).first, g->hill_rec.as<uint32_t>(), g->cap, g->cnt());
@@ -502,8 +527,10 @@ static int phase_resolve(rala_b200_graph* g, bool first_pass) {
                              h + g->n_hills, h + 2 * (size_t) g->n_hills, g->n_hills,
                              g->hills.as<uint32_t>() + 3 * (size_t) g->n_hills, g->dbuf.as<uint32_t>(), g->cnt());
     }
+    FinalPassReset reset;
+    if (first_pass) reset = final_pass_reset(g);
     launch_apply_deaths(ctx->L, g->piles.as<uint2>(), g->dbuf.as<uint32_t>(), g->n_piles, g->alive_bits.as<uint32_t>(), fused_decode,
-                        nullptr, skip_if_empty ? g->cnt() + C_EV : nullptr);
+                        nullptr, skip_if_empty ? g->cnt() + C_EV : nullptr, reset);
     CU(ctx, cudaGetLastError());
     return RALA_B200_OK;
 }
@@ -515,19 +542,13 @@ int phase_survivors(rala_b200_graph* g) {
     g->slot_ovl = C_LIST0;
     g->slot_inl = C_LIST0 + 1;
     g->next_slot = C_LIST0 + 2;
-    CU(ctx, zero_counter(g, C_LIST0, 2));
+    if (!g->n_rec) CU(ctx, zero_counter(g, C_LIST0, 2));   // otherwise the last run writes both counts
     CU(ctx, stage_event(g, g->ev_start[ST_K1S_KERNEL]));
-    {
-        const size_t nr = align_up((size_t) classify_num_runs(g->n_rec) + 8, 64);
-        uint32_t* t = g->tiles.as<uint32_t>();
-        RunBufs runs{t, t + nr, t + 2 * nr};
-        unsigned long long* status;
-        uint32_t* ticket;
-        scan_state(g, nr, &status, &ticket);
-        launch_classify_survivors(ctx->L, g->recs.view, g->n_rec, g->piles.as<uint2>(), g->alive_bits.as<uint32_t>(), g->n_piles,
-                                  g->ovl[1].view, g->inl[1].view, g->ovl[0].view, g->cnt() + g->slot_ovl, g->inl[0].view,
-                                  g->cnt() + g->slot_inl, g->cap, runs, status, ticket);
-    }
+    unsigned long long* status;
+    uint32_t* ticket;
+    scan_words(g, classify_num_runs(g->n_rec), &status, &ticket);
+    launch_classify_survivors(ctx->L, g->recs.view, g->n_rec, g->piles.as<uint2>(), g->alive_bits.as<uint32_t>(), g->n_piles,
+                              g->ovl[0].view, g->cnt() + g->slot_ovl, g->inl[0].view, g->cnt() + g->slot_inl, g->cap, status, ticket);
     CU(ctx, end_stage(g, ST_K1S_KERNEL));
     CU(ctx, cudaGetLastError());
     CU(ctx, end_stage(g, ST_CLASSIFY));
@@ -631,8 +652,6 @@ int materialize_final_lists(rala_b200_graph* g) {
     unsigned long long* status;
     uint32_t* ticket;
     List none{};
-    g->scan_used = 0;
-    CU(ctx, cudaMemsetAsync(g->scan_pool.p, 0, g->scan_pool_words * 8, ctx->L.stream));
     scan_state(g, g->cap, &status, &ticket);
     int inl_out = g->new_slot();
     CU(ctx, zero_counter(g, inl_out));
@@ -658,11 +677,7 @@ int begin_final_pass(rala_b200_graph* g, int time_base_slot) {
     rala_b200_ctx* ctx = g->ctx;
     if (g->state != SS_CLASSIFIED) return fail(ctx, RALA_B200_ERR_STATE, "finalize: classify first");
     CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, begin_stage(g, ST_FINALIZE));
-    CU(ctx, cudaMemcpyAsync(g->cnt() + C_EV_FIRST, g->cnt() + C_EV, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    CU(ctx, cudaMemcpyAsync(g->cnt() + C_ROUNDS_FIRST, g->cnt() + C_ROUNDS, 4, cudaMemcpyDeviceToDevice, ctx->L.stream));
-    CU(ctx, zero_counter(g, C_EV));
-    CU(ctx, clear_earliest_events(g));
+    CU(ctx, begin_stage(g, ST_FINALIZE));   // the first pass's k_apply_deaths kept its counts and cleared the events (FinalPassReset)
     g->final_time_base_slot = time_base_slot;
     return RALA_B200_OK;
 }
@@ -706,10 +721,13 @@ int emit_edges(rala_b200_graph* g, bool csr) {
     rala_b200_ctx* ctx = g->ctx;
     CU(ctx, cudaSetDevice(ctx->device));
     CU(ctx, begin_stage(g, ST_BUILD));
-    CU(ctx, zero_counter(g, C_NODES, 4));   // C_NODES, C_ALIVE, C_DOVETAILS, C_EDGES
     GraphArrays ga = g->graph_view();
-    if (csr) CU(ctx, cudaMemsetAsync(ga.slot_degree, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
-    else ga.cursor = nullptr;
+    if (!(g->step_cleared & kStepBuild)) {   // not already cleared by the step prologue
+        CU(ctx, zero_counter(g, C_NODES, 4));   // C_NODES, C_ALIVE, C_DOVETAILS, C_EDGES
+        if (csr) CU(ctx, cudaMemsetAsync(ga.slot_degree, 0, ((size_t) g->n_nodes_max + 8) * 4, ctx->L.stream));
+    }
+    g->step_cleared &= ~kStepBuild;
+    if (!csr) ga.cursor = nullptr;
     unsigned long long* status;
     uint32_t* ticket;
     scan_state(g, g->n_piles, &status, &ticket);
@@ -776,9 +794,12 @@ extern "C" int rala_b200_graph_build(rala_b200_graph* g) {
 
 int transitive_stage(rala_b200_graph* g, const GraphArrays& ga, const uint32_t* node_range) {
     rala_b200_ctx* ctx = g->ctx;
-    CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
-    // the two node counters of K3 (a node range of the NCCL phase sits behind them, in words 4 and 5)
-    CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 8, ctx->L.stream));
+    if (!(g->step_cleared & kStepTransitive)) {   // not already cleared by the step prologue
+        CU(ctx, zero_counter(g, C_PAIRS, 5));   // C_PAIRS, C_HEAVY_NODES, C_HEAVY, C_HOP_LO, C_HOP_HI
+        // the two node counters of K3 (a node range of the NCCL phase sits behind them, in words 4 and 5)
+        CU(ctx, cudaMemsetAsync(g->work_counter.p, 0, 8, ctx->L.stream));
+    }
+    g->step_cleared &= ~kStepTransitive;
     CU(ctx, stage_event(g, g->ev_start[ST_K3_KERNELS]));
     launch_transitive(ctx->L, ga, g->n_nodes_max, g->heavy_view(), g->work_counter.as<uint32_t>(), g->cnt(), node_range);
     CU(ctx, end_stage(g, ST_K3_KERNELS));
@@ -834,7 +855,7 @@ static int run_eager(rala_b200_graph* g) {
 // operations (27 kernels, memsets, small copies) are identical from run to run: the second run with a key is
 // captured into a CUDA graph and later runs replay it with one launch.
 struct RunKey {
-    const void *rec, *recs, *piles, *piles_initial, *events, *segs, *dbuf, *edges, *col, *scan_pool, *tiles, *ovl0, *inl0, *hills, *heavy;
+    const void *rec, *recs, *piles, *piles_initial, *events, *segs, *dbuf, *edges, *col, *scan_pool, *ovl0, *inl0, *hills, *heavy;
     const void *out_edges, *out_marked;
     uint32_t n_rec, n_piles, n_hills, cap, ev_cap, edge_cap, heavy_cap, t0, out_edges_cap, out_marked_cap;
     int world, rank, coop_blocks;
@@ -848,6 +869,8 @@ struct RunHostState {
     bool final_lists_ready, piles_dirty, piles_fresh, promote_pending;
     uint32_t retrim_passes;
     size_t scan_used;
+    bool scan_zeroed;
+    uint32_t step_cleared;
 };
 
 struct RunGraph {
@@ -863,7 +886,7 @@ static RunKey run_key(const rala_b200_graph* g) {
     memset(&k, 0, sizeof(k));   // padding included: keys are compared with memcmp
     k.rec = g->rec.p; k.recs = g->recs.buf.p; k.piles = g->piles.p; k.piles_initial = g->piles_initial.p;
     k.events = g->events.p; k.segs = g->segs.p; k.dbuf = g->dbuf.p; k.edges = g->edges.p; k.col = g->col.p;
-    k.scan_pool = g->scan_pool.p; k.tiles = g->tiles.p; k.ovl0 = g->ovl[0].buf.p; k.inl0 = g->inl[0].buf.p; k.hills = g->hills.p;
+    k.scan_pool = g->scan_pool.p; k.ovl0 = g->ovl[0].buf.p; k.inl0 = g->inl[0].buf.p; k.hills = g->hills.p;
     k.heavy = g->heavy.p;   // sized from n_piles, which can shrink and grow back without a new allocation
     k.n_rec = g->n_rec; k.n_piles = g->n_piles; k.n_hills = g->n_hills; k.cap = g->cap; k.ev_cap = g->ev_cap;
     k.edge_cap = g->edge_cap; k.heavy_cap = g->heavy_cap; k.t0 = g->t0;
@@ -875,7 +898,8 @@ static RunKey run_key(const rala_b200_graph* g) {
 
 static RunHostState host_state(const rala_b200_graph* g) {
     return RunHostState{g->ovl_cur, g->inl_cur, g->slot_ovl, g->slot_inl, g->next_slot, g->final_time_base_slot, g->state,
-                        g->final_lists_ready, g->piles_dirty, g->piles_fresh, g->promote_pending, g->retrim_passes, g->scan_used};
+                        g->final_lists_ready, g->piles_dirty, g->piles_fresh, g->promote_pending, g->retrim_passes, g->scan_used,
+                        g->scan_zeroed, g->step_cleared};
 }
 
 static void drop_run_graphs(rala_b200_graph* g) {
@@ -942,6 +966,7 @@ extern "C" int rala_b200_graph_run(rala_b200_graph* g) {
     g->ovl_cur = a.ovl_cur; g->inl_cur = a.inl_cur; g->slot_ovl = a.slot_ovl; g->slot_inl = a.slot_inl; g->next_slot = a.next_slot;
     g->final_time_base_slot = a.final_time_base_slot; g->state = a.state; g->final_lists_ready = a.final_lists_ready;
     g->piles_dirty = a.piles_dirty; g->piles_fresh = a.piles_fresh; g->promote_pending = a.promote_pending; g->retrim_passes = a.retrim_passes; g->scan_used = a.scan_used;
+    g->scan_zeroed = a.scan_zeroed; g->step_cleared = a.step_cleared;
     for (int i = 0; i < RALA_B200_N_STAGES; ++i) g->ev_valid[i] = false;   // no stage timers inside a graph
     return RALA_B200_OK;
 }
@@ -953,7 +978,8 @@ int read_counters(rala_b200_graph* g, uint32_t* h) {
     CU(ctx, cudaStreamSynchronize(ctx->L.stream));
     if (g->scan_pool_exhausted)
         return fail(ctx, RALA_B200_ERR_LIMIT, "the look-back status pool was exhausted inside a stage (%zu words): the results are void", g->scan_pool_words);
-    if (h[C_OVERFLOW] || (g->state >= SS_CLASSIFIED && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap || h[C_HILL] > g->cap)
+    if (h[C_OVERFLOW] || (g->state >= SS_CLASSIFIED && (h[g->slot_ovl] > g->cap || h[g->slot_inl] > g->cap)) || h[C_EV] > g->ev_cap ||
+        h[C_EV_FIRST] > g->ev_cap || h[C_HILL] > g->cap)
         return fail(ctx, RALA_B200_ERR_LIMIT, "a device list overflowed its capacity (cap=%u events=%u hills=%u heavy items=%u)",
                     g->cap, h[C_EV], h[C_HILL], h[C_HEAVY]);
     return RALA_B200_OK;
@@ -969,8 +995,9 @@ extern "C" int rala_b200_graph_counts(rala_b200_graph* g, rala_b200_counts_t* ou
     out->n_records = g->n_rec;
     out->n_overlaps = g->state >= SS_CLASSIFIED ? h[g->slot_ovl] : 0;
     out->n_internals = g->state >= SS_CLASSIFIED ? h[g->slot_inl] : 0;
-    out->n_candidates = g->state >= SS_FINALIZED ? h[C_EV_FIRST] : h[C_EV];
-    out->n_rounds = g->state >= SS_FINALIZED ? h[C_ROUNDS_FIRST] : h[C_ROUNDS];
+    // the first pass's k_apply_deaths moved its counts to *_FIRST (FinalPassReset)
+    out->n_candidates = g->state >= SS_CLASSIFIED ? h[C_EV_FIRST] : h[C_EV];
+    out->n_rounds = g->state >= SS_CLASSIFIED ? h[C_ROUNDS_FIRST] : h[C_ROUNDS];
     out->n_final_candidates = g->state >= SS_FINALIZED ? h[C_EV] : 0;
     out->n_final_rounds = g->state >= SS_FINALIZED ? h[C_ROUNDS] : 0;
     out->n_piles = g->n_piles;
@@ -1143,8 +1170,6 @@ extern "C" int rala_b200_graph_get_adjacency(rala_b200_graph* g, int which, int 
     CU(ctx, tmp.reserve(((size_t) n_edges + 8) * 4));
     CU(ctx, sorted.reserve(((size_t) n_edges + 8) * 4));
     GraphArrays ga = g->graph_view();
-    g->scan_used = 0;
-    CU(ctx, cudaMemsetAsync(g->scan_pool.p, 0, g->scan_pool_words * 8, ctx->L.stream));
     unsigned long long* status;
     uint32_t* ticket;
     scan_state(g, (uint64_t) n_nodes + 1, &status, &ticket);

@@ -192,245 +192,154 @@ __global__ void __launch_bounds__(kTileThreads, MINB) k_classify_events(
     if (staged) flush();
 }
 
-// Scratch of the survivors pass: one 32-byte entry per slot, kept as two 16-byte halves in the two spare list buffers
-// (a list buffer holds 25 B per entry of capacity, a half needs 16): {a, b | ori << 31, ab, ae} and {bb, be, tag, -}.
-__device__ __forceinline__ uint4* scratch_lo(const List& spare_ovl) { return reinterpret_cast<uint4*>(spare_ovl.a); }
-__device__ __forceinline__ uint4* scratch_hi(const List& spare_inl) { return reinterpret_cast<uint4*>(spare_inl.a); }
-
-// Survivors pass.  Every warp owns RUNS of 512 consecutive records (4 x 4 per lane): it writes the survivors of a
-// run, in record order, to the run's own slot range of the scratch lists (slot = record index of the run's
-// first record: the scratch lists are as long as the record set) and stores the run's two counts.  No atomics,
-// no block barriers, no dependence between runs.  k_scan_runs turns the counts into file-order offsets
-// (single-pass look-back scan) and k_relocate_runs moves each run to its final place.
+// Survivors pass.  Every warp takes RUNS of 512 consecutive records (4 x 4 per lane) from an atomic ticket, so a run only
+// ever waits on runs whose warps are resident or finished.  The survivors of a run go straight to their file-order
+// places in `overlaps` and `internals`: the run publishes its two counts as its aggregate and takes its exclusive prefix
+// with the decoupled look-back (one status word per run); the last run writes both list lengths.
 //
-// Only ~7 % of the records have two live piles, so the pass is split in two phases per run:
+// Only ~7 % of the records have two live piles, so the pass is split in phases per run:
 //   1. liveness: 16 records per lane, both id columns as 16-byte loads, 32 bitmap gathers in flight per lane;
 //      the candidates' positions inside the run are COMPACTED into a per-warp queue in shared memory (one packed
 //      warp scan ranks all four 128-record groups at once: one byte per group, each <= 128);
 //   2. trim + type run over the queue with (almost) every lane busy, instead of sixteen times over mostly idle
-//      warps (the first version of this kernel executed 12 of 32 lanes per instruction, profiles/r01f).
-// 5 resident blocks per SM (48 registers, 28 bytes of spill) and a grid of two waves: survivors stage 83 us against 91 us at
-// 4 resident blocks (64 registers); one persistent wave loses 15 us, 6 resident blocks spill 104 bytes and win nothing
-// (profiles/r02ae_ab.json, r02af_ab.json)
+//      warps (the first version of this kernel executed 12 of 32 lanes per instruction, profiles/r01f); the type goes
+//      back into the queue entry beside the position, and the run's counts are published;
+//   3. the run's prefix is awaited only after phases 1 and 2 of the warp's NEXT run (two queues per warp), when the
+//      runs before it have long published theirs; then the survivors' coordinates are gathered again (L2 hits), trimmed
+//      again and written.
+// This replaced scratch slots per run plus a scan and a relocation kernel (one 32-byte write and read per survivor, two
+// launches).  Waiting for the prefix right after phase 2 instead keeps thousands of resident warps spinning on a
+// straggler: that fusion once cost +39 us (profiles/r02w_ab.json); see profiles/r02ap_* for this one.
+// 5 resident blocks per SM and a grid of two waves: survivors stage 83 us against 91 us at 4 resident blocks (64 registers);
+// one persistent wave loses 15 us, 6 resident blocks spill 104 bytes and win nothing (profiles/r02ae_ab.json, r02af_ab.json)
 constexpr int kSurvMinBlocks = 5;
 constexpr int kSurvBlocks = 10;   // grid = this many blocks per SM at most
+constexpr uint32_t kQueueTagShift = 9;   // queue entry: position in the run (9 bits) | type << 9 (kQueueRejected: no survivor)
+constexpr uint32_t kQueueRejected = 7;
+static_assert(kRunRecords <= (1u << kQueueTagShift) && kBA < kQueueRejected, "a queue entry holds a run position and a type");
+
+// phases 1 and 2 of `run`: the queue holds the candidates' positions and types; returns their number and the run's counts
+__device__ __forceinline__ uint32_t survivors_queue(const List& recs, uint32_t n, const uint2* __restrict__ piles,
+                                                    const uint32_t* __restrict__ alive_bits, uint32_t n_piles, uint32_t run,
+                                                    uint16_t* queue, uint32_t& n_a, uint32_t& n_b) {
+    const uint32_t lane = lane_id();
+    uint32_t a[kRunGroups][4], b[kRunGroups][4];
+#pragma unroll
+    for (int j = 0; j < kRunGroups; ++j) {
+        const uint32_t q = run * (kRunRecords / 4) + j * 32u + lane;     // this lane's j-th group of 4 records
+#pragma unroll
+        for (int r = 0; r < 4; ++r) { a[j][r] = kInvalidBit; b[j][r] = 0u; }
+        if (4u * q < n) {
+            unpack4(reinterpret_cast<const uint4*>(recs.a)[q], a[j]);
+            unpack4(reinterpret_cast<const uint4*>(recs.b)[q], b[j]);
+        }
+    }
+    uint32_t cand = 0;   // bit j * 4 + r
+#pragma unroll
+    for (int j = 0; j < kRunGroups; ++j) {
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {   // both piles alive at the end (graph.cpp:493-515)?  one L1-resident bit each
+            const uint32_t i = run * kRunRecords + j * 128u + 4u * lane + r, ida = a[j][r], idb = b[j][r] & 0x7FFFFFFFu;
+            const bool ok = i < n && !(ida & kInvalidBit) && ida < n_piles && idb < n_piles &&
+                            ((__ldg(alive_bits + (ida >> 5)) >> (ida & 31u)) & 1u) && ((__ldg(alive_bits + (idb >> 5)) >> (idb & 31u)) & 1u);
+            cand |= ok ? 1u << (j * 4 + r) : 0u;
+        }
+    }
+    // rank of every candidate in record order (group-major, then lane, then r)
+    uint32_t packed = 0;
+#pragma unroll
+    for (int j = 0; j < kRunGroups; ++j) packed |= (uint32_t) __popc((cand >> (4 * j)) & 0xFu) << (8 * j);
+    const uint32_t inc = warp_inclusive_scan(packed);
+    const uint32_t tot = __shfl_sync(0xFFFFFFFFu, inc, 31);
+    uint32_t group_base = 0;
+#pragma unroll
+    for (int j = 0; j < kRunGroups; ++j) {
+        uint32_t p = group_base + (((inc - packed) >> (8 * j)) & 0xFFu);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) {
+            if ((cand >> (j * 4 + r)) & 1u) queue[p++] = (uint16_t) (j * 128u + 4u * lane + r);
+        }
+        group_base += (tot >> (8 * j)) & 0xFFu;
+    }
+    const uint32_t total = group_base;
+    __syncwarp();
+    n_a = 0;
+    n_b = 0;
+    for (uint32_t k0 = 0; k0 < total; k0 += 32) {
+        const uint32_t k = k0 + lane;
+        uint8_t tag = kRejected;
+        if (k < total) {   // only now fetch the coordinates and the two piles
+            Entry e = load_entry(recs, run * kRunRecords + queue[k]);
+            const Pile pa = load_pile(piles, e.a), pb = load_pile(piles, e.b);
+            if (trim(e.c, e.ori, pa, pb)) tag = classify(e.c, relative(e.c, e.ori, pa, pb));   // a surviving kA/kB has a chimeric container (:470, :476)
+            queue[k] |= (uint16_t) ((tag == kRejected ? kQueueRejected : (uint32_t) tag) << kQueueTagShift);
+        }
+        n_a += __popc(__ballot_sync(0xFFFFFFFFu, tag != kRejected && tag != kX));
+        n_b += __popc(__ballot_sync(0xFFFFFFFFu, tag == kX));
+    }
+    __syncwarp();   // the types in the queue are visible to every lane
+    return total;
+}
+
+// phase 3 of `run`: its survivors to their places behind the exclusive prefix `excl`
+__device__ __forceinline__ void survivors_write(const List& recs, const uint2* __restrict__ piles, uint32_t run, const uint16_t* queue,
+                                                uint32_t total, unsigned long long excl, const List& ovl, const List& inl, uint32_t cap) {
+    const uint32_t lane = lane_id();
+    uint32_t pos_a = count_a(excl), pos_b = count_b(excl);
+    for (uint32_t k0 = 0; k0 < total; k0 += 32) {
+        const uint32_t k = k0 + lane;
+        const uint32_t qe = k < total ? queue[k] : kQueueRejected << kQueueTagShift;
+        const uint8_t tag = (uint8_t) (qe >> kQueueTagShift);
+        const int dest = tag == kQueueRejected ? 0 : tag == kX ? 2 : 1;
+        const uint32_t ma = __ballot_sync(0xFFFFFFFFu, dest == 1), mb = __ballot_sync(0xFFFFFFFFu, dest == 2);
+        const uint32_t below = (1u << lane) - 1u;
+        const uint32_t p = dest == 1 ? pos_a + __popc(ma & below) : pos_b + __popc(mb & below);
+        if (dest && p < cap) {
+            Entry e = load_entry(recs, run * kRunRecords + (qe & ((1u << kQueueTagShift) - 1u)));
+            const Pile pa = load_pile(piles, e.a), pb = load_pile(piles, e.b);
+            trim(e.c, e.ori, pa, pb);
+            store_entry(dest == 1 ? ovl : inl, p, e, tag);
+        }
+        pos_a += __popc(ma);
+        pos_b += __popc(mb);
+    }
+}
+
 __global__ void __launch_bounds__(kTileThreads, kSurvMinBlocks) k_classify_survivors(
     List recs, uint32_t n, const uint2* __restrict__ piles, const uint32_t* __restrict__ alive_bits, uint32_t n_piles,
-    List tmp_ovl, List tmp_inl, uint32_t cap, uint32_t* __restrict__ run_cnt) {
-    __shared__ uint16_t s_queue[kTileWarps][kRunRecords];
-    const uint32_t lane = lane_id();
-    uint16_t* queue = s_queue[warp_id()];
-    const uint32_t num_runs = (n + kRunRecords - 1) / kRunRecords;
-    const uint32_t warps = gridDim.x * kTileWarps;
-    for (uint32_t run = blockIdx.x * kTileWarps + warp_id(); run < num_runs; run += warps) {
-        uint32_t a[kRunGroups][4], b[kRunGroups][4];
-#pragma unroll
-        for (int j = 0; j < kRunGroups; ++j) {
-            const uint32_t q = run * (kRunRecords / 4) + j * 32u + lane;     // this lane's j-th group of 4 records
-#pragma unroll
-            for (int r = 0; r < 4; ++r) { a[j][r] = kInvalidBit; b[j][r] = 0u; }
-            if (4u * q < n) {
-                unpack4(reinterpret_cast<const uint4*>(recs.a)[q], a[j]);
-                unpack4(reinterpret_cast<const uint4*>(recs.b)[q], b[j]);
-            }
-        }
-        uint32_t cand = 0;   // bit j * 4 + r
-#pragma unroll
-        for (int j = 0; j < kRunGroups; ++j) {
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {   // both piles alive at the end (graph.cpp:493-515)?  one L1-resident bit each
-                const uint32_t i = run * kRunRecords + j * 128u + 4u * lane + r, ida = a[j][r], idb = b[j][r] & 0x7FFFFFFFu;
-                const bool ok = i < n && !(ida & kInvalidBit) && ida < n_piles && idb < n_piles &&
-                                ((__ldg(alive_bits + (ida >> 5)) >> (ida & 31u)) & 1u) && ((__ldg(alive_bits + (idb >> 5)) >> (idb & 31u)) & 1u);
-                cand |= ok ? 1u << (j * 4 + r) : 0u;
-            }
-        }
-        // rank of every candidate in record order (group-major, then lane, then r)
-        uint32_t packed = 0;
-#pragma unroll
-        for (int j = 0; j < kRunGroups; ++j) packed |= (uint32_t) __popc((cand >> (4 * j)) & 0xFu) << (8 * j);
-        const uint32_t inc = warp_inclusive_scan(packed);
-        const uint32_t tot = __shfl_sync(0xFFFFFFFFu, inc, 31);
-        uint32_t group_base = 0, total = 0;
-#pragma unroll
-        for (int j = 0; j < kRunGroups; ++j) {
-            uint32_t p = group_base + (((inc - packed) >> (8 * j)) & 0xFFu);
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                if ((cand >> (j * 4 + r)) & 1u) queue[p++] = (uint16_t) (j * 128u + 4u * lane + r);
-            }
-            group_base += (tot >> (8 * j)) & 0xFFu;
-        }
-        total = group_base;
-        __syncwarp();
-        uint32_t n_a = 0, n_b = 0;   // warp-uniform: survivors of the run so far (`overlaps`, `internals`)
-        const uint32_t run_len = min((uint32_t) kRunRecords, n - run * kRunRecords);
-        for (uint32_t k0 = 0; k0 < total; k0 += 32) {
-            const uint32_t k = k0 + lane;
-            int dest = 0;
-            uint8_t tag = kRejected;
-            Entry e;
-            if (k < total) {   // only now fetch the coordinates and the two piles
-                const uint32_t i = run * kRunRecords + queue[k];
-                const uint32_t vb = recs.b[i];
-                e.a = recs.a[i];
-                e.b = vb & 0x7FFFFFFFu;
-                e.ori = vb >> 31;
-                e.c.ab = recs.ab[i]; e.c.ae = recs.ae[i]; e.c.bb = recs.bb[i]; e.c.be = recs.be[i];
-                const Pile pa = load_pile(piles, e.a), pb = load_pile(piles, e.b);
-                if (trim(e.c, e.ori, pa, pb)) {
-                    tag = classify(e.c, relative(e.c, e.ori, pa, pb));
-                    dest = tag == kX ? 2 : 1;   // a surviving kA/kB has a chimeric container (:470, :476)
-                }
-            }
-            const uint32_t ma = __ballot_sync(0xFFFFFFFFu, dest == 1), mb = __ballot_sync(0xFFFFFFFFu, dest == 2);
-            const uint32_t below = (1u << lane) - 1u;
-            if (dest) {   // one 32-byte scratch entry, two 16-byte stores: `overlaps` fill the run's slots from the front, `internals` from the back
-                const uint32_t p = dest == 1 ? run * kRunRecords + n_a + __popc(ma & below)
-                                             : run * kRunRecords + run_len - 1u - (n_b + __popc(mb & below));
-                if (p < cap) {
-                    scratch_lo(tmp_ovl)[p] = make_uint4(e.a, e.b | (e.ori << 31), e.c.ab, e.c.ae);
-                    scratch_hi(tmp_inl)[p] = make_uint4(e.c.bb, e.c.be, tag, 0u);
-                }
-            }
-            n_a += __popc(ma);
-            n_b += __popc(mb);
-        }
-        if (lane == 0) run_cnt[run] = n_a | (n_b << 16);
-        __syncwarp();   // the queue is reused by the next run
-    }
-}
-
-// per-run survivor counts (A | B << 16) -> file-order offsets of both lists; single pass, decoupled look-back
-__global__ void __launch_bounds__(kTileThreads) k_scan_runs(const uint32_t* __restrict__ run_cnt, uint32_t num_runs,
-                                                           uint32_t* __restrict__ off_a, uint32_t* __restrict__ off_b,
-                                                           uint32_t* __restrict__ n_a, uint32_t* __restrict__ n_b,
-                                                           unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket) {
-    __shared__ unsigned long long s_warp[kTileWarps];
-    __shared__ unsigned long long s_base;
-    __shared__ uint32_t s_tile;
-    const uint32_t tid = threadIdx.x, lane = lane_id(), warp = warp_id();
-    const uint32_t num_tiles = (num_runs + kTile - 1) / kTile;
-    while (true) {
-        if (tid == 0) s_tile = atomicAdd(ticket, 1u);
-        __syncthreads();
-        const uint32_t tile = s_tile;
-        if (tile >= num_tiles) break;
-        const uint32_t i0 = tile * kTile + tid * 4;
-        unsigned long long v[4];
-        unsigned long long tsum = 0;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t c = i0 + k < num_runs ? run_cnt[i0 + k] : 0u;
-            v[k] = pack_counts(c & 0xFFFFu, c >> 16);
-            tsum += v[k];
-        }
-        unsigned long long inc = tsum;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            const unsigned long long x = __shfl_up_sync(0xFFFFFFFFu, inc, d);
-            if ((int) lane >= d) inc += x;
-        }
-        if (lane == 31) s_warp[warp] = inc;
-        __syncthreads();
-        if (warp == 0) {
-            const unsigned long long w = lane < kTileWarps ? s_warp[lane] : 0ull;
-            unsigned long long winc = w;
-#pragma unroll
-            for (int d = 1; d < kTileWarps; d <<= 1) {
-                const unsigned long long x = __shfl_up_sync(0xFFFFFFFFu, winc, d);
-                if ((int) lane >= d) winc += x;
-            }
-            const unsigned long long total = __shfl_sync(0xFFFFFFFFu, winc, kTileWarps - 1);
-            const unsigned long long excl = lookback_exclusive(status, tile, total);
-            if (lane < kTileWarps) s_warp[lane] = winc - w;
-            if (lane == 0) s_base = excl;
-        }
-        __syncthreads();
-        unsigned long long runv = s_base + s_warp[warp] + inc - tsum;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            if (i0 + k < num_runs) {
-                off_a[i0 + k] = count_a(runv);
-                off_b[i0 + k] = count_b(runv);
-            }
-            runv += v[k];
-        }
-        if (tile == num_tiles - 1 && tid == kTileThreads - 1) {
-            *n_a = count_a(runv);
-            *n_b = count_b(runv);
-        }
-        __syncthreads();
-    }
-}
-
-// Scratch runs -> final positions, one BLOCK per 32 consecutive runs.  The survivors of 32 runs are one contiguous piece of the final list
-// (~1 150 entries on clean data), so the threads take consecutive OUTPUT positions: every column is written fully
-// coalesced, and read in contiguous pieces of a run.  Each warp holds the 32 runs' offsets in its lanes and finds the
-// run of a position with a 5-step binary search over them (shuffles).  (One warp per run, ~36 entries each, was 28 000
-// short dependent chains: count / offset loads, then one and a bit half-empty iterations: 34 us, profiles/r02a.)
-constexpr uint32_t kRelocRuns = 32;
-constexpr int kRelocUnroll = 2;
-
-// The move out of the 32-byte scratch entries: two 16-byte loads per entry (consecutive output positions read consecutive
-// slots of a run), seven coalesced column stores.  U positions per thread and trip: the loads of all of them are issued
-// before the first store, the trips of a block are a chain of dependent memory latencies otherwise.
-template <bool BACK, int U>
-__device__ __forceinline__ void relocate_scratch_piece(const uint4* __restrict__ lo, const uint4* __restrict__ hi, const List& out,
-                                                       uint32_t cap, uint32_t n, uint32_t run0, uint32_t my_off, uint32_t first,
-                                                       uint32_t total) {
+    List ovl, uint32_t* __restrict__ n_ovl, List inl, uint32_t* __restrict__ n_inl, uint32_t cap,
+    unsigned long long* __restrict__ status, uint32_t* __restrict__ ticket) {
+    __shared__ uint16_t s_queue[kTileWarps][2][kRunRecords];
     const uint32_t lane = lane_id(), warp = warp_id();
-    for (uint32_t k = warp * 32u; k < total; k += kTileThreads * U) {   // block-uniform trip count per warp: all lanes shuffle
-        uint4 vlo[U], vhi[U];
-        uint32_t d[U];
-        bool ok[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            const uint32_t kk = k + u * kTileThreads + lane;
-            d[u] = first + kk;
-            uint32_t l = 0;   // the largest run l of the 32 whose first output position is <= d
-#pragma unroll
-            for (uint32_t step = 16; step > 0; step >>= 1) {
-                const uint32_t v = __shfl_sync(0xFFFFFFFFu, my_off, (l + step) & 31u);
-                if (l + step < kRelocRuns && v <= d[u]) l += step;
-            }
-            const uint32_t j = d[u] - __shfl_sync(0xFFFFFFFFu, my_off, l), base = (run0 + l) * kRunRecords;
-            const uint32_t s = BACK ? base + min((uint32_t) kRunRecords, n - base) - 1u - j : base + j;   // internals sit at the back of the run's slots
-            ok[u] = kk < total && s < cap && d[u] < cap;
-            if (ok[u]) {
-                vlo[u] = __ldg(lo + s);
-                vhi[u] = __ldg(hi + s);
-            }
+    const uint32_t num_runs = (n + kRunRecords - 1) / kRunRecords;
+    uint32_t cur = 0, prev_run = 0xFFFFFFFFu, prev_total = 0;   // warp-uniform; prev_run: the run awaiting its prefix
+    unsigned long long prev_agg = 0;
+    while (true) {
+        uint32_t run = 0;
+        if (lane == 0) run = atomicAdd(ticket, 1u);
+        run = __shfl_sync(0xFFFFFFFFu, run, 0);
+        uint32_t total = 0;
+        unsigned long long agg = 0;
+        if (run < num_runs) {
+            uint32_t n_a, n_b;
+            total = survivors_queue(recs, n, piles, alive_bits, n_piles, run, s_queue[warp][cur], n_a, n_b);
+            agg = pack_counts(n_a, n_b);
+            lookback_publish(status, run, agg);
         }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            if (ok[u]) {
-                out.a[d[u]] = vlo[u].x; out.b[d[u]] = vlo[u].y;
-                out.ab[d[u]] = vlo[u].z; out.ae[d[u]] = vlo[u].w;
-                out.bb[d[u]] = vhi[u].x; out.be[d[u]] = vhi[u].y;
-                out.tag[d[u]] = (uint8_t) vhi[u].z;
+        if (prev_run != 0xFFFFFFFFu) {
+            const unsigned long long excl = lookback_wait(status, prev_run, prev_agg);
+            if (prev_run == num_runs - 1 && lane == 0) {
+                *n_ovl = count_a(excl + prev_agg);
+                *n_inl = count_b(excl + prev_agg);
             }
+            survivors_write(recs, piles, prev_run, s_queue[warp][cur ^ 1], prev_total, excl, ovl, inl, cap);
+            __syncwarp();   // that queue is refilled by the next run
         }
-    }
-}
-
-__global__ void __launch_bounds__(kTileThreads) k_relocate_runs(List tmp_a, List out_a, List tmp_b, List out_b, uint32_t cap,
-                                                               const uint32_t* __restrict__ run_cnt, const uint32_t* __restrict__ off_a,
-                                                               const uint32_t* __restrict__ off_b, uint32_t num_runs, uint32_t n) {
-    const uint32_t lane = lane_id();
-    const uint32_t supers = (num_runs + kRelocRuns - 1) / kRelocRuns;
-    for (uint32_t sr = blockIdx.x; sr < supers; sr += gridDim.x) {
-        const uint32_t run0 = sr * kRelocRuns, run = run0 + lane;
-        // lanes behind the last run repeat its end, so the search never lands on them
-        const uint32_t last = num_runs - 1u, r = min(run, last);
-        const uint32_t c = __ldg(run_cnt + r);
-        uint32_t oa = __ldg(off_a + r), ob = __ldg(off_b + r);
-        if (run > last) { oa += c & 0xFFFFu; ob += c >> 16; }
-        const uint32_t na = run <= last ? (c & 0xFFFFu) : 0u, nb = run <= last ? (c >> 16) : 0u;
-        const uint32_t first_a = __shfl_sync(0xFFFFFFFFu, oa, 0), first_b = __shfl_sync(0xFFFFFFFFu, ob, 0);
-        const uint32_t total_a = __shfl_sync(0xFFFFFFFFu, oa + na, 31) - first_a, total_b = __shfl_sync(0xFFFFFFFFu, ob + nb, 31) - first_b;
-        relocate_scratch_piece<false, kRelocUnroll>(scratch_lo(tmp_a), scratch_hi(tmp_b), out_a, cap, n, run0, oa, first_a, total_a);
-        relocate_scratch_piece<true, 1>(scratch_lo(tmp_a), scratch_hi(tmp_b), out_b, cap, n, run0, ob, first_b, total_b);
+        if (run >= num_runs) break;
+        prev_run = run;
+        prev_total = total;
+        prev_agg = agg;
+        cur ^= 1;
     }
 }
 
@@ -475,9 +384,20 @@ __global__ void k_hill_coverage(List recs, uint32_t t0, const uint2* __restrict_
 // Also refreshes the one-bit-per-pile liveness bitmap the survivors pass tests first.
 // DECODE: dbuf still holds the resolution's state words (containment.cu: settled bit | death time, 0x7FFFFFFF = never);
 // they are turned into death times (kInf = never) on the way, which saves the separate k_decode_state launch.
+// reset (first pass only, also when the pass is skipped): nothing reads the first pass's earliest events or event count
+// any more, so this sweep clears them for the final pass and keeps the first pass's event and round counts.
 template <bool DECODE>
 __global__ void k_apply_deaths(uint2* __restrict__ piles, uint32_t* __restrict__ D, uint32_t n_piles, uint32_t* __restrict__ alive_bits,
-                               const uint32_t* __restrict__ skip, const uint32_t* __restrict__ run_if) {
+                               const uint32_t* __restrict__ skip, const uint32_t* __restrict__ run_if, FinalPassReset reset) {
+    if (reset.counters) {
+        for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < reset.n_first; i += gridDim.x * blockDim.x) reset.first[i] = ~0ull;
+        if (blockIdx.x == 0 && threadIdx.x == 0) {
+            uint32_t* c = reset.counters;
+            c[C_EV_FIRST] = c[C_EV];
+            c[C_ROUNDS_FIRST] = c[C_ROUNDS];
+            c[C_EV] = 0u;
+        }
+    }
     if ((skip && *skip) || (run_if && *run_if == 0u)) return;
     for (uint32_t base = blockIdx.x * blockDim.x; base < n_piles; base += gridDim.x * blockDim.x) {
         const uint32_t i = base + threadIdx.x;
@@ -495,6 +415,32 @@ __global__ void k_apply_deaths(uint2* __restrict__ piles, uint32_t* __restrict__
         const uint32_t m = __ballot_sync(0xFFFFFFFFu, alive);
         if (lane_id() == 0 && i < n_piles) alive_bits[i >> 5] = m;
     }
+}
+
+// n words of p set to v by the whole grid, 16 bytes per store where p allows
+__device__ __forceinline__ void fill_words(uint32_t* p, size_t n, uint32_t v, size_t tid, size_t threads) {
+    size_t head = ((16u - ((uintptr_t) p & 15u)) & 15u) / 4u;
+    head = head < n ? head : n;
+    const size_t n4 = (n - head) / 4;
+    uint4* q = reinterpret_cast<uint4*>(p + head);
+    for (size_t i = tid; i < head; i += threads) p[i] = v;
+    for (size_t i = tid; i < n4; i += threads) q[i] = make_uint4(v, v, v, v);
+    for (size_t i = head + 4 * n4 + tid; i < n; i += threads) p[i] = v;
+}
+
+// The clears and the copy a step starts from, in one launch (StepPrologue).
+__global__ void __launch_bounds__(256) k_step_prologue(StepPrologue p) {
+    const size_t tid = (size_t) blockIdx.x * blockDim.x + threadIdx.x, threads = (size_t) gridDim.x * blockDim.x;
+    const uint4* src = reinterpret_cast<const uint4*>(p.snapshot ? p.piles : p.piles_initial);   // 256-byte aligned tables
+    uint4* dst = reinterpret_cast<uint4*>(p.snapshot ? p.piles_initial : p.piles);
+    for (size_t i = tid; i < p.n_piles / 2; i += threads) dst[i] = src[i];
+    if (tid == 0 && (p.n_piles & 1u)) {
+        const uint2* s2 = reinterpret_cast<const uint2*>(src);
+        reinterpret_cast<uint2*>(dst)[p.n_piles - 1] = s2[p.n_piles - 1];
+    }
+    fill_words(reinterpret_cast<uint32_t*>(p.first), 2 * (size_t) p.n_first, ~0u, tid, threads);
+    for (int k = 0; k < StepPrologue::kZero; ++k)
+        if (p.zero[k]) fill_words(p.zero[k], p.zero_words[k], 0u, tid, threads);
 }
 
 // =============================================================================================
@@ -711,23 +657,18 @@ void launch_classify_events(Launch& L, List recs, uint32_t n, uint32_t t0, const
     L.count++;
 }
 
+uint32_t classify_num_runs(uint32_t n) { return (n + kRunRecords - 1) / kRunRecords; }
+
 void launch_classify_survivors(Launch& L, List recs, uint32_t n, const uint2* piles, const uint32_t* alive_bits, uint32_t n_piles,
-                               List tmp_ovl, List tmp_inl, List ovl, uint32_t* n_ovl, List inl, uint32_t* n_inl, uint32_t cap,
-                               RunBufs runs, unsigned long long* status, uint32_t* ticket) {
+                               List ovl, uint32_t* n_ovl, List inl, uint32_t* n_inl, uint32_t cap, unsigned long long* status,
+                               uint32_t* ticket) {
     if (n == 0) return;   // n_ovl / n_inl were zeroed by the caller
-    const uint32_t num_runs = (n + kRunRecords - 1) / kRunRecords;
+    const uint32_t num_runs = classify_num_runs(n);
     k_classify_survivors<<<grid_for(num_runs, kTileWarps, kNumSMs * kSurvBlocks), kTileThreads, 0, L.stream>>>(
-        recs, n, piles, alive_bits, n_piles, tmp_ovl, tmp_inl, cap, runs.cnt);
-    L.count++;
-    k_scan_runs<<<grid_for(num_runs, kTile, kNumSMs * 4), kTileThreads, 0, L.stream>>>(runs.cnt, num_runs, runs.off_a, runs.off_b, n_ovl,
-                                                                                       n_inl, status, ticket);
-    L.count++;
-    k_relocate_runs<<<grid_for(num_runs, kRelocRuns, kNumSMs * 8), kTileThreads, 0, L.stream>>>(tmp_ovl, ovl, tmp_inl, inl, cap, runs.cnt,
-                                                                                               runs.off_a, runs.off_b, num_runs, n);
+        recs, n, piles, alive_bits, n_piles, ovl, n_ovl, inl, n_inl, cap, status, ticket);
     L.count++;
 }
 
-uint32_t classify_num_runs(uint32_t n) { return (n + kRunRecords - 1) / kRunRecords; }
 
 void launch_hill_coverage(Launch& L, List recs, uint32_t t0, const uint2* piles, const uint32_t* hill_rec,
                           uint32_t hill_cap, const uint32_t* hill_pile, const uint32_t* hill_begin,
@@ -739,10 +680,16 @@ void launch_hill_coverage(Launch& L, List recs, uint32_t t0, const uint2* piles,
 }
 
 void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, uint32_t* alive_bits, bool decode,
-                         const uint32_t* skip, const uint32_t* run_if) {
-    if (n_piles == 0) return;
-    if (decode) k_apply_deaths<true><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if);
-    else k_apply_deaths<false><<<grid_for(n_piles, 256, kNumSMs * 8), 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if);
+                         const uint32_t* skip, const uint32_t* run_if, FinalPassReset reset) {
+    if (n_piles == 0 && !reset.counters) return;
+    const int grid = grid_for(n_piles > reset.n_first ? n_piles : reset.n_first, 256, kNumSMs * 8);
+    if (decode) k_apply_deaths<true><<<grid, 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if, reset);
+    else k_apply_deaths<false><<<grid, 256, 0, L.stream>>>(piles, dbuf, n_piles, alive_bits, skip, run_if, reset);
+    L.count++;
+}
+
+void launch_step_prologue(Launch& L, const StepPrologue& p) {
+    k_step_prologue<<<kNumSMs * 4, 256, 0, L.stream>>>(p);
     L.count++;
 }
 
@@ -813,11 +760,10 @@ void preload_classify() {
     cudaFuncGetAttributes(&a, k_unpack_records);
     cudaFuncGetAttributes(&a, k_classify_events<kEventsMinBlocks, kEventsItems>);
     cudaFuncGetAttributes(&a, k_classify_survivors);
-    cudaFuncGetAttributes(&a, k_scan_runs);
-    cudaFuncGetAttributes(&a, k_relocate_runs);
     cudaFuncGetAttributes(&a, k_hill_coverage);
     cudaFuncGetAttributes(&a, k_apply_deaths<true>);
     cudaFuncGetAttributes(&a, k_apply_deaths<false>);
+    cudaFuncGetAttributes(&a, k_step_prologue);
     cudaFuncGetAttributes(&a, k_list_pass<kRetrim>);
     cudaFuncGetAttributes(&a, k_list_pass<kPromote>);
     cudaFuncGetAttributes(&a, k_list_pass<kFinalOvl>);

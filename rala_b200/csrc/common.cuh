@@ -245,15 +245,15 @@ __device__ __forceinline__ void st_status(unsigned long long* p, unsigned long l
     asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
 }
 
-// Called by ONE full warp of the block.  Returns the exclusive prefix (packed counts) of `tile`.
-__device__ __forceinline__ unsigned long long lookback_exclusive(unsigned long long* status, uint32_t tile,
-                                                                  unsigned long long aggregate) {
+// The two halves of lookback_exclusive, for a warp that has other work between them: publish `tile`'s aggregate (lane 0
+// stores), then later wait for its exclusive prefix (ONE full warp) and publish the inclusive one.
+__device__ __forceinline__ void lookback_publish(unsigned long long* status, uint32_t tile, unsigned long long aggregate) {
+    if (lane_id() == 0) st_status(status + tile, (tile == 0 ? kStateInc : kStateAgg) | aggregate);
+}
+
+__device__ __forceinline__ unsigned long long lookback_wait(unsigned long long* status, uint32_t tile, unsigned long long aggregate) {
     const uint32_t lane = lane_id();
-    if (tile == 0) {
-        if (lane == 0) st_status(status, kStateInc | aggregate);
-        return 0ull;
-    }
-    if (lane == 0) st_status(status + tile, kStateAgg | aggregate);
+    if (tile == 0) return 0ull;
     unsigned long long exclusive = 0ull;
     int64_t look = (int64_t) tile - 1;
     while (true) {
@@ -272,6 +272,13 @@ __device__ __forceinline__ unsigned long long lookback_exclusive(unsigned long l
     }
     if (lane == 0) st_status(status + tile, kStateInc | ((exclusive + aggregate) & kCountMask));
     return exclusive;
+}
+
+// Called by ONE full warp of the block.  Returns the exclusive prefix (packed counts) of `tile`.
+__device__ __forceinline__ unsigned long long lookback_exclusive(unsigned long long* status, uint32_t tile,
+                                                                  unsigned long long aggregate) {
+    lookback_publish(status, tile, aggregate);
+    return lookback_wait(status, tile, aggregate);
 }
 
 }  // namespace rb

@@ -64,22 +64,41 @@ void launch_unpack_records(Launch& L, const uint32_t* query_id, const uint32_t* 
                            const uint32_t* b_span, uint32_t n, List recs);
 void launch_classify_events(Launch& L, List recs, uint32_t n, uint32_t t0, const uint2* piles, uint32_t n_piles,
                             Events ev, uint32_t ev_cap, unsigned long long* first, uint32_t* hill_rec, uint32_t hill_cap, uint32_t* counters);
-// runs of the survivors pass (128 records each): packed counts (overlaps | internals << 16) and the scanned offsets
-struct RunBufs {
-    uint32_t *cnt, *off_a, *off_b;   // num_runs each
-};
+// the survivors in file order straight into `overlaps` / `internals` with their counts; the look-back takes one status word
+// per run of classify_num_runs(n)
 void launch_classify_survivors(Launch& L, List recs, uint32_t n, const uint2* piles, const uint32_t* alive_bits, uint32_t n_piles,
-                               List tmp_ovl, List tmp_inl, List ovl, uint32_t* n_ovl, List inl, uint32_t* n_inl, uint32_t cap,
-                               RunBufs runs, unsigned long long* status, uint32_t* ticket);
+                               List ovl, uint32_t* n_ovl, List inl, uint32_t* n_inl, uint32_t cap, unsigned long long* status,
+                               uint32_t* ticket);
 uint32_t classify_num_runs(uint32_t n);
 void launch_hill_coverage(Launch& L, List recs, uint32_t t0, const uint2* piles, const uint32_t* hill_rec,
                           uint32_t hill_cap, const uint32_t* hill_pile, const uint32_t* hill_begin,
                           const uint32_t* hill_end, uint32_t n_hills, uint32_t* hill_cov, const uint32_t* dbuf,
                           const uint32_t* counters);
+// what the first pass's k_apply_deaths clears for the final pass: `first` (n_first words) to all ones, counters[C_EV] to
+// zero after C_EV / C_ROUNDS went to C_EV_FIRST / C_ROUNDS_FIRST.  counters == nullptr: nothing.
+struct FinalPassReset {
+    unsigned long long* first = nullptr;
+    uint32_t n_first = 0;
+    uint32_t* counters = nullptr;
+};
 // skip: optional device flag, non-zero = do nothing (multi-GPU: a containment pass without events); run_if: optional device
-// count, zero = do nothing (single GPU: the final containment pass when it has no events)
+// count, zero = do nothing (single GPU: the final containment pass when it has no events).  reset is done in either case.
 void launch_apply_deaths(Launch& L, uint2* piles, uint32_t* dbuf, uint32_t n_piles, uint32_t* alive_bits, bool decode,
-                         const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr);
+                         const uint32_t* skip = nullptr, const uint32_t* run_if = nullptr, FinalPassReset reset = {});
+// the device state a step starts from, in one launch: the pile table restored from piles_initial (snapshot: the other
+// way), the earliest events (n_first words) all ones, and the zero[k] regions (counters, hill coverage, look-back pool,
+// slot degrees, transitive work counters) cleared; a null region is left alone
+struct StepPrologue {
+    static constexpr int kZero = 5;
+    uint2 *piles, *piles_initial;
+    uint32_t n_piles;
+    bool snapshot;
+    unsigned long long* first;
+    uint32_t n_first;
+    uint32_t* zero[kZero];
+    size_t zero_words[kZero];
+};
+void launch_step_prologue(Launch& L, const StepPrologue& p);
 void launch_list_pass(Launch& L, int mode, List in, const uint32_t* n_in, uint32_t in_cap, const uint2* piles, List out_a,
                       uint32_t* n_out_a, List out_b, uint32_t* n_out_b, const uint32_t* b_base, uint32_t cap,
                       const uint32_t* dbuf, const uint32_t* time_base, unsigned long long* status, uint32_t* ticket);

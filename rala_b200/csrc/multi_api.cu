@@ -507,7 +507,8 @@ static int resolve_owned_piles(rala_b200_multi* m, FabricRank& fr, int pass, boo
     }
     // every replica now holds every pile's final state: piles with a finite death time die (graph.cpp:471,477,838,842)
     // (a skipped pass killed nobody: the table and the liveness bitmap stay as they are)
-    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->alive_bits.as<uint32_t>(), !hills, skip_flag(fr.P));
+    launch_apply_deaths(L, g->piles.as<uint2>(), fr.sec<uint32_t>(fr.A.S), g->n_piles, g->alive_bits.as<uint32_t>(), !hills, skip_flag(fr.P),
+                        nullptr, pass == 0 ? final_pass_reset(g) : FinalPassReset{});
     MCU(m, cudaGetLastError());
     return RALA_B200_OK;
 }

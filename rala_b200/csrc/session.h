@@ -92,6 +92,8 @@ enum TextFormat : uint8_t { kTextNone = 0, kTextPaf, kTextMhap };
 // how far the session's stages got on the current inputs
 enum SessionState { SS_EMPTY = 0, SS_INPUTS, SS_CLASSIFIED, SS_FINALIZED, SS_BUILT, SS_REDUCED };
 
+enum StepCleared : uint32_t { kStepBuild = 1, kStepTransitive = 2 };
+
 enum Stage { ST_CLASSIFY = 0, ST_RETRIM, ST_FINALIZE, ST_BUILD, ST_TRANSITIVE, ST_K1_KERNEL, ST_K1B_KERNEL, ST_K3_KERNELS, ST_K1S_KERNEL };
 
 struct rala_b200_graph {
@@ -115,10 +117,16 @@ struct rala_b200_graph {
     int ovl_cur = 0, inl_cur = 0;
     int slot_ovl = C_LIST0, slot_inl = C_LIST0 + 1, next_slot = C_LIST0 + 2;
     DevBuf events, hill_rec;
-    DevBuf dbuf, flags, segs, tiles;   // dbuf: S | vcursor | vstart | work0 | work1 | hidx | first (2 strides) ; segs: seg | hev ; tiles: info | off
+    DevBuf dbuf, flags, segs;   // dbuf: S | vcursor | vstart | work0 | work1 | hidx | first (2 strides) ; segs: seg | hev
     DevBuf counters;
+    // look-back status words: one region per step, zeroed by the step prologue (phase_events) and handed out in order by
+    // scan_state; words [scan_used, scan_pool_words) are zero while scan_zeroed holds
     DevBuf scan_pool;
     size_t scan_pool_words = 0, scan_used = 0;
+    bool scan_zeroed = false;
+    // counters and buffers of a later stage the step prologue cleared and no stage has used since (kStep*): that stage
+    // skips its own clears
+    uint32_t step_cleared = 0;
     // graph
     DevBuf edges_aos;
     DevBuf seq_to_node, edges, row_ptr, cursor, col, col_eid, T, marked, heavy, work_counter;
@@ -203,6 +211,8 @@ cudaError_t end_stage(rala_b200_graph* g, int stage);
 cudaError_t zero_counter(rala_b200_graph* g, int slot, int n = 1);
 ResolveBufs resolve_bufs(const rala_b200_graph* g);
 cudaError_t clear_earliest_events(rala_b200_graph* g);
+// handed to the first containment pass's launch_apply_deaths: it prepares the final pass (kernels.h)
+FinalPassReset final_pass_reset(const rala_b200_graph* g);
 int reserve_events(rala_b200_graph* g, uint32_t ev_cap);
 int reserve_edges(rala_b200_graph* g, uint32_t edge_cap);
 int read_counters(rala_b200_graph* g, uint32_t* h);
