@@ -274,6 +274,46 @@ int rala_b200_graph_set_piles(rala_b200_graph* g, const rala_pile_t* piles, cons
  * the sequence lengths transmute checks, overlap.cpp:54-59, 73-78); once per session.  Layout and refusals as
  * rala_b200_parse_paf.  The name table stays on the device.  MHAP text uses only the lengths and their order. */
 int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint64_t* name_end, const uint32_t* read_len, uint32_t n_reads);
+/* The same from the sequence file: FASTA or FASTQ text in host memory -> the read names and lengths, parsed on the device
+ * (the first half of Graph::initialize, graph.cpp:249-264).  After success every later call behaves exactly as after
+ * set_reads(names, name_end, read_len) with the names and lengths the text holds, read ids in file order.  After a
+ * refusal the session holds no reads (set_overlaps_paf / _mhap: RALA_B200_ERR_STATE) and no upload is in flight.
+ * Text contract (anything else is refused with RALA_B200_ERR_ARG and a message naming the 1-based line and column; the
+ * smallest offending line is reported, within it the smallest column):
+ *   - the first byte picks the format: '>' FASTA, '@' FASTQ, anything else is refused; empty text = 0 reads;
+ *   - lines end in '\n' (the last one may lack it); an empty line is refused; a '\r' anywhere is refused (CRLF handling
+ *     is not pinned);
+ *   - header line ('>' in FASTA, '@' in FASTQ): the name is the bytes after the marker up to the first space (0x20) or tab
+ *     (0x09) or the line's end; the rest, the description, is never read.  An empty name, or a name byte < 0x20 or 0x7F,
+ *     is refused.  Restated, NOT pinned: the cut at the first space or tab (the token minimap2 writes into PAF column 1);
+ *     n_described counts the headers it cut;
+ *   - FASTA: a line starting with '>' starts a read, every other line is a sequence line of the current read; a read's
+ *     length is the sum of its sequence lines' lengths (any wrapping width); sequence bytes lie in 0x21..0x7E, each one
+ *     base (case and IUPAC codes are never interpreted; a '>' inside a line is a base); a read without sequence is refused
+ *     at its header line;
+ *   - FASTQ: exactly four lines per read: '@' header, sequence (the FASTA byte rule, not empty), a line starting with '+'
+ *     (the rest never read), quality with exactly as many bytes as the sequence (content never read, so it may start with
+ *     '@' or '+').  Text that ends inside a read is refused at that read's header line; multi-line FASTQ is refused;
+ *   - a name listed twice is refused as set_reads refuses it ("same name"); a read of 2^32 bases or more and a count of
+ *     reads >= 2^31 are refused at the read's header line.
+ * Upload as for PAF: chunks of RALA_B200_PAF_CHUNK_BYTES cut behind their last '\n' (a longer line, an unwrapped read
+ * above 32 Mbp, is refused with RALA_B200_ERR_LIMIT), page-locked caller memory in place.  The text is below 2^34 bytes
+ * (RALA_B200_ERR_LIMIT).  Device memory kept after the call is set_reads' (names, ends, lengths, table) plus the upload
+ * staging shared with the overlap readers.  stats: nullable. */
+typedef struct {
+    uint32_t format;         /* 1 FASTA, 2 FASTQ, 0 empty text */
+    uint32_t n_reads;
+    uint64_t n_lines, n_bases, name_bytes;
+    uint32_t max_len, n_described;   /* headers whose name was cut at a space / tab (restated, not pinned) */
+    uint64_t n_bytes, n_chunks;
+    float device_ms;         /* kernels of the call (line scan, roles, byte rules, lengths, name table); uploads excluded */
+} rala_b200_reads_stats_t;
+int rala_b200_graph_set_reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_reads_stats_t* stats);
+/* After set_reads or set_reads_text: the session's reads in the set_reads layout (names back to back, u64 name ends,
+ * u32 lengths).  *n_reads and *name_bytes (nullable) receive the sizes; each NULL buffer is skipped, so a call with NULL
+ * buffers only returns the sizes.  RALA_B200_ERR_STATE when the session holds no reads. */
+int rala_b200_graph_get_reads(rala_b200_graph* g, char* names_out, uint64_t* name_end_out, uint32_t* read_len_out,
+                              uint32_t* n_reads, uint64_t* name_bytes);
 /* PAF text in FILE ORDER -> the session's records, replacing the host parse and transmute of graph.cpp:443-451 and the
  * records set_overlaps* would receive: the text is parsed as rala_b200_parse_paf does, the duplicate filter of
  * Graph::initialize (graph.cpp:273-303, :340-361) runs on the parsed columns, and a record leaves INVALID when a name did

@@ -57,6 +57,15 @@ class MhapStats(C.Structure):
         return {k: int(getattr(self, k)) for k, _ in self._fields_}
 
 
+class ReadsStats(C.Structure):
+    _fields_ = [("format", C.c_uint32), ("n_reads", C.c_uint32), ("n_lines", C.c_uint64), ("n_bases", C.c_uint64),
+                ("name_bytes", C.c_uint64), ("max_len", C.c_uint32), ("n_described", C.c_uint32), ("n_bytes", C.c_uint64),
+                ("n_chunks", C.c_uint64), ("device_ms", C.c_float)]
+
+    def as_dict(self):
+        return {k: (float(getattr(self, k)) if k == "device_ms" else int(getattr(self, k))) for k, _ in self._fields_}
+
+
 PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES (the MHAP reader uses the same chunks)
 
 
@@ -69,12 +78,12 @@ class PileStats(C.Structure):
 
 
 def _text(text):
-    """PAF / MHAP text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
+    """PAF / MHAP / FASTA / FASTQ text as bytes, a uint8 numpy array or a contiguous uint8 CPU tensor (pinned: uploaded in place)."""
     if isinstance(text, (bytes, bytearray, memoryview)):
         text = np.frombuffer(text, np.uint8)
     if hasattr(text, "data_ptr"):
         if not text.is_contiguous() or text.device.type != "cpu" or text.element_size() != 1:
-            raise RalaB200Error("overlap text must be a contiguous uint8 CPU tensor")
+            raise RalaB200Error("text must be a contiguous uint8 CPU tensor")
         return text, int(text.numel())
     text = np.ascontiguousarray(text, dtype=np.uint8).reshape(-1)
     return text, int(text.shape[0])
@@ -102,7 +111,7 @@ EXPORTS = [
     "rala_b200_launch_count", "rala_b200_event_record", "rala_b200_event_elapsed_ms", "rala_b200_synchronize",
     "rala_b200_trim_classify", "rala_b200_transitive_reduce", "rala_b200_filter_duplicates",
     "rala_b200_parse_paf", "rala_b200_graph_set_reads", "rala_b200_graph_set_overlaps_paf",
-    "rala_b200_parse_mhap", "rala_b200_graph_set_overlaps_mhap",
+    "rala_b200_parse_mhap", "rala_b200_graph_set_overlaps_mhap", "rala_b200_graph_set_reads_text", "rala_b200_graph_get_reads",
     "rala_b200_build_piles", "rala_b200_graph_build_piles", "rala_b200_graph_get_medians", "rala_b200_graph_get_coverage_runs",
     "rala_b200_graph_create", "rala_b200_graph_destroy", "rala_b200_graph_set_overlaps",
     "rala_b200_graph_set_piles", "rala_b200_graph_set_hills", "rala_b200_graph_classify",
@@ -437,6 +446,26 @@ class Graph:
         self._call("rala_b200_graph_set_reads", _ptr(blob), _ptr(ends), _ptr(rl), C.c_uint32(ends.shape[0]))
         self._n_reads = int(ends.shape[0])
         return self
+
+    def set_reads_text(self, text) -> dict:
+        """FASTA or FASTQ text (bytes, uint8 array or pinned CPU tensor) -> the read names and lengths, parsed on the device;
+        afterwards the session is as after set_reads with them.  Returns the stats (format, reads, lines, bases, name
+        bytes, longest read, headers with a description, bytes, upload chunks, device_ms)."""
+        buf, n_bytes = _text(text)
+        st = ReadsStats()
+        self._call("rala_b200_graph_set_reads_text", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
+        self._n_reads = int(st.n_reads)
+        return st.as_dict()
+
+    def reads(self):
+        """The session's reads as set_reads holds them: (names blob uint8, name_end uint64, read_len uint32)."""
+        n, nb = C.c_uint32(0), C.c_uint64(0)
+        self._call("rala_b200_graph_get_reads", None, None, None, C.byref(n), C.byref(nb))
+        blob = np.zeros(max(int(nb.value), 1), np.uint8)
+        ends = np.zeros(int(n.value), np.uint64)
+        rl = np.zeros(int(n.value), np.uint32)
+        self._call("rala_b200_graph_get_reads", _ptr(blob), _ptr(ends), _ptr(rl), None, None)
+        return blob[:int(nb.value)], ends, rl
 
     def set_overlaps_paf(self, text) -> dict:
         """PAF text in file order -> the session's records (parse, name lookup, duplicate filter on the device); returns

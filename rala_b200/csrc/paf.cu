@@ -9,6 +9,7 @@
 //                            k_paf_parse        one warp per line: tab positions by ballot, lane f parses field f
 //                         or k_mhap_parse       the same for MHAP: spaces, numeric ids checked against the read count
 //   per call (session):      k_filter_duplicates, k_paf_fold   is_valid_overlap_ folded into the INVALID bit
+// The upload and line scan (text_chunks) and the name table (names_table) also serve the FASTA / FASTQ reader (reads.cu).
 //
 // Input contracts (the library refuses what it cannot map onto the reference's reading without guessing; the full text
 // is in include/rala_b200.h).  PAF: tab-separated, at least 12 fields; columns 2, 3, 4, 7, 8, 9, 11 plain decimal below
@@ -30,22 +31,6 @@ constexpr uint32_t kUnknownId = 0x7FFFFFFFu;                           // a name
 constexpr uint32_t kMinPafLine = 19;                                   // 11 tabs + 7 digits + '\n': no valid line is shorter
 constexpr uint32_t kMinMhapLine = 22;                                  // 11 spaces + 10 digits + '\n' (fields 3, 4 empty)
 enum : uint32_t { kErrFields = 1, kErrEmpty = 2, kErrDigit = 3, kErrOverflow = 4, kErrReadId = 5, kErrStrand = 6 };
-// device words of one call: the first four start at ~0 (minima), the rest at 0; line bases of the chunks follow
-enum { W_ERR = 0, W_DUP, W_FIRST_MISMATCH, W_FIRST_BAD, W_UNRESOLVED, W_MISMATCH, W_QUERY_RC, W_BASES = 8 };
-
-struct NameTable {
-    const uint8_t* blob;
-    const unsigned long long* end;   // name i = blob[end[i-1], end[i])
-    const uint32_t* read_len;
-    unsigned long long* slots;       // hash >> 32 << 32 | id, ~0 = empty
-    uint32_t mask;
-};
-
-struct PafCols {
-    uint32_t *a, *b, *ab, *ae, *bb, *be, *len;
-    uint8_t* mismatch;
-};
-
 __device__ __forceinline__ unsigned long long name_hash(const uint8_t* p, uint32_t n) {
     unsigned long long h = 0xcbf29ce484222325ull;   // FNV-1a, then the murmur3 finaliser for the slot bits
     for (uint32_t i = 0; i < n; ++i) h = (h ^ p[i]) * 0x100000001b3ull;
@@ -353,41 +338,46 @@ void preload_paf() {
 // ---------------------------------------------------------------------------------------------
 // host side: the name table, the chunked upload and the call's bookkeeping
 // ---------------------------------------------------------------------------------------------
-struct PafReader {
-    DevBuf names;                 // blob | ends | read lengths | table slots
-    NameTable table{};
-    uint32_t n_reads = 0, max_len = 0;
-    bool have_names = false;
-    DevBuf text[2];               // device side of the staging pair
-    DevBuf line_end, status, words, cols, valid;
-    char* pinned[2] = {nullptr, nullptr};
-    cudaStream_t copy = nullptr;  // uploads: chunk k + 1 crosses PCIe while chunk k is parsed
-    cudaEvent_t copied[2]{}, parsed[2]{};
-    std::vector<cudaEvent_t> timing;   // (start, stop) around the kernels of every chunk
-    unsigned long long rec_cap = 0;
-    std::vector<unsigned long long> w;   // the words of the last call, read back
-
-    PafCols view() const {
-        const size_t col = align_up((size_t) rec_cap * 4, 256);
-        char* b = cols.as<char>();
-        return PafCols{(uint32_t*) b, (uint32_t*) (b + col), (uint32_t*) (b + 2 * col), (uint32_t*) (b + 3 * col),
-                       (uint32_t*) (b + 4 * col), (uint32_t*) (b + 5 * col), (uint32_t*) (b + 6 * col), (uint8_t*) (b + 7 * col)};
-    }
-    ~PafReader() {
-        if (copy) cudaStreamSynchronize(copy);
-        DevBuf* bufs[] = {&names, &text[0], &text[1], &line_end, &status, &words, &cols, &valid};
-        for (DevBuf* b : bufs) b->release();
-        for (int k = 0; k < 2; ++k) {
-            if (pinned[k]) cudaFreeHost(pinned[k]);
-            if (copied[k]) cudaEventDestroy(copied[k]);
-            if (parsed[k]) cudaEventDestroy(parsed[k]);
-        }
-        for (cudaEvent_t e : timing) cudaEventDestroy(e);
-        if (copy) cudaStreamDestroy(copy);
-    }
-};
-
 void destroy_paf_reader(PafReader* r) { delete r; }
+
+NamesLayout names_layout(uint32_t n_reads, uint64_t blob) {
+    NamesLayout L;
+    L.slots = 1024;
+    while (L.slots < 2ull * n_reads) L.slots <<= 1;
+    L.o_end = align_up(blob + 1, 256);
+    L.o_len = L.o_end + align_up((size_t) n_reads * 8 + 8, 256);
+    L.o_slots = L.o_len + align_up((size_t) n_reads * 4 + 4, 256);
+    L.bytes = L.o_slots + (size_t) L.slots * 8;
+    return L;
+}
+
+int names_table(rala_b200_ctx* ctx, PafReader& R, uint32_t n_reads, uint64_t blob, cudaEvent_t ev0, cudaEvent_t ev1) {
+    const NamesLayout L = names_layout(n_reads, blob);
+    CU(ctx, R.words.reserve(256));
+    char* b = R.names.as<char>();
+    cudaStream_t s = ctx->L.stream;
+    CU(ctx, cudaMemsetAsync(b + L.o_slots, 0xFF, (size_t) L.slots * 8, s));
+    CU(ctx, cudaMemsetAsync(R.words.p, 0xFF, 8 * (W_DUP + 1), s));
+    R.table = NameTable{(const uint8_t*) b, (const unsigned long long*) (b + L.o_end), (const uint32_t*) (b + L.o_len),
+                        (unsigned long long*) (b + L.o_slots), L.slots - 1};
+    if (ev0) CU(ctx, cudaEventRecord(ev0, s));
+    if (n_reads) {
+        k_paf_names<<<grid_for(n_reads, 256, kNumSMs * 8), 256, 0, s>>>(R.table, n_reads, R.words.as<unsigned long long>() + W_DUP);
+        ctx->L.count++;
+        CU(ctx, cudaGetLastError());
+    }
+    if (ev1) CU(ctx, cudaEventRecord(ev1, s));
+    unsigned long long dup = ~0ull;
+    CU(ctx, cudaMemcpyAsync(&dup, R.words.as<unsigned long long>() + W_DUP, 8, cudaMemcpyDeviceToHost, s));
+    CU(ctx, cudaStreamSynchronize(s));
+    if (dup != ~0ull)
+        return fail(ctx, RALA_B200_ERR_ARG, "set_reads: reads %u and %u have the same name (which one name_to_id_ keeps is not pinned)",
+                    (unsigned) dup, (unsigned) (dup >> 32));
+    R.n_reads = n_reads;
+    R.name_bytes = blob;
+    R.have_names = true;
+    return RALA_B200_OK;
+}
 
 static int paf_set_names(rala_b200_ctx* ctx, PafReader& R, const char* names, const uint64_t* name_end, const uint32_t* read_len,
                          uint32_t n_reads) {
@@ -403,40 +393,19 @@ static int paf_set_names(rala_b200_ctx* ctx, PafReader& R, const char* names, co
     }
     const uint64_t blob = n_reads ? name_end[n_reads - 1] : 0;
     if (blob && !names) return fail(ctx, RALA_B200_ERR_ARG, "set_reads: names are missing");
-    uint32_t slots = 1024;
-    while (slots < 2ull * n_reads) slots <<= 1;
-    const size_t o_end = align_up(blob + 1, 256), o_len = o_end + align_up((size_t) n_reads * 8 + 8, 256),
-                 o_slots = o_len + align_up((size_t) n_reads * 4 + 4, 256), bytes = o_slots + (size_t) slots * 8;
+    const NamesLayout L = names_layout(n_reads, blob);
     CU(ctx, cudaSetDevice(ctx->device));
-    CU(ctx, R.names.reserve(bytes));
-    CU(ctx, R.words.reserve(256));
+    CU(ctx, R.names.reserve(L.bytes));
     char* b = R.names.as<char>();
     cudaStream_t s = ctx->L.stream;
     if (blob) CU(ctx, cudaMemcpyAsync(b, names, blob, cudaMemcpyHostToDevice, s));
     if (n_reads) {
-        CU(ctx, cudaMemcpyAsync(b + o_end, name_end, (size_t) n_reads * 8, cudaMemcpyHostToDevice, s));
-        CU(ctx, cudaMemcpyAsync(b + o_len, read_len, (size_t) n_reads * 4, cudaMemcpyHostToDevice, s));
+        CU(ctx, cudaMemcpyAsync(b + L.o_end, name_end, (size_t) n_reads * 8, cudaMemcpyHostToDevice, s));
+        CU(ctx, cudaMemcpyAsync(b + L.o_len, read_len, (size_t) n_reads * 4, cudaMemcpyHostToDevice, s));
     }
-    CU(ctx, cudaMemsetAsync(b + o_slots, 0xFF, (size_t) slots * 8, s));
-    CU(ctx, cudaMemsetAsync(R.words.p, 0xFF, 8 * (W_DUP + 1), s));
-    R.table = NameTable{(const uint8_t*) b, (const unsigned long long*) (b + o_end), (const uint32_t*) (b + o_len),
-                        (unsigned long long*) (b + o_slots), slots - 1};
-    if (n_reads) {
-        k_paf_names<<<grid_for(n_reads, 256, kNumSMs * 8), 256, 0, s>>>(R.table, n_reads, R.words.as<unsigned long long>() + W_DUP);
-        ctx->L.count++;
-        CU(ctx, cudaGetLastError());
-    }
-    unsigned long long dup = ~0ull;
-    CU(ctx, cudaMemcpyAsync(&dup, R.words.as<unsigned long long>() + W_DUP, 8, cudaMemcpyDeviceToHost, s));
-    CU(ctx, cudaStreamSynchronize(s));
-    if (dup != ~0ull)
-        return fail(ctx, RALA_B200_ERR_ARG, "set_reads: reads %u and %u have the same name (which one name_to_id_ keeps is not pinned)",
-                    (unsigned) dup, (unsigned) (dup >> 32));
-    R.n_reads = n_reads;
     R.max_len = 0;
     for (uint32_t i = 0; i < n_reads; ++i) R.max_len = read_len[i] > R.max_len ? read_len[i] : R.max_len;
-    R.have_names = true;
-    return RALA_B200_OK;
+    return names_table(ctx, R, n_reads, blob);
 }
 
 static const char* text_error_text(uint32_t kind) {
@@ -453,25 +422,17 @@ struct TextStats {
     uint64_t n_records, n_unresolved, n_length_mismatch, first_length_mismatch, n_query_rc, n_bytes, n_chunks;
 };
 
-// Parses the whole text into R.cols (record index = line index, file order).  *n_out = records; kernel_ms (nullable) = device
-// time of the chunks' kernels (line scan + parse), uploads excluded.  The format decides the parse kernel, the shortest
-// valid line and the wording of refusals; upload, line scan and the call's words are the same for both.
-static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
-                            float* kernel_ms, uint64_t* n_out) {
+uint64_t text_max_chunks(uint64_t n_bytes) { return n_bytes ? 2 * (n_bytes / kPafChunk) + 2 : 0; }   // two consecutive chunks span >= one chunk size
+size_t text_status_words() { return tiles_of((uint64_t) kPafChunk + 1) + 1; }
+
+static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes,
+                            ChunkKernels kernels, void* self, float* kernel_ms, uint32_t* n_chunks) {
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->L.stream;
-    const bool mhap = fmt == kTextMhap;
-    const char* label = mhap ? "MHAP" : "PAF";
-    const char* field = mhap ? "field" : "column";
-    // no valid line is shorter than the format's minimum (the last one may lack its '\n'): more lines than that means a refusal
-    R.rec_cap = (n_bytes + 1) / (mhap ? kMinMhapLine : kMinPafLine) + 1;
-    if (R.rec_cap > (1ull << 31)) R.rec_cap = 1ull << 31;
-    const size_t col = align_up((size_t) R.rec_cap * 4, 256);
-    CU(ctx, R.cols.reserve(7 * col + align_up((size_t) R.rec_cap, 256)));
-    const uint64_t max_chunks = n_bytes ? 2 * (n_bytes / kPafChunk) + 2 : 0;   // two consecutive chunks span >= one chunk size
+    const uint64_t max_chunks = text_max_chunks(n_bytes);
     CU(ctx, R.words.reserve((W_BASES + max_chunks + 2) * 8));
     CU(ctx, R.line_end.reserve(((size_t) kPafChunk + 2) * 4));
-    const size_t status_words = tiles_of((uint64_t) kPafChunk + 1) + 1;
+    const size_t status_words = text_status_words();
     CU(ctx, R.status.reserve(status_words * 8));
     for (int k = 0; k < 2; ++k) {
         CU(ctx, R.text[k].reserve((size_t) kPafChunk + 1 + kPafPad));
@@ -497,7 +458,6 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, co
     CU(ctx, cudaMemsetAsync(words, 0xFF, 8 * W_UNRESOLVED, s));
     CU(ctx, cudaMemsetAsync(words + W_UNRESOLVED, 0, 8 * (W_BASES + 1 - W_UNRESOLVED), s));
     CU(ctx, cudaStreamSynchronize(s));   // the copy stream starts from settled words and buffers
-    const PafCols out = R.view();
     uint64_t pos = 0;
     uint32_t k = 0;
     for (; pos < n_bytes; ++k) {
@@ -538,14 +498,9 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, co
         k_paf_line_ends<<<grid_for(scan_len, kScanTile, kNumSMs * 8), kTileThreads, 0, s>>>(
             (const uint8_t*) dtext, scan_len, R.line_end.as<uint32_t>(), st_words + 1, (uint32_t*) st_words, words + W_BASES, k);
         ctx->L.count++;
-        if (mhap)
-            k_mhap_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
-                (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table.read_len, R.n_reads, out, R.rec_cap, words);
-        else
-            k_paf_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
-                (const uint8_t*) dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table, out, R.rec_cap, words);
-        ctx->L.count++;
         CU(ctx, cudaGetLastError());
+        const int rc = kernels(self, ctx, k, (const uint8_t*) dtext, scan_len);
+        if (rc) return rc;
         CU(ctx, cudaEventRecord(R.timing[2 * k + 1], s));
         CU(ctx, cudaEventRecord(R.parsed[slot], s));
         pos += len;
@@ -561,6 +516,61 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, co
             *kernel_ms += ms;
         }
     }
+    *n_chunks = k;
+    return RALA_B200_OK;
+}
+
+// A refused call returns with no upload in flight: the caller may free its text at once.
+int text_chunks(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, ChunkKernels kernels,
+                void* self, float* kernel_ms, uint32_t* n_chunks) {
+    const int rc = text_chunks_once(ctx, R, label, text, n_bytes, kernels, self, kernel_ms, n_chunks);
+    if (rc) {
+        if (R.copy) cudaStreamSynchronize(R.copy);
+        cudaStreamSynchronize(ctx->L.stream);
+    }
+    return rc;
+}
+
+// the parse kernel of one PAF or MHAP chunk (ChunkKernels)
+struct OverlapChunk {
+    PafReader* R;
+    bool mhap;
+};
+
+static int overlap_chunk(void* self, rala_b200_ctx* ctx, uint32_t k, const uint8_t* dtext, uint32_t scan_len) {
+    const OverlapChunk& c = *static_cast<const OverlapChunk*>(self);
+    PafReader& R = *c.R;
+    unsigned long long* words = R.words.as<unsigned long long>();
+    cudaStream_t s = ctx->L.stream;
+    if (c.mhap)
+        k_mhap_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
+            dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table.read_len, R.n_reads, R.view(), R.rec_cap, words);
+    else
+        k_paf_parse<<<grid_for(scan_len, kTileWarps * 64, kNumSMs * 8), 256, 0, s>>>(
+            dtext, R.line_end.as<uint32_t>(), words + W_BASES, k, R.table, R.view(), R.rec_cap, words);
+    ctx->L.count++;
+    CU(ctx, cudaGetLastError());
+    return RALA_B200_OK;
+}
+
+// Parses the whole text into R.cols (record index = line index, file order).  *n_out = records; kernel_ms (nullable) = device
+// time of the chunks' kernels (line scan + parse), uploads excluded.  The format decides the parse kernel, the shortest
+// valid line and the wording of refusals; upload, line scan and the call's words are the same for both.
+static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
+                      float* kernel_ms, uint64_t* n_out) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    const bool mhap = fmt == kTextMhap;
+    const char* label = mhap ? "MHAP" : "PAF";
+    const char* field = mhap ? "field" : "column";
+    // no valid line is shorter than the format's minimum (the last one may lack its '\n'): more lines than that means a refusal
+    R.rec_cap = (n_bytes + 1) / (mhap ? kMinMhapLine : kMinPafLine) + 1;
+    if (R.rec_cap > (1ull << 31)) R.rec_cap = 1ull << 31;
+    const size_t col = align_up((size_t) R.rec_cap * 4, 256);
+    CU(ctx, R.cols.reserve(7 * col + align_up((size_t) R.rec_cap, 256)));
+    OverlapChunk chunk{&R, mhap};
+    uint32_t k = 0;
+    const int rc = text_chunks(ctx, R, label, text, n_bytes, overlap_chunk, &chunk, kernel_ms, &k);
+    if (rc) return rc;
     if (R.w[W_ERR] != ~0ull) {
         const uint32_t code = (uint32_t) (R.w[W_ERR] & 0xFF), kind = code >> 4, column = code & 15;
         const unsigned long long line = (R.w[W_ERR] >> 8) + 1;
@@ -581,17 +591,6 @@ static int paf_parse_chunks(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, co
     st->n_chunks = k;
     *n_out = n;
     return RALA_B200_OK;
-}
-
-// A refused call returns with no upload in flight: the caller may free its text at once.
-static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
-                      float* kernel_ms, uint64_t* n_out) {
-    const int rc = paf_parse_chunks(ctx, R, fmt, text, n_bytes, st, kernel_ms, n_out);
-    if (rc) {
-        if (R.copy) cudaStreamSynchronize(R.copy);
-        cudaStreamSynchronize(ctx->L.stream);
-    }
-    return rc;
 }
 
 extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, const uint64_t* name_end, const uint32_t* read_len,

@@ -154,7 +154,7 @@ struct rala_b200_graph {
     // rala_b200_graph_run as a replayed CUDA graph (see run_key / RunGraph below)
     bool use_cuda_graph = true, capturing = false;
     struct RunGraph* run_graphs = nullptr;   // two cached instances: first run after set_piles / repeated run
-    struct PafReader* paf = nullptr;         // read-name table and text upload buffers (paf.cu), from the first set_reads
+    struct PafReader* paf = nullptr;         // read-name table and text upload buffers (paf.cu), from the first set_reads*
     TextFormat text_records = kTextNone;     // the records came from set_overlaps_paf / _mhap: its parsed columns are still there
     struct PileBuilder* pile_builder = nullptr;   // event, sort and run buffers of build_piles (piles.cu)
 
@@ -238,7 +238,79 @@ int end_build(rala_b200_graph* g);
 int transitive_stage(rala_b200_graph* g, const GraphArrays& ga, const uint32_t* node_range);
 int marks_stage(rala_b200_graph* g, const GraphArrays& ga, uint8_t* copy /* nullable */, uint32_t copy_cap);
 
-// ---- paf.cu ----------------------------------------------------------------------------------------------------
+// ---- paf.cu: the read names and the chunked text upload, shared by the overlap readers and reads.cu --------------
+// device name table: name i = blob[end[i-1], end[i]), slots = open addressing by name hash (k_paf_names)
+struct NameTable {
+    const uint8_t* blob;
+    const unsigned long long* end;   // name i = blob[end[i-1], end[i])
+    const uint32_t* read_len;
+    unsigned long long* slots;       // hash >> 32 << 32 | id, ~0 = empty
+    uint32_t mask;
+};
+
+struct PafCols {
+    uint32_t *a, *b, *ab, *ae, *bb, *be, *len;
+    uint8_t* mismatch;
+};
+
+// device words of one text call: the first four start at ~0 (minima), the rest at 0; line bases of the chunks follow
+enum { W_ERR = 0, W_DUP, W_FIRST_MISMATCH, W_FIRST_BAD, W_UNRESOLVED, W_MISMATCH, W_QUERY_RC, W_BASES = 8 };
+
+struct PafReader {
+    DevBuf names;                 // blob | ends | read lengths | table slots (NamesLayout)
+    NameTable table{};
+    uint32_t n_reads = 0, max_len = 0;
+    uint64_t name_bytes = 0;
+    bool have_names = false;
+    DevBuf text[2];               // device side of the staging pair
+    DevBuf line_end, status, words, cols, valid;
+    char* pinned[2] = {nullptr, nullptr};
+    cudaStream_t copy = nullptr;  // uploads: chunk k + 1 crosses PCIe while chunk k is parsed
+    cudaEvent_t copied[2]{}, parsed[2]{};
+    std::vector<cudaEvent_t> timing;   // (start, stop) around the kernels of every chunk
+    unsigned long long rec_cap = 0;
+    std::vector<unsigned long long> w;   // the words of the last call, read back
+
+    PafCols view() const {
+        const size_t col = align_up((size_t) rec_cap * 4, 256);
+        char* b = cols.as<char>();
+        return PafCols{(uint32_t*) b, (uint32_t*) (b + col), (uint32_t*) (b + 2 * col), (uint32_t*) (b + 3 * col),
+                       (uint32_t*) (b + 4 * col), (uint32_t*) (b + 5 * col), (uint32_t*) (b + 6 * col), (uint8_t*) (b + 7 * col)};
+    }
+    ~PafReader() {
+        if (copy) cudaStreamSynchronize(copy);
+        DevBuf* bufs[] = {&names, &text[0], &text[1], &line_end, &status, &words, &cols, &valid};
+        for (DevBuf* b : bufs) b->release();
+        for (int k = 0; k < 2; ++k) {
+            if (pinned[k]) cudaFreeHost(pinned[k]);
+            if (copied[k]) cudaEventDestroy(copied[k]);
+            if (parsed[k]) cudaEventDestroy(parsed[k]);
+        }
+        for (cudaEvent_t e : timing) cudaEventDestroy(e);
+        if (copy) cudaStreamDestroy(copy);
+    }
+};
+
+// byte offsets of the read names in PafReader::names for n reads with `blob` name bytes
+struct NamesLayout {
+    size_t o_end, o_len, o_slots, bytes;
+    uint32_t slots;
+};
+NamesLayout names_layout(uint32_t n_reads, uint64_t blob);
+// R.names holds the names, ends and lengths of n_reads reads in names_layout(n_reads, blob) and R.max_len is set: builds
+// the name table (k_paf_names; ev0 / ev1 nullable, recorded around it) and refuses a name listed twice
+int names_table(rala_b200_ctx* ctx, PafReader& R, uint32_t n_reads, uint64_t blob, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr);
+// the launches of one upload chunk k after its line scan: text (scan_len bytes, ends in '\n') at dtext, its line ends in
+// R.line_end, the lines before it at words[W_BASES + k] and behind it at words[W_BASES + k + 1]
+typedef int (*ChunkKernels)(void* self, rala_b200_ctx* ctx, uint32_t k, const uint8_t* dtext, uint32_t scan_len);
+uint64_t text_max_chunks(uint64_t n_bytes);
+size_t text_status_words();
+// The whole text through the pinned staging pair (page-locked caller memory in place) in chunks of
+// RALA_B200_PAF_CHUNK_BYTES cut behind their last '\n', each one line-scanned and handed to `kernels`; R.w holds the
+// call's words afterwards (W_BASES + *n_chunks = lines).  W_ERR .. W_FIRST_BAD start at ~0, the rest at 0.
+// kernel_ms (nullable) = device time of the chunks' kernels.  A refused call returns with no upload in flight.
+int text_chunks(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, ChunkKernels kernels,
+                void* self, float* kernel_ms, uint32_t* n_chunks);
 void destroy_paf_reader(PafReader* r);
 // the overlap columns build_piles counts: the parsed records of the last successful set_overlaps_paf / _mhap, before the
 // duplicate filter was folded in (bit 31 of a = unresolved name), and the reads' lengths (device); returns the text format
