@@ -327,6 +327,47 @@ int rala_b200_graph_set_overlaps_paf(rala_b200_graph* g, const char* text, uint6
  * are numbers).  A record that stays valid while field 8 or 12 differs from set_reads' length is refused, naming its line.
  * After a refused call the session holds no records.  stats: nullable. */
 int rala_b200_graph_set_overlaps_mhap(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_mhap_stats_t* stats);
+/* BGZF input: the readers above on a BGZF file (htslib's bgzip output, the usual form of indexed FASTA / FASTQ), inflated on
+ * the device.  BGZF contract: the input is a series of gzip members, each with ID1 ID2 CM = 1f 8b 08, FLG = FEXTRA only,
+ * and a `BC` extra subfield of SLEN 2 (other subfields may stand before or after it) holding BSIZE - 1, the member's
+ * size; the members tile the input exactly; each member's trailer holds the CRC32 and ISIZE <= 65536 of its raw DEFLATE
+ * stream (RFC 1951: stored, fixed and dynamic Huffman blocks), which is decoded on its own (no distance reaches into the
+ * member before it).  Empty members and the end-of-file marker may stand anywhere.  The text is the concatenation of the
+ * inflated members.  Refusals (RALA_B200_ERR_ARG unless noted), all worded "BGZF block N (byte offset O): <reason>" with N
+ * the 0-based member and O its first byte; the smallest failing member is reported:
+ *   - the input ends inside a member header; the magic is not 1f 8b 08;
+ *   - a member without a BC subfield, e.g. plain `gzip` output: "the gzip member has no BC extra subfield: the input is
+ *     not BGZF (blocked gzip); compress it with bgzip";
+ *   - header flags other than FEXTRA; BSIZE smaller than the header and trailer, or past the end of the input;
+ *     ISIZE above 65536;
+ *   - in the DEFLATE stream: reading past BSIZE; BTYPE 3; a stored block whose LEN is not ~NLEN; more than 286
+ *     literal/length or 30 distance codes; an over-subscribed or incomplete code (one code of length 1 is accepted); a bad
+ *     code-length repeat; no end-of-block code; literal/length symbol 286 / 287 or a code not in the code; distance code
+ *     30 / 31 or a code not in the code; a distance before the start of the member; more or fewer bytes than ISIZE;
+ *     bytes between the end of the stream and the trailer; a CRC32 that differs from the trailer's.
+ * An inflated text of 2^34 bytes or more is refused with RALA_B200_ERR_LIMIT from the headers, before any upload.  The
+ * inflated text is then read exactly as the plain call reads the same text: the same chunks (RALA_B200_PAF_CHUNK_BYTES
+ * cut behind their last '\n', found on the device), the same stats (n_bytes = inflated bytes; device_ms of the reads
+ * stats covers the reader's kernels only), the same refusals with the same line and column, the same session afterwards.
+ * Device memory kept by the session after a _bgzf call, beside the plain reader's: the compressed input, the block table
+ * (40 B per member) and the inflated text, each grown to the largest call so far and freed with the session.
+ * rala_b200_inflate_bgzf is stateless: with out == NULL it only walks the headers and fills stats (inflate_ms 0);
+ * otherwise out receives the inflated bytes (cap smaller than the text: RALA_B200_ERR_ARG before any upload) and the
+ * device memory is freed before it returns.  stats / bgzf: nullable, filled when the call succeeds. */
+typedef struct {
+    uint64_t n_blocks;        /* BGZF members, empty ones and the end-of-file marker included */
+    uint64_t n_compressed;    /* input bytes */
+    uint64_t n_bytes;         /* inflated bytes = the text the reader parsed */
+    float inflate_ms;         /* device time of the inflate + CRC kernels; uploads excluded */
+} rala_b200_bgzf_stats_t;
+int rala_b200_inflate_bgzf(rala_b200_ctx* ctx, const uint8_t* data, uint64_t n, uint8_t* out, uint64_t cap,
+                           rala_b200_bgzf_stats_t* stats);
+int rala_b200_graph_set_reads_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_reads_stats_t* stats,
+                                   rala_b200_bgzf_stats_t* bgzf);
+int rala_b200_graph_set_overlaps_paf_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_paf_stats_t* stats,
+                                          rala_b200_bgzf_stats_t* bgzf);
+int rala_b200_graph_set_overlaps_mhap_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_mhap_stats_t* stats,
+                                           rala_b200_bgzf_stats_t* bgzf);
 /* The pile table of the reads given to set_reads, built on the device (rule and refusals as rala_b200_build_piles) from
  * the records of the last successful set_overlaps_paf or set_overlaps_mhap, counted as parsed: before the duplicate
  * filter.  A refused record is named by its line in that text ("PAF line N" / "MHAP line N").  It is installed as

@@ -66,6 +66,13 @@ class ReadsStats(C.Structure):
         return {k: (float(getattr(self, k)) if k == "device_ms" else int(getattr(self, k))) for k, _ in self._fields_}
 
 
+class BgzfStats(C.Structure):
+    _fields_ = [("n_blocks", C.c_uint64), ("n_compressed", C.c_uint64), ("n_bytes", C.c_uint64), ("inflate_ms", C.c_float)]
+
+    def as_dict(self):
+        return {k: (float(getattr(self, k)) if k == "inflate_ms" else int(getattr(self, k))) for k, _ in self._fields_}
+
+
 PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES (the MHAP reader uses the same chunks)
 
 
@@ -122,7 +129,8 @@ EXPORTS = [
     "rala_b200_graph_get_marked", "rala_b200_graph_stage_ms", "rala_b200_graph_set_kept_overlaps",
     "rala_b200_graph_use_cuda_graph", "rala_b200_graph_set_overlaps_columns", "rala_b200_graph_set_outputs",
     "rala_b200_graph_set_overlaps_packed", "rala_b200_multi_set_overlaps_packed", "rala_b200_graph_get_adjacency",
-    "rala_b200_graph_get_csr",
+    "rala_b200_graph_get_csr", "rala_b200_inflate_bgzf", "rala_b200_graph_set_reads_bgzf", "rala_b200_graph_set_overlaps_paf_bgzf",
+    "rala_b200_graph_set_overlaps_mhap_bgzf",
     # multi-GPU phases
     "rala_b200_create_on_stream", "rala_b200_graph_set_shard", "rala_b200_graph_phase_events",
     "rala_b200_graph_phase_resolve", "rala_b200_graph_phase_survivors", "rala_b200_graph_phase_emit_edges",
@@ -360,6 +368,18 @@ class Context:
         out = np.ascontiguousarray(cols[:, :stats["n_records"]])
         return (out, stats, float(ms.value)) if with_time else (out, stats)
 
+    def inflate_bgzf(self, data) -> tuple:
+        """A BGZF file (bytes, uint8 array or pinned CPU tensor) inflated on the device -> (text as a uint8 array, stats dict:
+        blocks, compressed bytes, inflated bytes, inflate_ms)."""
+        buf, n = _text(data)
+        st = BgzfStats()
+        self.check(self.lib.rala_b200_inflate_bgzf(self.handle, _ptr(buf), C.c_uint64(n), None, C.c_uint64(0), C.byref(st)),
+                   "inflate_bgzf")
+        out = np.zeros(max(int(st.n_bytes), 1), np.uint8)
+        self.check(self.lib.rala_b200_inflate_bgzf(self.handle, _ptr(buf), C.c_uint64(n), _ptr(out), C.c_uint64(int(st.n_bytes)),
+                                                   C.byref(st)), "inflate_bgzf")
+        return out[:int(st.n_bytes)], st.as_dict()
+
     def build_piles(self, columns, read_len, with_time: bool = False):
         """Graph::initialize's coverage half on the device: six host columns in the set_overlaps_columns layout (bit 31 of
         a_id = unresolved record; records the duplicate filter drops still count) + the read lengths -> (piles (n_reads, 2)
@@ -457,6 +477,14 @@ class Graph:
         self._n_reads = int(st.n_reads)
         return st.as_dict()
 
+    def set_reads_bgzf(self, data) -> tuple:
+        """set_reads_text on a BGZF file, inflated on the device -> (reads stats dict, BGZF stats dict)."""
+        buf, n = _text(data)
+        st, z = ReadsStats(), BgzfStats()
+        self._call("rala_b200_graph_set_reads_bgzf", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        self._n_reads = int(st.n_reads)
+        return st.as_dict(), z.as_dict()
+
     def reads(self):
         """The session's reads as set_reads holds them: (names blob uint8, name_end uint64, read_len uint32)."""
         n, nb = C.c_uint32(0), C.c_uint64(0)
@@ -482,6 +510,20 @@ class Graph:
         st = MhapStats()
         self._call("rala_b200_graph_set_overlaps_mhap", _ptr(buf), C.c_uint64(n_bytes), C.byref(st))
         return st.as_dict()
+
+    def set_overlaps_paf_bgzf(self, data) -> tuple:
+        """set_overlaps_paf on a BGZF file, inflated on the device -> (PAF stats dict, BGZF stats dict)."""
+        buf, n = _text(data)
+        st, z = PafStats(), BgzfStats()
+        self._call("rala_b200_graph_set_overlaps_paf_bgzf", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        return st.as_dict(), z.as_dict()
+
+    def set_overlaps_mhap_bgzf(self, data) -> tuple:
+        """set_overlaps_mhap on a BGZF file, inflated on the device -> (MHAP stats dict, BGZF stats dict)."""
+        buf, n = _text(data)
+        st, z = MhapStats(), BgzfStats()
+        self._call("rala_b200_graph_set_overlaps_mhap_bgzf", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        return st.as_dict(), z.as_dict()
 
     def build_piles(self) -> dict:
         """The pile table from the records of the last set_overlaps_paf / _mhap, built on the device and installed as

@@ -425,7 +425,7 @@ struct TextStats {
 uint64_t text_max_chunks(uint64_t n_bytes) { return n_bytes ? 2 * (n_bytes / kPafChunk) + 2 : 0; }   // two consecutive chunks span >= one chunk size
 size_t text_status_words() { return tiles_of((uint64_t) kPafChunk + 1) + 1; }
 
-static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes,
+static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, bool on_device,
                             ChunkKernels kernels, void* self, float* kernel_ms, uint32_t* n_chunks) {
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->L.stream;
@@ -447,17 +447,20 @@ static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label,
     }
     // caller memory that is page-locked is uploaded in place; anything else goes through the pinned staging pair
     bool direct = false;
-    if (n_bytes) {
+    if (n_bytes && !on_device) {
         cudaPointerAttributes attr;
         if (cudaPointerGetAttributes(&attr, text) == cudaSuccess) direct = attr.type == cudaMemoryTypeHost;
         cudaGetLastError();
     }
-    for (int k = 0; !direct && n_bytes && k < 2; ++k)
+    for (int k = 0; !direct && !on_device && n_bytes && k < 2; ++k)
         if (!R.pinned[k]) CU(ctx, cudaHostAlloc((void**) &R.pinned[k], kPafChunk + 1, cudaHostAllocDefault));
     unsigned long long* words = R.words.as<unsigned long long>();
     CU(ctx, cudaMemsetAsync(words, 0xFF, 8 * W_UNRESOLVED, s));
     CU(ctx, cudaMemsetAsync(words + W_UNRESOLVED, 0, 8 * (W_BASES + 1 - W_UNRESOLVED), s));
+    char tail = '\n';   // the text's last byte
+    if (n_bytes && on_device) CU(ctx, cudaMemcpyAsync(&tail, text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, s));
     CU(ctx, cudaStreamSynchronize(s));   // the copy stream starts from settled words and buffers
+    if (n_bytes && !on_device) tail = text[n_bytes - 1];
     uint64_t pos = 0;
     uint32_t k = 0;
     for (; pos < n_bytes; ++k) {
@@ -465,28 +468,36 @@ static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label,
         uint64_t len = n_bytes - pos < kPafChunk ? n_bytes - pos : kPafChunk;
         const bool last = pos + len == n_bytes;
         if (!last) {   // cut behind the last '\n' of the window; the tail goes with the next chunk
-            const void* nl = memrchr(text + pos, '\n', len);
-            if (!nl) {
+            uint64_t cut = 0;   // bytes up to and with the last '\n' of the window, 0 when there is none
+            if (on_device) {
+                const int rc = bgzf_text_cut(ctx, R, (const uint8_t*) text, pos, pos + len, &cut);
+                if (rc) return rc;
+                cut = cut ? cut - pos : 0;
+            } else {
+                const void* nl = memrchr(text + pos, '\n', len);
+                cut = nl ? (uint64_t) ((const char*) nl - (text + pos)) + 1 : 0;
+            }
+            if (!cut) {
                 unsigned long long lines = 0;
                 CU(ctx, cudaStreamSynchronize(R.copy));
                 CU(ctx, cudaMemcpyAsync(&lines, words + W_BASES + k, 8, cudaMemcpyDeviceToHost, s));
                 CU(ctx, cudaStreamSynchronize(s));
                 return fail(ctx, RALA_B200_ERR_LIMIT, "%s line %llu is longer than the upload chunk (%u bytes)", label, lines + 1, kPafChunk);
             }
-            len = (uint64_t) ((const char*) nl - (text + pos)) + 1;
+            len = cut;
         }
         const int slot = k & 1;
         const char* src = text + pos;
-        if (!direct) {
+        if (!direct && !on_device) {
             if (k >= 2) CU(ctx, cudaEventSynchronize(R.copied[slot]));   // the upload of chunk k - 2 has left the buffer
             memcpy(R.pinned[slot], src, len);
             src = R.pinned[slot];
         }
         if (k >= 2) CU(ctx, cudaStreamWaitEvent(R.copy, R.parsed[slot], 0));   // chunk k - 2 is parsed: its device buffer is free
         char* dtext = R.text[slot].as<char>();
-        CU(ctx, cudaMemcpyAsync(dtext, src, len, cudaMemcpyHostToDevice, R.copy));
+        CU(ctx, cudaMemcpyAsync(dtext, src, len, on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, R.copy));
         uint32_t scan_len = (uint32_t) len;
-        if (last && text[n_bytes - 1] != '\n') {   // the final line without its '\n'
+        if (last && tail != '\n') {   // the final line without its '\n'
             CU(ctx, cudaMemsetAsync(dtext + len, '\n', 1, R.copy));
             ++scan_len;
         }
@@ -521,9 +532,9 @@ static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label,
 }
 
 // A refused call returns with no upload in flight: the caller may free its text at once.
-int text_chunks(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, ChunkKernels kernels,
-                void* self, float* kernel_ms, uint32_t* n_chunks) {
-    const int rc = text_chunks_once(ctx, R, label, text, n_bytes, kernels, self, kernel_ms, n_chunks);
+int text_chunks(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, bool on_device,
+                ChunkKernels kernels, void* self, float* kernel_ms, uint32_t* n_chunks) {
+    const int rc = text_chunks_once(ctx, R, label, text, n_bytes, on_device, kernels, self, kernel_ms, n_chunks);
     if (rc) {
         if (R.copy) cudaStreamSynchronize(R.copy);
         cudaStreamSynchronize(ctx->L.stream);
@@ -556,8 +567,8 @@ static int overlap_chunk(void* self, rala_b200_ctx* ctx, uint32_t k, const uint8
 // Parses the whole text into R.cols (record index = line index, file order).  *n_out = records; kernel_ms (nullable) = device
 // time of the chunks' kernels (line scan + parse), uploads excluded.  The format decides the parse kernel, the shortest
 // valid line and the wording of refusals; upload, line scan and the call's words are the same for both.
-static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st,
-                      float* kernel_ms, uint64_t* n_out) {
+static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const char* text, uint64_t n_bytes, bool on_device,
+                      TextStats* st, float* kernel_ms, uint64_t* n_out) {
     CU(ctx, cudaSetDevice(ctx->device));
     const bool mhap = fmt == kTextMhap;
     const char* label = mhap ? "MHAP" : "PAF";
@@ -569,7 +580,7 @@ static int text_parse(rala_b200_ctx* ctx, PafReader& R, TextFormat fmt, const ch
     CU(ctx, R.cols.reserve(7 * col + align_up((size_t) R.rec_cap, 256)));
     OverlapChunk chunk{&R, mhap};
     uint32_t k = 0;
-    const int rc = text_chunks(ctx, R, label, text, n_bytes, overlap_chunk, &chunk, kernel_ms, &k);
+    const int rc = text_chunks(ctx, R, label, text, n_bytes, on_device, overlap_chunk, &chunk, kernel_ms, &k);
     if (rc) return rc;
     if (R.w[W_ERR] != ~0ull) {
         const uint32_t code = (uint32_t) (R.w[W_ERR] & 0xFF), kind = code >> 4, column = code & 15;
@@ -603,7 +614,9 @@ extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, 
 
 // Text in file order -> the session's records: parse, duplicate filter, INVALID bit folded in.  *counted = *st holds the
 // call's counts (also when a read-length refusal follows).
-static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st, bool* counted) {
+// bgzf (nullable): text[0, n_bytes) is a BGZF file, inflated on the device first; *bgzf receives its stats.
+static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st, bool* counted,
+                             rala_b200_bgzf_stats_t* bgzf = nullptr) {
     if (!g || (n_bytes && !text)) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     const bool mhap = fmt == kTextMhap;
@@ -614,8 +627,15 @@ static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* tex
     g->n_rec = 0;
     g->state = SS_EMPTY;
     g->text_records = kTextNone;
+    int rc;
+    if (bgzf) {
+        rc = bgzf_inflate(ctx, R, (const uint8_t*) text, n_bytes, bgzf);
+        if (rc) return rc;
+        text = R.bgzf_text.as<const char>();
+        n_bytes = bgzf->n_bytes;
+    }
     uint64_t n = 0;
-    int rc = text_parse(ctx, R, fmt, text, n_bytes, st, nullptr, &n);
+    rc = text_parse(ctx, R, fmt, text, n_bytes, bgzf != nullptr, st, nullptr, &n);
     if (rc) return rc;
     rc = reserve_for_records(g, n);
     if (rc) return rc;
@@ -668,6 +688,28 @@ extern "C" int rala_b200_graph_set_overlaps_mhap(rala_b200_graph* g, const char*
     return rc;
 }
 
+extern "C" int rala_b200_graph_set_overlaps_paf_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_paf_stats_t* stats,
+                                                     rala_b200_bgzf_stats_t* bgzf) {
+    TextStats st{};
+    rala_b200_bgzf_stats_t z{};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextPaf, (const char*) data, n, &st, &counted, &z);
+    if (stats && counted) paf_stats_of(st, stats);
+    if (bgzf && counted) *bgzf = z;
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_overlaps_mhap_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_mhap_stats_t* stats,
+                                                      rala_b200_bgzf_stats_t* bgzf) {
+    TextStats st{};
+    rala_b200_bgzf_stats_t z{};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextMhap, (const char*) data, n, &st, &counted, &z);
+    if (stats && counted) mhap_stats_of(st, stats);
+    if (bgzf && counted) *bgzf = z;
+    return rc;
+}
+
 TextFormat text_records_view(const rala_b200_graph* g, PileCols* cols, const uint32_t** read_len, uint32_t* n_reads, uint32_t* max_len) {
     if (g->text_records == kTextNone || !g->paf || !g->paf->have_names) return kTextNone;
     const PafCols c = g->paf->view();
@@ -701,7 +743,7 @@ extern "C" int rala_b200_parse_paf(rala_b200_ctx* ctx, const char* names, const 
     if (rc) return rc;
     uint64_t n = 0;
     TextStats st{};
-    rc = text_parse(ctx, R, kTextPaf, text, n_bytes, &st, device_ms, &n);
+    rc = text_parse(ctx, R, kTextPaf, text, n_bytes, false, &st, device_ms, &n);
     if (rc) return rc;
     paf_stats_of(st, stats);
     return download_columns(ctx, R, "parse_paf", n, cols_out, cap);
@@ -720,7 +762,7 @@ extern "C" int rala_b200_parse_mhap(rala_b200_ctx* ctx, const uint32_t* read_len
     R.n_reads = n_reads;
     uint64_t n = 0;
     TextStats st{};
-    int rc = text_parse(ctx, R, kTextMhap, text, n_bytes, &st, device_ms, &n);
+    int rc = text_parse(ctx, R, kTextMhap, text, n_bytes, false, &st, device_ms, &n);
     if (rc) return rc;
     mhap_stats_of(st, stats);
     return download_columns(ctx, R, "parse_mhap", n, cols_out, cap);

@@ -329,24 +329,37 @@ static const char* reads_error_text(uint32_t kind) {
     }
 }
 
-static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_reads_stats_t* st) {
+// bgzf (nullable): text[0, n_bytes) is a BGZF file, inflated on the device first; *bgzf receives its stats.
+static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_reads_stats_t* st,
+                      rala_b200_bgzf_stats_t* bgzf = nullptr) {
     rala_b200_ctx* ctx = g->ctx;
     if (!g->paf) g->paf = new PafReader();
     PafReader& R = *g->paf;
     R.have_names = false;
     g->text_records = kTextNone;   // the records' ids refer to the reads they were parsed against
     *st = rala_b200_reads_stats_t{};
-    st->n_bytes = n_bytes;
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->L.stream;
+    char first = n_bytes ? text[0] : 0;
+    if (bgzf) {
+        const int rc = bgzf_inflate(ctx, R, (const uint8_t*) text, n_bytes, bgzf);
+        if (rc) return rc;
+        text = R.bgzf_text.as<const char>();
+        n_bytes = bgzf->n_bytes;
+        if (n_bytes) {
+            CU(ctx, cudaMemcpyAsync(&first, text, 1, cudaMemcpyDeviceToHost, s));
+            CU(ctx, cudaStreamSynchronize(s));
+        }
+    }
+    st->n_bytes = n_bytes;
     if (n_bytes == 0) {   // no reads, as set_reads with n_reads = 0
         R.max_len = 0;
         CU(ctx, R.names.reserve(names_layout(0, 0).bytes));
         return names_table(ctx, R, 0, 0);
     }
-    if (text[0] != '>' && text[0] != '@')
+    if (first != '>' && first != '@')
         return fail(ctx, RALA_B200_ERR_ARG, "FASTA / FASTQ line 1, column 1: %s", reads_error_text(kRdFormat));
-    const bool fastq = text[0] == '@';
+    const bool fastq = first == '@';
     const char* label = fastq ? "FASTQ" : "FASTA";
     if (n_bytes >> 34) return fail(ctx, RALA_B200_ERR_LIMIT, "%s text of %llu bytes: 2^34 or more", label, (unsigned long long) n_bytes);
     ReadsCall c;
@@ -360,7 +373,7 @@ static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, ra
     for (cudaEvent_t& e : c.ev) CU(ctx, cudaEventCreate(&e));
     float ms = 0.f, part = 0.f;
     uint32_t k = 0;
-    int rc = text_chunks(ctx, R, label, text, n_bytes, reads_chunk, &c, &ms, &k);
+    int rc = text_chunks(ctx, R, label, text, n_bytes, bgzf != nullptr, reads_chunk, &c, &ms, &k);
     if (rc) return rc;
     // text_chunks ended with the stream synchronised: c.host holds the totals behind the last chunk
     const unsigned long long n_lines = R.w[W_BASES + k], n_reads = c.host[0], blob = c.host[1];
@@ -413,6 +426,17 @@ extern "C" int rala_b200_graph_set_reads_text(rala_b200_graph* g, const char* te
     rala_b200_reads_stats_t st;
     const int rc = reads_text(g, text, n_bytes, &st);
     if (stats && !rc) *stats = st;
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_reads_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_reads_stats_t* stats,
+                                               rala_b200_bgzf_stats_t* bgzf) {
+    if (!g || (n && !data)) return RALA_B200_ERR_ARG;
+    rala_b200_reads_stats_t st;
+    rala_b200_bgzf_stats_t z{};
+    const int rc = reads_text(g, (const char*) data, n, &st, &z);
+    if (stats && !rc) *stats = st;
+    if (bgzf && !rc) *bgzf = z;
     return rc;
 }
 

@@ -15,6 +15,8 @@ the reference's duplicate filter assumes (/root/reference/src/graph.cpp:343-350)
 """
 from __future__ import annotations
 
+import struct
+import zlib
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -405,3 +407,28 @@ def generate_duplicate_groups(n_reads: int = 300, n_groups: int = 500, max_group
             L.append(base + int(rng.integers(0, 4)))   # few distinct lengths: ties are common
     return DuplicateGroups(read_len, np.asarray(A, np.int64), np.asarray(B, np.int64), np.asarray(C, np.uint32),
                            np.asarray(O, np.uint8), np.asarray(L, np.uint32))
+
+
+BGZF_BLOCK = 65280   # input bytes per block, as htslib's bgzip cuts them (the compressed block then fits the 16-bit BSIZE)
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+def bgzf_block(data: bytes, level: int = 6, strategy: int = zlib.Z_DEFAULT_STRATEGY) -> bytes:
+    """One BGZF member: raw DEFLATE of `data` (<= 65536 bytes) with the BC subfield, CRC32 and ISIZE."""
+    c = zlib.compressobj(level, zlib.DEFLATED, -15, 8, strategy)
+    z = c.compress(data) + c.flush()
+    if len(z) + 26 > 65536:
+        raise ValueError(f"a block of {len(data)} bytes compresses to {len(z)}: BSIZE would not fit 16 bits")
+    head = b"\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00" + struct.pack("<H", len(z) + 25)
+    return head + z + struct.pack("<II", zlib.crc32(data), len(data))
+
+
+def write_bgzf(text, level: int = 6, strategy: int = zlib.Z_DEFAULT_STRATEGY, cuts=None) -> bytes:
+    """`text` as BGZF (what `bgzip` writes): blocks of at most BGZF_BLOCK input bytes, or cut at the offsets `cuts`
+    (ascending, each block <= 65536 bytes), raw DEFLATE from zlib.compressobj(level, DEFLATED, -15, 8, strategy), the
+    28-byte end-of-file marker at the end.  Blocks are independent, so a caller may compress them in a process pool."""
+    text = bytes(text)
+    bounds = list(range(0, len(text), BGZF_BLOCK)) if cuts is None else [0] + [int(c) for c in cuts]
+    bounds.append(len(text))
+    out = [bgzf_block(text[a:b], level, strategy) for a, b in zip(bounds[:-1], bounds[1:]) if b > a or cuts is not None]
+    return b"".join(out) + BGZF_EOF
