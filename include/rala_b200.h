@@ -368,6 +368,47 @@ int rala_b200_graph_set_overlaps_paf_bgzf(rala_b200_graph* g, const uint8_t* dat
                                           rala_b200_bgzf_stats_t* bgzf);
 int rala_b200_graph_set_overlaps_mhap_bgzf(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_mhap_stats_t* stats,
                                            rala_b200_bgzf_stats_t* bgzf);
+/* Plain gzip input (what gzip, pigz and `cat a.gz b.gz` write), inflated on the device.  The input is one or more gzip
+ * members (RFC 1952): header 1f 8b 08 with FTEXT / FHCRC / FEXTRA / FNAME / FCOMMENT (FHCRC checked, reserved flags
+ * refused), a raw DEFLATE stream whose distances never reach before the member's start, then CRC32 and ISIZE (mod 2^32),
+ * both checked.  Zero bytes between and after members are skipped, as gzip.decompress does; the empty input is the empty
+ * text.  An input that is BGZF throughout (the BGZF header walk succeeds) takes the BGZF path (stats bgzf = 1).
+ * Refusals are RALA_B200_ERR_ARG, worded "gzip member M (byte offset O): <reason>" with M the 0-based member and O the
+ * failing header or trailer, or the first byte of the failing DEFLATE block; the error earliest in the stream is reported:
+ *   - bad magic or compression method; reserved flags; the input ends inside a header, a DEFLATE stream or a trailer;
+ *   - every DEFLATE refusal of the BGZF path; a distance before the member's start;
+ *   - header CRC; CRC32; ISIZE; non-zero bytes after the last member that start no member.
+ * An inflated text of 2^34 bytes or more: RALA_B200_ERR_LIMIT.  The BGZF path refuses as the _bgzf calls do.
+ * The stream is cut into chunks of chunk_bytes compressed bytes; each chunk's decode starts at the first block or member
+ * boundary the finder proposes inside it and is accepted only when the decode of the chunk before it stops exactly there
+ * (chunk 0 starts at the stream's start), so the output never depends on the finder being right.
+ * The readers' _gzip calls read the inflated text exactly as the _bgzf calls do.  Device memory kept by the session
+ * beside the BGZF path's: the per-chunk table, the decoded symbols of at most 1 GiB of text or of the longest chunk
+ * (2 bytes per byte) and the member trailers, each grown to the largest call so far and freed with the session.
+ * rala_b200_inflate_gzip is stateless: with out == NULL it runs the finder and the counting pass only and fills stats
+ * (a stream they find malformed is decoded in full, to refuse it as the filling call does); otherwise out receives the
+ * text (cap smaller than the text: RALA_B200_ERR_ARG before any of
+ * it is written).  stats / gzip: nullable, filled when the call succeeds. */
+typedef struct {
+    uint64_t n_members;       /* gzip members (BGZF path: BGZF blocks) */
+    uint64_t n_compressed;    /* input bytes */
+    uint64_t n_bytes;         /* inflated bytes = the text the reader parsed */
+    uint64_t n_chunks;        /* decode chunks (0 when the BGZF path ran) */
+    uint64_t n_corrected;     /* chunk decodes redone because the chunk's proposed entry was not where its predecessor stopped */
+    uint64_t chunk_bytes;     /* compressed bytes per chunk */
+    uint32_t rounds;          /* counting rounds */
+    uint32_t bgzf;            /* 1: the input was BGZF and took the block-table path */
+    float inflate_ms;         /* device time of every inflate kernel; uploads excluded */
+    float stage_ms[5];        /* of which: finder, counting, symbols, window chain, resolve + CRC32 */
+} rala_b200_gzip_stats_t;
+int rala_b200_inflate_gzip(rala_b200_ctx* ctx, const uint8_t* data, uint64_t n, uint8_t* out, uint64_t cap,
+                           rala_b200_gzip_stats_t* stats);
+int rala_b200_graph_set_reads_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_reads_stats_t* stats,
+                                   rala_b200_gzip_stats_t* gzip);
+int rala_b200_graph_set_overlaps_paf_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_paf_stats_t* stats,
+                                          rala_b200_gzip_stats_t* gzip);
+int rala_b200_graph_set_overlaps_mhap_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_mhap_stats_t* stats,
+                                           rala_b200_gzip_stats_t* gzip);
 /* The pile table of the reads given to set_reads, built on the device (rule and refusals as rala_b200_build_piles) from
  * the records of the last successful set_overlaps_paf or set_overlaps_mhap, counted as parsed: before the duplicate
  * filter.  A refused record is named by its line in that text ("PAF line N" / "MHAP line N").  It is installed as

@@ -73,6 +73,21 @@ class BgzfStats(C.Structure):
         return {k: (float(getattr(self, k)) if k == "inflate_ms" else int(getattr(self, k))) for k, _ in self._fields_}
 
 
+GZIP_STAGES = ("finder", "counting", "symbols", "chain", "resolve_crc")
+
+
+class GzipStats(C.Structure):
+    _fields_ = [("n_members", C.c_uint64), ("n_compressed", C.c_uint64), ("n_bytes", C.c_uint64), ("n_chunks", C.c_uint64),
+                ("n_corrected", C.c_uint64), ("chunk_bytes", C.c_uint64), ("rounds", C.c_uint32), ("bgzf", C.c_uint32),
+                ("inflate_ms", C.c_float), ("stage_ms", C.c_float * 5)]
+
+    def as_dict(self):
+        d = {k: int(getattr(self, k)) for k, _ in self._fields_[:8]}
+        d["inflate_ms"] = float(self.inflate_ms)
+        d["stage_ms"] = {name: float(v) for name, v in zip(GZIP_STAGES, self.stage_ms)}
+        return d
+
+
 PAF_CHUNK_BYTES = 32 << 20   # RALA_B200_PAF_CHUNK_BYTES (the MHAP reader uses the same chunks)
 
 
@@ -130,7 +145,8 @@ EXPORTS = [
     "rala_b200_graph_use_cuda_graph", "rala_b200_graph_set_overlaps_columns", "rala_b200_graph_set_outputs",
     "rala_b200_graph_set_overlaps_packed", "rala_b200_multi_set_overlaps_packed", "rala_b200_graph_get_adjacency",
     "rala_b200_graph_get_csr", "rala_b200_inflate_bgzf", "rala_b200_graph_set_reads_bgzf", "rala_b200_graph_set_overlaps_paf_bgzf",
-    "rala_b200_graph_set_overlaps_mhap_bgzf",
+    "rala_b200_graph_set_overlaps_mhap_bgzf", "rala_b200_inflate_gzip", "rala_b200_graph_set_reads_gzip",
+    "rala_b200_graph_set_overlaps_paf_gzip", "rala_b200_graph_set_overlaps_mhap_gzip",
     # multi-GPU phases
     "rala_b200_create_on_stream", "rala_b200_graph_set_shard", "rala_b200_graph_phase_events",
     "rala_b200_graph_phase_resolve", "rala_b200_graph_phase_survivors", "rala_b200_graph_phase_emit_edges",
@@ -380,6 +396,19 @@ class Context:
                                                    C.byref(st)), "inflate_bgzf")
         return out[:int(st.n_bytes)], st.as_dict()
 
+    def inflate_gzip(self, data) -> tuple:
+        """A gzip file of one or more members (bytes, uint8 array or pinned CPU tensor) inflated on the device -> (text as a
+        uint8 array, stats dict: members, compressed and inflated bytes, chunks, corrected chunk decodes, chunk bytes,
+        rounds, bgzf (1: the BGZF path ran), inflate_ms and its stage_ms)."""
+        buf, n = _text(data)
+        st = GzipStats()
+        self.check(self.lib.rala_b200_inflate_gzip(self.handle, _ptr(buf), C.c_uint64(n), None, C.c_uint64(0), C.byref(st)),
+                   "inflate_gzip")
+        out = np.zeros(max(int(st.n_bytes), 1), np.uint8)
+        self.check(self.lib.rala_b200_inflate_gzip(self.handle, _ptr(buf), C.c_uint64(n), _ptr(out), C.c_uint64(int(st.n_bytes)),
+                                                   C.byref(st)), "inflate_gzip")
+        return out[:int(st.n_bytes)], st.as_dict()
+
     def build_piles(self, columns, read_len, with_time: bool = False):
         """Graph::initialize's coverage half on the device: six host columns in the set_overlaps_columns layout (bit 31 of
         a_id = unresolved record; records the duplicate filter drops still count) + the read lengths -> (piles (n_reads, 2)
@@ -485,6 +514,14 @@ class Graph:
         self._n_reads = int(st.n_reads)
         return st.as_dict(), z.as_dict()
 
+    def set_reads_gzip(self, data) -> tuple:
+        """set_reads_text on a gzip file (BGZF included), inflated on the device -> (reads stats dict, gzip stats dict)."""
+        buf, n = _text(data)
+        st, z = ReadsStats(), GzipStats()
+        self._call("rala_b200_graph_set_reads_gzip", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        self._n_reads = int(st.n_reads)
+        return st.as_dict(), z.as_dict()
+
     def reads(self):
         """The session's reads as set_reads holds them: (names blob uint8, name_end uint64, read_len uint32)."""
         n, nb = C.c_uint32(0), C.c_uint64(0)
@@ -523,6 +560,20 @@ class Graph:
         buf, n = _text(data)
         st, z = MhapStats(), BgzfStats()
         self._call("rala_b200_graph_set_overlaps_mhap_bgzf", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        return st.as_dict(), z.as_dict()
+
+    def set_overlaps_paf_gzip(self, data) -> tuple:
+        """set_overlaps_paf on a gzip file (BGZF included), inflated on the device -> (PAF stats dict, gzip stats dict)."""
+        buf, n = _text(data)
+        st, z = PafStats(), GzipStats()
+        self._call("rala_b200_graph_set_overlaps_paf_gzip", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
+        return st.as_dict(), z.as_dict()
+
+    def set_overlaps_mhap_gzip(self, data) -> tuple:
+        """set_overlaps_mhap on a gzip file (BGZF included), inflated on the device -> (MHAP stats dict, gzip stats dict)."""
+        buf, n = _text(data)
+        st, z = MhapStats(), GzipStats()
+        self._call("rala_b200_graph_set_overlaps_mhap_gzip", _ptr(buf), C.c_uint64(n), C.byref(st), C.byref(z))
         return st.as_dict(), z.as_dict()
 
     def build_piles(self) -> dict:

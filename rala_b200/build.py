@@ -14,8 +14,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librala_b200.so")
-SOURCES = ["classify.cu", "containment.cu", "graph_build.cu", "transitive.cu", "api.cu", "fabric.cu", "multi_api.cu", "frontend.cu", "paf.cu", "piles.cu", "reads.cu", "bgzf.cu"]
-HEADERS = ["common.cuh", "lists.cuh", "kernels.h", "session.h", "fabric.cuh", "bgzf.cuh", os.path.join("..", "..", "include", "rala_b200.h")]
+SOURCES = ["classify.cu", "containment.cu", "graph_build.cu", "transitive.cu", "api.cu", "fabric.cu", "multi_api.cu", "frontend.cu", "paf.cu", "piles.cu", "reads.cu", "bgzf.cu", "gzip.cu"]
+HEADERS = ["common.cuh", "lists.cuh", "kernels.h", "session.h", "fabric.cuh", "bgzf.cuh", "deflate.cuh", os.path.join("..", "..", "include", "rala_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

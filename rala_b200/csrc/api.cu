@@ -40,6 +40,7 @@ extern "C" int rala_b200_create(rala_b200_ctx** out, int device) {
     preload_paf();
     preload_reads();
     preload_bgzf();
+    preload_gzip();
     preload_piles();
     cudaGetLastError();
     cudaEventCreate(&ctx->ev[0]);

@@ -48,16 +48,7 @@ __global__ void __launch_bounds__(kInflateWarps * 32) k_bgzf_inflate(const uint8
         rc = __shfl_sync(0xFFFFFFFFu, rc, 0);
         __syncwarp();   // lane 0's output is visible to the warp
         if (rc == 0) {
-            const uint32_t slice = (B.isize + 31) / 32, lo = min(lane * slice, B.isize), hi = min(lo + slice, B.isize);
-            uint32_t crc = bgzf::crc_update(0, out + lo, hi - lo, s_crc), len = hi - lo;
-#pragma unroll
-            for (uint32_t d = 1; d < 32; d <<= 1) {   // lane 2dk absorbs lane 2dk + d: the CRC of the slices behind it
-                const uint32_t c2 = __shfl_down_sync(0xFFFFFFFFu, crc, d), l2 = __shfl_down_sync(0xFFFFFFFFu, len, d);
-                if ((lane & (2 * d - 1)) == 0) {
-                    crc = bgzf::crc_combine(crc, c2, l2, s_x2n);
-                    len += l2;
-                }
-            }
+            const uint32_t crc = bgzf::warp_crc(out, B.isize, lane, s_crc, s_x2n);
             if (lane == 0 && crc != B.crc) rc = bgzf::kCrc;
         }
         if (lane == 0 && rc) atomicMin(err, (unsigned long long) b << 8 | rc);
@@ -191,9 +182,9 @@ static int bgzf_inflate_once(rala_b200_ctx* ctx, PafReader& R, const uint8_t* da
     const size_t nb = blocks.size();
     if (total == 0) return RALA_B200_OK;   // only empty blocks: nothing to decode
     cudaStream_t s = ctx->L.stream;
-    CU(ctx, R.bgzf_in.reserve(n));
+    CU(ctx, R.packed.reserve(n));
     CU(ctx, R.bgzf_meta.reserve(nb * sizeof(BgzfBlock) + 8));
-    CU(ctx, R.bgzf_text.reserve(total));
+    CU(ctx, R.inflated.reserve(total));
     if (!R.copy) CU(ctx, cudaStreamCreateWithFlags(&R.copy, cudaStreamNonBlocking));
     for (int k = 0; k < 2; ++k)
         if (!R.copied[k]) CU(ctx, cudaEventCreateWithFlags(&R.copied[k], cudaEventDisableTiming));
@@ -209,7 +200,7 @@ static int bgzf_inflate_once(rala_b200_ctx* ctx, PafReader& R, const uint8_t* da
     CU(ctx, cudaMemsetAsync(err, 0xFF, 8, s));
     CU(ctx, cudaStreamSynchronize(s));   // the block table has left the host vector; the copy stream starts from settled buffers
     TimingEvents T;
-    uint8_t* din = R.bgzf_in.as<uint8_t>();
+    uint8_t* din = R.packed.as<uint8_t>();
     size_t b = 0, launched = 0;
     for (uint32_t k = 0; b < nb; ++k) {
         const size_t first = b;   // a piece: whole blocks, at most kPiece bytes unless one block is longer
@@ -235,7 +226,7 @@ static int bgzf_inflate_once(rala_b200_ctx* ctx, PafReader& R, const uint8_t* da
         CU(ctx, cudaEventRecord(e[0], s));
         const uint32_t n_run = (uint32_t) (b - launched);
         k_bgzf_inflate<<<grid_for(n_run, kInflateWarps, kNumSMs * 8), kInflateWarps * 32, 0, s>>>(
-            din, meta, (uint32_t) launched, (uint32_t) b, R.bgzf_text.as<uint8_t>(), err);
+            din, meta, (uint32_t) launched, (uint32_t) b, R.inflated.as<uint8_t>(), err);
         ctx->L.count++;
         CU(ctx, cudaGetLastError());
         CU(ctx, cudaEventRecord(e[1], s));
@@ -254,7 +245,7 @@ static int bgzf_inflate_once(rala_b200_ctx* ctx, PafReader& R, const uint8_t* da
         return walk_fail(ctx, RALA_B200_ERR_ARG, k, blocks[k].at, "%s", inflate_error_text((uint32_t) bad & 0xFFu));
     }
     if (host_out) {
-        CU(ctx, cudaMemcpyAsync(host_out, R.bgzf_text.p, total, cudaMemcpyDeviceToHost, s));
+        CU(ctx, cudaMemcpyAsync(host_out, R.inflated.p, total, cudaMemcpyDeviceToHost, s));
         CU(ctx, cudaStreamSynchronize(s));
     }
     return RALA_B200_OK;
@@ -270,7 +261,7 @@ int bgzf_inflate(rala_b200_ctx* ctx, PafReader& R, const uint8_t* data, uint64_t
     return rc;
 }
 
-int bgzf_text_cut(rala_b200_ctx* ctx, PafReader& R, const uint8_t* text, uint64_t lo, uint64_t hi, uint64_t* found) {
+int inflated_cut(rala_b200_ctx* ctx, PafReader& R, const uint8_t* text, uint64_t lo, uint64_t hi, uint64_t* found) {
     CU(ctx, R.bgzf_cut.reserve(8));
     if (!R.cut_host) CU(ctx, cudaHostAlloc((void**) &R.cut_host, 8, cudaHostAllocDefault));
     unsigned long long* d = R.bgzf_cut.as<unsigned long long>();
@@ -300,4 +291,10 @@ extern "C" int rala_b200_inflate_bgzf(rala_b200_ctx* ctx, const uint8_t* data, u
     }
     if (stats && !rc) *stats = st;
     return rc;
+}
+
+bool is_bgzf(const uint8_t* data, uint64_t n) {
+    std::vector<BgzfBlock> blocks;
+    uint64_t total = 0;
+    return bgzf_walk(nullptr, data, n, blocks, &total) == RALA_B200_OK;
 }

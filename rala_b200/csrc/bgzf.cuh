@@ -111,9 +111,10 @@ BGZF_HD uint32_t build(Code<kSymbols, kFast>& c, const uint8_t* lens, uint32_t n
     return kOk;
 }
 
-// one symbol of c, or -1 (not a code, or the stream ends inside it: err = kPastEnd)
-template <int kSymbols, int kFast>
-BGZF_HD int decode(const Code<kSymbols, kFast>& c, Bits& b, uint32_t& err) {
+// one symbol of c, or -1 (not a code, or the stream ends inside it: err = kPastEnd); B: Bits or another reader with
+// the same refill / buf / cnt
+template <int kSymbols, int kFast, class B>
+BGZF_HD int decode(const Code<kSymbols, kFast>& c, B& b, uint32_t& err) {
     b.refill();
     const uint32_t e = c.fast[b.buf & ((1u << kFast) - 1)];
     uint32_t len = e >> 9;
@@ -157,7 +158,8 @@ BGZF_HD void fixed_codes(Tables& t) {
     build(t.dist, t.lens, 32);
 }
 
-BGZF_HD uint32_t dynamic_codes(Tables& t, Bits& b) {
+template <class B>
+BGZF_HD uint32_t dynamic_codes(Tables& t, B& b) {
     uint32_t err = kOk;
     const uint32_t nlen = b.take(5, err) + 257, ndist = b.take(5, err) + 1, ncode = b.take(4, err) + 4;
     if (err) return err;
@@ -321,5 +323,22 @@ BGZF_HD void x2n_table(uint32_t* x2n) {
 BGZF_HD uint32_t crc_combine(uint32_t crc_a, uint32_t crc_b, uint32_t len_b, const uint32_t* x2n) {
     return multmodp(x2nmodp(len_b, 3, x2n), crc_a) ^ crc_b;
 }
+
+#if defined(__CUDACC__)
+// CRC32 of p[0, len) by the 32 lanes of a warp, one slice each, joined by the GF(2) shift; lane 0 returns it
+__device__ __forceinline__ uint32_t warp_crc(const uint8_t* p, uint32_t len, uint32_t lane, const uint32_t* table, const uint32_t* x2n) {
+    const uint32_t slice = (len + 31) / 32, lo = min(lane * slice, len), hi = min(lo + slice, len);
+    uint32_t crc = crc_update(0, p + lo, hi - lo, table), n = hi - lo;
+#pragma unroll
+    for (uint32_t d = 1; d < 32; d <<= 1) {   // lane 2dk absorbs lane 2dk + d: the CRC of the slices behind it
+        const uint32_t c2 = __shfl_down_sync(0xFFFFFFFFu, crc, d), l2 = __shfl_down_sync(0xFFFFFFFFu, n, d);
+        if ((lane & (2 * d - 1)) == 0) {
+            crc = crc_combine(crc, c2, l2, x2n);
+            n += l2;
+        }
+    }
+    return crc;
+}
+#endif
 
 }  // namespace bgzf

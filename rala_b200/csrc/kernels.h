@@ -210,6 +210,7 @@ void preload_paf();
 void preload_piles();
 void preload_reads();
 void preload_bgzf();
+void preload_gzip();
 
 // frontend.cu
 void launch_filter_duplicates(Launch& L, const uint32_t* a, const uint32_t* b, const uint32_t* len, uint32_t n, uint8_t* valid);

@@ -470,7 +470,7 @@ static int text_chunks_once(rala_b200_ctx* ctx, PafReader& R, const char* label,
         if (!last) {   // cut behind the last '\n' of the window; the tail goes with the next chunk
             uint64_t cut = 0;   // bytes up to and with the last '\n' of the window, 0 when there is none
             if (on_device) {
-                const int rc = bgzf_text_cut(ctx, R, (const uint8_t*) text, pos, pos + len, &cut);
+                const int rc = inflated_cut(ctx, R, (const uint8_t*) text, pos, pos + len, &cut);
                 if (rc) return rc;
                 cut = cut ? cut - pos : 0;
             } else {
@@ -614,9 +614,9 @@ extern "C" int rala_b200_graph_set_reads(rala_b200_graph* g, const char* names, 
 
 // Text in file order -> the session's records: parse, duplicate filter, INVALID bit folded in.  *counted = *st holds the
 // call's counts (also when a read-length refusal follows).
-// bgzf (nullable): text[0, n_bytes) is a BGZF file, inflated on the device first; *bgzf receives its stats.
+// z (nullable): text[0, n_bytes) is a BGZF or gzip file, inflated on the device first.
 static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* text, uint64_t n_bytes, TextStats* st, bool* counted,
-                             rala_b200_bgzf_stats_t* bgzf = nullptr) {
+                             const Packed* z = nullptr) {
     if (!g || (n_bytes && !text)) return RALA_B200_ERR_ARG;
     rala_b200_ctx* ctx = g->ctx;
     const bool mhap = fmt == kTextMhap;
@@ -628,14 +628,13 @@ static int set_overlaps_text(rala_b200_graph* g, TextFormat fmt, const char* tex
     g->state = SS_EMPTY;
     g->text_records = kTextNone;
     int rc;
-    if (bgzf) {
-        rc = bgzf_inflate(ctx, R, (const uint8_t*) text, n_bytes, bgzf);
+    if (z) {
+        rc = inflate_packed(ctx, R, (const uint8_t*) text, n_bytes, *z, &n_bytes);
         if (rc) return rc;
-        text = R.bgzf_text.as<const char>();
-        n_bytes = bgzf->n_bytes;
+        text = R.inflated.as<const char>();
     }
     uint64_t n = 0;
-    rc = text_parse(ctx, R, fmt, text, n_bytes, bgzf != nullptr, st, nullptr, &n);
+    rc = text_parse(ctx, R, fmt, text, n_bytes, z != nullptr, st, nullptr, &n);
     if (rc) return rc;
     rc = reserve_for_records(g, n);
     if (rc) return rc;
@@ -692,10 +691,23 @@ extern "C" int rala_b200_graph_set_overlaps_paf_bgzf(rala_b200_graph* g, const u
                                                      rala_b200_bgzf_stats_t* bgzf) {
     TextStats st{};
     rala_b200_bgzf_stats_t z{};
+    const Packed p{&z, nullptr};
     bool counted = false;
-    const int rc = set_overlaps_text(g, kTextPaf, (const char*) data, n, &st, &counted, &z);
+    const int rc = set_overlaps_text(g, kTextPaf, (const char*) data, n, &st, &counted, &p);
     if (stats && counted) paf_stats_of(st, stats);
     if (bgzf && counted) *bgzf = z;
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_overlaps_paf_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_paf_stats_t* stats,
+                                                     rala_b200_gzip_stats_t* gzip) {
+    TextStats st{};
+    rala_b200_gzip_stats_t z{};
+    const Packed p{nullptr, &z};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextPaf, (const char*) data, n, &st, &counted, &p);
+    if (stats && counted) paf_stats_of(st, stats);
+    if (gzip && counted) *gzip = z;
     return rc;
 }
 
@@ -703,10 +715,23 @@ extern "C" int rala_b200_graph_set_overlaps_mhap_bgzf(rala_b200_graph* g, const 
                                                       rala_b200_bgzf_stats_t* bgzf) {
     TextStats st{};
     rala_b200_bgzf_stats_t z{};
+    const Packed p{&z, nullptr};
     bool counted = false;
-    const int rc = set_overlaps_text(g, kTextMhap, (const char*) data, n, &st, &counted, &z);
+    const int rc = set_overlaps_text(g, kTextMhap, (const char*) data, n, &st, &counted, &p);
     if (stats && counted) mhap_stats_of(st, stats);
     if (bgzf && counted) *bgzf = z;
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_overlaps_mhap_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_mhap_stats_t* stats,
+                                                     rala_b200_gzip_stats_t* gzip) {
+    TextStats st{};
+    rala_b200_gzip_stats_t z{};
+    const Packed p{nullptr, &z};
+    bool counted = false;
+    const int rc = set_overlaps_text(g, kTextMhap, (const char*) data, n, &st, &counted, &p);
+    if (stats && counted) mhap_stats_of(st, stats);
+    if (gzip && counted) *gzip = z;
     return rc;
 }
 

@@ -329,9 +329,8 @@ static const char* reads_error_text(uint32_t kind) {
     }
 }
 
-// bgzf (nullable): text[0, n_bytes) is a BGZF file, inflated on the device first; *bgzf receives its stats.
-static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_reads_stats_t* st,
-                      rala_b200_bgzf_stats_t* bgzf = nullptr) {
+// z (nullable): text[0, n_bytes) is a BGZF or gzip file, inflated on the device first.
+static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, rala_b200_reads_stats_t* st, const Packed* z = nullptr) {
     rala_b200_ctx* ctx = g->ctx;
     if (!g->paf) g->paf = new PafReader();
     PafReader& R = *g->paf;
@@ -341,11 +340,10 @@ static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, ra
     CU(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->L.stream;
     char first = n_bytes ? text[0] : 0;
-    if (bgzf) {
-        const int rc = bgzf_inflate(ctx, R, (const uint8_t*) text, n_bytes, bgzf);
+    if (z) {
+        const int rc = inflate_packed(ctx, R, (const uint8_t*) text, n_bytes, *z, &n_bytes);
         if (rc) return rc;
-        text = R.bgzf_text.as<const char>();
-        n_bytes = bgzf->n_bytes;
+        text = R.inflated.as<const char>();
         if (n_bytes) {
             CU(ctx, cudaMemcpyAsync(&first, text, 1, cudaMemcpyDeviceToHost, s));
             CU(ctx, cudaStreamSynchronize(s));
@@ -373,7 +371,7 @@ static int reads_text(rala_b200_graph* g, const char* text, uint64_t n_bytes, ra
     for (cudaEvent_t& e : c.ev) CU(ctx, cudaEventCreate(&e));
     float ms = 0.f, part = 0.f;
     uint32_t k = 0;
-    int rc = text_chunks(ctx, R, label, text, n_bytes, bgzf != nullptr, reads_chunk, &c, &ms, &k);
+    int rc = text_chunks(ctx, R, label, text, n_bytes, z != nullptr, reads_chunk, &c, &ms, &k);
     if (rc) return rc;
     // text_chunks ended with the stream synchronised: c.host holds the totals behind the last chunk
     const unsigned long long n_lines = R.w[W_BASES + k], n_reads = c.host[0], blob = c.host[1];
@@ -434,9 +432,22 @@ extern "C" int rala_b200_graph_set_reads_bgzf(rala_b200_graph* g, const uint8_t*
     if (!g || (n && !data)) return RALA_B200_ERR_ARG;
     rala_b200_reads_stats_t st;
     rala_b200_bgzf_stats_t z{};
-    const int rc = reads_text(g, (const char*) data, n, &st, &z);
+    const Packed p{&z, nullptr};
+    const int rc = reads_text(g, (const char*) data, n, &st, &p);
     if (stats && !rc) *stats = st;
     if (bgzf && !rc) *bgzf = z;
+    return rc;
+}
+
+extern "C" int rala_b200_graph_set_reads_gzip(rala_b200_graph* g, const uint8_t* data, uint64_t n, rala_b200_reads_stats_t* stats,
+                                               rala_b200_gzip_stats_t* gzip) {
+    if (!g || (n && !data)) return RALA_B200_ERR_ARG;
+    rala_b200_reads_stats_t st;
+    rala_b200_gzip_stats_t z{};
+    const Packed p{nullptr, &z};
+    const int rc = reads_text(g, (const char*) data, n, &st, &p);
+    if (stats && !rc) *stats = st;
+    if (gzip && !rc) *gzip = z;
     return rc;
 }
 

@@ -270,8 +270,9 @@ struct PafReader {
     std::vector<cudaEvent_t> timing;   // (start, stop) around the kernels of every chunk
     unsigned long long rec_cap = 0;
     std::vector<unsigned long long> w;   // the words of the last call, read back
-    // BGZF input (bgzf.cu): compressed bytes, block table + error word, inflated text, the chunk cut and its read-back
-    DevBuf bgzf_in, bgzf_meta, bgzf_text, bgzf_cut;
+    // compressed input (bgzf.cu, gzip.cu): the compressed bytes, the BGZF block table + error word, the inflated text,
+    // the chunk cut and its read-back; gzip's chunk table, decoded symbols, member trailers and CRC32 segments
+    DevBuf packed, bgzf_meta, inflated, bgzf_cut, gz_meta, gz_sym, gz_trailers, gz_seg;
     unsigned long long* cut_host = nullptr;
 
     PafCols view() const {
@@ -282,7 +283,8 @@ struct PafReader {
     }
     ~PafReader() {
         if (copy) cudaStreamSynchronize(copy);
-        DevBuf* bufs[] = {&names, &text[0], &text[1], &line_end, &status, &words, &cols, &valid, &bgzf_in, &bgzf_meta, &bgzf_text, &bgzf_cut};
+        DevBuf* bufs[] = {&names, &text[0], &text[1], &line_end, &status, &words, &cols, &valid, &packed, &bgzf_meta, &inflated, &bgzf_cut,
+                          &gz_meta, &gz_sym, &gz_trailers, &gz_seg};
         for (DevBuf* b : bufs) b->release();
         for (int k = 0; k < 2; ++k) {
             if (pinned[k]) cudaFreeHost(pinned[k]);
@@ -313,18 +315,32 @@ size_t text_status_words();
 // RALA_B200_PAF_CHUNK_BYTES cut behind their last '\n', each one line-scanned and handed to `kernels`; R.w holds the
 // call's words afterwards (W_BASES + *n_chunks = lines).  W_ERR .. W_FIRST_BAD start at ~0, the rest at 0.
 // kernel_ms (nullable) = device time of the chunks' kernels.  A refused call returns with no upload in flight.
-// on_device: text is device memory (an inflated BGZF file); the cuts are found on the device and the chunks copied
+// on_device: text is device memory (an inflated BGZF or gzip file); the cuts are found on the device and the chunks copied
 // device to device into the same buffers, so chunks, line numbers and refusals are those of the host text.
 int text_chunks(rala_b200_ctx* ctx, PafReader& R, const char* label, const char* text, uint64_t n_bytes, bool on_device,
                 ChunkKernels kernels, void* self, float* kernel_ms, uint32_t* n_chunks);
 void destroy_paf_reader(PafReader* r);
 // ---- bgzf.cu: BGZF input --------------------------------------------------------------------------------------
-// The BGZF file data[0, n) inflated into R.bgzf_text (stats: blocks, bytes, inflate_ms); host_out (nullable, cap bytes)
+// The BGZF file data[0, n) inflated into R.inflated (stats: blocks, bytes, inflate_ms); host_out (nullable, cap bytes)
 // also receives the text.  A refused call returns with no upload in flight.
 int bgzf_inflate(rala_b200_ctx* ctx, PafReader& R, const uint8_t* data, uint64_t n, rala_b200_bgzf_stats_t* st,
                  uint8_t* host_out = nullptr, uint64_t cap = 0);
 // position + 1 of the last '\n' in device text[lo, hi), 0 when there is none (on R.copy, synchronised)
-int bgzf_text_cut(rala_b200_ctx* ctx, PafReader& R, const uint8_t* text, uint64_t lo, uint64_t hi, uint64_t* found);
+int inflated_cut(rala_b200_ctx* ctx, PafReader& R, const uint8_t* text, uint64_t lo, uint64_t hi, uint64_t* found);
+// whether the BGZF header walk accepts data[0, n) (sets no error text)
+bool is_bgzf(const uint8_t* data, uint64_t n);
+// ---- gzip.cu: plain gzip input -----------------------------------------------------------------------------------
+// The gzip file data[0, n) inflated into R.inflated (BGZF input through bgzf_inflate); host_out as for bgzf_inflate;
+// size_only: the finder and the counting pass only, R.inflated untouched.  A refused call returns with no upload in flight.
+int gzip_inflate(rala_b200_ctx* ctx, PafReader& R, const uint8_t* data, uint64_t n, rala_b200_gzip_stats_t* st,
+                 uint8_t* host_out = nullptr, uint64_t cap = 0, bool size_only = false);
+// A compressed input of the readers' _bgzf / _gzip calls (exactly one of the two set): inflated into R.inflated, whose
+// length goes to *n_bytes, before the reader parses it.
+struct Packed {
+    rala_b200_bgzf_stats_t* bgzf;
+    rala_b200_gzip_stats_t* gzip;
+};
+int inflate_packed(rala_b200_ctx* ctx, PafReader& R, const uint8_t* data, uint64_t n, const Packed& z, uint64_t* n_bytes);
 // the overlap columns build_piles counts: the parsed records of the last successful set_overlaps_paf / _mhap, before the
 // duplicate filter was folded in (bit 31 of a = unresolved name), and the reads' lengths (device); returns the text format
 // they came from, kTextNone when there are none

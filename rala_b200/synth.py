@@ -432,3 +432,51 @@ def write_bgzf(text, level: int = 6, strategy: int = zlib.Z_DEFAULT_STRATEGY, cu
     bounds.append(len(text))
     out = [bgzf_block(text[a:b], level, strategy) for a, b in zip(bounds[:-1], bounds[1:]) if b > a or cuts is not None]
     return b"".join(out) + BGZF_EOF
+
+
+def gzip_deflate(text, level: int = 6, strategy: int = zlib.Z_DEFAULT_STRATEGY, dictionary: bytes = b"", final: bool = True) -> bytes:
+    """Raw DEFLATE of `text`, primed with `dictionary` (at most the last 32 KiB count); not final: ends with Z_SYNC_FLUSH
+    (an empty stored block, byte-aligned), so that the next piece's stream can follow it, as pigz joins its pieces."""
+    c = zlib.compressobj(level, zlib.DEFLATED, -15, 8, strategy, **({"zdict": dictionary[-32768:]} if dictionary else {}))
+    return c.compress(bytes(text)) + c.flush(zlib.Z_FINISH if final else zlib.Z_SYNC_FLUSH)
+
+
+def write_gzip(text, level: int = 6, strategy: int = zlib.Z_DEFAULT_STRATEGY, members=1, sync_every=None, fname=None,
+               comment=None, extra=None, hcrc: bool = False, pool=None) -> bytes:
+    """`text` as plain gzip: `members` members (a count of equal parts, or a list of cut offsets), each one raw DEFLATE
+    stream, or with sync_every=N pigz-style pieces of N bytes, each compressed with the 32 KiB before it as dictionary and
+    joined by Z_SYNC_FLUSH (pool: an executor with .map to compress the pieces in parallel).  fname / comment (bytes
+    without NUL), extra (the FEXTRA payload) and hcrc (FHCRC) go into every member header."""
+    text = bytes(text)
+    if isinstance(members, int):
+        step = -(-len(text) // max(members, 1)) if text else 0
+        cuts = [min(i * step, len(text)) for i in range(1, max(members, 1))]
+    else:
+        cuts = [int(c) for c in members]
+    bounds = [0] + cuts + [len(text)]
+    flg = (4 if extra is not None else 0) | (8 if fname is not None else 0) | (16 if comment is not None else 0) | (2 if hcrc else 0)
+    head = b"\x1f\x8b\x08" + bytes([flg]) + b"\x00\x00\x00\x00\x00\xff"
+    if extra is not None:
+        head += struct.pack("<H", len(extra)) + bytes(extra)
+    if fname is not None:
+        head += bytes(fname) + b"\x00"
+    if comment is not None:
+        head += bytes(comment) + b"\x00"
+    if hcrc:
+        head += struct.pack("<H", zlib.crc32(head) & 0xFFFF)
+    out = []
+    for a, b in zip(bounds[:-1], bounds[1:]):
+        part = text[a:b]
+        if sync_every:
+            starts = list(range(0, len(part), sync_every)) or [0]
+            args = [(part[s:s + sync_every], level, strategy, part[max(0, s - 32768):s], s + sync_every >= len(part)) for s in starts]
+            pieces = list((pool.map if pool else map)(_gzip_piece, args))
+            body = b"".join(pieces)
+        else:
+            body = gzip_deflate(part, level, strategy)
+        out.append(head + body + struct.pack("<II", zlib.crc32(part), len(part) & 0xFFFFFFFF))
+    return b"".join(out)
+
+
+def _gzip_piece(a):
+    return gzip_deflate(*a)
